@@ -307,6 +307,8 @@ int keds_consumer_check(keds_consumer_t* c, void* cuda_stream, int64_t* launches
  *                   dropout multipliers (0 or 1/(1-p); rows ordered queries | image neighbours |
  *                   text neighbours), applied between Linear and ReLU as in IM2TEXT
  *                   (src/model/model.py:110-116); they must stay alive until the backward.
+ *                   Refuses (before queuing anything) a k whose attention backward, heads x
+ *                   (2 dim_head + 2k) floats of shared memory, would not fit one block.
  *   backward        dtokens [B][3][d_tok] -> grads (param_count floats, same layout, overwritten).
  *                   One backward per forward_train. tf32 tensor-core products, fp32 accumulation. */
 int64_t keds_consumer_param_count(const keds_consumer_t* c);
@@ -357,6 +359,20 @@ int keds_debug_scores(keds_index_t* idx, const float* q, int64_t nq, float* out,
  * rows each, nq queries, k neighbours on a device with num_sms SMs.
  * out = {exact_only, cta_pair, slices S, query tiles, work items, grid (CTAs)}. */
 int keds_debug_plan(int n_db, int64_t nq, int k, int64_t n_rows, int num_sms, int32_t out[6]);
+/* Host only, needs no GPU: which kernel the consumer's tf32 linear product C[M][N] (nz independent
+ * problems) takes on num_sms SMs. variant = 1: 128-column tiles, 2: 256-column tiles, 3: persistent
+ * 256-column tiles, 4 / 5: 32-column tiles with K split over a cluster of 2 / 4 CTAs. */
+int keds_debug_linear_plan(int64_t M, int N, int nz, int num_sms, int32_t* variant);
+/* Test hook for the tf32 linear product alone: C[z] = act(A[z] W[z]^T + b[z]) for z < nz (1 or 2),
+ * act = ReLU if relu else identity. A[z] [M][K] with lda floats between rows (lda a multiple of 4,
+ * >= K); W[z] [N][K] with round4(K) floats between rows; b[z] [N] or NULL; C[z] [M][N] with ldc
+ * floats between rows (ldc >= N). A and W 16-byte aligned, C 4-byte aligned; all device memory.
+ * variant 0 = the production choice (keds_debug_linear_plan), 1..5 forces one kernel.
+ * Asynchronous on cuda_stream; keds_consumer_check reports device-side errors. */
+int keds_consumer_debug_linear(keds_consumer_t* c, int variant, const float* A0, const float* A1, int64_t lda,
+                               int64_t M, int K, const float* W0, const float* W1, const float* b0,
+                               const float* b1, int N, int relu, float* C0, float* C1, int64_t ldc, int nz,
+                               void* cuda_stream);
 /* Programmatic dependent launch between the kernels of a search (default on; env KEDS_NO_PDL=1
  * turns the default off). Tuning/diagnostic switch; results do not depend on it. */
 int keds_index_set_pdl(keds_index_t* idx, int enable);

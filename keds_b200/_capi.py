@@ -137,6 +137,12 @@ SIGNATURES = {
     "keds_clip_loss_check": (C.c_int, [_vp, _vp]),
     "keds_debug_scores": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp]),
     "keds_debug_plan": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_int32)]),
+    "keds_debug_linear_plan": (C.c_int, [C.c_int64, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int32)]),
+    "keds_consumer_debug_linear": (
+        C.c_int,
+        [_vp, C.c_int, _vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp,
+         C.c_int64, C.c_int, _vp],
+    ),
     "keds_index_set_eps_scale": (C.c_int, [_vp, C.c_float]),
     "keds_index_set_pdl": (C.c_int, [_vp, C.c_int]),
     "keds_last_error": (C.c_char_p, []),

@@ -45,16 +45,7 @@ int keds_clip_loss_create(int device, keds_clip_loss_t** out) {
   h->device = device;
   h->lin.device = device;
   auto init = [&]() -> int {
-    CK(cudaFuncSetAttribute(k_linear_tf32<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)LinCfg<128>::kSmemBytes));
-    CK(cudaFuncSetAttribute(k_linear_tf32<256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)LinCfg<256>::kSmemBytes));
-    CK(cudaFuncSetAttribute(k_linear_tf32_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)PL_SMEM_BYTES));
-    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK_SMEM_BYTES));
-    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK_SMEM_BYTES));
-    CK(cudaDeviceGetAttribute(&h->lin.num_sms, cudaDevAttrMultiProcessorCount, device));
-    CKS(h->lin.err.ensure(16));
-    CK(cudaMemset(h->lin.err.p, 0, 16));
+    CKS(linear_init(&h->lin));
     CKS(h->accum.ensure(16));
     CK(cudaDeviceSynchronize());  // the memset above is on the legacy stream; callers may use any stream
     return 0;

@@ -18,7 +18,8 @@ struct LinearW {
 };
 
 // fp32 [rows][cols] with `ld` floats between rows -> boxes of {32 columns x 128 rows}, 128-byte
-// swizzle; the TMA unit rounds to tf32 and zero-fills out-of-range rows / columns.
+// swizzle; the TMA unit rounds to tf32 (to nearest, ties to even) and zero-fills out-of-range rows /
+// columns.
 int encode_f32_map(CUtensorMap* tm, const void* base, int64_t rows, int64_t cols, int64_t ld,
                    int box_rows = LIN_M) {
   EncodeTiledFn fn = get_encode_fn();
@@ -41,6 +42,7 @@ struct keds_consumer {
   int d_in = 0, d_mid = 0, d_tok = 0, n_hidden = 0, n_layers = 0, heads = 0, dim_head = 0, inner = 0;
   bool finalized = false, attrs_set = false;
   int num_sms = 0;
+  int attend_max = 0;  // dynamic shared memory the attention kernels may use (the device's opt-in limit)
   LinearW mlp[CONS_MAX_MLP + 1];               // n_hidden x (Linear + ReLU), then fc_out
   LinearW wq[2][CONS_MAX_LAYERS], wk[2][CONS_MAX_LAYERS], wv[2][CONS_MAX_LAYERS], wo[2][CONS_MAX_LAYERS];
   LinearW wkv[2];                              // all layers' to_k / to_v stacked: [L][k | v][inner] x d_tok
@@ -125,6 +127,87 @@ int consumer_cached_map(keds_consumer* c, const float* A, int64_t rows, int K, i
   return 0;
 }
 
+// The five kernels behind one linear product (keds_debug_linear_plan reports these numbers).
+enum LinearVariant { LIN_AUTO = 0, LIN_TILE128 = 1, LIN_TILE256 = 2, LIN_PERSISTENT = 3, LIN_SPLITK2 = 4, LIN_SPLITK4 = 5 };
+
+// Which kernel runs C[M][N] (nz problems) on num_sms SMs. Host only.
+int linear_variant(int64_t M, int N, int nz, int num_sms) {
+  // tile width: fewer, wider tiles re-read A half as often but fill the SMs worse; pick by waves x
+  // bytes per k-block (32 KB for 128 columns, 48 KB for 256)
+  const long long mt = (M + LIN_M - 1) / LIN_M;
+  const long long c128 = mt * ((N + 127) / 128) * nz, c256 = mt * ((N + 255) / 256) * nz;
+  const long long sms = std::max(1, num_sms);
+  const bool wide = ((c256 + sms - 1) / sms) * 48 < ((c128 + sms - 1) / sms) * 32;
+  // a handful of tiles only: 32-column tiles with the K range split over a cluster of SK_SPLIT CTAs
+  if (c128 * 6 <= sms && num_sms >= SK_MAX_SPLIT) {
+    const long long tiles = mt * ((N + SK_BN - 1) / SK_BN) * nz;
+    return tiles * 4 <= sms ? LIN_SPLITK4 : LIN_SPLITK2;  // keep it to one wave
+  }
+  // more than two waves of wide tiles: one persistent CTA per SM with the epilogue of a tile
+  // hidden under the main loop of the next
+  if (wide && c256 > 2 * sms) return LIN_PERSISTENT;
+  return wide ? LIN_TILE256 : LIN_TILE128;
+}
+
+// Launch one variant: C[z] = act(A[z] W[z]^T + b[z]) for z < nz, C[z] [M][N] with ldc floats between
+// rows. ta*: A maps with LIN_M-row boxes; tw*: W maps with SK_BN-row boxes for the split-K variants,
+// LIN_WBOX-row boxes otherwise.
+int linear_launch(keds_consumer* c, int variant, const CUtensorMap& ta0, const CUtensorMap& ta1, const CUtensorMap& tw0,
+                  const CUtensorMap& tw1, int64_t M, int N, int K, const float* b0, const float* b1, int relu, float* C0,
+                  float* C1, int64_t ldc, int nz, cudaStream_t st) {
+  LinearParams p;
+  memset(&p, 0, sizeof p);
+  p.M = static_cast<int>(M);
+  p.N = N;
+  p.K = K;
+  p.relu = relu;
+  p.bias[0] = b0;
+  p.bias[1] = nz > 1 ? b1 : nullptr;
+  p.C[0] = C0;
+  p.C[1] = C1;
+  p.ldc = ldc;
+  p.err = c->err.as<uint32_t>();
+  p.nz = nz;
+  const long long mt = (M + LIN_M - 1) / LIN_M;
+  if (variant == LIN_SPLITK2 || variant == LIN_SPLITK4) {
+    const int split = variant == LIN_SPLITK4 ? 4 : 2;
+    const dim3 gs(static_cast<unsigned>(split * ((p.N + SK_BN - 1) / SK_BN)), static_cast<unsigned>(mt),
+                  static_cast<unsigned>(nz));
+    if (c->debug && c->dbg_launch < CONS_DBG_LAUNCHES && gs.x * gs.y * gs.z <= (unsigned)CONS_DBG_CTAS)
+      p.tdump = c->tdump.as<unsigned long long>() + static_cast<size_t>(c->dbg_launch) * CONS_DBG_CTAS * 5;
+    c->dbg_launch++;
+    if (split == 4)
+      CKS(launch_kc(true, 4, k_linear_tf32_splitk<4>, gs, dim3(SK_THREADS), SK_SMEM_BYTES, st, ta0, ta1, tw0, tw1, p));
+    else
+      CKS(launch_kc(true, 2, k_linear_tf32_splitk<2>, gs, dim3(SK_THREADS), SK_SMEM_BYTES, st, ta0, ta1, tw0, tw1, p));
+    c->launches++;
+    return 0;
+  }
+  const int bn = variant == LIN_TILE128 ? 128 : 256;
+  const dim3 grid(static_cast<unsigned>((p.N + bn - 1) / bn), static_cast<unsigned>(mt), static_cast<unsigned>(nz));
+  if (c->debug && c->dbg_launch < CONS_DBG_LAUNCHES && grid.x * grid.y * grid.z <= (unsigned)CONS_DBG_CTAS)
+    p.tdump = c->tdump.as<unsigned long long>() + static_cast<size_t>(c->dbg_launch) * CONS_DBG_CTAS * 5;
+  c->dbg_launch++;
+  if (variant == LIN_PERSISTENT) {
+    p.tdump = nullptr;  // (no per-CTA stamps: one CTA walks many tiles)
+    CKS(launch_k(true, k_linear_tf32_persistent, dim3(static_cast<unsigned>(std::max(1, c->num_sms))), dim3(PL_THREADS),
+                 PL_SMEM_BYTES, st, ta0, ta1, tw0, tw1, p));
+  } else if (variant == LIN_TILE256) {
+    CKS(launch_k(true, k_linear_tf32<256>, grid, dim3(LIN_THREADS), LinCfg<256>::kSmemBytes, st, ta0, ta1, tw0, tw1, p));
+  } else {
+    CKS(launch_k(true, k_linear_tf32<128>, grid, dim3(LIN_THREADS), LinCfg<128>::kSmemBytes, st, ta0, ta1, tw0, tw1, p));
+  }
+  c->launches++;
+  return 0;
+}
+
+int64_t round4(int64_t x) { return (x + 3) & ~int64_t(3); }
+
+// dynamic shared memory of k_cross_attend and of k_cross_attend_bwd (twice as much): forward_train
+// accepts only what its backward can also launch
+size_t attend_smem(const keds_consumer* c, int k) { return static_cast<size_t>(c->heads) * (c->dim_head + k) * 4; }
+size_t attend_bwd_smem(const keds_consumer* c, int k) { return 2 * attend_smem(c, k); }
+
 // C[z] = act(A[z] W[z]^T + b[z]) for z < nz; A[z]: [M][K] with lda floats between rows
 int consumer_linear(keds_consumer* c, const float* A0, const float* A1, int64_t lda, int64_t M,
                     const LinearW* W0, const LinearW* W1, int relu, float* C0, float* C1, int64_t ldc,
@@ -132,64 +215,31 @@ int consumer_linear(keds_consumer* c, const float* A0, const float* A1, int64_t 
   CUtensorMap ta0, ta1;
   CKS(consumer_cached_map(c, A0, M, W0->in, lda, LIN_M, &ta0));
   if (nz > 1) CKS(consumer_cached_map(c, A1, M, W1->in, lda, LIN_M, &ta1)); else ta1 = ta0;
-  LinearParams p;
-  memset(&p, 0, sizeof p);
-  p.M = static_cast<int>(M);
-  p.N = W0->out;
-  p.K = W0->in;
-  p.relu = relu;
-  p.bias[0] = W0->b.as<float>();
-  p.bias[1] = nz > 1 ? W1->b.as<float>() : nullptr;
-  p.C[0] = C0;
-  p.C[1] = C1;
-  p.ldc = ldc;
-  p.err = c->err.as<uint32_t>();
-  p.nz = nz;
-  // tile width: fewer, wider tiles re-read A half as often but fill the SMs worse; pick by waves x
-  // bytes per k-block (32 KB for 128 columns, 48 KB for 256)
-  const long long mt = (M + LIN_M - 1) / LIN_M;
-  const long long c128 = mt * ((p.N + 127) / 128) * nz, c256 = mt * ((p.N + 255) / 256) * nz;
-  const long long sms = std::max(1, c->num_sms);
-  const bool wide = ((c256 + sms - 1) / sms) * 48 < ((c128 + sms - 1) / sms) * 32;
-  // a handful of tiles only: 32-column tiles with the K range split over a cluster of SK_SPLIT CTAs
-  if (c128 * 6 <= sms && c->num_sms >= SK_MAX_SPLIT) {
-    const long long tiles = mt * ((p.N + SK_BN - 1) / SK_BN) * nz;
-    const int split = tiles * 4 <= sms ? 4 : 2;  // keep it to one wave
-    const dim3 gs(static_cast<unsigned>(split * ((p.N + SK_BN - 1) / SK_BN)), static_cast<unsigned>(mt),
-                  static_cast<unsigned>(nz));
-    if (c->debug && c->dbg_launch < CONS_DBG_LAUNCHES && gs.x * gs.y * gs.z <= (unsigned)CONS_DBG_CTAS)
-      p.tdump = c->tdump.as<unsigned long long>() + static_cast<size_t>(c->dbg_launch) * CONS_DBG_CTAS * 5;
-    c->dbg_launch++;
-    if (split == 4)
-      CKS(launch_kc(true, 4, k_linear_tf32_splitk<4>, gs, dim3(SK_THREADS), SK_SMEM_BYTES, st, ta0, ta1, W0->tm32,
-                    nz > 1 ? W1->tm32 : W0->tm32, p));
-    else
-      CKS(launch_kc(true, 2, k_linear_tf32_splitk<2>, gs, dim3(SK_THREADS), SK_SMEM_BYTES, st, ta0, ta1, W0->tm32,
-                    nz > 1 ? W1->tm32 : W0->tm32, p));
-    c->launches++;
-    return 0;
+  const int v = linear_variant(M, W0->out, nz, c->num_sms);
+  const bool sk = v == LIN_SPLITK2 || v == LIN_SPLITK4;
+  const LinearW* W1e = nz > 1 ? W1 : W0;
+  return linear_launch(c, v, ta0, ta1, sk ? W0->tm32 : W0->tm, sk ? W1e->tm32 : W1e->tm, M, W0->out, W0->in,
+                       W0->b.as<float>(), nz > 1 ? W1->b.as<float>() : nullptr, relu, C0, C1, ldc, nz, st);
+}
+
+// kernel attributes, SM count and the error word: what any linear launch on `c` needs
+int linear_init(keds_consumer* c) {
+  if (!c->attrs_set) {
+    CK(cudaFuncSetAttribute(k_linear_tf32<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)LinCfg<128>::kSmemBytes));
+    CK(cudaFuncSetAttribute(k_linear_tf32<256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)LinCfg<256>::kSmemBytes));
+    CK(cudaFuncSetAttribute(k_linear_tf32_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)PL_SMEM_BYTES));
+    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)SK_SMEM_BYTES));
+    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            (int)SK_SMEM_BYTES));
+    CK(cudaDeviceGetAttribute(&c->num_sms, cudaDevAttrMultiProcessorCount, c->device));
+    c->attrs_set = true;
   }
-  const int bn = wide ? 256 : 128;
-  const dim3 grid(static_cast<unsigned>((p.N + bn - 1) / bn), static_cast<unsigned>(mt), static_cast<unsigned>(nz));
-  if (c->debug && c->dbg_launch < CONS_DBG_LAUNCHES && grid.x * grid.y * grid.z <= (unsigned)CONS_DBG_CTAS)
-    p.tdump = c->tdump.as<unsigned long long>() + static_cast<size_t>(c->dbg_launch) * CONS_DBG_CTAS * 5;
-  c->dbg_launch++;
-  // more than two waves of wide tiles: one persistent CTA per SM with the epilogue of a tile
-  // hidden under the main loop of the next
-  if (wide && c256 > 2 * sms) {
-    p.tdump = nullptr;  // (no per-CTA stamps: one CTA walks many tiles)
-    CKS(launch_k(true, k_linear_tf32_persistent, dim3(static_cast<unsigned>(sms)), dim3(PL_THREADS), PL_SMEM_BYTES,
-                 st, ta0, ta1, W0->tm, nz > 1 ? W1->tm : W0->tm, p));
-    c->launches++;
-    return 0;
-  }
-  if (wide)
-    CKS(launch_k(true, k_linear_tf32<256>, grid, dim3(LIN_THREADS), LinCfg<256>::kSmemBytes, st, ta0, ta1,
-                 W0->tm, nz > 1 ? W1->tm : W0->tm, p));
-  else
-    CKS(launch_k(true, k_linear_tf32<128>, grid, dim3(LIN_THREADS), LinCfg<128>::kSmemBytes, st, ta0, ta1,
-                 W0->tm, nz > 1 ? W1->tm : W0->tm, p));
-  c->launches++;
+  CKS(c->err.ensure(16));
+  CK(cudaMemset(c->err.p, 0, 16));
   return 0;
 }
 
@@ -296,22 +346,15 @@ int keds_consumer_finalize(keds_consumer_t* c) {
     for (int l = 0; l < c->n_layers; ++l)
       if (!c->wq[z][l].set || !c->wk[z][l].set || !c->wv[z][l].set || !c->wo[z][l].set)
         return fail(KEDS_ERR_ARG, "consumer_finalize: attention stack %d layer %d incomplete", z, l);
-  if (!c->attrs_set) {
-    CK(cudaFuncSetAttribute(k_linear_tf32<128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)LinCfg<128>::kSmemBytes));
-    CK(cudaFuncSetAttribute(k_linear_tf32<256>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)LinCfg<256>::kSmemBytes));
-    CK(cudaFuncSetAttribute(k_linear_tf32_persistent, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)PL_SMEM_BYTES));
-    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)SK_SMEM_BYTES));
-    CK(cudaFuncSetAttribute(k_linear_tf32_splitk<4>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                            (int)SK_SMEM_BYTES));
-    CK(cudaDeviceGetAttribute(&c->num_sms, cudaDevAttrMultiProcessorCount, c->device));
-    c->attrs_set = true;
+  CKS(linear_init(c));
+  if (c->attend_max == 0) {
+    int optin = 0;
+    CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    CK(cudaFuncSetAttribute(k_cross_attend<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+    CK(cudaFuncSetAttribute(k_cross_attend<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+    CK(cudaFuncSetAttribute(k_cross_attend_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+    c->attend_max = optin;
   }
-  CKS(c->err.ensure(16));
-  CK(cudaMemset(c->err.p, 0, 16));
   const size_t wl = static_cast<size_t>(c->inner) * c->d_tok;  // one to_k or to_v matrix
   for (int z = 0; z < 2; ++z) {
     LinearW& kv = c->wkv[z];
@@ -363,8 +406,10 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_
   if (B < 0 || k <= 0 || k > 1024 || n_img < 0 || n_txt < 0) return fail(KEDS_ERR_ARG, "consumer_forward: bad B or k");
   if (B == 0) return 0;
   if (B * (1 + 2 * (int64_t)k) > (int64_t(1) << 30)) return fail(KEDS_ERR_ARG, "consumer_forward: batch too large");
-  if (static_cast<size_t>(c->heads) * (c->dim_head + k) * 4 > 48 * 1024)
+  if (attend_smem(c, k) > static_cast<size_t>(c->attend_max))
     return fail(KEDS_ERR_ARG, "consumer_forward: heads * (dim_head + k) too large for the attention kernel");
+  if (train && attend_bwd_smem(c, k) > static_cast<size_t>(c->attend_max))
+    return fail(KEDS_ERR_ARG, "consumer_forward_train: heads * (dim_head + k) too large for the attention backward");
   for (const void* ptr : {(const void*)q, (const void*)base_img, (const void*)base_txt, (const void*)I_img,
                           (const void*)I_txt, (const void*)tokens})
     if (!is_device_ptr(ptr)) return fail(KEDS_ERR_ARG, "consumer_forward: all buffers must be device memory");
@@ -472,7 +517,7 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_
     // fast path: the reference's dim_head = 64 with 16-byte aligned key / value rows
     const bool dh64 = c->dim_head == 64 && (kvw & 3) == 0;
     CKS(launch_k(true, dh64 ? k_cross_attend<64> : k_cross_attend<0>, dim3(static_cast<unsigned>(B), 2),
-                 dim3(32 * c->heads), static_cast<size_t>(c->heads) * (c->dim_head + k) * 4, st, ap));
+                 dim3(32 * c->heads), attend_smem(c, k), st, ap));
     c->launches++;
     float *o0, *o1;
     int64_t ldo;
@@ -543,6 +588,51 @@ int keds_consumer_check(keds_consumer_t* c, void* stream, int64_t* launches) {
     return fail(KEDS_ERR_KERNEL, "consumer kernel pipeline timed out (code 0x%x)", e);
   }
   return 0;
+}
+
+int keds_debug_linear_plan(int64_t M, int N, int nz, int num_sms, int32_t* variant) {
+  if (!variant || M <= 0 || N <= 0 || nz < 1 || nz > 2 || num_sms <= 0)
+    return fail(KEDS_ERR_ARG, "debug_linear_plan: bad argument");
+  *variant = linear_variant(M, N, nz, num_sms);
+  return 0;
+}
+
+int keds_consumer_debug_linear(keds_consumer_t* c, int variant, const float* A0, const float* A1, int64_t lda,
+                               int64_t M, int K, const float* W0, const float* W1, const float* b0, const float* b1,
+                               int N, int relu, float* C0, float* C1, int64_t ldc, int nz, void* stream) {
+  if (!c || variant < LIN_AUTO || variant > LIN_SPLITK4 || nz < 1 || nz > 2 || M <= 0 || K <= 0 || N <= 0)
+    return fail(KEDS_ERR_ARG, "consumer_debug_linear: bad handle, variant, nz or shape");
+  if ((M + LIN_M - 1) / LIN_M > 65535 || ldc < N)
+    return fail(KEDS_ERR_ARG, "consumer_debug_linear: M too large or ldc < N");
+  const int64_t ldw = round4(K);
+  if ((lda & 3) || lda < K) return fail(KEDS_ERR_ARG, "consumer_debug_linear: lda must be a multiple of 4 and >= K");
+  for (int z = 0; z < nz; ++z) {
+    const float* A = z ? A1 : A0;
+    const float* W = z ? W1 : W0;
+    const float* b = z ? b1 : b0;
+    const float* C = z ? C1 : C0;
+    if (!A || !W || !C || (reinterpret_cast<uintptr_t>(A) & 15) || (reinterpret_cast<uintptr_t>(W) & 15) ||
+        (reinterpret_cast<uintptr_t>(C) & 3))
+      return fail(KEDS_ERR_ARG, "consumer_debug_linear: A, W 16-byte and C 4-byte aligned, none NULL");
+    if (!is_device_ptr(A) || !is_device_ptr(W) || !is_device_ptr(C) || (b && !is_device_ptr(b)))
+      return fail(KEDS_ERR_ARG, "consumer_debug_linear: all buffers must be device memory");
+  }
+  DeviceGuard g(c->device);
+  if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  if (!c->attrs_set) CKS(linear_init(c));
+  if (variant == LIN_AUTO) variant = linear_variant(M, N, nz, c->num_sms);
+  const bool sk = variant == LIN_SPLITK2 || variant == LIN_SPLITK4;
+  CUtensorMap ta[2], tw[2];
+  for (int z = 0; z < nz; ++z) {
+    CKS(encode_f32_map(&ta[z], z ? A1 : A0, M, K, lda, LIN_M));
+    CKS(encode_f32_map(&tw[z], z ? W1 : W0, N, K, ldw, sk ? SK_BN : LIN_WBOX));
+  }
+  if (nz == 1) {
+    ta[1] = ta[0];
+    tw[1] = tw[0];
+  }
+  return linear_launch(c, variant, ta[0], ta[1], tw[0], tw[1], M, N, K, b0, b1, relu, C0, C1, ldc, nz,
+                       static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -54,8 +54,6 @@ ConsLayout consumer_layout(const keds_consumer* c) {
   return y;
 }
 
-int64_t round4(int64_t x) { return (x + 3) & ~int64_t(3); }
-
 // a weight-like operand [out][in] with `ld` floats between rows, living in scratch memory
 int train_weight(keds_consumer* c, const float* W, int out, int in, int64_t ld, LinearW* w) {
   w->out = out;
@@ -234,6 +232,8 @@ int keds_consumer_backward(keds_consumer_t* c, const float* dtokens, float* grad
   const int k = c->tr.k, L = c->n_layers, inner = c->inner, dt = c->d_tok, dm = c->d_mid, din = c->d_in;
   const int64_t kvw = static_cast<int64_t>(L) * 2 * inner;
   const int64_t ldB = round4(B), ldBk = round4(Bk), ldM = round4(M);
+  if (attend_bwd_smem(c, k) > static_cast<size_t>(c->attend_max))  // (forward_train refuses such k first)
+    return fail(KEDS_ERR_ARG, "consumer_backward: heads * (dim_head + k) too large for the attention backward");
 
   CKS(consumer_refresh_transposes(c, st));
   CKS(c->tr.dq[0].ensure(static_cast<size_t>(2) * B * dt * 4));
@@ -304,9 +304,8 @@ int keds_consumer_backward(keds_consumer_t* c, const float* dtokens, float* grad
     ap.k_off = (2 * l) * inner;
     ap.v_off = (2 * l + 1) * inner;
     ap.scale = 1.0f / sqrtf(static_cast<float>(c->dim_head));
-    const size_t at_smem = static_cast<size_t>(c->heads) * (2 * c->dim_head + 2 * k) * 4;
-    if (at_smem > 48 * 1024) return fail(KEDS_ERR_ARG, "consumer_backward: heads * (dim_head + k) too large");
-    CKS(launch_k(true, k_cross_attend_bwd, dim3(static_cast<unsigned>(B), 2), dim3(32 * c->heads), at_smem, st, ap));
+    CKS(launch_k(true, k_cross_attend_bwd, dim3(static_cast<unsigned>(B), 2), dim3(32 * c->heads), attend_bwd_smem(c, k),
+                 st, ap));
     c->launches++;
     // to_q: dWq = dQ^T q_in, dbq, dq_in = dQ Wq
     CKS(train_weight_grad(c, dQ0, dQ1, inner, in0, in1, dt, B, inner, dt, grads + y.q_w[0][l], grads + y.q_w[1][l], 2, st));

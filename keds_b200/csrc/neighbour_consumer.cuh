@@ -6,7 +6,9 @@
 // Two kernels:
 //   k_linear_tf32   C = act(A W^T + bias), nn.Linear layout (W: [out][in]), fp32 in / fp32 out,
 //                   tcgen05.mma kind::tf32 with TMA-staged operands (the TMA unit rounds fp32 to
-//                   tf32 on the way in), accumulators in TMEM, bias (+ReLU) fused in the epilogue.
+//                   tf32 on the way in: to nearest, ties to even, subnormals kept -- measured by
+//                   tests/test_gpu_consumer_kernels.py), accumulators in TMEM, bias (+ReLU) fused
+//                   in the epilogue.
 //                   blockIdx.z selects one of two independent problems of the same shape (the two
 //                   attention stacks), so both run in one launch.
 //   k_cross_attend  softmax(q K^T / sqrt(dh)) V for ONE query token per batch row over its k

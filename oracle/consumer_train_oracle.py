@@ -24,6 +24,8 @@ from typing import Dict, Mapping, Optional, Sequence
 import numpy as np
 import torch
 
+from .consumer_oracle import round_tf32
+
 
 def _t(a) -> torch.Tensor:
     if isinstance(a, torch.Tensor):
@@ -31,15 +33,41 @@ def _t(a) -> torch.Tensor:
     return torch.from_numpy(np.asarray(a, dtype=np.float64))
 
 
+class _Tf32Linear(torch.autograd.Function):
+    """x W^T with both operands rounded to tf32 in every product, as the native GEMMs compute them:
+    forward x W^T, backward dX = dY W and dW = dY^T X."""
+
+    @staticmethod
+    def forward(ctx, x, W):
+        ctx.save_for_backward(x, W)
+        return _tf32(x) @ _tf32(W).t()
+
+    @staticmethod
+    def backward(ctx, g):
+        x, W = ctx.saved_tensors
+        g2 = _tf32(g.reshape(-1, g.shape[-1]))
+        dx = (g2 @ _tf32(W)).reshape(x.shape)
+        dW = g2.t() @ _tf32(x.reshape(-1, x.shape[-1]))
+        return dx, dW
+
+
+def _tf32(t: torch.Tensor) -> torch.Tensor:
+    return torch.from_numpy(round_tf32(t.detach().numpy()))
+
+
+def _matmul_wt(x: torch.Tensor, W: torch.Tensor, tf32: bool) -> torch.Tensor:
+    return _Tf32Linear.apply(x, W) if tf32 else x @ W.t()
+
+
 def _params(sd: Mapping[str, object]) -> Dict[str, torch.Tensor]:
     return {k: _t(v).clone().requires_grad_(True) for k, v in sd.items()}
 
 
 def _im2text(p: Dict[str, torch.Tensor], x: torch.Tensor, masks: Optional[Sequence[Optional[torch.Tensor]]],
-             gates: Optional[Sequence[torch.Tensor]] = None) -> torch.Tensor:
+             gates: Optional[Sequence[torch.Tensor]] = None, tf32: bool = False) -> torch.Tensor:
     i = 0
     while f"layers.{i}.0.weight" in p:
-        z = x @ p[f"layers.{i}.0.weight"].t() + p[f"layers.{i}.0.bias"]
+        z = _matmul_wt(x, p[f"layers.{i}.0.weight"], tf32) + p[f"layers.{i}.0.bias"]
         if masks is not None and masks[i] is not None:
             z = z * masks[i]
         # gates: the ReLU decisions of another evaluation of the same network (0 / 1 per unit). A
@@ -49,17 +77,18 @@ def _im2text(p: Dict[str, torch.Tensor], x: torch.Tensor, masks: Optional[Sequen
         # tiny pre-activation only).
         x = torch.relu(z) if gates is None else z * gates[i]
         i += 1
-    return x @ p["fc_out.weight"].t() + p["fc_out.bias"]
+    return _matmul_wt(x, p["fc_out.weight"], tf32) + p["fc_out.bias"]
 
 
-def _crossformer(p: Dict[str, torch.Tensor], q: torch.Tensor, kv: torch.Tensor, heads: int) -> torch.Tensor:
+def _crossformer(p: Dict[str, torch.Tensor], q: torch.Tensor, kv: torch.Tensor, heads: int,
+                 tf32: bool = False) -> torch.Tensor:
     B, n, _ = kv.shape
     l = 0
     while f"cross_layers.{l}.to_q.weight" in p:
         pre = f"cross_layers.{l}."
-        Q = q @ p[pre + "to_q.weight"].t() + p[pre + "to_q.bias"]
-        K = kv @ p[pre + "to_k.weight"].t() + p[pre + "to_k.bias"]
-        V = kv @ p[pre + "to_v.weight"].t() + p[pre + "to_v.bias"]
+        Q = _matmul_wt(q, p[pre + "to_q.weight"], tf32) + p[pre + "to_q.bias"]
+        K = _matmul_wt(kv, p[pre + "to_k.weight"], tf32) + p[pre + "to_k.bias"]
+        V = _matmul_wt(kv, p[pre + "to_v.weight"], tf32) + p[pre + "to_v.bias"]
         inner = Q.shape[-1]
         dh = inner // heads
         Qh = Q.reshape(B, 1, heads, dh).permute(0, 2, 1, 3)
@@ -67,15 +96,18 @@ def _crossformer(p: Dict[str, torch.Tensor], q: torch.Tensor, kv: torch.Tensor, 
         Vh = V.reshape(B, n, heads, dh).permute(0, 2, 1, 3)
         attn = torch.softmax(torch.einsum("bhid,bhjd->bhij", Qh, Kh) * dh ** -0.5, dim=-1)
         out = torch.einsum("bhij,bhjd->bhid", attn, Vh).permute(0, 2, 1, 3).reshape(B, 1, inner)
-        q = out @ p[pre + "to_out.0.weight"].t() + p[pre + "to_out.0.bias"]
+        q = _matmul_wt(out, p[pre + "to_out.0.weight"], tf32) + p[pre + "to_out.0.bias"]
         l += 1
     return q
 
 
 def tokens_and_grads(img2text_sd, retrieval_fuse_sd, text_condition_sd, heads: int, feature, nb_img_rows, nb_txt_rows,
-                     dtokens, masks: Optional[Sequence[Optional[object]]] = None, gates: Optional[Sequence[object]] = None):
+                     dtokens, masks: Optional[Sequence[Optional[object]]] = None, gates: Optional[Sequence[object]] = None,
+                     tf32: bool = False):
     """feature [B, d_in]; nb_*_rows [B, k, d_in] the gathered neighbour rows; masks: per hidden layer
     None or [B(1+2k), d_mid] multipliers over the rows (queries | image neighbours | text neighbours).
+    tf32: every nn.Linear product, forward and backward, with tf32-rounded operands as the native
+    GEMMs compute them (attention, softmax, bias adds and bias gradients stay exact).
     Returns (tokens [B,3,d_tok] float64 numpy, {"img2text/<name>": grad, "retrieval_fuse/<name>": ...})."""
     pm, pf, pc = _params(img2text_sd), _params(retrieval_fuse_sd), _params(text_condition_sd)
     feat, ni, nt = _t(feature), _t(nb_img_rows), _t(nb_txt_rows)
@@ -83,12 +115,12 @@ def tokens_and_grads(img2text_sd, retrieval_fuse_sd, text_condition_sd, heads: i
     x = torch.cat([feat, ni.reshape(B * k, d_in), nt.reshape(B * k, d_in)], dim=0)
     mk = None if masks is None else [None if m is None else _t(m) for m in masks]
     gt = None if gates is None else [_t(gv) for gv in gates]
-    y = _im2text(pm, x, mk, gt)
+    y = _im2text(pm, x, mk, gt, tf32)
     mapped = y[:B]
     nb_img = y[B:B + B * k].reshape(B, k, -1)
     nb_txt = y[B + B * k:].reshape(B, k, -1)
-    fused = _crossformer(pf, mapped[:, None, :], nb_img, heads)
-    text_c = _crossformer(pc, mapped[:, None, :], nb_txt, heads)
+    fused = _crossformer(pf, mapped[:, None, :], nb_img, heads, tf32)
+    text_c = _crossformer(pc, mapped[:, None, :], nb_txt, heads, tf32)
     tokens = torch.cat([fused, text_c, mapped[:, None, :]], dim=1)
     tokens.backward(_t(dtokens))
     grads = {}

@@ -4,10 +4,12 @@ the float64 oracle (oracle/consumer_train_oracle.py, pinned to the reference's o
 tests/golden/consumer_train.npz).
 
 Tolerance: every product runs on tf32 tensor cores (10-bit mantissa operands, fp32 accumulation);
-the reference trains in fp32 (fp16 under amp autocast, src/trainer.py:462-465). Asserted per
-tensor: max |got - oracle| <= 1e-2 * max |oracle| (measured: 5e-4 at the reference's widths on
-unit-norm inputs, 5e-3 on unnormalised inputs after an SGD step), with the ReLU gates of the native
-forward (see check_against_oracle).
+the reference trains in fp32 (fp16 under amp autocast, src/trainer.py:462-465). The native path is
+compared with the oracle in its tf32 mode (every Linear product, forward and backward, with
+tf32-rounded operands), with the ReLU gates of the native forward (see check_against_oracle):
+tokens within TF32_TOK_TOL and every gradient within TF32_GRAD_TOL of the tensor's maximum. Against
+the reference's own modules in float64 (tests/golden/consumer_train.npz), which do not round, the
+bounds are TOK_TOL and GRAD_TOL.
 """
 import os
 
@@ -24,6 +26,13 @@ from oracle import consumer_oracle as corc  # noqa: E402
 from oracle import consumer_train_oracle as cto  # noqa: E402
 
 TOK_TOL, GRAD_TOL = 4e-3, 1e-2
+# With tf32 rounding modelled, what is left is fp32 accumulation (K up to B(1+2k) rows in dW) and
+# fp32 attention and its backward, amplified by sharp softmaxes as in tests/test_gpu_consumer.py.
+# A gradient is measured against the larger of its own maximum and 1e-3 of the largest gradient (the
+# to_k biases have an exactly zero gradient). Measured on a B200 (1000 W): tokens at most 1.3e-4,
+# gradients at most 4.1e-4, the latter in the SGD-step case on unnormalised inputs, which differs
+# from the plain oracle by 5e-3: that excess is tf32 operand rounding, not a defect.
+TF32_TOK_TOL, TF32_GRAD_TOL = 4e-4, 1e-3
 
 
 def to_torch(sd):
@@ -52,7 +61,7 @@ def run(sds, heads, feat, base_img, base_txt, I_img, I_txt, dtok, masks=None, dr
     return mod, ix_i, ix_t, f, Ii, It
 
 
-def check_against_oracle(sds, heads, feat, base_img, base_txt, I_img, I_txt, dtok, masks=None):
+def check_against_oracle(sds, heads, feat, base_img, base_txt, I_img, I_txt, dtok, masks=None, tf32=True):
     mod, ix_i, ix_t, f, Ii, It = run(sds, heads, feat, base_img, base_txt, I_img, I_txt, dtok)
     from keds_b200.consumer import _ConsumerFn
     mk = None if masks is None else [None if m is None else torch.from_numpy(m.astype(np.float32)).cuda() for m in masks]
@@ -69,18 +78,20 @@ def check_against_oracle(sds, heads, feat, base_img, base_txt, I_img, I_txt, dto
     M = B * (1 + 2 * k)
     n_hidden = sum(1 for name in sds[0] if name.endswith(".0.weight"))
     gates = [(mod.debug_hidden(i, M) > 0).double().cpu().numpy() for i in range(n_hidden)]
-    _, free = cto.tokens_and_grads(sds[0], sds[1], sds[2], heads, feat, nb_i, nb_t, dtok, masks)
-    want_tok, want = cto.tokens_and_grads(sds[0], sds[1], sds[2], heads, feat, nb_i, nb_t, dtok, masks, gates)
+    tok_tol, grad_tol = (TF32_TOK_TOL, TF32_GRAD_TOL) if tf32 else (TOK_TOL, GRAD_TOL)
+    _, free = cto.tokens_and_grads(sds[0], sds[1], sds[2], heads, feat, nb_i, nb_t, dtok, masks, tf32=tf32)
+    want_tok, want = cto.tokens_and_grads(sds[0], sds[1], sds[2], heads, feat, nb_i, nb_t, dtok, masks, gates,
+                                          tf32=tf32)
     assert rel(want["img2text/fc_out.weight"], free["img2text/fc_out.weight"]) < 1e-2   # same network, same gates almost everywhere
     errs = {"tokens": rel(tokens.detach().cpu().numpy(), want_tok)}
-    assert errs["tokens"] < TOK_TOL, errs
+    assert errs["tokens"] < tok_tol, errs
     gi, gf, gc = mod.state_dicts(grads=True)
     scale = 1e-3 * max(float(np.abs(v).max()) for v in want.values())
     for prefix, gsd in (("img2text", gi), ("retrieval_fuse", gf), ("text_condition", gc)):
         for name, t in gsd.items():
             errs[f"{prefix}/{name}"] = rel(t.cpu().numpy(), want[f"{prefix}/{name}"], scale)
     worst = max(errs, key=errs.get)
-    assert errs[worst] < GRAD_TOL, "\n".join(f"{v:.3e}  {k_}" for k_, v in sorted(errs.items(), key=lambda kv: -kv[1])[:14])
+    assert errs[worst] < grad_tol, "\n".join(f"{v:.3e}  {k_}" for k_, v in sorted(errs.items(), key=lambda kv: -kv[1])[:14])
     return errs, mod
 
 
@@ -94,7 +105,9 @@ def test_reference_module_gradients_small_widths(golden_dir):
     base_img = g["topk_image"].reshape(B * k, d_in).astype(np.float32)
     base_txt = g["topk_text"].reshape(B * k, d_in).astype(np.float32)
     I = np.arange(B * k, dtype=np.int64).reshape(B, k)
-    errs, mod = check_against_oracle(sds, heads, g["feat"].astype(np.float32), base_img, base_txt, I, I, g["dtokens"])
+    errs, mod = check_against_oracle(sds, heads, g["feat"].astype(np.float32), base_img, base_txt, I, I, g["dtokens"],
+                                     tf32=False)
+    check_against_oracle(sds, heads, g["feat"].astype(np.float32), base_img, base_txt, I, I, g["dtokens"])
     gi, gf, gc = mod.state_dicts(grads=True)
     scale = 1e-3 * max(float(np.abs(g[k_]).max()) for k_ in g.files if k_.startswith("grad/"))
     for prefix, gsd in (("img2text", gi), ("retrieval_fuse", gf), ("text_condition", gc)):
@@ -154,14 +167,18 @@ def test_optimizer_updates_are_read_through_and_eval_matches_the_forward_only_co
     nb_i = base[I1.reshape(-1)].reshape(B, k, -1)
     nb_t = base[I2.reshape(-1)].reshape(B, k, -1)
     gates = [(mod.debug_hidden(i, B * (1 + 2 * k)) > 0).double().cpu().numpy() for i in range(2)]
-    want_tok, want = cto.tokens_and_grads(new_sds[0], new_sds[1], new_sds[2], 4, feat, nb_i, nb_t, dtok, None, gates)
-    assert rel(t1.detach().cpu().numpy(), want_tok) < TOK_TOL
+    want_tok, want = cto.tokens_and_grads(new_sds[0], new_sds[1], new_sds[2], 4, feat, nb_i, nb_t, dtok, None, gates,
+                                          tf32=True)
+    assert rel(t1.detach().cpu().numpy(), want_tok) < TF32_TOK_TOL
     assert not torch.equal(t1.detach(), t0.detach())
     gi, gf, gc = mod.state_dicts(grads=True)
     scale = 1e-3 * max(float(np.abs(v).max()) for v in want.values())
+    errs = {}
     for prefix, gsd in (("img2text", gi), ("retrieval_fuse", gf), ("text_condition", gc)):
         for name, t in gsd.items():
-            assert rel(t.cpu().numpy(), want[f"{prefix}/{name}"], scale) < GRAD_TOL, (prefix, name)
+            errs[f"{prefix}/{name}"] = rel(t.cpu().numpy(), want[f"{prefix}/{name}"], scale)
+    print("after an SGD step, worst:", sorted(errs.items(), key=lambda kv: -kv[1])[:4])
+    assert max(errs.values()) < TF32_GRAD_TOL, sorted(errs.items(), key=lambda kv: -kv[1])[:6]
     # train() mode draws dropout masks: outputs differ from eval, gradients still flow
     mod.train()
     mod.dropout = 0.5
@@ -169,3 +186,57 @@ def test_optimizer_updates_are_read_through_and_eval_matches_the_forward_only_co
     assert not torch.equal(t2.detach(), t1.detach())
     t2.sum().backward()
     assert torch.isfinite(mod.flat.grad).all() and float(mod.flat.grad.abs().max()) > 0
+
+
+# (B, k, heads, dim_head, n_hidden, n_layers): see tests/test_gpu_consumer.py ATTENTION_SHAPES
+TRAIN_SHAPES = [
+    (1, 31, 16, 64, 1, 1),
+    (129, 32, 32, 16, 3, 4),
+    (129, 33, 6, 40, 1, 4),
+    (1, 64, 2, 96, 3, 1),
+    (129, 100, 1, 4, 1, 1),
+    (129, 64, 16, 64, 3, 4),
+]
+
+
+@pytest.mark.parametrize("B,k,heads,dim_head,n_hidden,n_layers", TRAIN_SHAPES)
+def test_attention_shapes_gradients_match_the_tf32_oracle(B, k, heads, dim_head, n_hidden, n_layers):
+    sds = corc.random_state_dicts(96, 64, 80, n_hidden, n_layers, heads, dim_head, seed=B * k)
+    rng = np.random.default_rng(B + k)
+    n = 700
+    base_img = rng.standard_normal((n, 96)).astype(np.float32)
+    base_txt = rng.standard_normal((n, 96)).astype(np.float32)
+    feat = rng.standard_normal((B, 96)).astype(np.float32)
+    I_img = rng.integers(0, n, (B, k)).astype(np.int64)
+    I_txt = rng.integers(0, n, (B, k)).astype(np.int64)
+    dtok = rng.standard_normal((B, 3, 80)).astype(np.float32)
+    M = B * (1 + 2 * k)
+    masks = [((rng.random((M, 64)) < 0.9) / 0.9).astype(np.float32) for _ in range(n_hidden)]
+    errs, _ = check_against_oracle(sds, heads, feat, base_img, base_txt, I_img, I_txt, dtok, masks)
+    print(f"B={B} k={k} heads={heads} dim_head={dim_head}: worst", sorted(errs.items(), key=lambda kv: -kv[1])[:3])
+
+
+def test_forward_train_accepts_only_what_the_backward_can_run():
+    """The attention backward needs heads (2 dim_head + 2k) floats of shared memory, twice the
+    forward's. At the reference's 8 heads x 64 every k the forward accepts (up to 1024; 705 was the
+    first beyond the default 48 KB) must train; at 32 heads x 64 and k = 1024 the backward needs more
+    than a B200 block can have, so forward_train must refuse up front while the eval forward, which
+    needs half, still runs."""
+    rng = np.random.default_rng(4)
+    n, B = 3000, 2
+    base = rng.standard_normal((n, 64)).astype(np.float32)
+    feat = rng.standard_normal((B, 64)).astype(np.float32)
+    sds = corc.random_state_dicts(64, 32, 64, 1, 1, 8, 64, seed=4)
+    for k in (705, 1024):
+        I1 = rng.integers(0, n, (B, k)).astype(np.int64)
+        I2 = rng.integers(0, n, (B, k)).astype(np.int64)
+        dtok = rng.standard_normal((B, 3, 64)).astype(np.float32)
+        check_against_oracle(sds, 8, feat, base, base, I1, I2, dtok)
+    sds = corc.random_state_dicts(64, 32, 64, 1, 1, 32, 64, seed=5)
+    I = rng.integers(0, n, (B, 1024)).astype(np.int64)
+    mod, ix_i, ix_t, f, Ii, It = run(sds, 32, feat, base, base, I, I, None)
+    with pytest.raises(RuntimeError, match="attention backward"):
+        mod(f, ix_i, ix_t, Ii, It)
+    assert mod.flat.grad is None
+    ref = NeighbourConsumer(*mod.state_dicts(), heads=32, device=0)
+    assert torch.isfinite(ref(f, ix_i, ix_t, Ii, It)).all()

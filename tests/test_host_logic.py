@@ -150,3 +150,71 @@ def test_parallel_runner_keeps_order_and_raises_the_first_error():
 
     with pytest.raises(RuntimeError, match="shard 1 failed"):
         _run_parallel([job(0, 0.0), boom, job(2, 0.0)])
+
+
+# ------------------------------------------------------------------ the consumer's GEMM chooser (host only)
+TILE128, TILE256, PERSISTENT, SPLITK2, SPLITK4 = 1, 2, 3, 4, 5
+
+
+def _linear_plan(M, N, nz, sms=148):
+    import ctypes as C
+
+    from keds_b200 import _capi
+    v = C.c_int32(-1)
+    _capi.check(_capi.load().keds_debug_linear_plan(M, N, nz, sms, C.byref(v)))
+    return v.value
+
+
+@pytest.mark.parametrize("what,M,N,nz,variant", [
+    # B = 128, k = 16 at the reference's widths (768 -> 512 -> 512 -> 768, inner 512, 3 layers)
+    ("MLP hidden", 128 * 33, 512, 1, TILE128),
+    ("fc_out", 128 * 33, 768, 1, TILE256),
+    ("K/V of every layer", 128 * 16, 3072, 2, PERSISTENT),
+    ("to_q", 128, 512, 2, SPLITK4),
+    ("to_out", 128, 768, 2, SPLITK2),
+    ("MLP dW", 512, 768, 1, SPLITK2),
+    # B = 37: fewer tiles move fc_out and K/V to narrower variants
+    ("fc_out B=37", 37 * 33, 768, 1, TILE128),
+    ("K/V B=37", 37 * 16, 3072, 2, TILE256),
+    ("to_q B=37", 37, 512, 2, SPLITK4),
+    # the contrastive loss: N = 1024 logits (K = 3 x 768, nz = 2), its gradient for 256 local rows
+    ("clip logits", 1024, 1024, 2, TILE128),
+    ("clip gradient", 256, 768, 2, SPLITK2),
+])
+def test_linear_chooser_at_the_consumer_products(what, M, N, nz, variant):
+    assert _linear_plan(M, N, nz) == variant, what
+
+
+def test_linear_chooser_sweep_reaches_every_variant_and_respects_its_rules():
+    seen = set()
+    for M in (1, 37, 128, 129, 592, 1221, 2048, 4224, 20000):
+        for N in (4, 32, 260, 512, 768, 1024, 3072):
+            for nz in (1, 2):
+                v = _linear_plan(M, N, nz)
+                seen.add(v)
+                mt = -(-M // 128)
+                c128, c256 = mt * -(-N // 128) * nz, mt * -(-N // 256) * nz
+                if c128 * 6 <= 148:
+                    tiles32 = mt * -(-N // 32) * nz
+                    assert v == (SPLITK4 if tiles32 * 4 <= 148 else SPLITK2), (M, N, nz)
+                else:
+                    assert v in (TILE128, TILE256, PERSISTENT), (M, N, nz)
+                    assert (v == PERSISTENT) == (v != TILE128 and c256 > 2 * 148), (M, N, nz)
+    assert seen == {TILE128, TILE256, PERSISTENT, SPLITK2, SPLITK4}
+
+
+@pytest.mark.parametrize("sms", [1, 2, 3])
+def test_linear_chooser_without_four_sms_never_takes_split_k(sms):
+    for M, N, nz in [(1, 4, 1), (1, 32, 2), (128, 512, 2), (4224, 768, 1), (2048, 3072, 2)]:
+        assert _linear_plan(M, N, nz, sms) in (TILE128, TILE256, PERSISTENT)
+
+
+def test_linear_chooser_rejects_bad_arguments():
+    import ctypes as C
+
+    from keds_b200 import _capi
+    v = C.c_int32(-1)
+    lib = _capi.load()
+    for args in [(0, 4, 1, 148), (4, 0, 1, 148), (4, 4, 3, 148), (4, 4, 1, 0)]:
+        assert lib.keds_debug_linear_plan(*args, C.byref(v)) == -1
+    assert lib.keds_debug_linear_plan(4, 4, 1, 148, None) == -1

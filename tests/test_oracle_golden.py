@@ -172,3 +172,78 @@ def test_consumer_training_oracle_matches_reference_modules(golden_dir):
     _, grads0 = cto.tokens_and_grads(sds[0], sds[1], sds[2], int(g["dims"][5]), g["feat"], g["topk_image"],
                                      g["topk_text"], g["dtokens"], zeros)
     assert np.abs(grads0["img2text/layers.0.0.weight"]).max() == 0.0
+
+
+# ------------------------------------------------------------------ tf32 operand rounding of the oracles
+def test_round_tf32_ties_signs_subnormals_and_overflow():
+    from oracle.consumer_oracle import round_tf32
+
+    h = 2.0 ** -11                    # half a tf32 unit in the last place at 1.0
+    x = np.array([1 + h, 1 + 3 * h, 1 + h * 0.999, 1 + h * 1.001, -(1 + h), -(1 + 3 * h), 0.0, -0.0])
+    assert list(round_tf32(x, "rne")) == [1, 1 + 4 * h, 1, 1 + 2 * h, -1, -(1 + 4 * h), 0, 0]
+    assert list(round_tf32(x, "rz")) == [1, 1 + 2 * h, 1, 1, -1, -(1 + 2 * h), 0, 0]
+    assert np.signbit(round_tf32(np.float32(-0.0), "rne"))
+    # subnormals round on the same 13-bit grid: 0x1000 x 2^-149 is a tie between 0 and 0x2000 x 2^-149
+    sub = np.array([0x1000, 0x1001, 0x2FFF, 0x3000], np.uint32).view(np.float32)
+    assert list(round_tf32(sub, "rz")) == list(2.0 ** -149 * np.array([0, 0, 0x2000, 0x2000]))
+    assert list(round_tf32(sub, "rne")) == list(2.0 ** -149 * np.array([0, 0x2000, 0x2000, 0x4000]))
+    # FLT_MAX lies above the largest tf32 value by more than half a unit: nearest overflows
+    fmax = np.finfo(np.float32).max
+    tf32_max = (2 - 2.0 ** -10) * 2.0 ** 127
+    assert round_tf32(fmax, "rne") == np.inf and round_tf32(-fmax, "rne") == -np.inf
+    assert round_tf32(fmax, "rz") == tf32_max and round_tf32(np.float32(tf32_max), "rne") == tf32_max
+    special = round_tf32(np.array([np.inf, -np.inf, np.nan], np.float32))
+    assert special[0] == np.inf and special[1] == -np.inf and np.isnan(special[2])
+    # float64 input is first rounded to float32, as the native operands are stored
+    assert round_tf32(1 + 2.0 ** -30, "rz") == 1.0
+    with pytest.raises(ValueError):
+        round_tf32(x, "up")
+
+
+def test_round_tf32_matches_the_bit_masks_on_random_values():
+    from oracle.consumer_oracle import round_tf32
+
+    rng = np.random.default_rng(0)
+    bits = rng.integers(0, 2 ** 32, 100_000, dtype=np.uint64).astype(np.uint32)
+    x = bits.view(np.float32)
+    fin = np.isfinite(x)
+    for mode in ("rne", "rz"):
+        r = round_tf32(x, mode).astype(np.float32)
+        rb = r.view(np.uint32)
+        ok = fin & np.isfinite(r)
+        assert np.all(rb[ok] & 0x1FFF == 0)                                  # representable
+        d = np.abs(r[ok].astype(np.float64) - x[ok].astype(np.float64))
+        ulp = np.spacing(np.abs(x[ok])).astype(np.float64) * 2 ** 13         # tf32 unit of x's binade
+        assert np.all(d <= (ulp if mode == "rz" else ulp / 2) * (1 + 1e-12))  # within a (half) unit
+        if mode == "rz":
+            assert np.all(np.abs(r[ok]) <= np.abs(x[ok]))
+
+
+def test_tf32_oracles_equal_the_plain_ones_on_tf32_values():
+    """Small integers are tf32 numbers and their products and sums stay exact: with such operands the
+    tf32 mode changes nothing, forward (numpy oracle) and backward (the autograd Function)."""
+    import torch
+
+    from oracle import consumer_oracle as co
+    from oracle import consumer_train_oracle as cto
+
+    rng = np.random.default_rng(1)
+    sd = {"layers.0.0.weight": rng.integers(-3, 4, (6, 8)), "layers.0.0.bias": rng.integers(-3, 4, 6),
+          "fc_out.weight": rng.integers(-3, 4, (5, 6)), "fc_out.bias": rng.integers(-3, 4, 5)}
+    x = rng.integers(-4, 5, (7, 8)).astype(np.float32)
+    assert np.array_equal(co.im2text(sd, x, tf32=True), co.im2text(sd, x))
+    xt = torch.from_numpy(x.astype(np.float64)).requires_grad_(True)
+    W = torch.from_numpy(rng.integers(-3, 4, (5, 8)).astype(np.float64)).requires_grad_(True)
+    g = torch.from_numpy(rng.integers(-3, 4, (7, 5)).astype(np.float64))
+    y = cto._Tf32Linear.apply(xt, W)
+    y.backward(g)
+    assert torch.equal(y, xt @ W.t()) and torch.equal(xt.grad, g @ W) and torch.equal(W.grad, g.t() @ xt)
+    # on general values every product of the backward sees rounded operands
+    xt = torch.from_numpy(rng.standard_normal((2, 3, 8))).requires_grad_(True)
+    W = torch.from_numpy(rng.standard_normal((5, 8))).requires_grad_(True)
+    g = torch.from_numpy(rng.standard_normal((2, 3, 5)))
+    cto._Tf32Linear.apply(xt, W).backward(g)
+    r = co.round_tf32
+    g2, x2 = g.numpy().reshape(6, 5), xt.detach().numpy().reshape(6, 8)
+    assert np.array_equal(xt.grad.numpy(), (r(g2) @ r(W.detach().numpy())).reshape(2, 3, 8))
+    assert np.array_equal(W.grad.numpy(), r(g2).T @ r(x2))
