@@ -130,6 +130,32 @@ int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, 
                           int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img,
                           float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags,
                           void* cuda_stream);
+/* ---- search with exclusion -------------------------------------------------------------------
+ * The four calls above with rows left out per query (training without self-retrieval: a query
+ * whose own pair is in the knowledge base must not retrieve it). exclude: int64 [nq][n_exclude],
+ * 1 <= n_exclude <= 8, labels as I returns them (id_offset included); -1 = unused slot, a label the
+ * index does not hold excludes nothing. Device memory of the index's GPU; the hostio variant also
+ * takes page-locked host memory, read through the mapping once per call, like q. In two-database
+ * calls one array applies to both databases (aligned row for row: a pair's image row and caption
+ * row share a label). Each query's result equals an exact fp32 flat search over the rows it does
+ * not exclude: same order, same ties, -1 / -+FLT_MAX padding when fewer than k rows remain; an
+ * excluded row is never returned. Gather, pool and host mirrors follow the returned I. */
+int keds_index_search_exclude(keds_index_t* idx, const float* q, int64_t nq, int k, float* D, int64_t* I,
+                              const int64_t* exclude, int n_exclude, uint32_t flags, void* cuda_stream);
+int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k,
+                               float* Da, int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude,
+                               int n_exclude, uint32_t flags, void* cuda_stream);
+int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                           const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                           float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
+                           float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude,
+                           int n_exclude, uint32_t flags, void* cuda_stream);
+int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                                  const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                                  float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
+                                  int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img,
+                                  float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude,
+                                  int n_exclude, uint32_t flags, void* cuda_stream);
 /* Wait for the last asynchronous search on idx and report its device status. */
 int keds_index_sync(keds_index_t* idx, void* cuda_stream);
 int keds_index_last_stats(const keds_index_t* idx, keds_search_stats* out);

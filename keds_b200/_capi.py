@@ -74,6 +74,21 @@ SIGNATURES = {
         [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
          _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint32, _vp],
     ),
+    "keds_index_search_exclude": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp]),
+    "keds_index_search2_exclude": (
+        C.c_int,
+        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
+    ),
+    "keds_retrieve2_exclude": (
+        C.c_int,
+        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
+         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
+    ),
+    "keds_retrieve2_hostio_exclude": (
+        C.c_int,
+        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
+         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
+    ),
     "keds_index_label_hits": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp, C.c_int, _vp, _vp]),
     "keds_index_sync": (C.c_int, [_vp, _vp]),
     "keds_index_last_stats": (C.c_int, [_vp, C.POINTER(SearchStats)]),

@@ -135,19 +135,21 @@ class NeighbourConsumer:
         return out
 
     def from_features(self, image_features: torch.Tensor, database, topk: int = 16,
-                      shuffle: bool = True) -> torch.Tensor:
+                      shuffle: bool = True, exclude=None) -> torch.Tensor:
         """The whole block of src/trainer.py:53-69 / src/eval_utils.py:373-383 for one batch:
         retrieve the topk image / text neighbours of `image_features` from `database`
         (KnowledgeBase or the reference's 5-item sequence with native indices) and return
         tokens [B, 3, d_tok]. The search normalises its copy of the features (src/trainer.py:206);
         img2text sees them as given. shuffle: the batch-shared randperm of :218-219 (it cannot
-        change the result beyond fp32 summation order)."""
+        change the result beyond fp32 summation order). exclude: int64 [B] or [B, E] rows each query
+        must not retrieve (e.g. database.rows_of(names), training without self-retrieval); None:
+        the reference's search."""
         from .index import search2
 
         image_index, text_index = database[3], database[4]
         feats = image_features.detach().to(device=torch.device("cuda", self.device), dtype=torch.float32).contiguous()
         q = feats / feats.norm(dim=1, keepdim=True)
-        (_, I_img), (_, I_txt) = search2(image_index, text_index, q, topk)
+        (_, I_img), (_, I_txt) = search2(image_index, text_index, q, topk, exclude=exclude)
         perm = torch.randperm(topk) if shuffle else None
         return self(feats, image_index, text_index, I_img, I_txt, perm)
 

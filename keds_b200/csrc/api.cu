@@ -245,6 +245,7 @@ struct keds_index {
   bool use_pair = true;
   // per-call scratch (one search in flight per handle)
   DevBuf q_f32, q_bf16, qstat, cand, cand_cnt, cand_theta, flagged[2], ctrl, exact_scratch, rk, theta0;
+  DevBuf ex_rows;  // search with exclusion: the staged local row ids [n_db][nq][n_ex] of the pass
   bool warm_start = true;  // lists start at a finished list's threshold (KEDS_NO_WARM_START=1: every list cold)
   DevBuf D_stage[2], I_stage[2];
   HostBuf h_q, h_out;  // pinned staging for host-pointer calls
@@ -282,6 +283,10 @@ int set_kernel_attrs(keds_index* ix) {
                           (int)SCORE_SMEM_BYTES));
 
   CK(cudaFuncSetAttribute(k_score_topk<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)SCORE_PAIR_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(k_score_topk<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)SCORE_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(k_score_topk<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)SCORE_PAIR_SMEM_BYTES));
   const char* no_pair = getenv("KEDS_NO_PAIR");
   ix->use_pair = !(no_pair && no_pair[0] == '1');
@@ -458,9 +463,15 @@ int prof_mark(keds_index* a, cudaStream_t st, int tag) {
 // of the flagged list is empty.
 int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_dev, int64_t nq, int k,
                  float* D[2], long long* I[2], int metric, const ConsumeParams& cons,
-                 unsigned long long* timing, cudaStream_t st, const PeerOut* peer = nullptr) {
+                 unsigned long long* timing, cudaStream_t st, const PeerOut* peer = nullptr,
+                 const ExcludeStage* ex = nullptr) {
   ExactParams ep;
   memset(&ep, 0, sizeof ep);
+  if (ex) {
+    ep.ex_rows = ex->rows;
+    ep.n_ex = ex->n_ex;
+    ep.ex_ld = ex->nq * ex->n_ex;
+  }
   ep.cons = cons;
   ep.n_db = n_db;
   ep.d = ix->d;
@@ -543,9 +554,12 @@ int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_de
 int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int k, float* D[2],
                 long long* I[2], uint32_t flags, cudaStream_t st, float* dump, int64_t ld_dump,
                 const ConsumeParams* cons_in, const PeerOut* peer = nullptr, int pass_idx = 0,
-                const float* q_src = nullptr, const HitsMode* hm = nullptr) {
+                const float* q_src = nullptr, const HitsMode* hm = nullptr, const long long* ex_src = nullptr,
+                int n_ex = 0) {
   // q_src (nullable): the queries in page-locked host memory, addressed through the mapping;
   // k_prep_rows reads them there once and leaves the fp32 copy the other kernels use in q_dev
+  // ex_src (nullable): [nq][n_ex] labels to leave out of each query's result (device memory or
+  // mapped host memory); k_prep_rows stages them as local row ids in a->ex_rows
   keds_index* a = ix[0];
   const int metric = (flags & KEDS_SEARCH_FORCE_IP) ? METRIC_IP : a->metric;
   CKS(set_kernel_attrs(a));
@@ -573,6 +587,20 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
   const unsigned int band_hint = a->h_feedback ? *static_cast<volatile unsigned int*>(a->h_feedback) : 0u;
   Plan pl = make_plan(a, n_db, nq, k, n_min, n_max, flags, band_hint);
   if (dump && pl.exact_only) return fail(KEDS_ERR_ARG, "debug_scores needs at least one 256-row tile");
+  ExcludeStage exs;
+  memset(&exs, 0, sizeof exs);
+  if (ex_src) {
+    CKS(a->ex_rows.ensure(static_cast<size_t>(n_db) * nq * n_ex * 4));
+    exs.labels = ex_src;
+    exs.nq = nq;
+    exs.n_ex = n_ex;
+    exs.n_db = n_db;
+    exs.rows = a->ex_rows.as<int>();
+    for (int i = 0; i < n_db; ++i) {
+      exs.id_offset[i] = ix[i]->id_offset;
+      exs.n_rows[i] = ix[i]->n;
+    }
+  }
   a->stats.exact_only = pl.exact_only;
   a->stats.slices = pl.S;
   a->stats.items = pl.n_items;
@@ -584,6 +612,13 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     for (int i = 0; i < n_db; ++i) {
       k_flag_all<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, st>>>(
           a->flagged[i].as<int>(), reinterpret_cast<int*>(a->ctrl_cur) + i, static_cast<int>(nq));
+      a->stats.launches++;
+    }
+    if (ex_src) {
+      // the staging half of k_prep_rows alone (no query rows to prepare on this route)
+      const unsigned blocks = static_cast<unsigned>(std::min<long long>((nq + 255) / 256, 1024));
+      k_prep_rows<<<blocks, 256, 0, st>>>(nullptr, 0, a->d, a->d_pad, a->fmt, nullptr, nullptr, nullptr, nullptr,
+                                          nullptr, 0, nullptr, 0, nullptr, nullptr, exs);
       a->stats.launches++;
     }
   } else {
@@ -603,7 +638,7 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
                    static_cast<long long>(nq), a->d, a->d_pad, a->fmt, a->q_bf16.as<uint16_t>(),
                    a->qstat.as<float4>(), static_cast<float*>(nullptr), static_cast<unsigned int*>(nullptr),
                    a->ctrl_cur, CTRL_STRIDE, a->theta0.as<float>(), static_cast<int>(n_db * theta_ld), tchain,
-                   q_src ? const_cast<float*>(q_dev) : static_cast<float*>(nullptr)));
+                   q_src ? const_cast<float*>(q_dev) : static_cast<float*>(nullptr), exs));
       a->stats.launches++;
     }
     // candidate lines are indexed by (db, slice, query tile) whatever the work-item grouping
@@ -636,13 +671,21 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     sp.dump = dump;
     sp.ld_dump = ld_dump;
     sp.timing = tchain ? tchain + 2 : nullptr;
+    if (ex_src) {
+      sp.ex_rows = exs.rows;
+      sp.n_ex = n_ex;
+      sp.ex_ld = static_cast<long long>(nq) * n_ex;
+    }
     CKS(prof_mark(a, st, 1));
+    // (with exclusion: the instantiation that tests each tile against the query's excluded rows)
     if (pl.pair)
-      CKS(launch_kc(a->use_pdl, 2, k_score_topk<true>, dim3(pl.grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES,
-                    st, a->tm_q, ix[0]->tm_xh, n_db > 1 ? ix[1]->tm_xh : ix[0]->tm_xh, sp));
+      CKS(launch_kc(a->use_pdl, 2, ex_src ? k_score_topk<true, false, true> : k_score_topk<true>, dim3(pl.grid),
+                    dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, ix[0]->tm_xh,
+                    n_db > 1 ? ix[1]->tm_xh : ix[0]->tm_xh, sp));
     else
-      CKS(launch_k(a->use_pdl, k_score_topk<false>, dim3(pl.grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st,
-                   a->tm_q, ix[0]->tm_x, n_db > 1 ? ix[1]->tm_x : ix[0]->tm_x, sp));
+      CKS(launch_k(a->use_pdl, ex_src ? k_score_topk<false, false, true> : k_score_topk<false>, dim3(pl.grid),
+                   dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, ix[0]->tm_x,
+                   n_db > 1 ? ix[1]->tm_x : ix[0]->tm_x, sp));
     CKS(prof_mark(a, st, 2));
     a->stats.launches++;
     CK(cudaGetLastError());
@@ -755,7 +798,8 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     }
   }
   if (!(flags & KEDS_SEARCH_NO_FALLBACK) || pl.exact_only) {
-    CKS(launch_exact(a, ix, n_db, q_dev, nq, k, D, I, metric, cons, tchain ? tchain + 6 : nullptr, st, peer));
+    CKS(launch_exact(a, ix, n_db, q_dev, nq, k, D, I, metric, cons, tchain ? tchain + 6 : nullptr, st, peer,
+                     ex_src ? &exs : nullptr));
     CKS(prof_mark(a, st, 4));
   }
   if (hm) {
@@ -827,9 +871,13 @@ int finish_sync(keds_index* a, cudaStream_t st) {
 
 int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, float* D[2],
                 int64_t* I[2], uint32_t flags, void* stream, const ConsumeParams* cons = nullptr,
-                const PeerOut* peer = nullptr, bool q_mapped = false) {
+                const PeerOut* peer = nullptr, bool q_mapped = false, const int64_t* exclude = nullptr,
+                int n_ex = 0) {
   keds_index* a = ix[0];
   if (!a || !q || nq < 0 || k <= 0) return fail(KEDS_ERR_ARG, "search: null handle/query or bad nq/k");
+  if (n_ex != 0 && (!exclude || n_ex < 1 || n_ex > EXCLUDE_MAX))
+    return fail(KEDS_ERR_ARG, "search: exclude must be a non-null [nq][n_exclude] array, 1 <= n_exclude <= %d",
+                EXCLUDE_MAX);
   if (k > K_MAX) return fail(KEDS_ERR_ARG, "search: k=%d exceeds the maximum %d", k, K_MAX);
   for (int i = 0; i < n_db; ++i) {
     if (!ix[i] || !D[i] || !I[i]) return fail(KEDS_ERR_ARG, "search: null index or output pointer");
@@ -861,6 +909,24 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
     CKS(a->q_f32.ensure(static_cast<size_t>(nq) * a->d * 4));
   }
   const bool q_dev = q_map != nullptr || is_device_ptr(q);
+  // the exclusion labels: device memory, or (retrieve2_hostio) page-locked host memory that
+  // k_prep_rows reads through the mapping
+  const long long* ex_dev = nullptr;
+  if (n_ex != 0 && nq > 0) {
+    if (device_of(exclude) == a->device) {
+      ex_dev = reinterpret_cast<const long long*>(exclude);
+    } else {
+      cudaPointerAttributes at;
+      if (!q_mapped || cudaPointerGetAttributes(&at, exclude) != cudaSuccess || at.type != cudaMemoryTypeHost ||
+          !at.devicePointer) {
+        cudaGetLastError();
+        return fail(KEDS_ERR_ARG, q_mapped ? "retrieve2_hostio: exclude is neither device memory of the index's GPU "
+                                             "nor page-locked host memory"
+                                           : "search: exclude must be device memory of the index's GPU");
+      }
+      ex_dev = static_cast<const long long*>(at.devicePointer);
+    }
+  }
   bool out_dev = true;
   for (int i = 0; i < n_db; ++i) {
     const bool dd = is_device_ptr(D[i]), di = is_device_ptr(I[i]);
@@ -927,7 +993,8 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
           // (stream order keeps the passes apart: every kernel of a chain waits for its predecessor)
           CKS(one[0]->ctrl.ensure(static_cast<size_t>(n_passes) * CTRL_STRIDE * 4));
           CKS(search_pass(one, 1, qd + q0 * a->d, nb, k, Dp, Ip, flags, st, nullptr, 0, nullptr, nullptr,
-                          static_cast<int>(q0 / Q_PASS_MAX)));
+                          static_cast<int>(q0 / Q_PASS_MAX), nullptr, nullptr, ex_dev ? ex_dev + q0 * n_ex : nullptr,
+                          n_ex));
         }
       } else {
         const long long tot = static_cast<long long>(nq) * k;
@@ -963,7 +1030,8 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
       // every pass has its own status block and the scratch is reused in stream order (each kernel
       // of a chain waits for its predecessor to complete), so the passes queue without a host round trip
       CKS(search_pass(ix, n_db, qd + q0 * a->d, nb, k, Dp, Ip, flags, st, nullptr, 0, cons ? &cp : nullptr,
-                      peer ? &pp : nullptr, static_cast<int>(q0 / Q_PASS_MAX), q_map ? q_map + q0 * a->d : nullptr));
+                      peer ? &pp : nullptr, static_cast<int>(q0 / Q_PASS_MAX), q_map ? q_map + q0 * a->d : nullptr,
+                      nullptr, ex_dev ? ex_dev + q0 * n_ex : nullptr, n_ex));
     }
   }
   if (!out_dev) {
@@ -1071,7 +1139,7 @@ int keds_index_create(int d, int metric, int device, keds_index_t** out) {
   DevBuf* tracked[] = {&ix->x_f32, &ix->x_bf16, &ix->bias, &ix->q_f32, &ix->q_bf16, &ix->qstat, &ix->cand,
                        &ix->cand_cnt, &ix->cand_theta, &ix->flagged[0], &ix->flagged[1], &ix->ctrl,
                        &ix->exact_scratch, &ix->D_stage[0], &ix->D_stage[1], &ix->I_stage[0], &ix->I_stage[1],
-                       &ix->rk, &ix->theta0};
+                       &ix->rk, &ix->theta0, &ix->ex_rows};
   for (DevBuf* b : tracked) b->gen = &ix->generation;
   *out = ix;
   return 0;
@@ -1083,7 +1151,8 @@ void keds_index_free(keds_index_t* ix) {
   DevBuf* bufs[] = {&ix->x_f32, &ix->x_bf16, &ix->bias, &ix->dbstat, &ix->q_f32, &ix->q_bf16,
                     &ix->qstat, &ix->cand, &ix->cand_cnt, &ix->cand_theta, &ix->flagged[0],
                     &ix->flagged[1], &ix->ctrl, &ix->exact_scratch, &ix->D_stage[0], &ix->D_stage[1],
-                    &ix->I_stage[0], &ix->I_stage[1], &ix->timing, &ix->probe, &ix->rk, &ix->theta0};
+                    &ix->I_stage[0], &ix->I_stage[1], &ix->timing, &ix->probe, &ix->rk, &ix->theta0,
+                    &ix->ex_rows};
   for (DevBuf* b : bufs) b->release();
   ix->h_q.release();
   ix->h_out.release();
@@ -1120,7 +1189,8 @@ static int prep_db_rows(keds_index* ix, int64_t r0, int64_t r1) {
   const unsigned blocks = static_cast<unsigned>(std::min<int64_t>((n * 32 + 255) / 256, ix->num_sms * 16));
   k_prep_rows<<<blocks, 256>>>(ix->x_f32.as<float>() + r0 * d, n, ix->d, ix->d_pad, ix->fmt,
                                ix->x_bf16.as<uint16_t>() + r0 * dp, nullptr, ix->bias.as<float>() + r0,
-                               ix->dbstat.as<unsigned int>(), nullptr, 0, nullptr, 0, nullptr, nullptr);
+                               ix->dbstat.as<unsigned int>(), nullptr, 0, nullptr, 0, nullptr, nullptr,
+                               ExcludeStage{});
   CK(cudaGetLastError());
   return 0;
 }
@@ -1263,6 +1333,27 @@ int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t
   return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream);
 }
 
+int keds_index_search_exclude(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
+                              const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
+  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
+    return fail(KEDS_ERR_ARG, "search_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
+  keds_index* v[2] = {ix, nullptr};
+  float* Dv[2] = {D, nullptr};
+  int64_t* Iv[2] = {I, nullptr};
+  return search_impl(v, 1, q, nq, k, Dv, Iv, flags, stream, nullptr, nullptr, false, exclude, n_exclude);
+}
+
+int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
+                               int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude, int n_exclude,
+                               uint32_t flags, void* stream) {
+  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
+    return fail(KEDS_ERR_ARG, "search2_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
+  keds_index* v[2] = {a, b};
+  float* Dv[2] = {Da, Db};
+  int64_t* Iv[2] = {Ia, Ib};
+  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream, nullptr, nullptr, false, exclude, n_exclude);
+}
+
 }  // extern "C"
 
 namespace {
@@ -1271,7 +1362,8 @@ int retrieve2_impl(keds_index_t* img, keds_index_t* txt, const float* q, int64_t
                    const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
                    float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
                    float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags, void* stream,
-                   bool hostio, float* Dh_img, int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt) {
+                   bool hostio, float* Dh_img, int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt,
+                   const int64_t* exclude = nullptr, int n_exclude = 0) {
   if (!img || !txt || !q || !D_img || !I_img || !D_txt || !I_txt)
     return fail(KEDS_ERR_ARG, "retrieve2: null handle, query or result pointer");
   if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "retrieve2: pool_mode must be 0, 1 or 2");
@@ -1310,7 +1402,8 @@ int retrieve2_impl(keds_index_t* img, keds_index_t* txt, const float* q, int64_t
   // one warp per neighbour row; per-warp partial pools meet in shared memory ([warps][d/4] float4)
   static_assert(RERANK_THREADS == EXACT_THREADS, "the consumer scratch is sized for one block shape");
   cp.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
-  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream, cp.enabled ? &cp : nullptr, nullptr, hostio);
+  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream, cp.enabled ? &cp : nullptr, nullptr, hostio, exclude,
+                     n_exclude);
 }
 
 }  // namespace
@@ -1332,6 +1425,32 @@ int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, 
                           float* pool_img, float* pool_txt, uint32_t flags, void* stream) {
   return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
                         feat_txt, pool_img, pool_txt, flags, stream, true, Dh_img, Ih_img, Dh_txt, Ih_txt);
+}
+
+int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                           const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                           float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
+                           float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
+                           uint32_t flags, void* stream) {
+  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
+    return fail(KEDS_ERR_ARG, "retrieve2_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
+  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
+                        feat_txt, pool_img, pool_txt, flags, stream, false, nullptr, nullptr, nullptr, nullptr, exclude,
+                        n_exclude);
+}
+
+int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                                  const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                                  float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
+                                  int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
+                                  float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
+                                  uint32_t flags, void* stream) {
+  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
+    return fail(KEDS_ERR_ARG, "retrieve2_hostio_exclude: exclude must be non-null and 1 <= n_exclude <= %d",
+                EXCLUDE_MAX);
+  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
+                        feat_txt, pool_img, pool_txt, flags, stream, true, Dh_img, Ih_img, Dh_txt, Ih_txt, exclude,
+                        n_exclude);
 }
 
 int keds_index_sync(keds_index_t* ix, void* stream) {
@@ -1790,7 +1909,7 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
                    ix->d_pad, ix->fmt, ix->q_bf16.as<uint16_t>(), ix->qstat.as<float4>(), static_cast<float*>(nullptr),
                    static_cast<unsigned int*>(nullptr), ix->ctrl.as<unsigned int>(), CTRL_WORDS,
                    static_cast<float*>(nullptr), 0, static_cast<unsigned long long*>(nullptr),
-                   static_cast<float*>(nullptr)));
+                   static_cast<float*>(nullptr), ExcludeStage{}));
     }
     const unsigned wblocks = static_cast<unsigned>((nb * 32 + 255) / 256);
     CKS(launch_k(ix->use_pdl, k_rank_targets, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,

@@ -166,16 +166,56 @@ __device__ __forceinline__ unsigned int round_pair(int fmt, float a, float b, fl
   return *reinterpret_cast<const unsigned int*>(&h);
 }
 
+// Search with exclusion, staged by k_prep_rows: the caller's labels (as the search returns them,
+// id_offset included; device memory or page-locked host memory read through the mapping, once)
+// become local row ids per database in handle scratch, so that no later kernel reads the caller's
+// array. A label that is -1, outside the database or a repeat of an earlier slot becomes EX_NONE.
+struct ExcludeStage {
+  const long long* labels;  // [nq][n_ex]; nullptr: no exclusion
+  long long nq;
+  int n_ex;                 // 1 .. EXCLUDE_MAX
+  int n_db;
+  long long id_offset[2];
+  long long n_rows[2];
+  int* rows;                // [n_db][nq][n_ex]
+};
+
 __global__ void k_prep_rows(const float* __restrict__ x, long long n, int d, int d_pad, int fmt,
                             uint16_t* __restrict__ out, float4* __restrict__ stat,
                             float* __restrict__ bias, unsigned int* __restrict__ gmax,
                             unsigned int* __restrict__ zero_words, int n_zero,
                             float* __restrict__ neg_inf_words, int n_neg_inf,
-                            unsigned long long* timing, float* __restrict__ copy_f32) {
+                            unsigned long long* timing, float* __restrict__ copy_f32, const ExcludeStage ex) {
   const int lane = threadIdx.x & 31;
   griddep_wait();               // earlier kernels of the stream may still read what is rewritten here
   griddep_launch_dependents();  // the scoring kernel may start its prologue
   const unsigned long long t_start = ktimer_begin(timing);
+  if (ex.labels != nullptr) {
+    for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < ex.nq;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+      int r[2][EXCLUDE_MAX];  // every loop below is unrolled: the arrays stay in registers
+#pragma unroll
+      for (int e = 0; e < EXCLUDE_MAX; ++e) {
+        const long long lab = e < ex.n_ex ? ex.labels[i * ex.n_ex + e] : -1ll;
+#pragma unroll
+        for (int db = 0; db < 2; ++db) {
+          const long long loc = lab - ex.id_offset[db];
+          r[db][e] = (lab != -1ll && loc >= 0 && loc < ex.n_rows[db]) ? static_cast<int>(loc) : EX_NONE;
+#pragma unroll
+          for (int f = 0; f < e; ++f)
+            if (r[db][f] == r[db][e]) r[db][e] = EX_NONE;
+        }
+      }
+#pragma unroll
+      for (int db = 0; db < 2; ++db) {
+        if (db >= ex.n_db) break;
+        int* o = ex.rows + (static_cast<long long>(db) * ex.nq + i) * ex.n_ex;
+#pragma unroll
+        for (int e = 0; e < EXCLUDE_MAX; ++e)
+          if (e < ex.n_ex) o[e] = r[db][e];
+      }
+    }
+  }
   // per-call control words (flag counters, error word) are cleared here instead of by a separate
   // memset node in front of every search; the shared per-query thresholds start at -inf
   if (zero_words != nullptr && blockIdx.x == 0)

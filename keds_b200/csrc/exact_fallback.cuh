@@ -44,9 +44,24 @@ struct ExactParams {
   unsigned int* band_host;     // nullable: mapped host word that receives it (planner feedback, no copy node)
   PeerOut peer;                // row-sharded exchange (database 0 only); n == 0: off
   unsigned long long* timing;  // nullable in-kernel launch timer
+  // search with exclusion: staged local row ids (ScoreParams::ex_rows); nullptr: nothing excluded
+  const int* ex_rows;
+  int n_ex;
+  long long ex_ld;
 };
 
 constexpr unsigned int EXACT_ERR_BARRIER = 0xEB000000u;
+// Score an excluded row gets in the scratch: the NaN whose order key is 0, below every real score,
+// so the selection never takes it while keff (k capped at the rows left) rows remain; fmaxf drops
+// it from the chunk maxima.
+constexpr unsigned int EXACT_EXCLUDED_BITS = 0xFFFFFFFFu;
+
+__device__ __forceinline__ bool row_in(const int* ex, int n_ex, long long row) {
+  bool hit = false;
+#pragma unroll
+  for (int e = 0; e < EXCLUDE_MAX; ++e) hit = hit || (e < n_ex && ex[e] == row);
+  return hit;
+}
 constexpr int EXACT_LIST_CAP = 2048;  // rows at or above the pre-filter threshold held in shared memory
 
 // Work is handed out through counters, never by block index: the blocks that are resident drain
@@ -95,6 +110,7 @@ __device__ __forceinline__ void exact_scores(const ExactParams& p, const ExactSh
   const int wpb = blockDim.x >> 5;
   const int r0 = p.pass * p.f_cap;
   const unsigned int total = sh.units[0] + sh.units[1];
+  __shared__ int qex[EXACT_QG * EXCLUDE_MAX];  // the group's excluded rows (search with exclusion)
   int have_db = -1, have_g0 = -1;
   for (;;) {
     unsigned int u = exact_claim(p.work, slot);
@@ -110,6 +126,11 @@ __device__ __forceinline__ void exact_scores(const ExactParams& p, const ExactSh
         const int qi = i / dq, c = i % dq;
         const int q = e.flagged[r0 + g0 + qi];
         qs[i] = c < p.d ? p.q_f32[static_cast<long long>(q) * p.d + c] : 0.f;
+      }
+      if (p.ex_rows != nullptr && tid < G * p.n_ex) {
+        const int q = e.flagged[r0 + g0 + tid / p.n_ex];
+        qex[(tid / p.n_ex) * EXCLUDE_MAX + tid % p.n_ex] =
+            p.ex_rows[dbi * p.ex_ld + static_cast<long long>(q) * p.n_ex + tid % p.n_ex];
       }
       __syncthreads();
       have_db = dbi;
@@ -141,6 +162,8 @@ __device__ __forceinline__ void exact_scores(const ExactParams& p, const ExactSh
 #pragma unroll
         for (int i = 0; i < EXACT_QG; ++i) {
           if (i < G) {
+            if (p.ex_rows != nullptr && row_in(qex + i * EXCLUDE_MAX, p.n_ex, row))
+              keep[i] = __uint_as_float(EXACT_EXCLUDED_BITS);
             e.scratch[static_cast<long long>(g0 + i) * e.n_rows + row] = keep[i];
             best[i] = fmaxf(best[i], keep[i]);
           }
@@ -209,7 +232,13 @@ __device__ __forceinline__ void exact_select(const ExactParams& p, uint8_t* ex_s
     const int q = e.flagged[r0 + f];
     const float* sc = e.scratch + static_cast<long long>(f) * e.n_rows;
     const long long n = e.n_rows;
-    const int keff = static_cast<int>(min(static_cast<long long>(p.k), n));
+    // excluded rows (distinct and in range once staged) are not candidates: k is capped at the rest
+    int n_out = 0;
+    if (p.ex_rows != nullptr) {
+      const int* xr = p.ex_rows + dbi * p.ex_ld + static_cast<long long>(q) * p.n_ex;
+      for (int j = 0; j < p.n_ex; ++j) n_out += xr[j] != EX_NONE;
+    }
+    const int keff = static_cast<int>(min(static_cast<long long>(p.k), n - n_out));
     __syncthreads();
     for (int r = tid; r < p.k; r += blockDim.x) top_id[r] = 0xFFFFFFFFu;
     // Pre-filter: the k-th best row is at least as good as the k-th best chunk maximum t0 (each of
@@ -217,8 +246,8 @@ __device__ __forceinline__ void exact_select(const ExactParams& p, uint8_t* ex_s
     // answer, and only their rows at or above t0 are candidates. A handful of chunks instead of
     // five passes over the whole score row; the dense path below stays for k > chunks and for
     // candidate lists that do not fit (heavily duplicated data).
-    bool filled = false;
-    if (e.chunks >= keff && e.chunks <= p.ck_cap && 2 * keff <= EXACT_LIST_CAP) {
+    bool filled = keff == 0;  // every row excluded: padding only
+    if (!filled && e.chunks >= keff && e.chunks <= p.ck_cap && 2 * keff <= EXACT_LIST_CAP) {
       const float* cm = e.cmax + static_cast<long long>(f) * e.chunks;
       for (int c = tid; c < e.chunks; c += blockDim.x) {
         float v = __ldcg(cm + c);

@@ -43,6 +43,10 @@ constexpr int SCORE_THREADS = 192;       // single-CTA variant: producer, issuer
 constexpr int SCORE_PAIR_THREADS = 320;  // CTA-pair variant: 8 epilogue warps
 constexpr uint32_t Q_STAGE_BYTES = BM * BK * 2;
 constexpr uint32_t TMEM_COLS = 512;
+// Search with exclusion: at most EXCLUDE_MAX rows left out per query. k_prep_rows stages them as
+// local row ids per database, EX_NONE where a slot excludes nothing (unused, out of range, repeat).
+constexpr int EXCLUDE_MAX = 8;
+constexpr int EX_NONE = -1;
 
 template <bool kPair>
 struct ScoreCfg {
@@ -99,6 +103,11 @@ struct ScoreParams {
   const float* rk_hi;
   const int* rk_target;
   const int* rk_exclude;     // -1: none
+  // top-k search with exclusion (kRank = false): per database [nq][n_ex] local row ids that must
+  // never enter a candidate list (EX_NONE: unused slot); nullptr / n_ex = 0: nothing excluded
+  const int* ex_rows;
+  int n_ex;
+  long long ex_ld;           // ints per database
 };
 
 struct ItemCoord {
@@ -192,10 +201,13 @@ __device__ __noinline__ CandState compact_candidates(uint32_t slot0, int cnt, fl
 //                overflow mark and the query is recounted exactly). The target and the excluded row
 //                are skipped by id. Output: the same 128-byte lines (band rows), cand_cnt = band
 //                rows or -1 (overflow), cand_theta = the certain count (as int bits).
-template <bool kPair, bool kRank = false>
+// kExclude = true (top-k search only): rows listed per query in p.ex_rows never enter a list. A
+//                separate instantiation, so that the plain search keeps its code and registers.
+template <bool kPair, bool kRank = false, bool kExclude = false>
 __global__ void __launch_bounds__(ScoreCfg<kPair>::kThreads, 1)
 k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_x0,
              const __grid_constant__ CUtensorMap tm_x1, const ScoreParams p) {
+  static_assert(!(kRank && kExclude), "exclusion is a top-k search option");
   using Cfg = ScoreCfg<kPair>;
   constexpr int NSTAGE = Cfg::kStages;
   extern __shared__ uint8_t smem_raw[];
@@ -407,9 +419,36 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
           rk_e = p.rk_exclude != nullptr ? p.rk_exclude[q_glob] : -1;
         }
       }
+      // Exclusion: this query's excluded rows of this database, in registers (statically indexed:
+      // every loop over them is unrolled). An excluded row is not a row of this query's problem --
+      // it never enters a list, so no list's theta depends on it (DESIGN.md section 3).
+      [[maybe_unused]] int ex[EXCLUDE_MAX];
+      [[maybe_unused]] bool has_ex = false;
+      if constexpr (kExclude) {
+#pragma unroll
+        for (int e = 0; e < EXCLUDE_MAX; ++e) ex[e] = EX_NONE;
+        if (active && p.ex_rows != nullptr) {
+          const int* xr = p.ex_rows + c.db * p.ex_ld + static_cast<long long>(q_glob) * p.n_ex;
+#pragma unroll
+          for (int e = 0; e < EXCLUDE_MAX; ++e) {
+            if (e < p.n_ex) ex[e] = __ldg(xr + e);
+            has_ex = has_ex || ex[e] != EX_NONE;
+          }
+        }
+      }
       const float* bias = p.bias[c.db];
       const int n_rows = p.n_rows[c.db];
       for (int tile = c.t0; tile < c.t1; ++tile) {
+        // one test per tile and query; the per-column path below runs only for a tile that holds
+        // an excluded row
+        [[maybe_unused]] bool tile_ex = false;
+        if constexpr (kExclude) {
+          if (has_ex) {
+#pragma unroll
+            for (int e = 0; e < EXCLUDE_MAX; ++e)
+              tile_ex = tile_ex || static_cast<unsigned>(ex[e] - tile * BN) < static_cast<unsigned>(BN);
+          }
+        }
         if (bias != nullptr) {
           if constexpr (SUB == 2) {
             sbias[acc * BN + et] = bias[static_cast<long long>(tile) * BN + et];
@@ -452,6 +491,20 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
 #pragma unroll
             for (int j = 0; j < CHUNK; ++j)
               if (static_cast<int>(idx0) + j < n_rows) drow[idx0 + j] = __uint_as_float(v[j]);
+          }
+          if constexpr (kExclude) {
+            if (tile_ex) {
+              // rare: the chunk's excluded columns as a bit mask, then -inf there (never > theta)
+              uint32_t xm = 0;
+#pragma unroll
+              for (int e = 0; e < EXCLUDE_MAX; ++e) {
+                const unsigned o = static_cast<unsigned>(ex[e] - static_cast<int>(idx0));
+                xm |= o < static_cast<unsigned>(CHUNK) ? (1u << o) : 0u;
+              }
+#pragma unroll
+              for (int j = 0; j < CHUNK; ++j)
+                if ((xm >> j) & 1u) v[j] = 0xff800000u;
+            }
           }
           if constexpr (kRank) {
             // count the certain winners; rows inside the band are rare and take a plain branch

@@ -49,6 +49,50 @@ def _as_f32_matrix(x, d: int, what: str) -> np.ndarray:
     return np.ascontiguousarray(a)
 
 
+EXCLUDE_MAX = 8  # rows one query may leave out (include/keds_knn.h, search with exclusion)
+
+
+def check_exclude(exclude, nq: int):
+    """Validate a per-query exclusion array: labels as `search` returns them, -1 = unused slot.
+    Accepts a numpy array or a torch tensor of int64, shaped [nq] or [nq, E] with 1 <= E <= 8.
+    Returns it as [nq, E] (a view, nothing is copied or moved); raises TypeError / ValueError."""
+    if _is_tensor(exclude):
+        if exclude.dtype != torch.int64:
+            raise TypeError(f"exclude: expected int64 labels, got {exclude.dtype}")
+    elif isinstance(exclude, np.ndarray):
+        if exclude.dtype != np.int64:
+            raise TypeError(f"exclude: expected int64 labels, got {exclude.dtype}")
+    else:
+        raise TypeError(f"exclude: expected a numpy array or a torch tensor, got {type(exclude).__name__}")
+    shape = tuple(exclude.shape)
+    if len(shape) == 1:
+        exclude = exclude.reshape(-1, 1)
+    elif len(shape) != 2:
+        raise ValueError(f"exclude: expected shape [nq] or [nq, E], got {shape}")
+    if exclude.shape[0] != nq:
+        raise ValueError(f"exclude: {exclude.shape[0]} rows for {nq} queries")
+    if not 1 <= exclude.shape[1] <= EXCLUDE_MAX:
+        raise ValueError(f"exclude: E = {exclude.shape[1]} labels per query, expected 1..{EXCLUDE_MAX}")
+    return exclude
+
+
+def _exclude_arg(exclude, nq: int, device: int, pinned_ok: bool = False):
+    """check_exclude, then a contiguous int64 tensor the native call can read: on `device`, or a
+    pinned host tensor as it is when `pinned_ok` (the hostio path reads it through the mapping)."""
+    ex = check_exclude(exclude, nq)
+    if torch is None:
+        raise RuntimeError("search with exclusion needs torch for the device copy of `exclude`")
+    if isinstance(ex, np.ndarray):
+        ex = torch.from_numpy(np.ascontiguousarray(ex))
+    if ex.is_cuda:
+        if ex.device.index != device:
+            raise ValueError(f"exclude: on cuda:{ex.device.index}, index on cuda:{device}")
+        return ex.contiguous()
+    if pinned_ok and ex.is_pinned() and ex.is_contiguous():
+        return ex
+    return ex.to(torch.device("cuda", device), non_blocking=False).contiguous()
+
+
 def _stream_ptr(device: int) -> int:
     if torch is not None and torch.cuda.is_available():
         return int(torch.cuda.current_stream(device).cuda_stream)
@@ -197,12 +241,22 @@ class GpuIndexFlat:
         return out
 
     # -- search
-    def search(self, x, k: int, flags: int = 0, out=None):
+    def search(self, x, k: int, flags: int = 0, out=None, exclude=None):
         """numpy in -> numpy (D, I) out, synchronous. CUDA tensor in -> CUDA tensors out,
-        stream-ordered; `out=(D, I)` may name preallocated contiguous CUDA tensors to fill."""
+        stream-ordered; `out=(D, I)` may name preallocated contiguous CUDA tensors to fill.
+        exclude: int64 [nq] or [nq, E] (E <= 8) labels each query must not get back (e.g. its own
+        row), -1 = unused; the result is the exact search over the remaining rows."""
         k = int(k)
         if k <= 0:
             raise ValueError("k must be positive")
+
+        def call(qp, nq, Dp, Ip):
+            if exclude is None:
+                return self._lib.keds_index_search_ex(self._h, qp, nq, k, Dp, Ip, flags, _stream_ptr(self.device))
+            ex = _exclude_arg(exclude, nq, self.device)
+            return self._lib.keds_index_search_exclude(self._h, qp, nq, k, Dp, Ip, ex.data_ptr(), ex.shape[1], flags,
+                                                       _stream_ptr(self.device))
+
         if _is_tensor(x) and x.is_cuda:
             q = self._check_q_tensor(x)
             if out is not None:
@@ -213,22 +267,12 @@ class GpuIndexFlat:
             else:
                 D = torch.empty((q.shape[0], k), dtype=torch.float32, device=q.device)
                 I = torch.empty((q.shape[0], k), dtype=torch.int64, device=q.device)
-            _capi.check(
-                self._lib.keds_index_search_ex(
-                    self._h, q.data_ptr(), q.shape[0], k, D.data_ptr(), I.data_ptr(), flags,
-                    _stream_ptr(self.device),
-                )
-            )
+            _capi.check(call(q.data_ptr(), q.shape[0], D.data_ptr(), I.data_ptr()))
             return D, I
         a = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, self.d, "search")
         D = np.empty((a.shape[0], k), dtype=np.float32)
         I = np.empty((a.shape[0], k), dtype=np.int64)
-        _capi.check(
-            self._lib.keds_index_search_ex(
-                self._h, a.ctypes.data, a.shape[0], k, D.ctypes.data, I.ctypes.data, flags,
-                _stream_ptr(self.device),
-            )
-        )
+        _capi.check(call(a.ctypes.data, a.shape[0], D.ctypes.data, I.ctypes.data))
         return D, I
 
     def _check_q_tensor(self, x):
@@ -302,32 +346,34 @@ class GpuIndexFlat:
         return out
 
 
-def search2(a: GpuIndexFlat, b: GpuIndexFlat, x, k: int, flags: int = 0):
-    """Both databases against one query batch in one pass (src/trainer.py:213 + :221)."""
+def search2(a: GpuIndexFlat, b: GpuIndexFlat, x, k: int, flags: int = 0, exclude=None):
+    """Both databases against one query batch in one pass (src/trainer.py:213 + :221).
+    exclude: as GpuIndexFlat.search; one array for both databases (aligned row for row)."""
     lib = _capi.load()
     k = int(k)
+
+    def call(qp, nq, Da, Ia, Db, Ib):
+        if exclude is None:
+            return lib.keds_index_search2(a._h, b._h, qp, nq, k, Da, Ia, Db, Ib, flags, _stream_ptr(a.device))
+        ex = _exclude_arg(exclude, nq, a.device)
+        return lib.keds_index_search2_exclude(a._h, b._h, qp, nq, k, Da, Ia, Db, Ib, ex.data_ptr(), ex.shape[1],
+                                              flags, _stream_ptr(a.device))
+
     if _is_tensor(x) and x.is_cuda:
         q = a._check_q_tensor(x)
         outs = []
         for _ in range(2):
             outs.append(torch.empty((q.shape[0], k), dtype=torch.float32, device=q.device))
             outs.append(torch.empty((q.shape[0], k), dtype=torch.int64, device=q.device))
-        _capi.check(
-            lib.keds_index_search2(a._h, b._h, q.data_ptr(), q.shape[0], k, outs[0].data_ptr(),
-                                   outs[1].data_ptr(), outs[2].data_ptr(), outs[3].data_ptr(),
-                                   flags, _stream_ptr(a.device))
-        )
+        _capi.check(call(q.data_ptr(), q.shape[0], outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(),
+                         outs[3].data_ptr()))
         return (outs[0], outs[1]), (outs[2], outs[3])
     arr = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, a.d, "search2")
     Da = np.empty((arr.shape[0], k), np.float32)
     Ia = np.empty((arr.shape[0], k), np.int64)
     Db = np.empty_like(Da)
     Ib = np.empty_like(Ia)
-    _capi.check(
-        lib.keds_index_search2(a._h, b._h, arr.ctypes.data, arr.shape[0], k, Da.ctypes.data,
-                               Ia.ctypes.data, Db.ctypes.data, Ib.ctypes.data, flags,
-                               _stream_ptr(a.device))
-    )
+    _capi.check(call(arr.ctypes.data, arr.shape[0], Da.ctypes.data, Ia.ctypes.data, Db.ctypes.data, Ib.ctypes.data))
     return (Da, Ia), (Db, Ib)
 
 

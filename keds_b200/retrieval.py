@@ -27,7 +27,7 @@ import numpy as np
 import torch
 
 from . import _capi
-from .index import GpuIndexFlat, METRIC_INNER_PRODUCT, METRIC_L2, search2, _stream_ptr
+from .index import GpuIndexFlat, METRIC_INNER_PRODUCT, METRIC_L2, check_exclude, search2, _exclude_arg, _stream_ptr
 
 
 def gather_rows(index: GpuIndexFlat, I: torch.Tensor, perm: Optional[torch.Tensor] = None) -> torch.Tensor:
@@ -133,18 +133,36 @@ class KnowledgeBase:
     def __len__(self) -> int:
         return 5
 
+    def rows_of(self, names: Sequence[str]) -> torch.Tensor:
+        """int64 [len(names)] rows of the pairs with these basenames, -1 for a name the base does not
+        hold: how a training loop turns its batch's file names into `exclude` (leave each query's
+        own pair out of its neighbours). The name -> row table is built once per basenames list."""
+        table = getattr(self, "_row_table", None)
+        if table is None or table[0] is not self.basenames or table[1] != len(self.basenames):
+            pos = {}
+            for i, n in enumerate(self.basenames):
+                pos.setdefault(n, i)  # a repeated name maps to its first row
+            table = (self.basenames, len(self.basenames), pos)
+            self._row_table = table
+        pos = table[2]
+        return torch.tensor([pos.get(n, -1) for n in names], dtype=torch.int64)
+
 
 def _native(ix) -> bool:
     return isinstance(ix, GpuIndexFlat)
 
 
-def get_retrieved_features(feature, database, args=None, topk: int = 16, use_faiss: bool = True):
+def get_retrieved_features(feature, database, args=None, topk: int = 16, use_faiss: bool = True, exclude=None):
     """Same contract as src/trainer.py:198-259: returns (topk_image_features, topk_text_features),
     each [B, topk, d] on feature.device; image neighbours permuted along k by one
     torch.randperm(topk) shared by the batch (:218-219), text neighbours in rank order.
 
     use_faiss=False in the reference is a dense torch matmul over the whole database; both
-    settings run the native search here (same answer: exact top-k by inner product / L2)."""
+    settings run the native search here (same answer: exact top-k by inner product / L2).
+
+    exclude (not in the reference; default None = its behaviour): int64 [B] or [B, E] rows each
+    query must not retrieve, -1 = none -- e.g. database.rows_of(batch_names) to train without
+    self-retrieval. One array for both bases (aligned row for row)."""
     image_base, text_base, basenames, image_index, text_index = (database[i] for i in range(5))
     if not (_native(image_index) and _native(text_index)):
         raise TypeError("database[3] and database[4] must be keds_b200 GPU indices (no CPU path)")
@@ -154,7 +172,8 @@ def get_retrieved_features(feature, database, args=None, topk: int = 16, use_fai
     q = feature.detach().to(device=dev, dtype=torch.float32).contiguous()
     flags = 0 if use_faiss else _capi.SEARCH_FORCE_IP  # the torch branch ranks by raw inner product
     perm = torch.randperm(topk) if use_faiss else None  # CPU generator, like the reference (:218)
-    out = retrieve2(image_index, text_index, q, topk, perm_img=perm, want_feats=True, pool_mode=0, flags=flags)
+    out = retrieve2(image_index, text_index, q, topk, perm_img=perm, want_feats=True, pool_mode=0, flags=flags,
+                    exclude=exclude)
     return out["feat_img"].to(feature.device), out["feat_txt"].to(feature.device)
 
 
@@ -164,7 +183,7 @@ POOL_NONE, POOL_MEAN, POOL_SOFTMAX = 0, 1, 2
 def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tensor, topk: int = 16,
               perm_img: Optional[torch.Tensor] = None, perm_txt: Optional[torch.Tensor] = None,
               want_feats: bool = True, pool_mode: int = POOL_NONE, tau: float = 100.0, flags: int = 0,
-              out: Optional[dict] = None, host_out: Optional[dict] = None) -> dict:
+              out: Optional[dict] = None, host_out: Optional[dict] = None, exclude=None) -> dict:
     """One native call for the whole operator: fused two-database search, then for each stream the
     gathered neighbours [B, k, d] (image stream permuted by perm_img) and/or the pooled stream
     [B, d].  `out` may carry preallocated tensors from a previous call (keys as returned) so a
@@ -173,7 +192,11 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
     Host I/O without copies (keds_retrieve2_hostio): `q` may be a pinned CPU tensor -- the first
     kernel reads it through the device mapping -- and `host_out` may hold pinned CPU tensors
     D_img / I_img / D_txt / I_txt ([B, k]) that the kernels fill next to the device results; they
-    are complete once the stream has been synchronised."""
+    are complete once the stream has been synchronised.
+
+    exclude: int64 [B] or [B, E] (E <= 8) labels each query must not retrieve from either base, -1 =
+    none; the neighbours, gathers and pools are those of the exact search over the remaining rows.
+    On the host-I/O path it may be a pinned CPU tensor, read through the mapping like `q`."""
     lib = _capi.load()
     hostio = host_out is not None or not q.is_cuda
     if q.is_cuda:
@@ -211,6 +234,7 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
     pi_ptr, _keep1 = perm_ptr(perm_img)
     pt_ptr, _keep2 = perm_ptr(perm_txt)
     ptr = lambda t: 0 if t is None else t.data_ptr()
+    ex = None if exclude is None else _exclude_arg(exclude, B, image_index.device, pinned_ok=hostio)
     if hostio:
         ho = host_out or {}
         hp = []
@@ -219,11 +243,27 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
             if t is not None and not (t.is_pinned() and t.dtype == dt and t.is_contiguous() and t.numel() == B * k):
                 raise TypeError(f"retrieve2: host_out[{name!r}] must be a pinned contiguous {dt} tensor of {B * k} elements")
             hp.append(0 if t is None else t.data_ptr())
+        if ex is not None:
+            _capi.check(
+                lib.keds_retrieve2_hostio_exclude(
+                    image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode), float(tau),
+                    Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), hp[0], hp[1], hp[2], hp[3], ptr(fi),
+                    ptr(ft), ptr(pi), ptr(pt), ex.data_ptr(), ex.shape[1], int(flags), _stream_ptr(image_index.device))
+            )
+            return o
         _capi.check(
             lib.keds_retrieve2_hostio(image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode),
                                       float(tau), Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(),
                                       hp[0], hp[1], hp[2], hp[3], ptr(fi), ptr(ft), ptr(pi), ptr(pt), int(flags),
                                       _stream_ptr(image_index.device))
+        )
+        return o
+    if ex is not None:
+        _capi.check(
+            lib.keds_retrieve2_exclude(image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr,
+                                       int(pool_mode), float(tau), Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(),
+                                       It.data_ptr(), ptr(fi), ptr(ft), ptr(pi), ptr(pt), ex.data_ptr(), ex.shape[1],
+                                       int(flags), _stream_ptr(image_index.device))
         )
         return o
     _capi.check(
@@ -243,11 +283,17 @@ class RetrievalStep:
     few microseconds. Write the batch into `q_host` (pinned, [batch, d]) or pass it to `run()`;
     after `run()` returns, `D_img/I_img/D_txt/I_txt` (pinned host) hold what `index.search` gives
     the host in the reference, and `out` holds the device tensors (gathered / pooled streams).
+
+    n_exclude > 0: every step also leaves rows out per query (search with exclusion). The step owns
+    a pinned `exclude_host` [batch, n_exclude] int64 (-1 = none) that `run(q, exclude=...)` fills or
+    the caller writes directly; the graph reads it on every replay, so changing it needs no
+    re-capture.
     """
 
     def __init__(self, image_index: GpuIndexFlat, text_index: GpuIndexFlat, batch: int, topk: int = 16,
                  perm_img: Optional[torch.Tensor] = None, want_feats: bool = True,
-                 pool_mode: int = POOL_NONE, tau: float = 100.0, copy_nodes: Optional[bool] = None) -> None:
+                 pool_mode: int = POOL_NONE, tau: float = 100.0, copy_nodes: Optional[bool] = None,
+                 n_exclude: int = 0) -> None:
         self.ia, self.ib = image_index, text_index
         # copy_nodes=False: no copies in the graph -- the first kernel reads the pinned queries through
         # the mapping and the ranking blocks store (D, I) into the pinned result block next to the
@@ -266,6 +312,13 @@ class RetrievalStep:
         d, k = image_index.d, int(topk)
         self.q_host = torch.empty((batch, d), dtype=torch.float32).pin_memory()
         self.q_dev = torch.empty((batch, d), dtype=torch.float32, device=dev)
+        self.n_exclude = int(n_exclude)
+        if not 0 <= self.n_exclude <= 8:
+            raise ValueError(f"n_exclude: expected 0..8, got {n_exclude}")
+        self.exclude_host = self.exclude_dev = None
+        if self.n_exclude:
+            self.exclude_host = torch.full((batch, self.n_exclude), -1, dtype=torch.int64).pin_memory()
+            self.exclude_dev = torch.full((batch, self.n_exclude), -1, dtype=torch.int64, device=dev)
         # (I_img | I_txt | D_img | D_txt) live in one device block mirrored by one pinned host block,
         # so the results leave the GPU with a single copy
         nI, nD = batch * k * 8, batch * k * 4
@@ -344,14 +397,26 @@ class RetrievalStep:
     def _body(self) -> None:
         if self.copy_nodes:
             self.q_dev.copy_(self.q_host, non_blocking=True)
-            retrieve2(self.ia, self.ib, self.q_dev, out=self.out, **self._args)
+            if self.n_exclude:
+                self.exclude_dev.copy_(self.exclude_host, non_blocking=True)
+            retrieve2(self.ia, self.ib, self.q_dev, out=self.out, exclude=self.exclude_dev, **self._args)
             self._res_host.copy_(self._res_dev, non_blocking=True)
         else:
-            retrieve2(self.ia, self.ib, self.q_host, out=self.out, host_out=self._host_out, **self._args)
+            retrieve2(self.ia, self.ib, self.q_host, out=self.out, host_out=self._host_out, exclude=self.exclude_host,
+                      **self._args)
 
-    def run(self, q: Optional[torch.Tensor] = None, sync: bool = True) -> dict:
+    def run(self, q: Optional[torch.Tensor] = None, sync: bool = True, exclude=None) -> dict:
+        """exclude (steps built with n_exclude > 0): [batch] or [batch, n_exclude] int64 labels to
+        leave out of each query's neighbours, copied into `exclude_host`; None keeps its contents."""
         if q is not None:
             self.q_host.copy_(q)
+        if exclude is not None:
+            if not self.n_exclude:
+                raise ValueError("run: this step was built without exclusion (n_exclude=0)")
+            ex = check_exclude(exclude, self.q_host.shape[0])
+            if ex.shape[1] != self.n_exclude:
+                raise ValueError(f"run: exclude has {ex.shape[1]} labels per query, the step {self.n_exclude}")
+            self.exclude_host.copy_(torch.as_tensor(ex))
         if (self.ia.generation, self.ib.generation) != self._gen:
             self._capture()  # reads q_host only; the batch just written stays in place
         self.graph.replay()
@@ -376,12 +441,13 @@ class RetrievalPipeline:
         self._events = [None, None]
         self._n = 0
 
-    def submit(self, q: Optional[torch.Tensor] = None) -> int:
+    def submit(self, q: Optional[torch.Tensor] = None, exclude=None) -> int:
+        """exclude: as RetrievalStep.run (pipelines built with n_exclude > 0)."""
         slot = self._n & 1
         if self._events[slot] is not None:      # the slot's previous batch must be done with its buffers
             self._events[slot].synchronize()
         st = self.steps[slot]
-        st.run(q, sync=False)
+        st.run(q, sync=False, exclude=exclude)
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream(st.q_dev.device))
         self._events[slot] = ev

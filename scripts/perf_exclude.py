@@ -1,0 +1,183 @@
+"""Cost of search with exclusion, and of the change on the plain entry points.
+
+Loads two builds of libkeds_knn.so into one process (ctypes, RTLD_LOCAL: their symbols do not mix)
+and times, round after round in rotating order on the same device-resident inputs:
+
+  base     the plain entry point of a reference build (--base-lib, e.g. the parent commit's)
+  plain    the plain entry point of this tree's build
+  exclude  this tree's *_exclude entry point, E = 1: every query is a row of the base and leaves
+           itself out (training without self-retrieval)
+
+on three shapes: config 2 (retrieve2, 128 queries x 2 databases x 0.5M rows, k = 16, gathered
+neighbours), config 1 (search, 4096 x 50k, k = 16) and 4096 x 0.5M. Times are per call from CUDA
+events around a back-to-back loop; the spread is the range over rounds, and the differences are
+the median (and quartiles) of the per-round ratios of variants that ran back to back. Also checks that base and
+plain return the same bits. Writes one JSON document (card name and power limit included).
+
+    python scripts/perf_exclude.py --base-lib /path/to/parent/libkeds_knn.so --out perf.json
+"""
+from __future__ import annotations
+
+import argparse
+import ctypes as C
+import json
+import os
+import statistics
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+import torch  # noqa: E402
+
+from keds_b200 import _capi  # noqa: E402
+
+D = 768
+K = 16
+
+
+def load(path: str) -> C.CDLL:
+    lib = C.CDLL(path)
+    for name, (res, args) in _capi.SIGNATURES.items():
+        if hasattr(lib, name):
+            fn = getattr(lib, name)
+            fn.restype, fn.argtypes = res, args
+    return lib
+
+
+def check(lib, rc):
+    if rc != 0:
+        raise RuntimeError(lib.keds_last_error().decode())
+
+
+def make_index(lib, rows: torch.Tensor):
+    h = C.c_void_p()
+    check(lib, lib.keds_index_create(D, _capi.METRIC_IP, 0, C.byref(h)))
+    check(lib, lib.keds_index_add_ex(h, rows.data_ptr(), rows.shape[0], 0))
+    return h
+
+
+def card() -> dict:
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                             capture_output=True, text=True, timeout=30).stdout.strip().splitlines()[0]
+        name, power, clock = [s.strip() for s in out.split(",")]
+        return {"name": name, "power_limit": power, "max_sm_clock": clock}
+    except Exception as e:  # pragma: no cover
+        return {"name": torch.cuda.get_device_name(0), "error": str(e)}
+
+
+def main() -> None:
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--base-lib", required=True, help="reference build of libkeds_knn.so (plain entry points)")
+    ap.add_argument("--lib", default=_capi.LIB_PATH, help="this tree's build")
+    ap.add_argument("--rounds", type=int, default=30)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    assert torch.cuda.is_available(), "needs a CUDA device"
+    libs = {"base": load(os.path.abspath(args.base_lib)), "new": load(os.path.abspath(args.lib))}
+    assert hasattr(libs["new"], "keds_index_search_exclude"), "--lib is not a build with exclusion"
+    dev = torch.device("cuda", 0)
+    st = torch.cuda.current_stream(dev).cuda_stream
+    g = torch.Generator(device=dev).manual_seed(0)
+
+    def unit(n):
+        x = torch.randn(n, D, generator=g, device=dev)
+        return x / x.norm(dim=1, keepdim=True)
+
+    big_a, big_b, small = unit(500_000), unit(500_000), unit(50_000)
+    idx = {name: {"a": make_index(lib, big_a), "b": make_index(lib, big_b), "s": make_index(lib, small)}
+           for name, lib in libs.items()}
+    torch.cuda.synchronize()
+
+    perm = torch.randperm(K, generator=torch.Generator().manual_seed(1)).to(dev, torch.int32)
+    shapes = {}
+    for cfg, nq, n in (("cfg2_retrieve2_128x2x500k", 128, 500_000), ("cfg1_search_4096x50k", 4096, 50_000),
+                       ("search_4096x500k", 4096, 500_000)):
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(nq + n))[:nq]
+        q = (big_a if n == 500_000 else small)[rows.to(dev)].contiguous()
+        ex = rows.to(dev, torch.int64).reshape(nq, 1).contiguous()
+        shapes[cfg] = (nq, q, ex)
+
+    def outputs(nq, feats):
+        o = [torch.empty((nq, K), dtype=torch.float32, device=dev), torch.empty((nq, K), dtype=torch.int64, device=dev),
+             torch.empty((nq, K), dtype=torch.float32, device=dev), torch.empty((nq, K), dtype=torch.int64, device=dev)]
+        if feats:
+            o += [torch.empty((nq, K, D), dtype=torch.float32, device=dev) for _ in range(2)]
+        return o
+
+    def call(cfg, variant):
+        nq, q, ex = shapes[cfg]
+        lib = libs["base" if variant == "base" else "new"]
+        ix = idx["base" if variant == "base" else "new"]
+        o = outs[(cfg, variant)]
+        p = [t.data_ptr() for t in o]
+        if cfg.startswith("cfg2"):
+            common = (ix["a"], ix["b"], q.data_ptr(), nq, K, perm.data_ptr(), None, 0, 100.0, p[0], p[1], p[2], p[3],
+                      p[4], p[5], None, None)
+            if variant == "exclude":
+                return lambda: check(lib, lib.keds_retrieve2_exclude(*common, ex.data_ptr(), 1, 0, st))
+            return lambda: check(lib, lib.keds_retrieve2(*common, 0, st))
+        h = ix["s"] if cfg.startswith("cfg1") else ix["a"]
+        if variant == "exclude":
+            return lambda: check(lib, lib.keds_index_search_exclude(h, q.data_ptr(), nq, K, p[0], p[1], ex.data_ptr(), 1,
+                                                                    0, st))
+        return lambda: check(lib, lib.keds_index_search_ex(h, q.data_ptr(), nq, K, p[0], p[1], 0, st))
+
+    variants = ("base", "plain", "exclude")
+    outs = {(c, v): outputs(shapes[c][0], c.startswith("cfg2")) for c in shapes for v in variants}
+    fns = {(c, v): call(c, v) for c in shapes for v in variants}
+    iters = {"cfg2_retrieve2_128x2x500k": 50, "cfg1_search_4096x50k": 20, "search_4096x500k": 5}
+    for f in fns.values():  # warm-up: modules, scratch sizes, planner feedback
+        for _ in range(5):
+            f()
+    torch.cuda.synchronize()
+
+    times = {key: [] for key in fns}
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for r in range(args.rounds):
+        for c in shapes:
+            order = variants[r % 3:] + variants[:r % 3]
+            for v in order:
+                f = fns[(c, v)]
+                f()
+                e0.record()
+                for _ in range(iters[c]):
+                    f()
+                e1.record()
+                e1.synchronize()
+                times[(c, v)].append(e0.elapsed_time(e1) * 1000.0 / iters[c])
+    for name, lib in libs.items():
+        for h in idx[name].values():
+            check(lib, lib.keds_index_sync(h, st))
+
+    result = {"card": card(), "rounds": args.rounds, "unit": "us per call", "configs": {}}
+    for c in shapes:
+        same = all(torch.equal(a, b) for a, b in zip(outs[(c, "base")], outs[(c, "plain")]))
+        nq, _, ex = shapes[c]
+        I_ex = outs[(c, "exclude")][1]
+        row = {"base_plain_outputs_identical": bool(same),
+               "exclude_never_returns_self": bool(not (I_ex == ex).any().item())}
+        for v in variants:
+            t = times[(c, v)]
+            row[v] = {"median": round(statistics.median(t), 2), "min": round(min(t), 2), "max": round(max(t), 2)}
+        # paired within each round (the three variants ran back to back): median and range of the ratios
+        for name, num, den in (("plain_vs_base_pct", "plain", "base"), ("exclude_vs_plain_pct", "exclude", "plain")):
+            r = [100.0 * (a / b - 1.0) for a, b in zip(times[(c, num)], times[(c, den)])]
+            row[name] = {"median": round(statistics.median(r), 2), "p25": round(statistics.quantiles(r, n=4)[0], 2),
+                         "p75": round(statistics.quantiles(r, n=4)[2], 2)}
+        result["configs"][c] = row
+    text = json.dumps(result, indent=1)
+    print(text)
+    if args.out:
+        os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
+        with open(args.out, "w") as f:
+            f.write(text + "\n")
+    for name, lib in libs.items():
+        for h in idx[name].values():
+            lib.keds_index_free(h)
+
+
+if __name__ == "__main__":
+    main()
