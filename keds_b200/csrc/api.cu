@@ -170,25 +170,26 @@ int encode_rows_map(CUtensorMap* tm, const void* base, int64_t rows, int d_pad, 
   return 0;
 }
 
-bool is_device_ptr(const void* p) {
-  if (!p) return false;
-  cudaPointerAttributes a;
-  if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-    cudaGetLastError();
-    return false;
-  }
-  return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
+// Where a caller's pointer lives: the device that owns it (-1: not device or managed memory) and,
+// for page-locked host memory, its device alias (kernels read and write it through the mapping).
+// Converts to true for device memory.
+struct PtrLoc {
+  int device = -1;
+  void* mapped = nullptr;
+  explicit operator bool() const { return device >= 0; }
+};
 
-// device that owns a device pointer (-1: not device memory)
-int device_of(const void* p) {
-  if (!p) return -1;
+PtrLoc locate(const void* p) {
+  PtrLoc l;
   cudaPointerAttributes a;
+  if (!p) return l;
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
     cudaGetLastError();
-    return -1;
+    return l;
   }
-  return (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) ? a.device : -1;
+  if (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) l.device = a.device;
+  if (a.type == cudaMemoryTypeHost) l.mapped = a.devicePointer;
+  return l;
 }
 
 // [0],[1] n_flagged per db, [2] err word, [3..5] spare, [6] largest candidate band |C| of the search
@@ -212,16 +213,28 @@ struct HitsMode {
   int nks;
   int ks[HITS_MAX_CUTS];
   const long long* row_labels;
-  const long long* qlabel;  // already offset to the pass's first query
-  int* hits;                // [nq][nks], likewise
+  const long long* qlabel;  // [nq]
+  int* hits;                // [nq][nks]
 };
 
-struct Plan {
-  int exact_only = 0;
+// How the scoring kernel covers nq queries: which kernel, its work units and query groups, and
+// the most row slices the candidate budget holds.
+struct Geometry {
   bool pair = false;  // CTA-pair scoring kernel (two query tiles per work item)
   int sub = 1;        // candidate lines per (slice, query): 2 in the pair kernel (one per column half)
-  int S = 1, n_qt = 1, n_qg = 1, n_items = 0, grid = 0;
+  int n_qt = 1, n_qg = 1, units = 0;
+  long long s_mem = 0;
+};
+
+struct Plan : Geometry {
+  int exact_only = 0;
+  int S = 1, n_items = 0, grid = 0;
   bool small_batch = true;  // one wave of re-rank blocks: the latency variant
+  void set_slices(int n_db, int slices) {
+    S = slices;
+    n_items = n_db * n_qg * S;
+    grid = std::min(n_items, units) * (pair ? 2 : 1);
+  }
 };
 
 }  // namespace
@@ -258,6 +271,7 @@ struct keds_index {
   bool use_pdl = true;
   unsigned int* ctrl_cur = nullptr;  // status block of the pass being launched
   int ctrl_passes = 1;             // status blocks the last call used (finish_sync reads them all)
+  int ctrl_slot = 0;               // n_flagged slot of the blocks' first count (1: only the call's second database ran)
   int rerank_threads_large = 128;  // block size of the throughput re-rank variant (KEDS_RERANK_THREADS)
   int rerank_variant = 0;          // 0: by batch size; 1 / 2: force the latency / throughput variant
   // in-kernel timing of the scoring kernel (bench.py's roofline leg): {min start, max end} ns
@@ -349,6 +363,19 @@ int launch_k(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
   return launch_kc(pdl, 1, kernel, grid, block, smem, st, std::forward<Args>(args)...);
 }
 
+Geometry geometry(const keds_index* ix, int n_db, int64_t nq) {
+  Geometry g;
+  g.n_qt = static_cast<int>((nq + BM - 1) / BM);
+  // more than one query tile: CTA pairs share each row tile (two query tiles per work item)
+  g.pair = ix->use_pair && g.n_qt >= 2 && ix->num_sms >= 2;
+  g.sub = g.pair ? ScoreCfg<true>::kSub : ScoreCfg<false>::kSub;
+  g.n_qg = g.pair ? (g.n_qt + 1) / 2 : g.n_qt;
+  g.units = g.pair ? ix->num_sms / 2 : ix->num_sms;
+  g.s_mem = static_cast<long long>(CAND_BUDGET / (size_t(LKEEP) * BM * 8)) /
+            (static_cast<long long>(n_db) * g.n_qt * g.sub);
+  return g;
+}
+
 // Pick the number of row slices: enough that no slice is expected to hold more than a third of
 // LKEEP of the top-k, enough work items to fill the SMs, then whatever minimises the longest CTA.
 // band_hint: the largest candidate band |C| a recent search on this handle reported (0: none).
@@ -358,24 +385,16 @@ int launch_k(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t s
 Plan make_plan(const keds_index* ix, int n_db, int64_t nq, int k, int64_t n_min, int64_t n_max,
                uint32_t flags, unsigned int band_hint = 0) {
   Plan pl;
-  pl.n_qt = static_cast<int>((nq + BM - 1) / BM);
+  static_cast<Geometry&>(pl) = geometry(ix, n_db, nq);
   const int T_min = static_cast<int>((n_min + BN - 1) / BN);
   const int T_max = static_cast<int>((n_max + BN - 1) / BN);
   // a slice hands over its best LKEEP-1 rows and drops the rest (theta = its LKEEP-th best): for
   // the certificate to pass, theta must sit well below the k-th best score overall, i.e. the
   // top-k must be spread over many slices (expected share per slice <= LKEEP / 6)
-  // more than one query tile: CTA pairs share each row tile (two query tiles per work item)
-  pl.pair = ix->use_pair && pl.n_qt >= 2 && ix->num_sms >= 2;
-  pl.sub = pl.pair ? ScoreCfg<true>::kSub : ScoreCfg<false>::kSub;
   // (in candidate lists: the pair kernel keeps one per column half of every slice)
   const int S_sel = std::max(1, ((6 * k + LKEEP - 1) / LKEEP + pl.sub - 1) / pl.sub);
-  pl.n_qg = pl.pair ? (pl.n_qt + 1) / 2 : pl.n_qt;
-  const int units = pl.pair ? ix->num_sms / 2 : ix->num_sms;
   const int groups = n_db * pl.n_qg;
-  int S_hi = std::min(T_min, S_MAX);
-  const long long by_mem = static_cast<long long>(CAND_BUDGET / (size_t(LKEEP) * BM * 8)) /
-                           (static_cast<long long>(n_db) * pl.n_qt * pl.sub);
-  S_hi = static_cast<int>(std::min<long long>(S_hi, by_mem));
+  const int S_hi = static_cast<int>(std::min<long long>(std::min(T_min, S_MAX), pl.s_mem));
   if ((flags & KEDS_SEARCH_EXACT_ONLY) || S_hi < S_sel || k > R_MAX / 2) {
     pl.exact_only = 1;
     return pl;
@@ -387,10 +406,10 @@ Plan make_plan(const keds_index* ix, int n_db, int64_t nq, int k, int64_t n_min,
   if (ix->rerank_variant == 2) pl.small_batch = false;
   double best = 1e300;
   // one exact scan of every fp32 row, in the cost unit below (one bf16 row tile per work unit)
-  const double scan_cost = 2.0 * T_max / units;
+  const double scan_cost = 2.0 * T_max / pl.units;
   for (int S = S_sel; S <= S_hi; ++S) {
     const long long items = static_cast<long long>(groups) * S;
-    const long long G = std::min<long long>(items, units);
+    const long long G = std::min<long long>(items, pl.units);
     const long long per_cta = (items + G - 1) / G;
     double cost = static_cast<double>(per_cta) * ((T_max + S - 1) / S) + 0.35 * per_cta;
     // expected fallbacks: a query is flagged when one list holds LKEEP or more of the rows at or
@@ -416,8 +435,7 @@ Plan make_plan(const keds_index* ix, int n_db, int64_t nq, int k, int64_t n_min,
     const int v = atoi(dbg);
     if (v >= S_sel && v <= S_hi) pl.S = v;
   }
-  pl.n_items = groups * pl.S;
-  pl.grid = std::min(pl.n_items, units) * (pl.pair ? 2 : 1);
+  pl.set_slices(n_db, pl.S);
   return pl;
 }
 
@@ -459,25 +477,78 @@ int prof_mark(keds_index* a, cudaStream_t st, int tag) {
   return 0;
 }
 
+// One search call. The entry points fill it with the caller's arrays; search_impl puts host
+// queries and results into device staging before the first pass, and every pass gets a slice.
+struct Call {
+  keds_index* owner = nullptr;  // scratch, status blocks, stats and tuning switches: the call's first handle
+  keds_index* dbs[2] = {nullptr, nullptr};
+  int n_db = 1;
+  int slot0 = 0;  // which of the call's databases dbs[0] is: its flagged count is reported there
+  int64_t nq = 0;
+  int k = 0;
+  uint32_t flags = 0;
+  int pass = 0;                  // status block of this pass
+  const float* q = nullptr;      // fp32 [nq][d]
+  const float* q_src = nullptr;  // device alias of page-locked host queries, or null: k_prep_rows reads
+                                 // them through the mapping and leaves the fp32 copy in q
+  float* D[2] = {nullptr, nullptr};  // [nq][k] per database
+  long long* I[2] = {nullptr, nullptr};
+  // optional parts, absent while zero
+  ConsumeParams cons{};           // the fused neighbour consumer (retrieve2)
+  PeerOut peer{};                 // the sharded search's push to the other ranks
+  const long long* ex = nullptr;  // [nq][n_ex] labels to leave out (device memory or a mapped host alias);
+  int n_ex = 0;                   // k_prep_rows stages them as local row ids in owner->ex_rows
+  HitsMode hits{};                // label hits at cut points in the re-rank's place
+  float* dump = nullptr;          // debug_scores: the raw scores, ld_dump per query
+  int64_t ld_dump = 0;
+
+  int metric() const { return (flags & KEDS_SEARCH_FORCE_IP) ? METRIC_IP : owner->metric; }
+  int exclude(const int64_t* labels, int n) {
+    if (!labels || n < 1 || n > EXCLUDE_MAX)
+      return fail(KEDS_ERR_ARG, "exclude must be a non-null [nq][n_exclude] array, 1 <= n_exclude <= %d", EXCLUDE_MAX);
+    ex = reinterpret_cast<const long long*>(labels);
+    n_ex = n;
+    return 0;
+  }
+};
+
+Call call(int n_db, keds_index* a, keds_index* b, const float* q, int64_t nq, int k, float* Da, int64_t* Ia,
+          float* Db, int64_t* Ib, uint32_t flags) {
+  Call c;
+  c.owner = c.dbs[0] = a;
+  c.dbs[1] = b;
+  c.n_db = n_db;
+  c.q = q;
+  c.nq = nq;
+  c.k = k;
+  c.D[0] = Da;
+  c.I[0] = reinterpret_cast<long long*>(Ia);
+  c.D[1] = Db;
+  c.I[1] = reinterpret_cast<long long*>(Ib);
+  c.flags = flags;
+  return c;
+}
+
 // The exact-fallback kernel, ceil(nq / f_cap) passes; every launch returns at once when its slice
 // of the flagged list is empty.
-int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_dev, int64_t nq, int k,
-                 float* D[2], long long* I[2], int metric, const ConsumeParams& cons,
-                 unsigned long long* timing, cudaStream_t st, const PeerOut* peer = nullptr,
-                 const ExcludeStage* ex = nullptr) {
+int launch_exact(const Call& c, unsigned long long* timing, cudaStream_t st) {
+  keds_index* ix = c.owner;
+  keds_index* const* dbs = c.dbs;
+  const int n_db = c.n_db, k = c.k;
+  const int64_t nq = c.nq;
   ExactParams ep;
   memset(&ep, 0, sizeof ep);
-  if (ex) {
-    ep.ex_rows = ex->rows;
-    ep.n_ex = ex->n_ex;
-    ep.ex_ld = ex->nq * ex->n_ex;
+  if (c.ex) {
+    ep.ex_rows = ix->ex_rows.as<int>();
+    ep.n_ex = c.n_ex;
+    ep.ex_ld = nq * c.n_ex;
   }
-  ep.cons = cons;
+  ep.cons = c.cons;
   ep.n_db = n_db;
   ep.d = ix->d;
-  ep.metric = metric;
+  ep.metric = c.metric();
   ep.k = k;
-  ep.q_f32 = q_dev;
+  ep.q_f32 = c.q;
   // Queries per launch: as many as the score scratch holds (it is allocated for the batch at hand,
   // never beyond the budget). Up to 1 GB always -- all of a 128-query batch at 2 x 0.5M rows, all of
   // 4,096 queries at 50k rows in ONE launch; large batches get up to 4 GB so that a search is followed
@@ -514,14 +585,14 @@ int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_de
     scratch += static_cast<size_t>(fc) * dbs[i]->n;
     e.cmax = scratch;
     scratch += static_cast<size_t>(fc) * e.chunks;
-    e.D = D[i];
-    e.I = I[i];
+    e.D = c.D[i];
+    e.I = c.I[i];
     e.id_offset = dbs[i]->id_offset;
   }
   const int dq = (ix->d + 3) & ~3;
   const size_t smem_sc = static_cast<size_t>(EXACT_QG) * dq * 4 + (EXACT_THREADS / 32) * EXACT_QG * 4;
   ep.ck_cap = std::min(chunks_max, 8192);
-  const size_t smem_sel = static_cast<size_t>(cons.part4) * 16 + static_cast<size_t>(k) * 20 + 256 * 4 + 16 + 16 + 32 +
+  const size_t smem_sel = static_cast<size_t>(c.cons.part4) * 16 + static_cast<size_t>(k) * 20 + 256 * 4 + 16 + 16 + 32 +
                           static_cast<size_t>(EXACT_LIST_CAP) * 8 + static_cast<size_t>(ep.ck_cap) * 4;
   const size_t smem = std::max(smem_sc, smem_sel);
   if (smem > 160 * 1024) return fail(KEDS_ERR_ARG, "d=%d / k=%d too large for the exact fallback", ix->d, k);
@@ -532,10 +603,8 @@ int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_de
   for (int pass = 0; pass < passes; ++pass) {
     ep.pass = pass;
     ep.band_host = pass == passes - 1 ? ix->h_feedback : nullptr;
-    if (peer) {
-      ep.peer = *peer;
-      ep.peer.publish = peer->publish && pass == passes - 1;  // only the step's very last launch publishes
-    }
+    ep.peer = c.peer;
+    ep.peer.publish = c.peer.publish && pass == passes - 1;  // only the step's very last launch publishes
     ep.timing = pass == 0 ? timing : nullptr;
     // work counters of this launch: its own zeroed set (the last set is shared, with a memset, by
     // launches beyond EXACT_CTR_SETS)
@@ -549,34 +618,83 @@ int launch_exact(keds_index* ix, keds_index* dbs[2], int n_db, const float* q_de
   return 0;
 }
 
-// One pass (<= Q_PASS_MAX queries). q_dev: device fp32 [nq][d]. D/I: device outputs.
-// cons_in (nullable): neighbour-consumer outputs for this pass, already offset to its first query.
-int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int k, float* D[2],
-                long long* I[2], uint32_t flags, cudaStream_t st, float* dump, int64_t ld_dump,
-                const ConsumeParams* cons_in, const PeerOut* peer = nullptr, int pass_idx = 0,
-                const float* q_src = nullptr, const HitsMode* hm = nullptr, const long long* ex_src = nullptr,
-                int n_ex = 0) {
-  // q_src (nullable): the queries in page-locked host memory, addressed through the mapping;
-  // k_prep_rows reads them there once and leaves the fp32 copy the other kernels use in q_dev
-  // ex_src (nullable): [nq][n_ex] labels to leave out of each query's result (device memory or
-  // mapped host memory); k_prep_rows stages them as local row ids in a->ex_rows
-  keds_index* a = ix[0];
-  const int metric = (flags & KEDS_SEARCH_FORCE_IP) ? METRIC_IP : a->metric;
+// Candidate lines of a pass, indexed by (db, slice, query tile) whatever the work-item grouping.
+int ensure_cand(keds_index* a, size_t lines) {
+  CKS(a->cand.ensure(lines * LKEEP * BM * 8));
+  CKS(a->cand_cnt.ensure(lines * BM * 4));
+  CKS(a->cand_theta.ensure(lines * BM * 4));
+  return 0;
+}
+
+// What every launch of the scoring kernel is given: the plan, the databases, the candidate lists
+// and the error word. The rest is zero: the caller adds its epilogue's inputs.
+ScoreParams score_params(const keds_index* a, keds_index* const* dbs, int n_db, const Plan& pl, int64_t nq,
+                         unsigned int* err) {
+  ScoreParams sp;
+  memset(&sp, 0, sizeof sp);
+  sp.n_db = n_db;
+  sp.n_qt = pl.n_qt;
+  sp.n_qg = pl.n_qg;
+  sp.S = pl.S;
+  sp.n_items = pl.n_items;
+  sp.kblocks = a->d_pad / BK;
+  sp.fmt_bits = a->fmt == FMT_BF16 ? kIdescBf16Bits : 0u;
+  sp.nq = static_cast<int>(nq);
+  for (int i = 0; i < n_db; ++i) {
+    sp.n_rows[i] = static_cast<int>(dbs[i]->n);
+    sp.n_tiles[i] = static_cast<int>((dbs[i]->n + BN - 1) / BN);
+  }
+  sp.cand = a->cand.as<uint2>();
+  sp.cand_cnt = a->cand_cnt.as<int>();
+  sp.cand_theta = a->cand_theta.as<float>();
+  sp.err = err;
+  return sp;
+}
+
+// The scoring kernel in the instantiation sp asks for: gallery ranking (rk_lo), top-k with
+// exclusion (ex_rows: tests each tile against the query's excluded rows) or the plain top-k.
+int launch_score(keds_index* a, keds_index* const* dbs, int n_db, const Plan& pl, const ScoreParams& sp,
+                 cudaStream_t st) {
+  const keds_index* x1 = n_db > 1 ? dbs[1] : dbs[0];
+  if (pl.pair)
+    return launch_kc(a->use_pdl, 2,
+                     sp.rk_lo ? k_score_topk<true, true> : sp.ex_rows ? k_score_topk<true, false, true> : k_score_topk<true>,
+                     dim3(pl.grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, dbs[0]->tm_xh,
+                     x1->tm_xh, sp);
+  return launch_k(a->use_pdl,
+                  sp.rk_lo ? k_score_topk<false, true> : sp.ex_rows ? k_score_topk<false, false, true> : k_score_topk<false>,
+                  dim3(pl.grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, dbs[0]->tm_x, x1->tm_x, sp);
+}
+
+// Candidate capacity per query of the re-rank and hits blocks: room for the band a recent search
+// reported (a query that does not fit is answered by the exact fallback and raises the next call's figure).
+int cand_capacity(int k, unsigned int band_hint) {
+  const unsigned int want =
+      std::max<unsigned int>(static_cast<unsigned int>(k + k / 2 + 64), band_hint + band_hint / 2);
+  int rmax = 256;
+  while (rmax < static_cast<int>(std::min<unsigned int>(want, R_MAX))) rmax *= 2;
+  return rmax;
+}
+
+// One pass (<= Q_PASS_MAX queries) of a call; q, D and I are device memory.
+int search_pass(const Call& c, cudaStream_t st) {
+  keds_index* a = c.owner;
+  keds_index* const* ix = c.dbs;
+  const int n_db = c.n_db, k = c.k, metric = c.metric();
+  const int64_t nq = c.nq;
   CKS(set_kernel_attrs(a));
-  ConsumeParams cons;
-  memset(&cons, 0, sizeof cons);
-  if (cons_in) cons = *cons_in;
   // in-kernel %globaltimer stamps, one {min start, max end} pair per kernel of this chain
   // (prep, score, rerank, exact scores, exact select); the first TIMING_RING searches are timed
   unsigned long long* tchain = nullptr;
-  if (a->timing_on && a->timing_launches < TIMING_RING && !dump) {
+  if (a->timing_on && a->timing_launches < TIMING_RING && !c.dump) {
     tchain = a->timing.as<unsigned long long>() + TIMING_PAIRS * 2 * a->timing_launches;
     a->timing_launches++;
   }
   // (a multi-pass call sizes the status blocks of all its passes before the first launch)
-  CKS(a->ctrl.ensure(static_cast<size_t>(pass_idx + 1) * CTRL_STRIDE * 4));
-  a->ctrl_cur = a->ctrl.as<unsigned int>() + static_cast<size_t>(pass_idx) * CTRL_STRIDE;
-  a->ctrl_passes = pass_idx + 1;
+  CKS(a->ctrl.ensure(static_cast<size_t>(c.pass + 1) * CTRL_STRIDE * 4));
+  a->ctrl_cur = a->ctrl.as<unsigned int>() + static_cast<size_t>(c.pass) * CTRL_STRIDE;
+  a->ctrl_passes = c.pass + 1;
+  a->ctrl_slot = c.slot0;
   for (int i = 0; i < n_db; ++i) CKS(a->flagged[i].ensure(static_cast<size_t>(nq) * 4));
 
   int64_t n_min = ix[0]->n, n_max = ix[0]->n;
@@ -585,15 +703,15 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     n_max = std::max(n_max, ix[1]->n);
   }
   const unsigned int band_hint = a->h_feedback ? *static_cast<volatile unsigned int*>(a->h_feedback) : 0u;
-  Plan pl = make_plan(a, n_db, nq, k, n_min, n_max, flags, band_hint);
-  if (dump && pl.exact_only) return fail(KEDS_ERR_ARG, "debug_scores needs at least one 256-row tile");
+  Plan pl = make_plan(a, n_db, nq, k, n_min, n_max, c.flags, band_hint);
+  if (c.dump && pl.exact_only) return fail(KEDS_ERR_ARG, "debug_scores needs at least one 256-row tile");
   ExcludeStage exs;
   memset(&exs, 0, sizeof exs);
-  if (ex_src) {
-    CKS(a->ex_rows.ensure(static_cast<size_t>(n_db) * nq * n_ex * 4));
-    exs.labels = ex_src;
+  if (c.ex) {
+    CKS(a->ex_rows.ensure(static_cast<size_t>(n_db) * nq * c.n_ex * 4));
+    exs.labels = c.ex;
     exs.nq = nq;
-    exs.n_ex = n_ex;
+    exs.n_ex = c.n_ex;
     exs.n_db = n_db;
     exs.rows = a->ex_rows.as<int>();
     for (int i = 0; i < n_db; ++i) {
@@ -607,14 +725,14 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
   a->stats.grid = pl.grid;
 
   if (pl.exact_only) {
-    if (q_src) CK(cudaMemcpyAsync(const_cast<float*>(q_dev), q_src, static_cast<size_t>(nq) * a->d * 4, cudaMemcpyDefault, st));
+    if (c.q_src) CK(cudaMemcpyAsync(const_cast<float*>(c.q), c.q_src, static_cast<size_t>(nq) * a->d * 4, cudaMemcpyDefault, st));
     CK(cudaMemsetAsync(a->ctrl_cur, 0, CTRL_STRIDE * 4, st));
     for (int i = 0; i < n_db; ++i) {
       k_flag_all<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, st>>>(
           a->flagged[i].as<int>(), reinterpret_cast<int*>(a->ctrl_cur) + i, static_cast<int>(nq));
       a->stats.launches++;
     }
-    if (ex_src) {
+    if (c.ex) {
       // the staging half of k_prep_rows alone (no query rows to prepare on this route)
       const unsigned blocks = static_cast<unsigned>(std::min<long long>((nq + 255) / 256, 1024));
       k_prep_rows<<<blocks, 256, 0, st>>>(nullptr, 0, a->d, a->d_pad, a->fmt, nullptr, nullptr, nullptr, nullptr,
@@ -634,66 +752,37 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
       const long long warps_needed = nq;
       const unsigned blocks =
           static_cast<unsigned>(std::min<long long>((warps_needed * 32 + threads - 1) / threads, 4096));
-      CKS(launch_k(a->use_pdl, k_prep_rows, dim3(blocks), dim3(threads), 0, st, q_src ? q_src : q_dev,
+      CKS(launch_k(a->use_pdl, k_prep_rows, dim3(blocks), dim3(threads), 0, st, c.q_src ? c.q_src : c.q,
                    static_cast<long long>(nq), a->d, a->d_pad, a->fmt, a->q_bf16.as<uint16_t>(),
                    a->qstat.as<float4>(), static_cast<float*>(nullptr), static_cast<unsigned int*>(nullptr),
                    a->ctrl_cur, CTRL_STRIDE, a->theta0.as<float>(), static_cast<int>(n_db * theta_ld), tchain,
-                   q_src ? const_cast<float*>(q_dev) : static_cast<float*>(nullptr), exs));
+                   c.q_src ? const_cast<float*>(c.q) : static_cast<float*>(nullptr), exs));
       a->stats.launches++;
     }
-    // candidate lines are indexed by (db, slice, query tile) whatever the work-item grouping
-    const size_t items = static_cast<size_t>(n_db) * pl.S * pl.sub * pl.n_qt;
-    CKS(a->cand.ensure(items * LKEEP * BM * 8));
-    CKS(a->cand_cnt.ensure(items * BM * 4));
-    CKS(a->cand_theta.ensure(items * BM * 4));
-
-    ScoreParams sp;
-    memset(&sp, 0, sizeof sp);
-    sp.n_db = n_db;
-    sp.n_qt = pl.n_qt;
-    sp.n_qg = pl.n_qg;
-    sp.S = pl.S;
-    sp.n_items = pl.n_items;
-    sp.kblocks = a->d_pad / BK;
-    sp.fmt_bits = a->fmt == FMT_BF16 ? kIdescBf16Bits : 0u;
-    sp.nq = static_cast<int>(nq);
-    for (int i = 0; i < n_db; ++i) {
-      sp.n_rows[i] = static_cast<int>(ix[i]->n);
-      sp.n_tiles[i] = static_cast<int>((ix[i]->n + BN - 1) / BN);
-      sp.bias[i] = metric == METRIC_L2 ? ix[i]->bias.as<float>() : nullptr;
-    }
-    sp.cand = a->cand.as<uint2>();
-    sp.cand_cnt = a->cand_cnt.as<int>();
-    sp.cand_theta = a->cand_theta.as<float>();
+    CKS(ensure_cand(a, static_cast<size_t>(n_db) * pl.S * pl.sub * pl.n_qt));
+    ScoreParams sp = score_params(a, ix, n_db, pl, nq, a->ctrl_cur + 2);
+    for (int i = 0; i < n_db; ++i) sp.bias[i] = metric == METRIC_L2 ? ix[i]->bias.as<float>() : nullptr;
     sp.theta0 = a->warm_start ? a->theta0.as<float>() : nullptr;
     sp.theta_ld = static_cast<int>(theta_ld);
-    sp.err = a->ctrl_cur + 2;
-    sp.dump = dump;
-    sp.ld_dump = ld_dump;
+    sp.dump = c.dump;
+    sp.ld_dump = c.ld_dump;
     sp.timing = tchain ? tchain + 2 : nullptr;
-    if (ex_src) {
+    if (c.ex) {
       sp.ex_rows = exs.rows;
-      sp.n_ex = n_ex;
-      sp.ex_ld = static_cast<long long>(nq) * n_ex;
+      sp.n_ex = c.n_ex;
+      sp.ex_ld = static_cast<long long>(nq) * c.n_ex;
     }
     CKS(prof_mark(a, st, 1));
-    // (with exclusion: the instantiation that tests each tile against the query's excluded rows)
-    if (pl.pair)
-      CKS(launch_kc(a->use_pdl, 2, ex_src ? k_score_topk<true, false, true> : k_score_topk<true>, dim3(pl.grid),
-                    dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, ix[0]->tm_xh,
-                    n_db > 1 ? ix[1]->tm_xh : ix[0]->tm_xh, sp));
-    else
-      CKS(launch_k(a->use_pdl, ex_src ? k_score_topk<false, false, true> : k_score_topk<false>, dim3(pl.grid),
-                   dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, ix[0]->tm_x,
-                   n_db > 1 ? ix[1]->tm_x : ix[0]->tm_x, sp));
+    CKS(launch_score(a, ix, n_db, pl, sp, st));
     CKS(prof_mark(a, st, 2));
     a->stats.launches++;
     CK(cudaGetLastError());
-    if (dump) return 0;
+    if (c.dump) return 0;
 
-    if (hm) {
+    if (c.hits.nks) {
       // label hits at the cut points instead of the ranked rows (label_hits.cuh): same lists, same
       // certificate, exact scores only for the rows inside the error band around a cut
+      const HitsMode& hm = c.hits;
       HitsParams hp;
       memset(&hp, 0, sizeof hp);
       hp.n_qt = pl.n_qt;
@@ -701,22 +790,20 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
       hp.nq = static_cast<int>(nq);
       hp.d = a->d;
       hp.metric = metric;
-      hp.nks = hm->nks;
-      for (int j = 0; j < hm->nks; ++j) hp.ks[j] = hm->ks[j];
-      unsigned int want = std::max<unsigned int>(static_cast<unsigned int>(k + k / 2 + 64), band_hint + band_hint / 2);
-      int rmax = 256;
-      while (rmax < static_cast<int>(std::min<unsigned int>(want, R_MAX))) rmax *= 2;
+      hp.nks = hm.nks;
+      for (int j = 0; j < hm.nks; ++j) hp.ks[j] = hm.ks[j];
+      const int rmax = cand_capacity(k, band_hint);
       hp.rmax = rmax;
       hp.cand = sp.cand;
       hp.cand_cnt = sp.cand_cnt;
       hp.cand_theta = sp.cand_theta;
-      hp.q_f32 = q_dev;
+      hp.q_f32 = c.q;
       hp.qstat = a->qstat.as<float4>();
-      hp.x_f32 = a->x_f32.as<float>();
-      hp.dbstat = a->dbstat.as<unsigned int>();
-      hp.row_labels = hm->row_labels;
-      hp.qlabel = hm->qlabel;
-      hp.hits = hm->hits;
+      hp.x_f32 = ix[0]->x_f32.as<float>();
+      hp.dbstat = ix[0]->dbstat.as<unsigned int>();
+      hp.row_labels = hm.row_labels;
+      hp.qlabel = hm.qlabel;
+      hp.hits = hm.hits;
       hp.flagged = a->flagged[0].as<int>();
       hp.n_flagged = reinterpret_cast<int*>(a->ctrl_cur);
       hp.eps_scale = a->eps_scale;
@@ -745,13 +832,13 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     rp.cand = sp.cand;
     rp.cand_cnt = sp.cand_cnt;
     rp.cand_theta = sp.cand_theta;
-    rp.q_f32 = q_dev;
+    rp.q_f32 = c.q;
     rp.qstat = a->qstat.as<float4>();
     for (int i = 0; i < n_db; ++i) {
       rp.x_f32[i] = ix[i]->x_f32.as<float>();
       rp.dbstat[i] = ix[i]->dbstat.as<unsigned int>();
-      rp.D[i] = D[i];
-      rp.I[i] = I[i];
+      rp.D[i] = c.D[i];
+      rp.I[i] = c.I[i];
       rp.id_offset[i] = ix[i]->id_offset;
       rp.flagged[i] = a->flagged[i].as<int>();
       rp.n_flagged[i] = reinterpret_cast<int*>(a->ctrl_cur) + i;
@@ -760,23 +847,16 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     rp.band_max = a->ctrl_cur + CTRL_BAND;
     // one wave of blocks (two per SM): the latency variant; more: the four-per-SM throughput variant
     const bool small_batch = pl.small_batch;
-    // Candidate capacity. A single wave has the shared memory to spare: full size. Large batches
-    // live on blocks per SM, so they start small and follow the band a recent search reported (a
-    // query that does not fit is answered by the exact fallback and raises the next call's figure).
-    int rmax = R_MAX;
-    if (!small_batch) {
-      const unsigned int want =
-          std::max<unsigned int>(static_cast<unsigned int>(k + k / 2 + 64), band_hint + band_hint / 2);
-      rmax = 256;
-      while (rmax < static_cast<int>(std::min<unsigned int>(want, R_MAX))) rmax *= 2;
-    }
+    // A single wave has the shared memory to spare: full candidate capacity. Large batches live on
+    // blocks per SM, so they start small and follow the band a recent search reported.
+    const int rmax = small_batch ? R_MAX : cand_capacity(k, band_hint);
     rp.rmax = rmax;
-    if (peer) rp.peer = *peer;
-    rp.cons = cons;
+    rp.peer = c.peer;
+    rp.cons = c.cons;
     rp.timing = tchain ? tchain + 4 : nullptr;
     const size_t slots = static_cast<size_t>(pl.S) * pl.sub * LKEEP;
     // qvec | part | okey | keys, ids | smax | a_key, a_id, sel_id, sel_sc | hist | red | bcast | counters | top_*
-    const size_t smem = static_cast<size_t>((a->d + 3) & ~3) * 4 + static_cast<size_t>(cons.part4) * 16 +
+    const size_t smem = static_cast<size_t>((a->d + 3) & ~3) * 4 + static_cast<size_t>(c.cons.part4) * 16 +
                         static_cast<size_t>(rmax) * 24 + slots * 8 + pl.S * pl.sub * 4 + 256 * 4 + 32 * 4 + 16 + 16 +
                         static_cast<size_t>(k) * 12;
     if (smem > 200 * 1024) return fail(KEDS_ERR_ARG, "re-rank shared memory %zu too large", smem);
@@ -797,22 +877,21 @@ int search_pass(keds_index* ix[2], int n_db, const float* q_dev, int64_t nq, int
     CK(cudaGetLastError());
     }
   }
-  if (!(flags & KEDS_SEARCH_NO_FALLBACK) || pl.exact_only) {
-    CKS(launch_exact(a, ix, n_db, q_dev, nq, k, D, I, metric, cons, tchain ? tchain + 6 : nullptr, st, peer,
-                     ex_src ? &exs : nullptr));
+  if (!(c.flags & KEDS_SEARCH_NO_FALLBACK) || pl.exact_only) {
+    CKS(launch_exact(c, tchain ? tchain + 6 : nullptr, st));
     CKS(prof_mark(a, st, 4));
   }
-  if (hm) {
+  if (c.hits.nks) {
     // the queued queries' exact rows (written by the fallback just now) -> their hits
     HitsParams hp;
     memset(&hp, 0, sizeof hp);
-    hp.nks = hm->nks;
-    for (int j = 0; j < hm->nks; ++j) hp.ks[j] = hm->ks[j];
-    hp.hits = hm->hits;
+    hp.nks = c.hits.nks;
+    for (int j = 0; j < c.hits.nks; ++j) hp.ks[j] = c.hits.ks[j];
+    hp.hits = c.hits.hits;
     CKS(launch_k(a->use_pdl, k_hits_from_rows, dim3(static_cast<unsigned>(std::min<int64_t>((nq + 127) / 128, 64))),
                  dim3(128), 0, st, static_cast<const int*>(a->flagged[0].as<int>()),
-                 static_cast<const int*>(reinterpret_cast<int*>(a->ctrl_cur)), static_cast<const long long*>(I[0]), k,
-                 static_cast<long long>(a->id_offset), hm->row_labels, hm->qlabel, hp));
+                 static_cast<const int*>(reinterpret_cast<int*>(a->ctrl_cur)), static_cast<const long long*>(c.I[0]), k,
+                 static_cast<long long>(ix[0]->id_offset), c.hits.row_labels, c.hits.qlabel, hp));
     a->stats.launches++;
   }
   CK(cudaGetLastError());
@@ -827,39 +906,56 @@ __global__ void k_fill_pad(float* D, long long* I, long long n, float dv) {
   }
 }
 
-// device alias of a page-locked host result block (nullptr in: nullptr out)
-template <class T>
-int mapped_alias(T* host, T** out) {
-  *out = nullptr;
-  if (!host) return 0;
-  cudaPointerAttributes at;
-  if (cudaPointerGetAttributes(&at, host) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) {
-    cudaGetLastError();
-    return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host result pointer is not page-locked (cudaHostAlloc / pin_memory)");
+// Queries [q0, q0 + nb) of a call: every per-query pointer moved to q0, and only the call's last
+// pass publishes to the peers.
+Call slice(const Call& c, int64_t q0, int64_t nb) {
+  Call p = c;
+  const int64_t d = c.owner->d, k = c.k;
+  p.nq = nb;
+  p.pass = static_cast<int>(q0 / Q_PASS_MAX);
+  p.q += q0 * d;
+  if (p.q_src) p.q_src += q0 * d;
+  // (label hits: D and I hold the fallback's rows of the queued queries, scratch every pass reuses)
+  for (int i = 0; i < c.n_db && !c.hits.nks; ++i) {
+    p.D[i] += q0 * k;
+    p.I[i] += q0 * k;
   }
-  *out = static_cast<T*>(at.devicePointer);
+  for (int s = 0; s < 2; ++s) {
+    if (p.cons.feat[s]) p.cons.feat[s] += q0 * k * d;
+    if (p.cons.pool[s]) p.cons.pool[s] += q0 * d;
+    if (p.cons.host_D[s]) p.cons.host_D[s] += q0 * k;
+    if (p.cons.host_I[s]) p.cons.host_I[s] += q0 * k;
+  }
+  for (int r = 0; r < p.peer.n; ++r) {
+    if (p.peer.D[r]) p.peer.D[r] += q0 * k;
+    if (p.peer.I[r]) p.peer.I[r] += q0 * k;
+  }
+  if (p.peer.n) p.peer.publish = q0 + nb >= c.nq;  // the flags go out behind the step's last pass
+  if (p.ex) p.ex += q0 * c.n_ex;
+  if (p.hits.nks) {
+    p.hits.qlabel += q0;
+    p.hits.hits += q0 * p.hits.nks;
+  }
+  return p;
+}
+
+// Every pass of a call, queued back to back: each pass has its own status block and the scratch is
+// reused in stream order (each kernel of a chain waits for its predecessor to complete), so the
+// passes need no host round trip between them.
+int run_passes(const Call& c, cudaStream_t st) {
+  for (int64_t q0 = 0; q0 < c.nq; q0 += Q_PASS_MAX)
+    CKS(search_pass(slice(c, q0, std::min<int64_t>(Q_PASS_MAX, c.nq - q0)), st));
   return 0;
 }
 
 // Status of a call = its passes' status blocks folded: flagged queries summed, first error word.
-void read_status(const keds_index* a, const uint32_t* blocks, uint32_t h[CTRL_WORDS]) {
-  for (int i = 0; i < CTRL_WORDS; ++i) h[i] = 0;
-  if (!blocks) return;
-  for (int p = 0; p < a->ctrl_passes; ++p) {
+// Sets last_stats; a fired watchdog is the call's error.
+int fold_status(keds_index* a, const uint32_t* blocks) {
+  uint32_t h[3] = {0, 0, 0};
+  for (int p = 0; blocks && p < a->ctrl_passes; ++p) {
     const uint32_t* b = blocks + static_cast<size_t>(p) * CTRL_STRIDE;
-    h[0] += b[0];
-    h[1] += b[1];
+    for (int i = a->ctrl_slot; i < 2; ++i) h[i] += b[i - a->ctrl_slot];
     if (h[2] == 0) h[2] = b[2];
-  }
-}
-
-int finish_sync(keds_index* a, cudaStream_t st) {
-  CK(cudaStreamSynchronize(st));
-  uint32_t h[CTRL_WORDS] = {0};
-  if (a->ctrl.p) {
-    std::vector<uint32_t> all(static_cast<size_t>(a->ctrl_passes) * CTRL_STRIDE);
-    CK(cudaMemcpy(all.data(), a->ctrl.p, all.size() * 4, cudaMemcpyDeviceToHost));
-    read_status(a, all.data(), h);
   }
   a->stats.n_flagged[0] = static_cast<int32_t>(h[0]);
   a->stats.n_flagged[1] = static_cast<int32_t>(h[1]);
@@ -869,18 +965,31 @@ int finish_sync(keds_index* a, cudaStream_t st) {
   return 0;
 }
 
-int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, float* D[2],
-                int64_t* I[2], uint32_t flags, void* stream, const ConsumeParams* cons = nullptr,
-                const PeerOut* peer = nullptr, bool q_mapped = false, const int64_t* exclude = nullptr,
-                int n_ex = 0) {
-  keds_index* a = ix[0];
-  if (!a || !q || nq < 0 || k <= 0) return fail(KEDS_ERR_ARG, "search: null handle/query or bad nq/k");
-  if (n_ex != 0 && (!exclude || n_ex < 1 || n_ex > EXCLUDE_MAX))
-    return fail(KEDS_ERR_ARG, "search: exclude must be a non-null [nq][n_exclude] array, 1 <= n_exclude <= %d",
-                EXCLUDE_MAX);
+int finish_sync(keds_index* a, cudaStream_t st) {
+  CK(cudaStreamSynchronize(st));
+  if (!a->ctrl.p) return fold_status(a, nullptr);
+  std::vector<uint32_t> all(static_cast<size_t>(a->ctrl_passes) * CTRL_STRIDE);
+  CK(cudaMemcpy(all.data(), a->ctrl.p, all.size() * 4, cudaMemcpyDeviceToHost));
+  return fold_status(a, all.data());
+}
+
+// Where a call's caller arrays may live.
+enum Io {
+  IO_HOST,    // q, D and I host or device memory (host arrays are staged through the handle)
+  IO_DEVICE,  // device memory, checked by the caller
+  IO_MAPPED,  // D and I device memory, checked by the caller; q and the exclusion labels device or
+              // page-locked host memory (read through the mapping)
+};
+
+int search_impl(Call c, Io io, void* stream) {
+  keds_index** ix = c.dbs;
+  keds_index* a = c.owner;
+  const int n_db = c.n_db, k = c.k;
+  const int64_t nq = c.nq;
+  if (!a || !c.q || nq < 0 || k <= 0) return fail(KEDS_ERR_ARG, "search: null handle/query or bad nq/k");
   if (k > K_MAX) return fail(KEDS_ERR_ARG, "search: k=%d exceeds the maximum %d", k, K_MAX);
   for (int i = 0; i < n_db; ++i) {
-    if (!ix[i] || !D[i] || !I[i]) return fail(KEDS_ERR_ARG, "search: null index or output pointer");
+    if (!ix[i] || !c.D[i] || !c.I[i]) return fail(KEDS_ERR_ARG, "search: null index or output pointer");
     if (ix[i]->d != a->d || ix[i]->metric != a->metric || ix[i]->device != a->device)
       return fail(KEDS_ERR_ARG, "search2: indices differ in d, metric or device");
     if (ix[i]->n > 0x7fffffffll - BN) return fail(KEDS_ERR_ARG, "index too large for 32-bit row ids");
@@ -896,48 +1005,26 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
     for (int i = 0; i < 2; ++i)
       if (ix[i]->fmt != FMT_BF16) CKS(keds_index_set_operand_format(ix[i], FMT_BF16));
 
-  // q_mapped: the queries sit in page-locked host memory and the first kernel of the chain reads
-  // them through the mapping (no copy in front of the search); it leaves an fp32 copy in q_f32
-  const float* q_map = nullptr;
-  if (q_mapped && !is_device_ptr(q)) {
-    cudaPointerAttributes at;
-    if (cudaPointerGetAttributes(&at, q) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) {
-      cudaGetLastError();
-      return fail(KEDS_ERR_ARG, "retrieve2_hostio: q is neither device memory nor page-locked host memory");
-    }
-    q_map = static_cast<const float*>(at.devicePointer);
-    CKS(a->q_f32.ensure(static_cast<size_t>(nq) * a->d * 4));
-  }
-  const bool q_dev = q_map != nullptr || is_device_ptr(q);
-  // the exclusion labels: device memory, or (retrieve2_hostio) page-locked host memory that
-  // k_prep_rows reads through the mapping
-  const long long* ex_dev = nullptr;
-  if (n_ex != 0 && nq > 0) {
-    if (device_of(exclude) == a->device) {
-      ex_dev = reinterpret_cast<const long long*>(exclude);
-    } else {
-      cudaPointerAttributes at;
-      if (!q_mapped || cudaPointerGetAttributes(&at, exclude) != cudaSuccess || at.type != cudaMemoryTypeHost ||
-          !at.devicePointer) {
-        cudaGetLastError();
-        return fail(KEDS_ERR_ARG, q_mapped ? "retrieve2_hostio: exclude is neither device memory of the index's GPU "
-                                             "nor page-locked host memory"
-                                           : "search: exclude must be device memory of the index's GPU");
-      }
-      ex_dev = static_cast<const long long*>(at.devicePointer);
-    }
-  }
+  const PtrLoc lq = io == IO_DEVICE ? PtrLoc{a->device, nullptr} : locate(c.q);
+  if (!lq && io == IO_MAPPED && !lq.mapped)
+    return fail(KEDS_ERR_ARG, "retrieve2_hostio: q is neither device memory nor page-locked host memory");
   bool out_dev = true;
-  for (int i = 0; i < n_db; ++i) {
-    const bool dd = is_device_ptr(D[i]), di = is_device_ptr(I[i]);
+  for (int i = 0; io == IO_HOST && i < n_db; ++i) {
+    const bool dd = static_cast<bool>(locate(c.D[i])), di = static_cast<bool>(locate(c.I[i]));
     if (dd != di) return fail(KEDS_ERR_ARG, "search: D and I must both be host or both be device memory");
-    out_dev = out_dev && dd;
-    if (i > 0 && dd != is_device_ptr(D[0]))
-      return fail(KEDS_ERR_ARG, "search2: outputs must all be host or all be device memory");
+    if (i > 0 && dd != out_dev) return fail(KEDS_ERR_ARG, "search2: outputs must all be host or all be device memory");
+    out_dev = dd;
   }
-  const float* qd = q_map ? a->q_f32.as<float>() : q;
-  bool any_empty = false;
-  for (int i = 0; i < n_db; ++i) any_empty = any_empty || ix[i]->n == 0;
+  if (c.ex) {
+    const PtrLoc lex = locate(c.ex);
+    if (lex.device != a->device) {
+      if (io != IO_MAPPED || !lex.mapped)
+        return fail(KEDS_ERR_ARG, io == IO_MAPPED ? "retrieve2_hostio: exclude is neither device memory of the index's GPU "
+                                                    "nor page-locked host memory"
+                                                  : "search: exclude must be device memory of the index's GPU");
+      c.ex = static_cast<const long long*>(lex.mapped);
+    }
+  }
   // Host in, host out (the reference's numpy call): the call synchronises before it returns, so
   // page-locked staging buffers can be reused call after call (one real DMA each way instead of
   // the driver's chunked pageable copies). Letting the kernels work on those buffers through the
@@ -946,94 +1033,60 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
   // the call is dominated by its host side.
   // one database's I (8 B) and D (4 B) blocks in the staged result, labels first (8-byte aligned)
   const size_t res_per = (static_cast<size_t>(nq) * k * 12 + 15) & ~size_t(15);
-  if (!q_dev) {
+  const float* q = c.q;
+  if (!lq) {
     const size_t qb = static_cast<size_t>(nq) * a->d * 4;
     CKS(a->q_f32.ensure(qb));
-    const void* src = q;
-    if (!out_dev && qb <= (size_t(64) << 20)) {
-      CKS(a->h_q.ensure(qb));
-      memcpy(a->h_q.p, q, qb);
-      src = a->h_q.p;
-    }
-    CK(cudaMemcpyAsync(a->q_f32.p, src, qb, cudaMemcpyHostToDevice, st));
-    qd = a->q_f32.as<float>();
-  }
-  float* Dd[2] = {nullptr, nullptr};
-  long long* Id[2] = {nullptr, nullptr};
-  for (int i = 0; i < n_db; ++i) {
-    if (out_dev) {
-      Dd[i] = D[i];
-      Id[i] = reinterpret_cast<long long*>(I[i]);
+    c.q = a->q_f32.as<float>();
+    if (io == IO_MAPPED) {
+      c.q_src = static_cast<const float*>(lq.mapped);
     } else {
-      CKS(a->D_stage[i].ensure(static_cast<size_t>(nq) * k * 4));
-      CKS(a->I_stage[i].ensure(static_cast<size_t>(nq) * k * 8));
-      Dd[i] = a->D_stage[i].as<float>();
-      Id[i] = a->I_stage[i].as<long long>();
+      const void* src = q;
+      if (!out_dev && qb <= (size_t(64) << 20)) {
+        CKS(a->h_q.ensure(qb));
+        memcpy(a->h_q.p, q, qb);
+        src = a->h_q.p;
+      }
+      CK(cudaMemcpyAsync(a->q_f32.p, src, qb, cudaMemcpyHostToDevice, st));
     }
+  }
+  float* D[2] = {c.D[0], c.D[1]};
+  long long* I[2] = {c.I[0], c.I[1]};
+  for (int i = 0; i < n_db && !out_dev; ++i) {
+    CKS(a->D_stage[i].ensure(static_cast<size_t>(nq) * k * 4));
+    CKS(a->I_stage[i].ensure(static_cast<size_t>(nq) * k * 8));
+    c.D[i] = a->D_stage[i].as<float>();
+    c.I[i] = a->I_stage[i].as<long long>();
   }
   // status blocks of every pass, sized before the first launch (growing them later would free
   // memory that kernels of an earlier pass still write)
   const int n_passes = static_cast<int>((nq + Q_PASS_MAX - 1) / Q_PASS_MAX);
   CKS(a->ctrl.ensure(static_cast<size_t>(n_passes) * CTRL_STRIDE * 4));
-  // empty databases answer with padding only
-  if (any_empty) {
-    if (cons) return fail(KEDS_ERR_ARG, "retrieve2: both databases must hold rows");
-    // no kernel of a chain may run on this handle: its status blocks read as clean
+  if (ix[0]->n == 0 || (n_db > 1 && ix[1]->n == 0)) {
+    // empty databases answer with padding only; a non-empty one is searched alone, still with the
+    // owner's scratch, status blocks and switches
+    if (c.cons.enabled) return fail(KEDS_ERR_ARG, "retrieve2: both databases must hold rows");
+    // (with every database empty no chain runs: the status blocks must read clean)
     CK(cudaMemsetAsync(a->ctrl.p, 0, static_cast<size_t>(n_passes) * CTRL_STRIDE * 4, st));
     a->ctrl_passes = n_passes;
+    Call rest = c;
+    rest.n_db = 0;
     for (int i = 0; i < n_db; ++i) {
       if (ix[i]->n != 0) {
-        keds_index* one[2] = {ix[i], nullptr};
-        float* D1[2] = {Dd[i], nullptr};
-        long long* I1[2] = {Id[i], nullptr};
-        for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
-          const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
-          float* Dp[2] = {D1[0] + q0 * k, nullptr};
-          long long* Ip[2] = {I1[0] + q0 * k, nullptr};
-          // (stream order keeps the passes apart: every kernel of a chain waits for its predecessor)
-          CKS(one[0]->ctrl.ensure(static_cast<size_t>(n_passes) * CTRL_STRIDE * 4));
-          CKS(search_pass(one, 1, qd + q0 * a->d, nb, k, Dp, Ip, flags, st, nullptr, 0, nullptr, nullptr,
-                          static_cast<int>(q0 / Q_PASS_MAX), nullptr, nullptr, ex_dev ? ex_dev + q0 * n_ex : nullptr,
-                          n_ex));
-        }
+        rest.n_db = 1;
+        rest.slot0 = i;
+        rest.dbs[0] = ix[i];
+        rest.D[0] = c.D[i];
+        rest.I[0] = c.I[i];
       } else {
         const long long tot = static_cast<long long>(nq) * k;
         k_fill_pad<<<static_cast<unsigned>((tot + 255) / 256), 256, 0, st>>>(
-            Dd[i], Id[i], tot,
-            (a->metric == METRIC_L2 && !(flags & KEDS_SEARCH_FORCE_IP)) ? FLT_MAX : -FLT_MAX);
+            c.D[i], c.I[i], tot, c.metric() == METRIC_L2 ? FLT_MAX : -FLT_MAX);
       }
     }
-  } else {
-    for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
-      const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
-      float* Dp[2] = {Dd[0] + q0 * k, n_db > 1 ? Dd[1] + q0 * k : nullptr};
-      long long* Ip[2] = {Id[0] + q0 * k, n_db > 1 ? Id[1] + q0 * k : nullptr};
-      ConsumeParams cp;
-      if (cons) {
-        cp = *cons;
-        for (int s = 0; s < 2; ++s) {
-          if (cp.feat[s]) cp.feat[s] += q0 * k * a->d;
-          if (cp.pool[s]) cp.pool[s] += q0 * a->d;
-          if (cp.host_D[s]) cp.host_D[s] += q0 * k;
-          if (cp.host_I[s]) cp.host_I[s] += q0 * k;
-        }
-      }
-      PeerOut pp;
-      if (peer) {
-        pp = *peer;
-        for (int r = 0; r < pp.n; ++r) {
-          if (pp.D[r]) pp.D[r] += q0 * k;
-          if (pp.I[r]) pp.I[r] += q0 * k;
-        }
-        pp.publish = q0 + nb >= nq;  // the flags go out behind the step's last pass
-      }
-      // every pass has its own status block and the scratch is reused in stream order (each kernel
-      // of a chain waits for its predecessor to complete), so the passes queue without a host round trip
-      CKS(search_pass(ix, n_db, qd + q0 * a->d, nb, k, Dp, Ip, flags, st, nullptr, 0, cons ? &cp : nullptr,
-                      peer ? &pp : nullptr, static_cast<int>(q0 / Q_PASS_MAX), q_map ? q_map + q0 * a->d : nullptr,
-                      nullptr, ex_dev ? ex_dev + q0 * n_ex : nullptr, n_ex));
-    }
+    c = rest;
   }
+  if (c.n_db) CKS(run_passes(c, st));
   if (!out_dev) {
     // results and status words into pinned memory with asynchronous copies, ONE synchronisation,
     // then plain memcpy into the caller's arrays
@@ -1042,8 +1095,8 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
     if (per * n_db > (size_t(256) << 20)) {
       // very large result blocks: not worth pinning that much host memory, copy straight out
       for (int i = 0; i < n_db; ++i) {
-        CK(cudaMemcpyAsync(D[i], Dd[i], db_, cudaMemcpyDeviceToHost, st));
-        CK(cudaMemcpyAsync(I[i], Id[i], ib_, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(D[i], a->D_stage[i].p, db_, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(I[i], a->I_stage[i].p, ib_, cudaMemcpyDeviceToHost, st));
       }
       return finish_sync(a, st);
     }
@@ -1051,24 +1104,18 @@ int search_impl(keds_index* ix[2], int n_db, const float* q, int64_t nq, int k, 
     CKS(a->h_out.ensure(per * n_db + ctrl_bytes));
     uint8_t* h = static_cast<uint8_t*>(a->h_out.p);
     for (int i = 0; i < n_db; ++i) {
-      CK(cudaMemcpyAsync(h + per * i, Id[i], ib_, cudaMemcpyDeviceToHost, st));
-      CK(cudaMemcpyAsync(h + per * i + ib_, Dd[i], db_, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(h + per * i, a->I_stage[i].p, ib_, cudaMemcpyDeviceToHost, st));
+      CK(cudaMemcpyAsync(h + per * i + ib_, a->D_stage[i].p, db_, cudaMemcpyDeviceToHost, st));
     }
     uint32_t* hall = reinterpret_cast<uint32_t*>(h + per * n_db);
     memset(hall, 0, ctrl_bytes);
     if (a->ctrl.p) CK(cudaMemcpyAsync(hall, a->ctrl.p, ctrl_bytes, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    uint32_t hc[CTRL_WORDS];
-    read_status(a, hall, hc);
     for (int i = 0; i < n_db; ++i) {
       memcpy(I[i], h + per * i, ib_);
       memcpy(D[i], h + per * i + ib_, db_);
     }
-    a->stats.n_flagged[0] = static_cast<int32_t>(hc[0]);
-    a->stats.n_flagged[1] = static_cast<int32_t>(hc[1]);
-    a->stats.err_word = hc[2];
-    if (hc[2] != 0) return fail(KEDS_ERR_KERNEL, "device watchdog fired (scoring pipeline or fallback barrier): error word 0x%x", hc[2]);
-    return 0;
+    return fold_status(a, hall);
   }
   return 0;
 }
@@ -1319,76 +1366,66 @@ int keds_index_search(keds_index_t* ix, const float* q, int64_t nq, int k, float
 
 int keds_index_search_ex(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
                          uint32_t flags, void* stream) {
-  keds_index* v[2] = {ix, nullptr};
-  float* Dv[2] = {D, nullptr};
-  int64_t* Iv[2] = {I, nullptr};
-  return search_impl(v, 1, q, nq, k, Dv, Iv, flags, stream);
+  Call c = call(1, ix, nullptr, q, nq, k, D, I, nullptr, nullptr, flags);
+  return search_impl(c, IO_HOST, stream);
 }
 
 int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
                        int64_t* Ia, float* Db, int64_t* Ib, uint32_t flags, void* stream) {
-  keds_index* v[2] = {a, b};
-  float* Dv[2] = {Da, Db};
-  int64_t* Iv[2] = {Ia, Ib};
-  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream);
+  Call c = call(2, a, b, q, nq, k, Da, Ia, Db, Ib, flags);
+  return search_impl(c, IO_HOST, stream);
 }
 
 int keds_index_search_exclude(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
                               const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
-  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
-    return fail(KEDS_ERR_ARG, "search_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
-  keds_index* v[2] = {ix, nullptr};
-  float* Dv[2] = {D, nullptr};
-  int64_t* Iv[2] = {I, nullptr};
-  return search_impl(v, 1, q, nq, k, Dv, Iv, flags, stream, nullptr, nullptr, false, exclude, n_exclude);
+  Call c = call(1, ix, nullptr, q, nq, k, D, I, nullptr, nullptr, flags);
+  CKS(c.exclude(exclude, n_exclude));
+  return search_impl(c, IO_HOST, stream);
 }
 
 int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
                                int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude, int n_exclude,
                                uint32_t flags, void* stream) {
-  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
-    return fail(KEDS_ERR_ARG, "search2_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
-  keds_index* v[2] = {a, b};
-  float* Dv[2] = {Da, Db};
-  int64_t* Iv[2] = {Ia, Ib};
-  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream, nullptr, nullptr, false, exclude, n_exclude);
+  Call c = call(2, a, b, q, nq, k, Da, Ia, Db, Ib, flags);
+  CKS(c.exclude(exclude, n_exclude));
+  return search_impl(c, IO_HOST, stream);
 }
 
 }  // extern "C"
 
 namespace {
 
-int retrieve2_impl(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                   const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                   float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
-                   float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags, void* stream,
-                   bool hostio, float* Dh_img, int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt,
-                   const int64_t* exclude = nullptr, int n_exclude = 0) {
-  if (!img || !txt || !q || !D_img || !I_img || !D_txt || !I_txt)
+// The fused consumer on top of a two-database call (c: both handles, q, the device results and
+// the exclusion); hostio: q may be page-locked host memory and the results get host mirrors.
+int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                   float* feat_img, float* feat_txt, float* pool_img, float* pool_txt, float* Dh_img, int64_t* Ih_img,
+                   float* Dh_txt, int64_t* Ih_txt, void* stream) {
+  keds_index* img = c.dbs[0];
+  if (!img || !c.dbs[1] || !c.q || !c.D[0] || !c.I[0] || !c.D[1] || !c.I[1])
     return fail(KEDS_ERR_ARG, "retrieve2: null handle, query or result pointer");
   if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "retrieve2: pool_mode must be 0, 1 or 2");
-  if ((!hostio && !is_device_ptr(q)) || !is_device_ptr(D_img) || !is_device_ptr(I_img) || !is_device_ptr(D_txt) ||
-      !is_device_ptr(I_txt))
+  if ((!hostio && !locate(c.q)) || !locate(c.D[0]) || !locate(c.I[0]) || !locate(c.D[1]) || !locate(c.I[1]))
     return fail(KEDS_ERR_ARG, "retrieve2: device pointers only");
   if ((Dh_img == nullptr) != (Ih_img == nullptr) || (Dh_txt == nullptr) != (Ih_txt == nullptr))
     return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host mirror needs both its D and its I block");
-  if (k > 1024) return fail(KEDS_ERR_ARG, "retrieve2: k=%d too large for the fused consumer", k);
-  keds_index* v[2] = {img, txt};
-  float* Dv[2] = {D_img, D_txt};
-  int64_t* Iv[2] = {I_img, I_txt};
+  if (c.k > 1024) return fail(KEDS_ERR_ARG, "retrieve2: k=%d too large for the fused consumer", c.k);
   const bool want_pool = pool_mode != 0 && (pool_img || pool_txt);
   ConsumeParams cp;
   memset(&cp, 0, sizeof cp);
   {
     DeviceGuard g(img->device);
     if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", img->device);
-    long long* ih[2] = {nullptr, nullptr};
-    CKS(mapped_alias(Dh_img, &cp.host_D[0]));
-    CKS(mapped_alias(reinterpret_cast<long long*>(Ih_img), &ih[0]));
-    CKS(mapped_alias(Dh_txt, &cp.host_D[1]));
-    CKS(mapped_alias(reinterpret_cast<long long*>(Ih_txt), &ih[1]));
-    cp.host_I[0] = ih[0];
-    cp.host_I[1] = ih[1];
+    // the host mirrors: written through their device aliases
+    void* mirror[4] = {Dh_img, Ih_img, Dh_txt, Ih_txt};
+    for (void*& m : mirror) {
+      if (!m) continue;
+      m = locate(m).mapped;
+      if (!m) return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host result pointer is not page-locked (cudaHostAlloc / pin_memory)");
+    }
+    cp.host_D[0] = static_cast<float*>(mirror[0]);
+    cp.host_I[0] = static_cast<long long*>(mirror[1]);
+    cp.host_D[1] = static_cast<float*>(mirror[2]);
+    cp.host_I[1] = static_cast<long long*>(mirror[3]);
   }
   cp.enabled = (feat_img || feat_txt || want_pool || Dh_img || Dh_txt) ? 1 : 0;
   cp.mode = want_pool ? pool_mode : 0;
@@ -1402,8 +1439,8 @@ int retrieve2_impl(keds_index_t* img, keds_index_t* txt, const float* q, int64_t
   // one warp per neighbour row; per-warp partial pools meet in shared memory ([warps][d/4] float4)
   static_assert(RERANK_THREADS == EXACT_THREADS, "the consumer scratch is sized for one block shape");
   cp.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
-  return search_impl(v, 2, q, nq, k, Dv, Iv, flags, stream, cp.enabled ? &cp : nullptr, nullptr, hostio, exclude,
-                     n_exclude);
+  if (cp.enabled) c.cons = cp;
+  return search_impl(c, hostio ? IO_MAPPED : IO_DEVICE, stream);
 }
 
 }  // namespace
@@ -1414,8 +1451,9 @@ int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t
                    const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
                    float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
                    float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags, void* stream) {
-  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
-                        feat_txt, pool_img, pool_txt, flags, stream, false, nullptr, nullptr, nullptr, nullptr);
+  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
+  return retrieve2_impl(c, false, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, nullptr,
+                        nullptr, nullptr, nullptr, stream);
 }
 
 int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
@@ -1423,8 +1461,9 @@ int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, 
                           float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
                           int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
                           float* pool_img, float* pool_txt, uint32_t flags, void* stream) {
-  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
-                        feat_txt, pool_img, pool_txt, flags, stream, true, Dh_img, Ih_img, Dh_txt, Ih_txt);
+  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
+  return retrieve2_impl(c, true, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, Dh_img,
+                        Ih_img, Dh_txt, Ih_txt, stream);
 }
 
 int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
@@ -1432,11 +1471,10 @@ int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q,
                            float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
                            float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
                            uint32_t flags, void* stream) {
-  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
-    return fail(KEDS_ERR_ARG, "retrieve2_exclude: exclude must be non-null and 1 <= n_exclude <= %d", EXCLUDE_MAX);
-  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
-                        feat_txt, pool_img, pool_txt, flags, stream, false, nullptr, nullptr, nullptr, nullptr, exclude,
-                        n_exclude);
+  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
+  CKS(c.exclude(exclude, n_exclude));
+  return retrieve2_impl(c, false, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, nullptr,
+                        nullptr, nullptr, nullptr, stream);
 }
 
 int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
@@ -1445,12 +1483,10 @@ int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const fl
                                   int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
                                   float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
                                   uint32_t flags, void* stream) {
-  if (!exclude || n_exclude < 1 || n_exclude > EXCLUDE_MAX)
-    return fail(KEDS_ERR_ARG, "retrieve2_hostio_exclude: exclude must be non-null and 1 <= n_exclude <= %d",
-                EXCLUDE_MAX);
-  return retrieve2_impl(img, txt, q, nq, k, perm_img, perm_txt, pool_mode, tau, D_img, I_img, D_txt, I_txt, feat_img,
-                        feat_txt, pool_img, pool_txt, flags, stream, true, Dh_img, Ih_img, Dh_txt, Ih_txt, exclude,
-                        n_exclude);
+  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
+  CKS(c.exclude(exclude, n_exclude));
+  return retrieve2_impl(c, true, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, Dh_img,
+                        Ih_img, Dh_txt, Ih_txt, stream);
 }
 
 int keds_index_sync(keds_index_t* ix, void* stream) {
@@ -1563,15 +1599,15 @@ int keds_index_last_stats(const keds_index_t* ix, keds_search_stats* out) {
 
 int keds_debug_scores(keds_index_t* ix, const float* q, int64_t nq, float* out, void* stream) {
   if (!ix || !q || !out || nq <= 0 || nq > Q_PASS_MAX) return fail(KEDS_ERR_ARG, "debug_scores: bad argument");
-  if (!is_device_ptr(q) || !is_device_ptr(out)) return fail(KEDS_ERR_ARG, "debug_scores: device pointers only");
+  if (!locate(q) || !locate(out)) return fail(KEDS_ERR_ARG, "debug_scores: device pointers only");
   if (ix->n == 0) return fail(KEDS_ERR_ARG, "debug_scores: empty index");
   DeviceGuard g(ix->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   memset(&ix->stats, 0, sizeof ix->stats);
-  keds_index* v[2] = {ix, nullptr};
-  float* Dv[2] = {nullptr, nullptr};
-  long long* Iv[2] = {nullptr, nullptr};
-  CKS(search_pass(v, 1, q, nq, 1, Dv, Iv, 0u, st, out, ix->n, nullptr));
+  Call c = call(1, ix, nullptr, q, nq, 1, nullptr, nullptr, nullptr, nullptr, 0u);
+  c.dump = out;
+  c.ld_dump = ix->n;
+  CKS(search_pass(c, st));
   return finish_sync(ix, st);
 }
 
@@ -1597,8 +1633,8 @@ int keds_gather_pool(const float* base, int64_t n_base, const int64_t* I, const 
   if (!base || !I || !out || B < 0 || k <= 0 || d <= 0 || n_base < 0)
     return fail(KEDS_ERR_ARG, "gather_pool: bad argument");
   if (B == 0) return 0;
-  const int dev = device_of(out);
-  if (dev < 0 || device_of(base) != dev) return fail(KEDS_ERR_ARG, "gather_pool: base and out must be memory of one device");
+  const int dev = locate(out).device;
+  if (dev < 0 || locate(base).device != dev) return fail(KEDS_ERR_ARG, "gather_pool: base and out must be memory of one device");
   DeviceGuard g(dev);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (!W) {
@@ -1630,7 +1666,7 @@ static int merge_impl(const float* Dp, const int64_t* Ip, int64_t stride_d, int6
   const size_t tot = static_cast<size_t>(parts) * k;
   const size_t smem = tot * 8 + tot * 4;  // labels, rank scores
   if (smem > 200 * 1024) return fail(KEDS_ERR_ARG, "topk_merge: parts*k too large");
-  const int dev = device_of(D);
+  const int dev = locate(D).device;
   if (dev < 0) return fail(KEDS_ERR_ARG, "topk_merge: device pointers only");
   DeviceGuard g(dev);
   // the attribute is per device; IndexShards / IndexReplicas search from one host thread per GPU
@@ -1675,7 +1711,7 @@ int keds_p2p_push(const void* src, int64_t bytes, void* const* peer_dst, uint32_
     if (r != my_rank && (!p.dst[r] || !p.flag[r])) return fail(KEDS_ERR_ARG, "p2p_push: null peer pointer");
   }
   p.ticket = ticket;
-  const int dev = device_of(src);
+  const int dev = locate(src).device;
   if (dev < 0) return fail(KEDS_ERR_ARG, "p2p_push: src must be device memory");
   DeviceGuard g(dev);
   const unsigned blocks = static_cast<unsigned>(std::min<long long>(64, (p.n16 + 255) / 256));
@@ -1762,8 +1798,7 @@ int keds_index_search_sharded(keds_index_t* ix, keds_exchange_t* ex, const float
   if (!ix || !ex || !q || !D || !I || nq <= 0 || k <= 0)
     return fail(KEDS_ERR_ARG, "search_sharded: null handle / pointer or bad nq / k");
   if (ex->device != ix->device) return fail(KEDS_ERR_ARG, "search_sharded: exchange and index live on different devices");
-  if (!is_device_ptr(q) || !is_device_ptr(D) || !is_device_ptr(I))
-    return fail(KEDS_ERR_ARG, "search_sharded: device pointers only");
+  if (!locate(q) || !locate(D) || !locate(I)) return fail(KEDS_ERR_ARG, "search_sharded: device pointers only");
   if (nq * k > ex->i_off / 4)
     return fail(KEDS_ERR_ARG, "search_sharded: nq*k = %lld exceeds the exchange capacity %lld", (long long)(nq * k),
                 (long long)(ex->i_off / 4));
@@ -1806,10 +1841,9 @@ int keds_index_search_sharded(keds_index_t* ix, keds_exchange_t* ex, const float
       CKS(keds_p2p_push(mine, ex->slot_bytes, dst, flg, R, me, epoch, po.ticket, stream));
     }
   } else {
-    keds_index* v[2] = {ix, nullptr};
-    float* Dv[2] = {Dl, nullptr};
-    int64_t* Iv[2] = {Il, nullptr};
-    CKS(search_impl(v, 1, q, nq, k, Dv, Iv, 0u, stream, nullptr, R > 1 ? &po : nullptr));
+    Call c = call(1, ix, nullptr, q, nq, k, Dl, Il, nullptr, nullptr, 0u);
+    if (R > 1) c.peer = po;
+    CKS(search_impl(c, IO_DEVICE, stream));
   }
   MergeWait mw;
   memset(&mw, 0, sizeof mw);
@@ -1853,7 +1887,7 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
   if (!ix || !q || !target || !rank_out || nq < 0) return fail(KEDS_ERR_ARG, "index_rank: null argument or bad nq");
   if (nq == 0) return 0;
   if (ix->n == 0) return fail(KEDS_ERR_ARG, "index_rank: empty index");
-  if (!is_device_ptr(q) || !is_device_ptr(target) || !is_device_ptr(rank_out) || (exclude && !is_device_ptr(exclude)))
+  if (!locate(q) || !locate(target) || !locate(rank_out) || (exclude && !locate(exclude)))
     return fail(KEDS_ERR_ARG, "index_rank: device pointers only");
   DeviceGuard g(ix->device);
   if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
@@ -1877,27 +1911,18 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
   for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
     const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
     const float* qp = q + q0 * d;
-    const int n_qt = static_cast<int>((nb + BM - 1) / BM);
-    const bool pair = ix->use_pair && n_qt >= 2 && ix->num_sms >= 2;
-    const int sub = pair ? ScoreCfg<true>::kSub : ScoreCfg<false>::kSub;
-    const int n_qg = pair ? (n_qt + 1) / 2 : n_qt;
-    const int units = pair ? ix->num_sms / 2 : ix->num_sms;
+    Plan pl{geometry(ix, 1, nb)};
     // as many candidate lists as the tiles allow: the band around a mid-ranked target is crowded
-    const long long by_mem = static_cast<long long>(CAND_BUDGET / (size_t(LKEEP) * BM * 8)) / (static_cast<long long>(n_qt) * sub);
-    const int S = static_cast<int>(std::max<long long>(1, std::min<long long>(std::min(T, S_MAX), by_mem)));
-    const int n_items = n_qg * S;
-    const int grid = std::min(n_items, units) * (pair ? 2 : 1);
-    const int n_lists = S * sub;
+    pl.set_slices(1, static_cast<int>(std::max<long long>(1, std::min<long long>(std::min(T, S_MAX), pl.s_mem))));
+    const int n_lists = pl.S * pl.sub;
     CKS(ix->ctrl.ensure(CTRL_STRIDE * 4));  // (finish_sync reads whole status blocks)
     ix->ctrl_passes = 1;
+    ix->ctrl_slot = 0;
     CKS(ix->flagged[0].ensure(static_cast<size_t>(nb) * 4));
-    CKS(ensure_q_map(ix, static_cast<int64_t>(n_qt) * BM, st));
+    CKS(ensure_q_map(ix, static_cast<int64_t>(pl.n_qt) * BM, st));
     CKS(ix->qstat.ensure(static_cast<size_t>(nb) * sizeof(float4)));
     CKS(ix->rk.ensure(static_cast<size_t>(nb) * 5 * 4));
-    const size_t lines = static_cast<size_t>(n_lists) * n_qt;
-    CKS(ix->cand.ensure(lines * LKEEP * BM * 8));
-    CKS(ix->cand_cnt.ensure(lines * BM * 4));
-    CKS(ix->cand_theta.ensure(lines * BM * 4));
+    CKS(ensure_cand(ix, static_cast<size_t>(n_lists) * pl.n_qt));
     float* rk_st = ix->rk.as<float>();
     float* rk_lo = rk_st + nb;
     float* rk_hi = rk_lo + nb;
@@ -1915,34 +1940,14 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
     CKS(launch_k(ix->use_pdl, k_rank_targets, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,
                  tg + q0, ex ? ex + q0 : nullptr, ix->qstat.as<float4>(), ix->dbstat.as<unsigned int>(), ix->eps_scale,
                  rk_st, rk_lo, rk_hi, rk_t, rk_e));
-    ScoreParams sp;
-    memset(&sp, 0, sizeof sp);
-    sp.n_db = 1;
-    sp.n_qt = n_qt;
-    sp.n_qg = n_qg;
-    sp.S = S;
-    sp.n_items = n_items;
-    sp.kblocks = ix->d_pad / BK;
-    sp.fmt_bits = ix->fmt == FMT_BF16 ? kIdescBf16Bits : 0u;
-    sp.nq = static_cast<int>(nb);
-    sp.n_rows[0] = static_cast<int>(ix->n);
-    sp.n_tiles[0] = T;
-    sp.cand = ix->cand.as<uint2>();
-    sp.cand_cnt = ix->cand_cnt.as<int>();
-    sp.cand_theta = ix->cand_theta.as<float>();
-    sp.err = ix->ctrl.as<uint32_t>() + 2;
+    ScoreParams sp = score_params(ix, &ix, 1, pl, nb, ix->ctrl.as<unsigned int>() + 2);
     sp.rk_lo = rk_lo;
     sp.rk_hi = rk_hi;
     sp.rk_target = rk_t;
     sp.rk_exclude = ex ? rk_e : nullptr;
-    if (pair)
-      CKS(launch_kc(ix->use_pdl, 2, k_score_topk<true, true>, dim3(grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES,
-                    st, ix->tm_q, ix->tm_xh, ix->tm_xh, sp));
-    else
-      CKS(launch_k(ix->use_pdl, k_score_topk<false, true>, dim3(grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st,
-                   ix->tm_q, ix->tm_x, ix->tm_x, sp));
+    CKS(launch_score(ix, &ix, 1, pl, sp, st));
     CKS(launch_k(ix->use_pdl, k_rank_finish, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,
-                 n_lists, n_qt, static_cast<const uint2*>(sp.cand), static_cast<const int*>(sp.cand_cnt),
+                 n_lists, pl.n_qt, static_cast<const uint2*>(sp.cand), static_cast<const int*>(sp.cand_cnt),
                  static_cast<const float*>(sp.cand_theta), static_cast<const float*>(rk_st),
                  static_cast<const int*>(rk_t), out + q0, ix->flagged[0].as<int>(), ix->ctrl.as<int>()));
     // exact recount of the queries whose band overflowed a list (none, normally: the blocks leave at once)
@@ -1950,9 +1955,9 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
                  static_cast<long long>(nb), G, static_cast<long long>(ix->n), d, tg + q0, ex ? ex + q0 : nullptr,
                  out + q0, static_cast<const int*>(ix->flagged[0].as<int>()), static_cast<const int*>(ix->ctrl.as<int>())));
     ix->stats.launches = 5;
-    ix->stats.slices = S;
-    ix->stats.items = n_items;
-    ix->stats.grid = grid;
+    ix->stats.slices = pl.S;
+    ix->stats.items = pl.n_items;
+    ix->stats.grid = pl.grid;
     if (q0 + nb < nq) CKS(finish_sync(ix, st));  // the scratch is reused by the next pass
   }
   CK(cudaGetLastError());
@@ -1969,7 +1974,7 @@ int keds_index_label_hits(keds_index_t* ix, const float* q, int64_t nq, const in
   if (nq == 0) return 0;
   if (ix->n == 0) return fail(KEDS_ERR_ARG, "index_label_hits: empty index");
   if (ix->n > 0x7fffffffll - BN) return fail(KEDS_ERR_ARG, "index too large for 32-bit row ids");
-  if (!is_device_ptr(q) || !is_device_ptr(row_labels) || !is_device_ptr(qlabel) || !is_device_ptr(hits))
+  if (!locate(q) || !locate(row_labels) || !locate(qlabel) || !locate(hits))
     return fail(KEDS_ERR_ARG, "index_label_hits: device pointers only");
   DeviceGuard g(ix->device);
   if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
@@ -1982,20 +1987,14 @@ int keds_index_label_hits(keds_index_t* ix, const float* q, int64_t nq, const in
   const int64_t nb_max = std::min<int64_t>(nq, Q_PASS_MAX);
   CKS(ix->D_stage[0].ensure(static_cast<size_t>(nb_max) * kmax * 4));
   CKS(ix->I_stage[0].ensure(static_cast<size_t>(nb_max) * kmax * 8));
-  keds_index* v[2] = {ix, nullptr};
-  for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
-    const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
-    HitsMode hm;
-    hm.nks = nks;
-    for (int j = 0; j < nks; ++j) hm.ks[j] = ks[j];
-    hm.row_labels = reinterpret_cast<const long long*>(row_labels);
-    hm.qlabel = reinterpret_cast<const long long*>(qlabel) + q0;
-    hm.hits = hits + q0 * nks;
-    float* Dp[2] = {ix->D_stage[0].as<float>(), nullptr};
-    long long* Ip[2] = {ix->I_stage[0].as<long long>(), nullptr};
-    CKS(search_pass(v, 1, q + q0 * ix->d, nb, kmax, Dp, Ip, 0u, st, nullptr, 0, nullptr, nullptr,
-                    static_cast<int>(q0 / Q_PASS_MAX), nullptr, &hm));
-  }
+  Call c = call(1, ix, nullptr, q, nq, kmax, ix->D_stage[0].as<float>(), ix->I_stage[0].as<int64_t>(), nullptr,
+                nullptr, 0u);
+  c.hits.nks = nks;
+  for (int j = 0; j < nks; ++j) c.hits.ks[j] = ks[j];
+  c.hits.row_labels = reinterpret_cast<const long long*>(row_labels);
+  c.hits.qlabel = reinterpret_cast<const long long*>(qlabel);
+  c.hits.hits = hits;
+  CKS(run_passes(c, st));
   CK(cudaGetLastError());
   return 0;
 }
@@ -2007,8 +2006,8 @@ int keds_gallery_rank(const float* Q, int64_t nq, const float* G, int64_t ng, in
   if (nq == 0) return 0;
   const size_t smem = static_cast<size_t>((d + 3) & ~3) * 4 * 8;  // 8 queries per block
   if (smem > 48 * 1024) return fail(KEDS_ERR_ARG, "gallery_rank: d too large");
-  const int dev = device_of(rank_out);
-  if (dev < 0 || device_of(Q) != dev || device_of(G) != dev)
+  const int dev = locate(rank_out).device;
+  if (dev < 0 || locate(Q).device != dev || locate(G).device != dev)
     return fail(KEDS_ERR_ARG, "gallery_rank: Q, G and rank_out must be memory of one device");
   DeviceGuard g(dev);
   if (ng >= 1024 && nq >= 64) {
@@ -2034,8 +2033,8 @@ int keds_label_hits(const int64_t* I, int64_t nq, int kmax, const int64_t* label
   if (!I || !labels || !qlabel || !ks || !hits || nq < 0 || kmax <= 0 || nks <= 0)
     return fail(KEDS_ERR_ARG, "label_hits: bad argument");
   if (nq == 0) return 0;
-  const int dev = device_of(hits);
-  if (dev < 0 || device_of(I) != dev) return fail(KEDS_ERR_ARG, "label_hits: I and hits must be memory of one device");
+  const int dev = locate(hits).device;
+  if (dev < 0 || locate(I).device != dev) return fail(KEDS_ERR_ARG, "label_hits: I and hits must be memory of one device");
   DeviceGuard g(dev);
   k_label_hits<<<static_cast<unsigned>((nq + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
       reinterpret_cast<const long long*>(I), nq, kmax, reinterpret_cast<const long long*>(labels),

@@ -81,7 +81,7 @@ int keds_clip_loss_forward_backward(keds_clip_loss_t* h, const float* I_all, con
   if (want_grad && (!dI_local || !dT_local || n_local == 0))
     return fail(KEDS_ERR_ARG, "clip_loss: pass both gradient buffers (and local rows) or neither");
   for (const void* p : {(const void*)I_all, (const void*)T_all, (const void*)loss, (const void*)scale})
-    if (!is_device_ptr(p)) return fail(KEDS_ERR_ARG, "clip_loss: all buffers must be device memory");
+    if (!locate(p)) return fail(KEDS_ERR_ARG, "clip_loss: all buffers must be device memory");
   DeviceGuard g(h->device);
   if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", h->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);

@@ -412,7 +412,7 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_
     return fail(KEDS_ERR_ARG, "consumer_forward_train: heads * (dim_head + k) too large for the attention backward");
   for (const void* ptr : {(const void*)q, (const void*)base_img, (const void*)base_txt, (const void*)I_img,
                           (const void*)I_txt, (const void*)tokens})
-    if (!is_device_ptr(ptr)) return fail(KEDS_ERR_ARG, "consumer_forward: all buffers must be device memory");
+    if (!locate(ptr)) return fail(KEDS_ERR_ARG, "consumer_forward: all buffers must be device memory");
   DeviceGuard g(c->device);
   if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -425,7 +425,7 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_
     for (int i = 0; i < c->n_hidden; ++i) {
       CKS(c->tr.h[i].ensure(static_cast<size_t>(M) * c->d_mid * 4));
       c->tr.masks[i] = masks ? masks[i] : nullptr;
-      if (c->tr.masks[i] && !is_device_ptr(c->tr.masks[i]))
+      if (c->tr.masks[i] && !locate(c->tr.masks[i]))
         return fail(KEDS_ERR_ARG, "consumer_forward_train: dropout masks must be device memory");
     }
     for (int l = 0; l < L; ++l) {
@@ -614,7 +614,7 @@ int keds_consumer_debug_linear(keds_consumer_t* c, int variant, const float* A0,
     if (!A || !W || !C || (reinterpret_cast<uintptr_t>(A) & 15) || (reinterpret_cast<uintptr_t>(W) & 15) ||
         (reinterpret_cast<uintptr_t>(C) & 3))
       return fail(KEDS_ERR_ARG, "consumer_debug_linear: A, W 16-byte and C 4-byte aligned, none NULL");
-    if (!is_device_ptr(A) || !is_device_ptr(W) || !is_device_ptr(C) || (b && !is_device_ptr(b)))
+    if (!locate(A) || !locate(W) || !locate(C) || (b && !locate(b)))
       return fail(KEDS_ERR_ARG, "consumer_debug_linear: all buffers must be device memory");
   }
   DeviceGuard g(c->device);

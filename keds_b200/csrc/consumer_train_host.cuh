@@ -165,7 +165,7 @@ int keds_consumer_param_offset(const keds_consumer_t* c, int kind, int stack, in
 
 int keds_consumer_bind_params(keds_consumer_t* c, float* params) {
   if (!c || !params) return fail(KEDS_ERR_ARG, "consumer_bind_params: NULL argument");
-  if (!is_device_ptr(params) || (reinterpret_cast<uintptr_t>(params) & 15))
+  if (!locate(params) || (reinterpret_cast<uintptr_t>(params) & 15))
     return fail(KEDS_ERR_ARG, "consumer_bind_params: params must be 16-byte aligned device memory");
   if ((c->inner * c->d_tok) & 3) return fail(KEDS_ERR_ARG, "consumer_bind_params: inner * d_tok must be a multiple of 4");
   DeviceGuard g(c->device);
@@ -222,7 +222,7 @@ int keds_consumer_debug_hidden(keds_consumer_t* c, int layer, float* out, int64_
 int keds_consumer_backward(keds_consumer_t* c, const float* dtokens, float* grads, void* stream) {
   if (!c || !dtokens || !grads) return fail(KEDS_ERR_ARG, "consumer_backward: NULL argument");
   if (!c->finalized || !c->tr.valid) return fail(KEDS_ERR_ARG, "consumer_backward: no keds_consumer_forward_train to differentiate");
-  if (!is_device_ptr(dtokens) || !is_device_ptr(grads) || (reinterpret_cast<uintptr_t>(grads) & 15))
+  if (!locate(dtokens) || !locate(grads) || (reinterpret_cast<uintptr_t>(grads) & 15))
     return fail(KEDS_ERR_ARG, "consumer_backward: dtokens / grads must be device memory (grads 16-byte aligned)");
   DeviceGuard g(c->device);
   if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);

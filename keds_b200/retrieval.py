@@ -235,42 +235,21 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
     pt_ptr, _keep2 = perm_ptr(perm_txt)
     ptr = lambda t: 0 if t is None else t.data_ptr()
     ex = None if exclude is None else _exclude_arg(exclude, B, image_index.device, pinned_ok=hostio)
+    mirrors = []
     if hostio:
         ho = host_out or {}
-        hp = []
         for name, dt in (("D_img", torch.float32), ("I_img", torch.int64), ("D_txt", torch.float32), ("I_txt", torch.int64)):
             t = ho.get(name)
             if t is not None and not (t.is_pinned() and t.dtype == dt and t.is_contiguous() and t.numel() == B * k):
                 raise TypeError(f"retrieve2: host_out[{name!r}] must be a pinned contiguous {dt} tensor of {B * k} elements")
-            hp.append(0 if t is None else t.data_ptr())
-        if ex is not None:
-            _capi.check(
-                lib.keds_retrieve2_hostio_exclude(
-                    image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode), float(tau),
-                    Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), hp[0], hp[1], hp[2], hp[3], ptr(fi),
-                    ptr(ft), ptr(pi), ptr(pt), ex.data_ptr(), ex.shape[1], int(flags), _stream_ptr(image_index.device))
-            )
-            return o
-        _capi.check(
-            lib.keds_retrieve2_hostio(image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode),
-                                      float(tau), Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(),
-                                      hp[0], hp[1], hp[2], hp[3], ptr(fi), ptr(ft), ptr(pi), ptr(pt), int(flags),
-                                      _stream_ptr(image_index.device))
-        )
-        return o
+            mirrors.append(ptr(t))
+    args = [image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode), float(tau),
+            Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), *mirrors, ptr(fi), ptr(ft), ptr(pi), ptr(pt)]
     if ex is not None:
-        _capi.check(
-            lib.keds_retrieve2_exclude(image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr,
-                                       int(pool_mode), float(tau), Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(),
-                                       It.data_ptr(), ptr(fi), ptr(ft), ptr(pi), ptr(pt), ex.data_ptr(), ex.shape[1],
-                                       int(flags), _stream_ptr(image_index.device))
-        )
-        return o
-    _capi.check(
-        lib.keds_retrieve2(image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode),
-                           float(tau), Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), ptr(fi),
-                           ptr(ft), ptr(pi), ptr(pt), int(flags), _stream_ptr(image_index.device))
-    )
+        args += [ex.data_ptr(), ex.shape[1]]
+    fn = {(False, False): lib.keds_retrieve2, (True, False): lib.keds_retrieve2_hostio,
+          (False, True): lib.keds_retrieve2_exclude, (True, True): lib.keds_retrieve2_hostio_exclude}[(hostio, ex is not None)]
+    _capi.check(fn(*args, int(flags), _stream_ptr(image_index.device)))
     return o
 
 
