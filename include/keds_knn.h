@@ -241,6 +241,36 @@ int keds_index_search_sharded(keds_index_t* idx, keds_exchange_t* ex, const floa
                               float* D, int64_t* I, void* cuda_stream);
 int keds_exchange_stats(keds_exchange_t* ex, void* cuda_stream, double* wait_us_avg, double* wait_us_max,
                         int64_t* steps, uint32_t* err_word);
+/* search_sharded with exclusion: exclude [nq][n_exclude] global labels (device memory, -1 = none,
+ * 1 <= n_exclude <= 8), the same on every rank; each shard leaves out the ones it holds, so the
+ * merged result equals keds_index_search_exclude on an unsharded index. */
+int keds_index_search_sharded_exclude(keds_index_t* idx, keds_exchange_t* ex, const float* q, int64_t nq, int k,
+                                      float* D, int64_t* I, const int64_t* exclude, int n_exclude,
+                                      void* cuda_stream);
+
+/* Row-sharded retrieval step: keds_retrieve2 over two row-sharded bases that share one exchange.
+ *   index_rows_ipc      cudaIpcMemHandle_t (64 bytes) of the index's fp32 rows; all zero for an
+ *                       empty index. Valid until the next add / reset of the index.
+ *   exchange_attach_rows  every rank's rows of database db (0 image, 1 text): handles[r] from
+ *                       index_rows_ipc on rank r, lo[r] its first global label, n[r] its row count
+ *                       (n = 0: no rows, handle ignored). Peers' rows are mapped (cudaIpc), this
+ *                       rank's own handle must come from index_rows_ipc in this process. Collective
+ *                       in effect: every rank re-attaches after every add on any rank.
+ *   retrieve2_sharded   q [nq][d] identical on every rank; every rank receives the merged
+ *                       D_* / I_* [nq][k] of all queries (bit-identical to keds_retrieve2 on an
+ *                       unsharded index, exclusion included), and feat_* [row_hi-row_lo][k][d] /
+ *                       pool_* [row_hi-row_lo][d] of queries [row_lo, row_hi) only, gathered from the
+ *                       owners' rows over NVLink (pools: the same weights; summation order fixed, so
+ *                       equal for every shard count). Device pointers only; exclude nullable;
+ *                       refuses to run if this rank's rows moved or grew since the attach. */
+int keds_index_rows_ipc(const keds_index_t* idx, void* handle64);
+int keds_exchange_attach_rows(keds_exchange_t* ex, int db, const void* const* handles, const int64_t* lo,
+                              const int64_t* n);
+int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t* ex, const float* q, int64_t nq,
+                           int k, const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                           int64_t row_lo, int64_t row_hi, float* D_img, int64_t* I_img, float* D_txt,
+                           int64_t* I_txt, float* feat_img, float* feat_txt, float* pool_img, float* pool_txt,
+                           const int64_t* exclude, int n_exclude, uint32_t flags, void* cuda_stream);
 
 /* ---- gallery ranking --------------------------------------------------------------------------
  * rank_out[q] = #{ g != target[q], g != exclude[q] : (s(q,g), -g) > (s(q,target), -target) } with

@@ -9,6 +9,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <mutex>
 #include <string>
 #include <vector>
 
@@ -1740,6 +1741,11 @@ struct keds_exchange {
   int64_t buf_bytes = 0, slot_bytes = 0, i_off = 0;
   uint32_t epoch = 0;
   DevBuf words;  // [0] ticket, [1] error word, [2..3] pad, then {sum, max, count} wait statistics (u64)
+  // every rank's fp32 rows per database (keds_exchange_attach_rows): the sharded consumer reads them
+  // in place. opened: a peer mapping this handle owns (cudaIpcCloseMemHandle on re-attach and free).
+  bool attached[2] = {false, false};
+  ShardRowsDb rows[2];
+  bool opened[2][P2P_MAX_RANKS] = {};
 };
 
 namespace {
@@ -1749,6 +1755,111 @@ uint8_t* ex_slot(const keds_exchange* ex, int owner, int parity, int r) {
 }
 uint32_t* ex_flag(const keds_exchange* ex, int owner, int parity, int r) {
   return reinterpret_cast<uint32_t*>(ex->base[owner]) + parity * P2P_MAX_RANKS + r;
+}
+
+// Handles keds_index_rows_ipc gave out in this process, with the rows they name: a process cannot
+// open its own handle, so attach_rows finds its own rank's pointer here.
+struct IpcExport {
+  cudaIpcMemHandle_t h;
+  const float* rows;
+};
+std::mutex g_ipc_mu;
+std::vector<IpcExport> g_ipc;
+
+void ex_detach_rows(keds_exchange* ex, int db) {
+  for (int r = 0; r < P2P_MAX_RANKS; ++r) {
+    if (ex->opened[db][r]) cudaIpcCloseMemHandle(const_cast<float*>(ex->rows[db].base[r]));
+    ex->opened[db][r] = false;
+  }
+  memset(&ex->rows[db], 0, sizeof ex->rows[db]);
+  ex->attached[db] = false;
+}
+
+// Every database of a sharded call must be attached and this rank's rows where they were then.
+int ex_check_rows(const keds_exchange* ex, keds_index* const* dbs, int n_db) {
+  for (int i = 0; i < n_db; ++i) {
+    const ShardRowsDb& rd = ex->rows[i];
+    const int me = ex->my_rank;
+    if (!ex->attached[i])
+      return fail(KEDS_ERR_ARG, "retrieve2_sharded: database %d has no rows attached to the exchange", i);
+    if (rd.n[me] != dbs[i]->n || rd.lo[me] != dbs[i]->id_offset ||
+        (dbs[i]->n > 0 && rd.base[me] != dbs[i]->x_f32.as<float>()))
+      return fail(KEDS_ERR_ARG,
+                  "retrieve2_sharded: the rows of database %d changed since keds_exchange_attach_rows "
+                  "(re-attach on every rank after each add)", i);
+  }
+  return 0;
+}
+
+// The local search of a row-sharded call (c: this rank's handles, the queries, flags and exclusion)
+// with every finished result row pushed to the peers, then one merge per database into D[i] / I[i].
+// Database i's [nq][k] blocks sit at i * nq * k in the D and I halves of the exchange slot.
+int sharded_search(Call c, keds_exchange* ex, float* const* D, int64_t* const* I, void* stream) {
+  const int64_t nq = c.nq, blk = c.nq * c.k;
+  if (c.n_db * blk > ex->i_off / 4)
+    return fail(KEDS_ERR_ARG, "sharded: %d x nq*k = %lld exceeds the exchange capacity %lld", c.n_db,
+                (long long)(c.n_db * blk), (long long)(ex->i_off / 4));
+  if (c.flags & KEDS_SEARCH_NO_FALLBACK)
+    return fail(KEDS_ERR_ARG, "sharded: KEDS_SEARCH_NO_FALLBACK is not supported (the fallback publishes the step)");
+  keds_index* ix = c.owner;
+  DeviceGuard g(ix->device);
+  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const uint32_t epoch = ++ex->epoch;
+  const int parity = static_cast<int>(epoch & 1u);
+  const int me = ex->my_rank, R = ex->n_ranks;
+  // this rank's blocks land in slot `me` of every rank's buffer (its own included: the merge reads them there)
+  uint8_t* mine = ex_slot(ex, me, parity, me);
+  for (int i = 0; i < c.n_db; ++i) {
+    c.D[i] = reinterpret_cast<float*>(mine) + i * blk;
+    c.I[i] = reinterpret_cast<long long*>(mine + ex->i_off) + i * blk;
+  }
+  PeerOut po;
+  memset(&po, 0, sizeof po);
+  po.n = R;
+  po.my_rank = me;
+  po.publish = 1;
+  po.epoch = epoch;
+  po.ticket = ex->words.as<unsigned int>();
+  po.db_stride = blk;
+  for (int r = 0; r < R; ++r) {
+    uint8_t* there = ex_slot(ex, r, parity, me);
+    po.D[r] = reinterpret_cast<float*>(there);
+    po.I[r] = reinterpret_cast<long long*>(there + ex->i_off);
+    po.flag[r] = ex_flag(ex, r, parity, me);
+  }
+  bool empty = false;
+  for (int i = 0; i < c.n_db; ++i) empty = empty || c.dbs[i]->n == 0;
+  if (!empty && R > 1) c.peer = po;
+  CKS(search_impl(c, IO_DEVICE, stream));
+  if (empty && R > 1) {
+    // an empty shard database runs no search chain to carry its padding (search_impl has filled it):
+    // the whole slot goes out with the stand-alone push, which publishes
+    void* dst[P2P_MAX_RANKS];
+    uint32_t* flg[P2P_MAX_RANKS];
+    for (int r = 0; r < R; ++r) {
+      dst[r] = ex_slot(ex, r, parity, me);
+      flg[r] = ex_flag(ex, r, parity, me);
+    }
+    CKS(keds_p2p_push(mine, ex->slot_bytes, dst, flg, R, me, epoch, po.ticket, stream));
+  }
+  uint8_t* parts = ex_slot(ex, me, parity, 0);
+  for (int i = 0; i < c.n_db; ++i) {
+    MergeWait mw;
+    memset(&mw, 0, sizeof mw);
+    if (R > 1) {
+      // both merges wait on the step's one set of flags; the first one reports the wait
+      mw.flags = ex_flag(ex, me, parity, 0);
+      mw.my_rank = me;
+      mw.epoch = epoch;
+      mw.err_word = ex->words.as<unsigned int>() + 1;
+      if (i == 0) mw.stats = reinterpret_cast<unsigned long long*>(ex->words.as<uint8_t>() + 16);
+    }
+    CKS(merge_impl(reinterpret_cast<const float*>(parts) + i * blk,
+                   reinterpret_cast<const int64_t*>(parts + ex->i_off) + i * blk, ex->slot_bytes / 4,
+                   ex->slot_bytes / 8, R, nq, c.k, c.metric(), D[i], I[i], mw, stream));
+  }
+  return 0;
 }
 }  // namespace
 
@@ -1773,6 +1884,7 @@ int keds_exchange_create(int n_ranks, int my_rank, int device, void* const* peer
   ex->buf_bytes = buf_bytes;
   ex->slot_bytes = slot;
   ex->i_off = slot / 3;
+  memset(ex->rows, 0, sizeof ex->rows);
   int s = ex->words.ensure(64);
   if (s == 0 && cudaMemset(ex->words.p, 0, 64) != cudaSuccess) s = fail(KEDS_ERR_CUDA, "memset failed");
   if (s != 0) {
@@ -1787,76 +1899,152 @@ int keds_exchange_create(int n_ranks, int my_rank, int device, void* const* peer
 void keds_exchange_free(keds_exchange_t* ex) {
   if (!ex) return;
   DeviceGuard g(ex->device);
+  for (int db = 0; db < 2; ++db) ex_detach_rows(ex, db);
   ex->words.release();
   delete ex;
 }
 
 int64_t keds_exchange_capacity(const keds_exchange_t* ex) { return ex ? ex->i_off / 4 : -1; }
 
+int keds_index_rows_ipc(const keds_index_t* ix, void* handle64) {
+  if (!ix || !handle64) return fail(KEDS_ERR_ARG, "index_rows_ipc: null handle or output");
+  memset(handle64, 0, sizeof(cudaIpcMemHandle_t));
+  if (ix->n == 0) return 0;  // no rows: nothing to map (the all-zero handle)
+  DeviceGuard g(ix->device);
+  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
+  IpcExport e;
+  CK(cudaIpcGetMemHandle(&e.h, ix->x_f32.p));
+  e.rows = ix->x_f32.as<float>();
+  memcpy(handle64, &e.h, sizeof e.h);
+  std::lock_guard<std::mutex> lk(g_ipc_mu);
+  for (IpcExport& o : g_ipc)
+    if (o.rows == e.rows) {
+      o = e;
+      return 0;
+    }
+  if (g_ipc.size() >= 256) g_ipc.erase(g_ipc.begin());
+  g_ipc.push_back(e);
+  return 0;
+}
+
+int keds_exchange_attach_rows(keds_exchange_t* ex, int db, const void* const* handles, const int64_t* lo,
+                              const int64_t* n) {
+  if (!ex || db < 0 || db > 1 || !handles || !lo || !n)
+    return fail(KEDS_ERR_ARG, "exchange_attach_rows: null argument or db outside 0..1");
+  for (int r = 0; r < ex->n_ranks; ++r)
+    if (lo[r] < 0 || n[r] < 0 || (n[r] > 0 && !handles[r]))
+      return fail(KEDS_ERR_ARG, "exchange_attach_rows: rank %d has a negative range or no handle", r);
+  DeviceGuard g(ex->device);
+  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ex->device);
+  ex_detach_rows(ex, db);
+  ShardRowsDb& rd = ex->rows[db];
+  for (int r = 0; r < ex->n_ranks; ++r) {
+    rd.lo[r] = lo[r];
+    rd.n[r] = n[r];
+    if (n[r] == 0) continue;
+    cudaIpcMemHandle_t h;
+    memcpy(&h, handles[r], sizeof h);
+    if (r == ex->my_rank) {
+      std::lock_guard<std::mutex> lk(g_ipc_mu);
+      for (const IpcExport& e : g_ipc)
+        if (!memcmp(&e.h, &h, sizeof h)) rd.base[r] = e.rows;
+      if (!rd.base[r]) {
+        ex_detach_rows(ex, db);
+        return fail(KEDS_ERR_ARG, "exchange_attach_rows: this rank's handle was not made by keds_index_rows_ipc here");
+      }
+      continue;
+    }
+    void* p = nullptr;
+    const cudaError_t e = cudaIpcOpenMemHandle(&p, h, cudaIpcMemLazyEnablePeerAccess);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      ex_detach_rows(ex, db);
+      return fail(KEDS_ERR_CUDA, "exchange_attach_rows: cudaIpcOpenMemHandle of rank %d failed: %s", r,
+                  cudaGetErrorString(e));
+    }
+    rd.base[r] = static_cast<const float*>(p);
+    ex->opened[db][r] = true;
+  }
+  ex->attached[db] = true;
+  return 0;
+}
+
 int keds_index_search_sharded(keds_index_t* ix, keds_exchange_t* ex, const float* q, int64_t nq, int k, float* D,
                               int64_t* I, void* stream) {
+  return keds_index_search_sharded_exclude(ix, ex, q, nq, k, D, I, nullptr, 0, stream);
+}
+
+int keds_index_search_sharded_exclude(keds_index_t* ix, keds_exchange_t* ex, const float* q, int64_t nq, int k,
+                                      float* D, int64_t* I, const int64_t* exclude, int n_exclude, void* stream) {
   if (!ix || !ex || !q || !D || !I || nq <= 0 || k <= 0)
     return fail(KEDS_ERR_ARG, "search_sharded: null handle / pointer or bad nq / k");
   if (ex->device != ix->device) return fail(KEDS_ERR_ARG, "search_sharded: exchange and index live on different devices");
   if (!locate(q) || !locate(D) || !locate(I)) return fail(KEDS_ERR_ARG, "search_sharded: device pointers only");
-  if (nq * k > ex->i_off / 4)
-    return fail(KEDS_ERR_ARG, "search_sharded: nq*k = %lld exceeds the exchange capacity %lld", (long long)(nq * k),
-                (long long)(ex->i_off / 4));
-  DeviceGuard g(ix->device);
-  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const uint32_t epoch = ++ex->epoch;
-  const int parity = static_cast<int>(epoch & 1u);
-  const int me = ex->my_rank, R = ex->n_ranks;
-  // this rank's block lands in slot `me` of every rank's buffer (its own included: the merge reads it there)
-  uint8_t* mine = ex_slot(ex, me, parity, me);
-  float* Dl = reinterpret_cast<float*>(mine);
-  int64_t* Il = reinterpret_cast<int64_t*>(mine + ex->i_off);
-  PeerOut po;
-  memset(&po, 0, sizeof po);
-  po.n = R;
-  po.my_rank = me;
-  po.publish = 1;
-  po.epoch = epoch;
-  po.ticket = ex->words.as<unsigned int>();
-  for (int r = 0; r < R; ++r) {
-    uint8_t* there = ex_slot(ex, r, parity, me);
-    po.D[r] = reinterpret_cast<float*>(there);
-    po.I[r] = reinterpret_cast<long long*>(there + ex->i_off);
-    po.flag[r] = ex_flag(ex, r, parity, me);
+  Call c = call(1, ix, nullptr, q, nq, k, nullptr, nullptr, nullptr, nullptr, 0u);
+  if (exclude) CKS(c.exclude(exclude, n_exclude));
+  return sharded_search(c, ex, &D, &I, stream);
+}
+
+int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t* ex, const float* q, int64_t nq,
+                           int k, const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                           int64_t row_lo, int64_t row_hi, float* D_img, int64_t* I_img, float* D_txt,
+                           int64_t* I_txt, float* feat_img, float* feat_txt, float* pool_img, float* pool_txt,
+                           const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
+  if (!img || !txt || !ex || !q || !D_img || !I_img || !D_txt || !I_txt || nq <= 0 || k <= 0)
+    return fail(KEDS_ERR_ARG, "retrieve2_sharded: null handle / pointer or bad nq / k");
+  if (k > 1024) return fail(KEDS_ERR_ARG, "retrieve2_sharded: k=%d too large for the fused consumer", k);
+  if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "retrieve2_sharded: pool_mode must be 0, 1 or 2");
+  if (row_lo < 0 || row_hi < row_lo || row_hi > nq)
+    return fail(KEDS_ERR_ARG, "retrieve2_sharded: rows [%lld, %lld) outside [0, %lld)", (long long)row_lo,
+                (long long)row_hi, (long long)nq);
+  if (ex->device != img->device || txt->device != img->device)
+    return fail(KEDS_ERR_ARG, "retrieve2_sharded: exchange and indices live on different devices");
+  const bool want_pool = pool_mode != 0 && (pool_img || pool_txt);
+  const void* dev_ptrs[] = {q, D_img, I_img, D_txt, I_txt, feat_img, feat_txt, want_pool ? pool_img : nullptr,
+                            want_pool ? pool_txt : nullptr, perm_img, perm_txt};
+  for (const void* p : dev_ptrs)
+    if (p && locate(p).device != img->device)
+      return fail(KEDS_ERR_ARG, "retrieve2_sharded: device pointers of the indices' GPU only");
+  Call c = call(2, img, txt, q, nq, k, nullptr, nullptr, nullptr, nullptr, flags);
+  if (exclude) CKS(c.exclude(exclude, n_exclude));
+  CKS(ex_check_rows(ex, c.dbs, 2));
+  float* D[2] = {D_img, D_txt};
+  int64_t* I[2] = {I_img, I_txt};
+  CKS(sharded_search(c, ex, D, I, stream));
+  const int64_t nb = row_hi - row_lo;
+  if (nb == 0 || !(feat_img || feat_txt || want_pool)) return 0;
+  ShardConsume sc;
+  memset(&sc, 0, sizeof sc);
+  sc.cons.enabled = 1;
+  sc.cons.mode = want_pool ? pool_mode : 0;
+  sc.cons.tau = tau;
+  sc.cons.perm[0] = perm_img;
+  sc.cons.perm[1] = perm_txt;
+  sc.cons.feat[0] = feat_img;
+  sc.cons.feat[1] = feat_txt;
+  sc.cons.pool[0] = want_pool ? pool_img : nullptr;
+  sc.cons.pool[1] = want_pool ? pool_txt : nullptr;
+  sc.cons.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
+  sc.n_ranks = ex->n_ranks;
+  sc.k = k;
+  sc.d = img->d;
+  sc.metric = c.metric();
+  sc.row_lo = row_lo;
+  for (int i = 0; i < 2; ++i) {
+    sc.D[i] = D[i];
+    sc.I[i] = reinterpret_cast<const long long*>(I[i]);
+    sc.db[i] = ex->rows[i];
   }
-  if (ix->n == 0) {
-    // an empty shard still has to deliver (padding) and publish: plain fill + the stand-alone push
-    const long long tot = static_cast<long long>(nq) * k;
-    k_fill_pad<<<static_cast<unsigned>((tot + 255) / 256), 256, 0, st>>>(
-        Dl, reinterpret_cast<long long*>(Il), tot, ix->metric == METRIC_L2 ? FLT_MAX : -FLT_MAX);
-    CK(cudaGetLastError());
-    if (R > 1) {
-      void* dst[P2P_MAX_RANKS];
-      uint32_t* flg[P2P_MAX_RANKS];
-      for (int r = 0; r < R; ++r) {
-        dst[r] = ex_slot(ex, r, parity, me);
-        flg[r] = ex_flag(ex, r, parity, me);
-      }
-      CKS(keds_p2p_push(mine, ex->slot_bytes, dst, flg, R, me, epoch, po.ticket, stream));
-    }
-  } else {
-    Call c = call(1, ix, nullptr, q, nq, k, Dl, Il, nullptr, nullptr, 0u);
-    if (R > 1) c.peer = po;
-    CKS(search_impl(c, IO_DEVICE, stream));
+  const size_t smem = static_cast<size_t>(sc.cons.part4) * 16 + static_cast<size_t>(k) * 20;
+  DeviceGuard g(img->device);
+  static std::atomic<bool> attr[64];
+  if (img->device >= 64 || !attr[img->device].load(std::memory_order_acquire)) {
+    CK(cudaFuncSetAttribute(k_shard_consume, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    if (img->device < 64) attr[img->device].store(true, std::memory_order_release);
   }
-  MergeWait mw;
-  memset(&mw, 0, sizeof mw);
-  if (R > 1) {
-    mw.flags = ex_flag(ex, me, parity, 0);
-    mw.my_rank = me;
-    mw.epoch = epoch;
-    mw.err_word = ex->words.as<unsigned int>() + 1;
-    mw.stats = reinterpret_cast<unsigned long long*>(ex->words.as<uint8_t>() + 16);
-  }
-  uint8_t* parts = ex_slot(ex, me, parity, 0);
-  return merge_impl(reinterpret_cast<const float*>(parts), reinterpret_cast<const int64_t*>(parts + ex->i_off),
-                    ex->slot_bytes / 4, ex->slot_bytes / 8, R, nq, k, ix->metric, D, I, mw, stream);
+  CKS(launch_k(img->use_pdl, k_shard_consume, dim3(static_cast<unsigned>(nb), 2), dim3(RERANK_THREADS), smem,
+               static_cast<cudaStream_t>(stream), sc));
+  return 0;
 }
 
 int keds_exchange_stats(keds_exchange_t* ex, void* stream, double* wait_us_avg, double* wait_us_max,

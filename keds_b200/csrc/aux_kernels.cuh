@@ -396,27 +396,28 @@ __device__ __forceinline__ void mirror_row_to_host(const ConsumeParams& c, int s
 }
 
 // Row-sharded exchange fused into the search (p2p_exchange.cuh): the block that has ranked query b
-// also stores that [k] result row into every peer's receive buffer (NVLink P2P stores), and the
-// last block of the search's last kernel publishes the epoch flag. n == 0: off.
+// of database s also stores that [k] result row into every peer's receive buffer (NVLink P2P
+// stores), and the last block of the search's last kernel publishes the epoch flag. n == 0: off.
 struct PeerOut {
   int n, my_rank;
   int publish;                          // this launch is the last writer of the step: publish the flags
   unsigned int epoch;
-  float* D[P2P_MAX_RANKS];              // where THIS rank's [nq][k] score block lives in rank r's buffer
+  float* D[P2P_MAX_RANKS];              // where THIS rank's [nq][k] score block of database 0 lives in rank r's buffer
   long long* I[P2P_MAX_RANKS];          // ... and its label block
+  long long db_stride;                  // database 1's blocks follow at D[r] + db_stride, I[r] + db_stride
   unsigned int* flag[P2P_MAX_RANKS];    // "rank my_rank has delivered `epoch`" word in rank r's buffer
   unsigned int* ticket;                 // local counter for "last block publishes" (zero between launches)
 };
 
-// Store one query's final row to the peers. top_id: local row ids in rank order (0xFFFFFFFF =
-// padding); called by every thread of the block after the row is complete in shared memory.
-__device__ __forceinline__ void push_row_to_peers(const PeerOut& po, long long q, int k,
+// Store one query's final row of database s to the peers. top_id: local row ids in rank order
+// (0xFFFFFFFF = padding); called by every thread of the block after the row is complete in shared memory.
+__device__ __forceinline__ void push_row_to_peers(const PeerOut& po, int s, long long q, int k,
                                                   const unsigned int* top_id, const float* top_d,
                                                   long long id_offset, int metric) {
   for (int r = 0; r < po.n; ++r) {
     if (r == po.my_rank) continue;
-    float* Dr = po.D[r] + q * k;
-    long long* Ir = po.I[r] + q * k;
+    float* Dr = po.D[r] + s * po.db_stride + q * k;
+    long long* Ir = po.I[r] + s * po.db_stride + q * k;
     for (int j = threadIdx.x; j < k; j += blockDim.x) {
       const unsigned int id = top_id[j];
       const bool pad = id == 0xFFFFFFFFu;
@@ -427,10 +428,22 @@ __device__ __forceinline__ void push_row_to_peers(const PeerOut& po, long long q
   __threadfence_system();  // ordered before the flag a later block publishes with release.sys
 }
 
-// top_id: local row ids in rank order (0xFFFFFFFF = padding), top_d: their D values.
+// Where the consumer finds neighbour row `id` (the id top_id holds). LocalRows: the search's own
+// database, row id of a [n][d] matrix. The sharded consumer (k_shard_consume) addresses rows that
+// live on several GPUs through a per-query table of row pointers instead.
+struct LocalRows {
+  const float* __restrict__ base;
+  int d;
+  __device__ __forceinline__ const float* operator()(unsigned int id) const {
+    return base + static_cast<long long>(id) * d;
+  }
+  __device__ __forceinline__ uintptr_t align_bits() const { return reinterpret_cast<uintptr_t>(base); }
+};
+
+// top_id: row ids in rank order (0xFFFFFFFF = padding) as `rows` resolves them, top_d: their D values.
 // NIF = neighbour rows in flight per warp (2 for latency, 1 where registers are scarce).
-template <int NIF>
-__device__ __forceinline__ void consume_query(const ConsumeParams& c, const float* __restrict__ rows,
+template <int NIF, class Rows>
+__device__ __forceinline__ void consume_query(const ConsumeParams& c, const Rows& rows,
                                               int s, long long b, int k, int d, int metric,
                                               const unsigned int* top_id, const float* top_d,
                                               float* w, float4* part) {
@@ -472,7 +485,7 @@ __device__ __forceinline__ void consume_query(const ConsumeParams& c, const floa
     }
   }
   __syncthreads();
-  const bool vec = c.part4 > 0 && ((reinterpret_cast<uintptr_t>(rows) | reinterpret_cast<uintptr_t>(c.feat[s]) |
+  const bool vec = c.part4 > 0 && ((rows.align_bits() | reinterpret_cast<uintptr_t>(c.feat[s]) |
                                     reinterpret_cast<uintptr_t>(c.pool[s])) & 15) == 0;
   if (vec) {
     // One warp per neighbour row, two neighbours per warp in flight: every lane issues all its
@@ -502,7 +515,7 @@ __device__ __forceinline__ void consume_query(const ConsumeParams& c, const floa
           for (int u = 0; u < U; ++u) {
             const int col = cb + u * 32 + lane;
             v[t][u] = (idv[t] != 0xFFFFFFFFu && col < d4)
-                          ? __ldg(reinterpret_cast<const float4*>(rows + static_cast<long long>(idv[t]) * d) + col)
+                          ? __ldg(reinterpret_cast<const float4*>(rows(idv[t])) + col)
                           : make_float4(0.f, 0.f, 0.f, 0.f);
           }
         }
@@ -552,7 +565,7 @@ __device__ __forceinline__ void consume_query(const ConsumeParams& c, const floa
         const bool j_ok = static_cast<unsigned int>(j) < static_cast<unsigned int>(k);
         if (!j_ok) j = 0;
         const unsigned int id = j_ok ? top_id[j] : 0xFFFFFFFFu;
-        const float v = id != 0xFFFFFFFFu ? rows[static_cast<long long>(id) * d + col] : 0.f;
+        const float v = id != 0xFFFFFFFFu ? rows(id)[col] : 0.f;
         if (feat) feat[static_cast<long long>(jo) * d + col] = v;
         acc = fmaf(w[j], v, acc);
       }

@@ -42,7 +42,7 @@ struct ExactParams {
   unsigned int* err;           // status word: EXACT_ERR_BARRIER if the barrier watchdog fired
   const unsigned int* band_dev;  // status word written by the re-rank kernel: largest |C| of this search
   unsigned int* band_host;     // nullable: mapped host word that receives it (planner feedback, no copy node)
-  PeerOut peer;                // row-sharded exchange (database 0 only); n == 0: off
+  PeerOut peer;                // row-sharded exchange; n == 0: off
   unsigned long long* timing;  // nullable in-kernel launch timer
   // search with exclusion: staged local row ids (ScoreParams::ex_rows); nullptr: nothing excluded
   const int* ex_rows;
@@ -406,13 +406,13 @@ __device__ __forceinline__ void exact_select(const ExactParams& p, uint8_t* ex_s
       Dq[r] = p.metric == METRIC_L2 ? FLT_MAX : -FLT_MAX;
       Iq[r] = -1;
     }
-    if (p.cons.enabled || (p.peer.n > 1 && dbi == 0)) {
+    if (p.cons.enabled || p.peer.n > 1) {
       __syncthreads();
-      if (p.peer.n > 1 && dbi == 0) push_row_to_peers(p.peer, q, p.k, top_id, top_d, e.id_offset, p.metric);
+      if (p.peer.n > 1) push_row_to_peers(p.peer, dbi, q, p.k, top_id, top_d, e.id_offset, p.metric);
       if (p.cons.enabled && p.cons.host_D[dbi] != nullptr)
         mirror_row_to_host(p.cons, dbi, q, p.k, top_id, top_d, e.id_offset, p.metric);
       if (p.cons.enabled)
-        consume_query<1>(p.cons, e.x_f32, dbi, q, p.k, p.d, p.metric, top_id, top_d, top_w, part);
+        consume_query<1>(p.cons, LocalRows{e.x_f32, p.d}, dbi, q, p.k, p.d, p.metric, top_id, top_d, top_w, part);
     }
   }
 }

@@ -61,4 +61,60 @@ __device__ __forceinline__ bool p2p_wait_flags(const unsigned int* flags, int n_
   return true;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Neighbour consumer of a row-sharded two-database step (keds_retrieve2_sharded): after the merges,
+// one block per (query of this rank's block [row_lo, row_lo + gridDim.x), database) looks up the
+// owner of each merged label in the lo table, reads the row in place from that rank's fp32 master
+// (its own, or a peer's over NVLink through a cudaIpc mapping) and runs the same gather / weights /
+// pool as the local consumer. The rows do not change between adds, so no flag guards them.
+struct ShardRowsDb {
+  const float* base[P2P_MAX_RANKS];  // rank r's [n][d] fp32 rows as mapped into this process (null: no rows)
+  long long lo[P2P_MAX_RANKS];       // global label of its first row
+  long long n[P2P_MAX_RANKS];
+};
+
+struct ShardConsume {
+  ConsumeParams cons;  // feat / pool of the output rows [0, gridDim.x)
+  int n_ranks, k, d, metric;
+  long long row_lo;
+  const float* D[2];  // merged [nq][k] per database
+  const long long* I[2];
+  ShardRowsDb db[2];
+};
+
+// Row `id` = slot id of a per-query table of row pointers (filled from the owners' bases).
+struct PtrRows {
+  const float* const* ptr;
+  uintptr_t bits;  // OR of every base the pointers derive from (alignment test)
+  __device__ __forceinline__ const float* operator()(unsigned int id) const { return ptr[id]; }
+  __device__ __forceinline__ uintptr_t align_bits() const { return bits; }
+};
+
+__global__ void __launch_bounds__(RERANK_THREADS)
+k_shard_consume(const ShardConsume p) {
+  extern __shared__ __align__(16) uint8_t sc_smem[];
+  float4* part = reinterpret_cast<float4*>(sc_smem);                          // cons.part4
+  const float** ptr = reinterpret_cast<const float**>(part + p.cons.part4);   // k
+  unsigned int* top_id = reinterpret_cast<unsigned int*>(ptr + p.k);          // k
+  float* top_d = reinterpret_cast<float*>(top_id + p.k);                      // k
+  float* w = top_d + p.k;                                                     // k
+  const int s = blockIdx.y;
+  const long long b = blockIdx.x, q = p.row_lo + b;
+  const ShardRowsDb& rd = p.db[s];
+  uintptr_t bits = 0;
+  for (int r = 0; r < p.n_ranks; ++r) bits |= reinterpret_cast<uintptr_t>(rd.base[r]);
+  griddep_wait();  // the merged rows are complete
+  for (int j = threadIdx.x; j < p.k; j += blockDim.x) {
+    const long long lab = p.I[s][q * p.k + j];
+    const float* row = nullptr;
+    for (int r = 0; r < p.n_ranks; ++r)
+      if (lab >= rd.lo[r] && lab < rd.lo[r] + rd.n[r]) row = rd.base[r] + (lab - rd.lo[r]) * p.d;
+    ptr[j] = row;
+    top_id[j] = row != nullptr ? static_cast<unsigned int>(j) : 0xFFFFFFFFu;  // -1 padding: a zero row
+    top_d[j] = p.D[s][q * p.k + j];
+  }
+  __syncthreads();
+  consume_query<2>(p.cons, PtrRows{ptr, bits}, s, b, p.k, p.d, p.metric, top_id, top_d, w, part);
+}
+
 }  // namespace keds

@@ -34,7 +34,7 @@ struct RerankParams {
   float eps_scale;           // 1.0 normally; tests shrink/grow it to exercise the fallback
   int rmax;                  // candidate capacity of this launch (<= R_MAX; sizes the shared arrays)
   unsigned int* band_max;    // status word: largest |C| of this search (feeds the planner's next slice count)
-  PeerOut peer;              // row-sharded exchange (database 0 only); n == 0: off
+  PeerOut peer;              // row-sharded exchange; n == 0: off
   unsigned long long* timing;  // nullable in-kernel launch timer
 };
 
@@ -348,14 +348,15 @@ k_select_rerank(const RerankParams p) {
   }
   // a flagged query is consumed (and sent to the peers) by the exact fallback instead, once its
   // answer is final
-  if (ok && (p.cons.enabled || (p.peer.n > 1 && db == 0))) {
+  if (ok && (p.cons.enabled || p.peer.n > 1)) {
     __syncthreads();  // (7)
-    if (p.peer.n > 1 && db == 0)
-      push_row_to_peers(p.peer, q, p.k, top_id, top_d, p.id_offset[db], p.metric);
+    if (p.peer.n > 1)
+      push_row_to_peers(p.peer, db, q, p.k, top_id, top_d, p.id_offset[db], p.metric);
     if (p.cons.enabled && p.cons.host_D[db] != nullptr)
       mirror_row_to_host(p.cons, db, q, p.k, top_id, top_d, p.id_offset[db], p.metric);
     if (p.cons.enabled)
-      consume_query<(R >= 2 ? 2 : 1)>(p.cons, xbase, db, q, p.k, p.d, p.metric, top_id, top_d, top_w, part);
+      consume_query<(R >= 2 ? 2 : 1)>(p.cons, LocalRows{xbase, p.d}, db, q, p.k, p.d, p.metric, top_id, top_d, top_w,
+                                      part);
   }
   ktimer_end(p.timing, t_start);
 }

@@ -162,10 +162,31 @@ def get_retrieved_features(feature, database, args=None, topk: int = 16, use_fai
 
     exclude (not in the reference; default None = its behaviour): int64 [B] or [B, E] rows each
     query must not retrieve, -1 = none -- e.g. database.rows_of(batch_names) to train without
-    self-retrieval. One array for both bases (aligned row for row)."""
+    self-retrieval. One array for both bases (aligned row for row).
+
+    Row-sharded bases (database[3], database[4] = the `image` and `text` indices of one
+    sharded.ShardedKnowledgeBase), called by every DDP rank with its own batch: the ranks all-gather
+    their batch sizes, their queries padded to the largest batch and their exclusion arrays, run one
+    sharded step over all of them and each gets the [B, topk, d] pair of its own block of rows, its
+    image stream permuted by its own torch.randperm(topk) as the reference does per rank."""
     image_base, text_base, basenames, image_index, text_index = (database[i] for i in range(5))
+    from .sharded import ShardedIndex, gather_ddp_step
+
+    if isinstance(image_index, ShardedIndex) and isinstance(text_index, ShardedIndex):
+        kb = image_index._kb
+        if kb is None or kb.image is not image_index or kb.text is not text_index:
+            raise TypeError("database[3] and database[4] must be the image and text indices of one ShardedKnowledgeBase")
+        if use_faiss:
+            feature = feature / feature.norm(dim=1, keepdim=True)  # src/trainer.py:206
+        flags = 0 if use_faiss else _capi.SEARCH_FORCE_IP
+        perm = torch.randperm(topk) if use_faiss else None
+        q_all, ex_all, rows = gather_ddp_step(feature.detach(), exclude, kb.group, kb.device)
+        out = kb.retrieve2(q_all, topk, perm_img=perm, want_feats=True, pool_mode=0, flags=flags, exclude=ex_all,
+                           rows=rows)
+        return out["feat_img"].to(feature.device), out["feat_txt"].to(feature.device)
     if not (_native(image_index) and _native(text_index)):
-        raise TypeError("database[3] and database[4] must be keds_b200 GPU indices (no CPU path)")
+        raise TypeError("database[3] and database[4] must be keds_b200 GPU indices or the two indices of a "
+                        "ShardedKnowledgeBase (no CPU path)")
     if use_faiss:
         feature = feature / feature.norm(dim=1, keepdim=True)  # src/trainer.py:206
     dev = torch.device("cuda", image_index.device)

@@ -21,7 +21,7 @@ import torch
 import torch.distributed as dist
 
 from . import _capi
-from .index import GpuIndexFlat, _stream_ptr
+from .index import GpuIndexFlat, _exclude_arg, _stream_ptr
 
 
 def shard_bounds(n: int, world: int, rank: int) -> Tuple[int, int]:
@@ -42,27 +42,47 @@ class _FusedExchange:
     """Symmetric (peer-mapped) receive buffers + the native exchange handle over them. The buffer
     is allocated with torch symmetric memory, so every rank holds raw pointers into every other
     rank's copy (NVLink P2P through NVSwitch); the library lays it out (flag words, two parities
-    of one slot per rank) and never sees torch types."""
+    of one slot per rank) and never sees torch types. Symmetric memory needs one GPU per rank:
+    ranks that share a GPU map each other's buffers with cudaIpc instead (torch's CUDA tensor
+    sharing), which gives the library the same kind of peer pointers."""
 
     def __init__(self, world: int, rank: int, capacity: int, device: torch.device, group) -> None:
         import ctypes as C
         import torch.distributed._symmetric_memory as symm_mem
 
         lib = _capi.load()
+        group = group if group is not None else dist.group.WORLD
         slot = -(-(12 * capacity) // 48) * 48
         total = (256 + 2 * world * slot + 255) // 256 * 256
-        self.buf = symm_mem.empty(total, dtype=torch.uint8, device=device)
-        self.buf.zero_()
-        torch.cuda.synchronize(device)
-        self.hdl = symm_mem.rendezvous(self.buf, group if group is not None else dist.group.WORLD)
-        peers = [int(p) for p in self.hdl.buffer_ptrs]
+        uuids = [None] * world
+        dist.all_gather_object(uuids, str(torch.cuda.get_device_properties(device).uuid), group=group)
+        self.hdl = None
+        if len(set(uuids)) == world:
+            self.buf = symm_mem.empty(total, dtype=torch.uint8, device=device)
+            self.buf.zero_()
+            torch.cuda.synchronize(device)
+            self.hdl = symm_mem.rendezvous(self.buf, group)
+            peers = [int(p) for p in self.hdl.buffer_ptrs]
+        else:
+            from torch.multiprocessing.reductions import reduce_tensor
+
+            self.buf = torch.zeros(total, dtype=torch.uint8, device=device)
+            torch.cuda.synchronize(device)
+            shared = [None] * world
+            dist.all_gather_object(shared, reduce_tensor(self.buf), group=group)
+            self._peer_bufs = [self.buf if r == rank else fn(*args) for r, (fn, args) in enumerate(shared)]
+            peers = [int(b.data_ptr()) for b in self._peer_bufs]
         assert peers[rank] == self.buf.data_ptr()
         h = C.c_void_p()
         _capi.check(lib.keds_exchange_create(world, rank, device.index, (C.c_void_p * world)(*peers), total, C.byref(h)))
         self.handle, self._lib = h, lib
         self.capacity = int(lib.keds_exchange_capacity(h))
         assert self.capacity >= capacity
-        self.hdl.barrier()  # every rank's buffer is zeroed before anyone pushes
+        # every rank's buffer is zeroed before anyone pushes
+        if self.hdl is not None:
+            self.hdl.barrier()
+        else:
+            dist.barrier(group=group)
 
     def stats(self, stream_ptr: int) -> dict:
         import ctypes as C
@@ -113,32 +133,45 @@ class ShardedIndex:
             self.device = torch.device("cuda", dev)
         self.ntotal = 0
         self.lo = self.hi = 0
+        self._kb: Optional["ShardedKnowledgeBase"] = None  # set when this index is a base of one
+        self._db = 0
 
     def add_local(self, x_local, lo: int, ntotal: int) -> None:
-        """This rank's rows (global row ids lo .. lo+len) of an ntotal-row database."""
+        """This rank's rows (global row ids lo .. lo+len) of an ntotal-row database. Collective:
+        every rank calls it (an index of a ShardedKnowledgeBase re-attaches the rows afterwards)."""
+        kb = self._kb
+        if kb is not None and kb._fx is not None and self.device.type == "cuda":
+            # peers may still be reading these rows for a step in flight
+            torch.cuda.synchronize(self.device)
+            dist.barrier(group=self.group)
         self.lo, self.hi, self.ntotal = int(lo), int(lo) + int(x_local.shape[0]), int(ntotal)
         self.local.set_id_offset(self.lo)
         if x_local.shape[0]:
             self.local.add(x_local)
+        if kb is not None:
+            kb._attach_rows(self._db)
 
     def add(self, x) -> None:
         """Every rank passes the same full matrix and keeps its own row range."""
         lo, hi = shard_bounds(int(x.shape[0]), self.world, self.rank)
         self.add_local(x[lo:hi], lo, int(x.shape[0]))
 
-    def search(self, q: torch.Tensor, k: int, out=None):
+    def search(self, q: torch.Tensor, k: int, out=None, exclude=None):
         """q: [nq, d] float32 on this rank's device, identical on all ranks. Returns (D, I);
-        `out=(D, I)` may name preallocated contiguous device tensors to fill (fused exchange)."""
+        `out=(D, I)` may name preallocated contiguous device tensors to fill (fused exchange).
+        exclude: int64 [nq] or [nq, E] (E <= 8) global labels each query must not get back, -1 =
+        none, the same on every rank; the result is that of an unsharded search with exclusion."""
         nq = int(q.shape[0])
         total, off_i, d_bytes = packed_layout(nq, k)
         if self.exchange == "fused" and isinstance(self.local, GpuIndexFlat):
-            return self._search_fused(q, nq, k, out)
+            return self._search_fused(q, nq, k, out, exclude)
         if isinstance(self.local, GpuIndexFlat):
             # the local search writes straight into the exchange buffer: no repacking copies
             send = torch.empty(total, dtype=torch.uint8, device=q.device)
-            self.local.search(q, k, out=(send[:d_bytes].view(torch.float32), send[off_i:].view(torch.int64)))
+            self.local.search(q, k, out=(send[:d_bytes].view(torch.float32), send[off_i:].view(torch.int64)),
+                              exclude=exclude)
         else:  # CPU test stand-in
-            D, I = self.local.search(q, k)
+            D, I = self.local.search(q, k) if exclude is None else self.local.search(q, k, exclude=exclude)
             D, I = torch.as_tensor(D), torch.as_tensor(I)
             send = torch.empty(total, dtype=torch.uint8, device=D.device)
             send[:d_bytes].view(torch.float32).copy_(D.reshape(-1))
@@ -161,13 +194,14 @@ class ShardedIndex:
         )
         return Dg, Ig
 
-    def _search_fused(self, q: torch.Tensor, nq: int, k: int, out=None):
+    def _search_fused(self, q: torch.Tensor, nq: int, k: int, out=None, exclude=None):
         """One native call: local search with the peer stores fused into its kernels, flag
         publication by the chain's last block, merge that waits on the peers' flags. Two buffer
         parities keep a fast rank from overwriting a block a slow rank is still merging (a rank can
         only publish step t+1 after finishing its merge of step t)."""
         lib = _capi.load()
         q = self.local._check_q_tensor(q)
+        ex = None if exclude is None else _exclude_arg(exclude, nq, self.device.index)
         if self._fx is None or self._fx.capacity < nq * k:
             # (re)allocation is collective: every rank sees the same shapes in the same order
             if self._fx is not None:
@@ -181,8 +215,13 @@ class ShardedIndex:
         else:
             Dg = torch.empty((nq, k), dtype=torch.float32, device=q.device)
             Ig = torch.empty((nq, k), dtype=torch.int64, device=q.device)
-        _capi.check(lib.keds_index_search_sharded(self.local._h, self._fx.handle, q.data_ptr(), nq, k, Dg.data_ptr(),
-                                                  Ig.data_ptr(), _stream_ptr(self.device.index)))
+        if ex is None:
+            _capi.check(lib.keds_index_search_sharded(self.local._h, self._fx.handle, q.data_ptr(), nq, k,
+                                                      Dg.data_ptr(), Ig.data_ptr(), _stream_ptr(self.device.index)))
+        else:
+            _capi.check(lib.keds_index_search_sharded_exclude(self.local._h, self._fx.handle, q.data_ptr(), nq, k,
+                                                              Dg.data_ptr(), Ig.data_ptr(), ex.data_ptr(), ex.shape[1],
+                                                              _stream_ptr(self.device.index)))
         return Dg, Ig
 
     def exchange_stats(self) -> dict:
@@ -194,3 +233,195 @@ class ShardedIndex:
 
     def check_exchange(self) -> None:
         self.exchange_stats()
+
+
+def rank_block(batch_sizes, rank: int) -> Tuple[int, int, int]:
+    """(padded batch Bmax, first row, end row) of `rank`'s queries in the all-gathered query matrix
+    of a DDP step: every rank pads its batch to the largest one, so rank r owns [r*Bmax, r*Bmax + B_r)."""
+    sizes = [int(b) for b in batch_sizes]
+    if not sizes or min(sizes) < 0 or not 0 <= rank < len(sizes):
+        raise ValueError(f"rank_block: rank {rank} of batch sizes {sizes}")
+    bmax = max(sizes)
+    return bmax, rank * bmax, rank * bmax + sizes[rank]
+
+
+class ShardedKnowledgeBase:
+    """The KEDs retrieval step over row-sharded image and text bases: two ShardedIndex (`image`,
+    `text`) over one fused exchange. Every rank holds rows [lo_r, hi_r) of each base; retrieve2
+    searches both bases for queries that are the same on every rank, merges the global top-k on every
+    rank, and gathers / pools the neighbour rows of the query rows a rank asks for straight from the
+    owners' fp32 rows over NVLink (mapped with cudaIpc, re-attached after every add). Results equal
+    retrieval.retrieve2 on an unsharded index bit for bit (D, I, gathered rows); pools use the same
+    weights and do not depend on the shard count.
+
+    Test hooks: `_local_index` (a factory of stand-in local indices, as ShardedIndex takes) and
+    `_retrieve` (a stand-in for the native step, called with the checked arguments) let the CPU
+    (gloo) tests drive the DDP plumbing of get_retrieved_features."""
+
+    def __init__(self, d: int, metric: int, device: Optional[int] = None, group=None, exchange: str = "fused",
+                 _local_index: Optional[Callable] = None, _retrieve: Optional[Callable] = None) -> None:
+        if exchange == "p2p":
+            exchange = "fused"
+        if exchange != "fused":
+            raise ValueError("ShardedKnowledgeBase: the retrieval step needs exchange='fused' (peer memory); "
+                             f"got {exchange!r}")
+        self.image = ShardedIndex(d, metric, device, group, exchange,
+                                  _local_index=_local_index() if _local_index else None)
+        self.text = ShardedIndex(d, metric, device, group, exchange,
+                                 _local_index=_local_index() if _local_index else None)
+        for db, ix in enumerate((self.image, self.text)):
+            ix._kb, ix._db = self, db
+        self.group, self.rank, self.world = group, self.image.rank, self.image.world
+        self.d, self.metric_type, self.device = int(d), int(metric), self.image.device
+        self._fx: Optional[_FusedExchange] = None
+        self._retrieve = _retrieve
+
+    def add(self, image_rows, text_rows) -> None:
+        """Every rank passes the same full matrices and keeps its own row ranges. Collective."""
+        self.image.add(image_rows)
+        self.text.add(text_rows)
+
+    def _native(self) -> bool:
+        return self._retrieve is None and isinstance(self.image.local, GpuIndexFlat)
+
+    def _attach_rows(self, db: int) -> None:
+        """Tell the exchange where every rank's rows of base `db` live (collective)."""
+        if self._fx is None or not self._native():
+            return
+        import ctypes as C
+
+        ix = (self.image, self.text)[db]
+        lib = _capi.load()
+        torch.cuda.synchronize(self.device)
+        h = (C.c_uint8 * 64)()
+        _capi.check(lib.keds_index_rows_ipc(ix.local._h, h))
+        mine = (bytes(h), ix.lo, ix.hi - ix.lo)
+        every = [None] * self.world
+        dist.all_gather_object(every, mine, group=self.group)
+        bufs = [(C.c_uint8 * 64).from_buffer_copy(e[0]) for e in every]
+        handles = (C.c_void_p * self.world)(*[C.addressof(b) for b in bufs])
+        lo = (C.c_int64 * self.world)(*[e[1] for e in every])
+        n = (C.c_int64 * self.world)(*[e[2] for e in every])
+        _capi.check(lib.keds_exchange_attach_rows(self._fx.handle, db, handles, lo, n))
+
+    def _exchange(self, need: int) -> "_FusedExchange":
+        if self._fx is None or self._fx.capacity < need:
+            # (re)allocation is collective: every rank sees the same shapes in the same order
+            if self._fx is not None:
+                torch.cuda.synchronize(self.device)
+                dist.barrier(group=self.group)
+            self._fx = _FusedExchange(self.world, self.rank, max(need, 16384), self.device, self.group)
+            for ix in (self.image, self.text):
+                ix._fx = self._fx
+            self._attach_rows(0)
+            self._attach_rows(1)
+        return self._fx
+
+    def retrieve2(self, q: torch.Tensor, k: int = 16, perm_img: Optional[torch.Tensor] = None,
+                  perm_txt: Optional[torch.Tensor] = None, want_feats: bool = True, pool_mode: int = 0,
+                  tau: float = 100.0, flags: int = 0, exclude=None, rows: Optional[Tuple[int, int]] = None,
+                  out: Optional[dict] = None) -> dict:
+        """One step for queries q [Bt, d] (float32, this rank's device, identical on every rank).
+        Returns D_img / I_img / D_txt / I_txt [Bt, k] for every query and, for the query rows
+        rows = (lo, hi) only (default: all), feat_img / feat_txt [hi-lo, k, d] (image stream permuted
+        by perm_img) and pool_img / pool_txt [hi-lo, d] (pool_mode 1 mean, 2 softmax(+-tau*D)).
+        exclude: int64 [Bt] or [Bt, E] (E <= 8) global labels each query must not retrieve from
+        either base, -1 = none. Collective: every rank calls it with the same q, k and exclusion.
+        `out` may carry the tensors of a previous call (keys as returned)."""
+        if not isinstance(q, torch.Tensor) or q.dtype != torch.float32 or q.dim() != 2 or q.shape[1] != self.d:
+            raise TypeError(f"retrieve2: q must be a float32 [Bt, {self.d}] tensor")
+        if q.device != self.device:
+            raise ValueError(f"retrieve2: q on {q.device}, the knowledge base on {self.device}")
+        Bt, k = int(q.shape[0]), int(k)
+        if Bt < 1:
+            raise ValueError("retrieve2: empty query batch")
+        if not 1 <= k <= 1024:
+            raise ValueError(f"retrieve2: k must be 1..1024, got {k}")
+        if pool_mode not in (0, 1, 2):
+            raise ValueError(f"retrieve2: pool_mode must be 0, 1 or 2, got {pool_mode}")
+        lo, hi = (0, Bt) if rows is None else (int(rows[0]), int(rows[1]))
+        if not 0 <= lo <= hi <= Bt:
+            raise ValueError(f"retrieve2: rows ({lo}, {hi}) outside [0, {Bt}]")
+        perms = []
+        for name, p in (("perm_img", perm_img), ("perm_txt", perm_txt)):
+            if p is not None and (not isinstance(p, torch.Tensor) or p.dim() != 1 or p.numel() != k
+                                  or p.dtype not in (torch.int32, torch.int64)):
+                raise TypeError(f"retrieve2: {name} must be an integer tensor of {k} entries")
+            perms.append(None if p is None else p.to(device=self.device, dtype=torch.int32).contiguous())
+        ex = None
+        if exclude is not None:
+            ex = _exclude_arg(exclude, Bt, self.device.index) if self.device.type == "cuda" else \
+                torch.as_tensor(_check_exclude_host(exclude, Bt))
+        q = q.contiguous()
+        if self._retrieve is not None:  # CPU test hook
+            return self._retrieve(q, k, perms[0], perms[1], want_feats, pool_mode, tau, flags, ex, (lo, hi))
+        fx = self._exchange(2 * Bt * k)
+        o = out if out is not None else {}
+        dev, d = self.device, self.d
+
+        def buf(name, shape, dtype):
+            t = o.get(name)
+            if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev:
+                t = torch.empty(shape, dtype=dtype, device=dev)
+                o[name] = t
+            return t
+
+        Di, Ii = buf("D_img", (Bt, k), torch.float32), buf("I_img", (Bt, k), torch.int64)
+        Dt, It = buf("D_txt", (Bt, k), torch.float32), buf("I_txt", (Bt, k), torch.int64)
+        fi = ft = pi = pt = None
+        if want_feats:
+            fi, ft = buf("feat_img", (hi - lo, k, d), torch.float32), buf("feat_txt", (hi - lo, k, d), torch.float32)
+        if pool_mode != 0:
+            pi, pt = buf("pool_img", (hi - lo, d), torch.float32), buf("pool_txt", (hi - lo, d), torch.float32)
+        ptr = lambda t: 0 if t is None else t.data_ptr()
+        lib = _capi.load()
+        _capi.check(lib.keds_retrieve2_sharded(
+            self.image.local._h, self.text.local._h, fx.handle, q.data_ptr(), Bt, k, ptr(perms[0]), ptr(perms[1]),
+            int(pool_mode), float(tau), lo, hi, Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(),
+            ptr(fi), ptr(ft), ptr(pi), ptr(pt), ptr(ex), 0 if ex is None else ex.shape[1], int(flags),
+            _stream_ptr(dev.index)))
+        return o
+
+    def exchange_stats(self) -> dict:
+        """Synchronise and report how long the merges waited for the peers; raises if a peer failed
+        to deliver within the watchdog window."""
+        return {} if self._fx is None else self._fx.stats(_stream_ptr(self.device.index))
+
+
+def _check_exclude_host(exclude, nq: int):
+    from .index import check_exclude
+
+    ex = check_exclude(exclude, nq)
+    return ex if isinstance(ex, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(ex))
+
+
+def gather_ddp_step(feature: torch.Tensor, exclude, group=None, device=None):
+    """The all-gathers of a sharded DDP retrieval step: every rank's batch size, then the queries
+    padded to the largest batch ([world * Bmax, d]) and, if any rank passes one, the exclusion arrays
+    padded with -1 ([world * Bmax, E_max]). Returns (queries, exclusion or None, (lo, hi)) with
+    [lo, hi) this rank's own rows."""
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    dev = feature.device if device is None else device
+    B, d = int(feature.shape[0]), int(feature.shape[1])
+    ex = None if exclude is None else _check_exclude_host(exclude, B)
+    meta = torch.tensor([B, 0 if ex is None else int(ex.shape[1])], dtype=torch.int64, device=dev)
+    # (flat receive buffers: the form every backend's all_gather_into_tensor takes)
+    metas = torch.empty(world * 2, dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(metas, meta, group=group)
+    sizes, widths = metas[0::2].tolist(), metas[1::2].tolist()
+    bmax, lo, hi = rank_block(sizes, rank)
+    qp = torch.zeros((bmax, d), dtype=torch.float32, device=dev)
+    qp[:B] = feature.to(device=dev, dtype=torch.float32)
+    q_all = torch.empty(world * bmax * d, dtype=torch.float32, device=dev)
+    dist.all_gather_into_tensor(q_all, qp.view(-1), group=group)
+    q_all = q_all.view(world * bmax, d)
+    e_max = max(widths)
+    ex_all = None
+    if e_max > 0:
+        ep = torch.full((bmax, e_max), -1, dtype=torch.int64, device=dev)
+        if ex is not None:
+            ep[:B, :ex.shape[1]] = ex.to(dev)
+        ex_all = torch.empty(world * bmax * e_max, dtype=torch.int64, device=dev)
+        dist.all_gather_into_tensor(ex_all, ep.view(-1), group=group)
+        ex_all = ex_all.view(world * bmax, e_max)
+    return q_all, ex_all, (lo, hi)
