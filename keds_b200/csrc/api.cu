@@ -2096,9 +2096,16 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
     CK(cudaGetLastError());
     return 0;
   }
+  // warp_exact_score sums in float4 chunks only when q is 16-byte aligned: a query tensor that
+  // starts elsewhere is scored from an aligned copy (left by k_prep_rows), so that its ranks do not
+  // depend on where it starts and equal those of the recount, which reads q from shared memory
+  const bool q_copy = (d & 3) == 0 && (reinterpret_cast<uintptr_t>(q) & 15) != 0;
   for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
     const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
-    const float* qp = q + q0 * d;
+    const float* qsrc = q + q0 * d;
+    if (q_copy) CKS(ix->q_f32.ensure(static_cast<size_t>(nb) * d * 4));
+    float* qcopy = q_copy ? ix->q_f32.as<float>() : nullptr;
+    const float* qp = q_copy ? qcopy : qsrc;
     Plan pl{geometry(ix, 1, nb)};
     // as many candidate lists as the tiles allow: the band around a mid-ranked target is crowded
     pl.set_slices(1, static_cast<int>(std::max<long long>(1, std::min<long long>(std::min(T, S_MAX), pl.s_mem))));
@@ -2118,11 +2125,11 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
     int* rk_e = rk_t + nb;
     {
       const unsigned blocks = static_cast<unsigned>(std::min<long long>((nb * 32 + 255) / 256, 4096));
-      CKS(launch_k(ix->use_pdl, k_prep_rows, dim3(blocks), dim3(256), 0, st, qp, static_cast<long long>(nb), d,
+      CKS(launch_k(ix->use_pdl, k_prep_rows, dim3(blocks), dim3(256), 0, st, qsrc, static_cast<long long>(nb), d,
                    ix->d_pad, ix->fmt, ix->q_bf16.as<uint16_t>(), ix->qstat.as<float4>(), static_cast<float*>(nullptr),
                    static_cast<unsigned int*>(nullptr), ix->ctrl.as<unsigned int>(), CTRL_WORDS,
-                   static_cast<float*>(nullptr), 0, static_cast<unsigned long long*>(nullptr),
-                   static_cast<float*>(nullptr), ExcludeStage{}));
+                   static_cast<float*>(nullptr), 0, static_cast<unsigned long long*>(nullptr), qcopy,
+                   ExcludeStage{}));
     }
     const unsigned wblocks = static_cast<unsigned>((nb * 32 + 255) / 256);
     CKS(launch_k(ix->use_pdl, k_rank_targets, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,

@@ -396,7 +396,8 @@ __device__ __forceinline__ void exact_select(const ExactParams& p, uint8_t* ex_s
         rank += other > mine;
       }
       const float v = key_to_f32(sel_key[c]);
-      const float dv = p.metric == METRIC_L2 ? -v : v;
+      // 0 - v, not -v: an exact match's distance is +0, as the re-rank writes it (v is +0 then)
+      const float dv = p.metric == METRIC_L2 ? 0.f - v : v;
       Dq[rank] = dv;
       Iq[rank] = static_cast<long long>(sel_id[c]) + e.id_offset;
       top_id[rank] = sel_id[c];
