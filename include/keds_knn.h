@@ -163,19 +163,14 @@ int keds_index_last_stats(const keds_index_t* idx, keds_search_stats* out);
  * set_profiling(1): every launch stamps %globaltimer at the start of its first CTA and the end of
  *   its last one -- no stream events, the launch chain (programmatic dependent launches) is left
  *   untouched; profile() returns the summed kernel duration in ms and the number of launches.
- * set_profiling(2): diagnostic stage marks (stream events between the kernels, which serialise
- *   them); profile_stages() splits stream time by stage.
- * set_profiling(0): off. */
+ * set_profiling(0): off; any other mode is KEDS_ERR_ARG. profile() and profile_chain() fail unless
+ *   mode 1 is on. */
 int keds_index_set_profiling(keds_index_t* idx, int enable);
 int keds_index_profile(keds_index_t* idx, double* score_ms_total, int64_t* score_launches);
 /* Mode 1, whole chain: average in-loop duration of each kernel of a search (0 k_prep_rows,
  * 1 k_score_topk, 2 k_select_rerank, 3 k_exact_fallback, 4 reserved = 0) and the average idle gap
  * in front of it (end of the previous kernel to its first CTA), in ms. n >= 5. Does not clear. */
 int keds_index_profile_chain(keds_index_t* idx, double* dur_ms, double* gap_ms, int64_t* searches, int n);
-/* Stage marks (mode 2): index 1 prep_rows, 2 score_topk, 3 select_rerank (+ neighbour consumer),
- * 4 exact-fallback pair (indices 0 and 5 unused); each entry is the stream time from the previous
- * mark to the end of that stage. n_stages >= 6. */
-int keds_index_profile_stages(keds_index_t* idx, double* ms_total, int64_t* launches, int n_stages);
 
 /* ---- neighbour gather / weighted pool ---------------------------------------------------------
  * W == NULL:  out[b][j][:] = base[I[b][perm ? perm[j] : j]][:]   (out: [B][k][d])

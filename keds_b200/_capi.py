@@ -105,7 +105,6 @@ SIGNATURES = {
     "keds_index_profile": (C.c_int, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "keds_index_profile_chain": (
         C.c_int, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int]),
-    "keds_index_profile_stages": (C.c_int, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_int64), C.c_int]),
     "keds_gather_pool": (
         C.c_int,
         [_vp, C.c_int64, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_int, _vp, _vp],

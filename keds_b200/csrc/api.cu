@@ -218,6 +218,14 @@ struct HitsMode {
   int* hits;                // [nq][nks]
 };
 
+// keds_index_rank: the scoring kernel counts the rows that beat each query's target (k_rank_targets
+// before it, k_rank_finish and the exact recount after it) instead of collecting the top-k
+struct RankMode {
+  const long long* target;   // [nq]
+  const long long* exclude;  // [nq] or nullptr
+  long long* out;            // [nq] ranks
+};
+
 // How the scoring kernel covers nq queries: which kernel, its work units and query groups, and
 // the most row slices the candidate budget holds.
 struct Geometry {
@@ -279,11 +287,6 @@ struct keds_index {
   bool timing_on = false;
   DevBuf timing;
   size_t timing_launches = 0;
-  // optional per-launch timing of the scoring kernel (bench.py's roofline leg)
-  bool profiling = false;
-  std::vector<cudaEvent_t> prof_ev;
-  std::vector<int> prof_tag;
-  size_t prof_used = 0;
 };
 
 namespace {
@@ -440,6 +443,15 @@ Plan make_plan(const keds_index* ix, int n_db, int64_t nq, int k, int64_t n_min,
   return pl;
 }
 
+// Gallery ranking: as many candidate lists as the tiles and the candidate budget allow (the band
+// around a mid-ranked target is crowded); never exact-only.
+Plan rank_plan(const keds_index* ix, int64_t nq) {
+  Plan pl{geometry(ix, 1, nq)};
+  const int T = static_cast<int>((ix->n + BN - 1) / BN);
+  pl.set_slices(1, static_cast<int>(std::max<long long>(1, std::min<long long>(std::min(T, S_MAX), pl.s_mem))));
+  return pl;
+}
+
 int ensure_q_map(keds_index* ix, int64_t rows_needed, cudaStream_t st) {
   const size_t bytes = static_cast<size_t>(rows_needed) * ix->d_pad * 2;
   if (bytes > ix->q_bf16.cap) {
@@ -460,24 +472,6 @@ int ensure_q_map(keds_index* ix, int64_t rows_needed, cudaStream_t st) {
   return 0;
 }
 
-// Stage marks (diagnostics; they sit between the kernels, so they suppress the programmatic
-// overlap they measure around): tag 0 opens a search, tag t closes stage t
-// (1 prep_rows, 2 score_topk, 3 select_rerank, 4 exact fallback pair).
-constexpr int PROF_STAGES = 6;
-int prof_mark(keds_index* a, cudaStream_t st, int tag) {
-  if (!a->profiling) return 0;
-  if (a->prof_used == a->prof_ev.size()) {
-    cudaEvent_t e;
-    CK(cudaEventCreate(&e));
-    a->prof_ev.push_back(e);
-    a->prof_tag.push_back(0);
-  }
-  CK(cudaEventRecord(a->prof_ev[a->prof_used], st));
-  a->prof_tag[a->prof_used] = tag;
-  a->prof_used++;
-  return 0;
-}
-
 // One search call. The entry points fill it with the caller's arrays; search_impl puts host
 // queries and results into device staging before the first pass, and every pass gets a slice.
 struct Call {
@@ -490,8 +484,8 @@ struct Call {
   uint32_t flags = 0;
   int pass = 0;                  // status block of this pass
   const float* q = nullptr;      // fp32 [nq][d]
-  const float* q_src = nullptr;  // device alias of page-locked host queries, or null: k_prep_rows reads
-                                 // them through the mapping and leaves the fp32 copy in q
+  const float* q_src = nullptr;  // page-locked host queries (device alias) or a misaligned query tensor
+                                 // (gallery ranking), or null: k_prep_rows reads them and leaves the fp32 copy in q
   float* D[2] = {nullptr, nullptr};  // [nq][k] per database
   long long* I[2] = {nullptr, nullptr};
   // optional parts, absent while zero
@@ -500,6 +494,7 @@ struct Call {
   const long long* ex = nullptr;  // [nq][n_ex] labels to leave out (device memory or a mapped host alias);
   int n_ex = 0;                   // k_prep_rows stages them as local row ids in owner->ex_rows
   HitsMode hits{};                // label hits at cut points in the re-rank's place
+  RankMode rank{};                // gallery ranks in the top-k's place (rank.out set)
   float* dump = nullptr;          // debug_scores: the raw scores, ld_dump per query
   int64_t ld_dump = 0;
 
@@ -627,44 +622,124 @@ int ensure_cand(keds_index* a, size_t lines) {
   return 0;
 }
 
-// What every launch of the scoring kernel is given: the plan, the databases, the candidate lists
-// and the error word. The rest is zero: the caller adds its epilogue's inputs.
-ScoreParams score_params(const keds_index* a, keds_index* const* dbs, int n_db, const Plan& pl, int64_t nq,
-                         unsigned int* err) {
+// What every launch of the scoring kernel of a pass is given: the plan, the databases, the
+// candidate lists and the error word, and a search's epilogue inputs (row bias, warm-start
+// thresholds, exclusion, debug dump). Gallery ranking adds its band edges (launch_rank_targets).
+ScoreParams score_params(const Call& c, const Plan& pl, unsigned long long* tchain) {
+  const keds_index* a = c.owner;
   ScoreParams sp;
   memset(&sp, 0, sizeof sp);
-  sp.n_db = n_db;
+  sp.n_db = c.n_db;
   sp.n_qt = pl.n_qt;
   sp.n_qg = pl.n_qg;
   sp.S = pl.S;
   sp.n_items = pl.n_items;
   sp.kblocks = a->d_pad / BK;
   sp.fmt_bits = a->fmt == FMT_BF16 ? kIdescBf16Bits : 0u;
-  sp.nq = static_cast<int>(nq);
-  for (int i = 0; i < n_db; ++i) {
-    sp.n_rows[i] = static_cast<int>(dbs[i]->n);
-    sp.n_tiles[i] = static_cast<int>((dbs[i]->n + BN - 1) / BN);
+  sp.nq = static_cast<int>(c.nq);
+  for (int i = 0; i < c.n_db; ++i) {
+    sp.n_rows[i] = static_cast<int>(c.dbs[i]->n);
+    sp.n_tiles[i] = static_cast<int>((c.dbs[i]->n + BN - 1) / BN);
   }
   sp.cand = a->cand.as<uint2>();
   sp.cand_cnt = a->cand_cnt.as<int>();
   sp.cand_theta = a->cand_theta.as<float>();
-  sp.err = err;
+  sp.err = a->ctrl_cur + 2;
+  if (c.rank.out) return sp;
+  for (int i = 0; i < c.n_db; ++i) sp.bias[i] = c.metric() == METRIC_L2 ? c.dbs[i]->bias.as<float>() : nullptr;
+  sp.theta0 = a->warm_start ? a->theta0.as<float>() : nullptr;
+  sp.theta_ld = pl.n_qt * BM;
+  sp.dump = c.dump;
+  sp.ld_dump = c.ld_dump;
+  sp.timing = tchain ? tchain + 2 : nullptr;
+  if (c.ex) {
+    sp.ex_rows = a->ex_rows.as<int>();
+    sp.n_ex = c.n_ex;
+    sp.ex_ld = static_cast<long long>(c.nq) * c.n_ex;
+  }
   return sp;
+}
+
+// The front of a pass: the status block cleared, the exclusion labels staged, and the queries'
+// 16-bit operand rows and statistics (with the fp32 device copy of queries read from q_src).
+// On the exact-only route no query rows are prepared: every query is flagged for the fallback.
+int launch_prep(const Call& c, const Plan& pl, unsigned long long* tchain, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const int n_db = c.n_db;
+  const int64_t nq = c.nq;
+  PrepParams pp;
+  memset(&pp, 0, sizeof pp);
+  pp.d = a->d;
+  pp.d_pad = a->d_pad;
+  pp.fmt = a->fmt;
+  if (c.ex) {
+    CKS(a->ex_rows.ensure(static_cast<size_t>(n_db) * nq * c.n_ex * 4));
+    pp.ex.labels = c.ex;
+    pp.ex.nq = nq;
+    pp.ex.n_ex = c.n_ex;
+    pp.ex.n_db = n_db;
+    pp.ex.rows = a->ex_rows.as<int>();
+    for (int i = 0; i < n_db; ++i) {
+      pp.ex.id_offset[i] = c.dbs[i]->id_offset;
+      pp.ex.n_rows[i] = c.dbs[i]->n;
+    }
+  }
+  if (pl.exact_only) {
+    if (c.q_src) CK(cudaMemcpyAsync(const_cast<float*>(c.q), c.q_src, static_cast<size_t>(nq) * a->d * 4, cudaMemcpyDefault, st));
+    CK(cudaMemsetAsync(a->ctrl_cur, 0, CTRL_STRIDE * 4, st));
+    for (int i = 0; i < n_db; ++i) {
+      k_flag_all<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, st>>>(
+          a->flagged[i].as<int>(), reinterpret_cast<int*>(a->ctrl_cur) + i, static_cast<int>(nq));
+      a->stats.launches++;
+    }
+    if (c.ex) {
+      // the staging half of k_prep_rows alone (no query rows to prepare on this route)
+      const unsigned blocks = static_cast<unsigned>(std::min<long long>((nq + 255) / 256, 1024));
+      k_prep_rows<<<blocks, 256, 0, st>>>(pp);
+      a->stats.launches++;
+    }
+    return 0;
+  }
+  // operands: bf16 queries + per-query residual norms
+  const int64_t q_rows = static_cast<int64_t>(pl.n_qt) * BM;
+  CKS(ensure_q_map(a, q_rows, st));
+  CKS(a->qstat.ensure(static_cast<size_t>(nq) * sizeof(float4)));
+  pp.x = c.q_src ? c.q_src : c.q;
+  pp.n = nq;
+  pp.out = a->q_bf16.as<uint16_t>();
+  pp.stat = a->qstat.as<float4>();
+  pp.zero_words = a->ctrl_cur;
+  pp.n_zero = CTRL_STRIDE;
+  pp.timing = tchain;
+  pp.copy_f32 = c.q_src ? const_cast<float*>(c.q) : nullptr;
+  if (!c.rank.out) {  // the lists' warm-start thresholds (gallery ranking starts from its band edges)
+    CKS(a->theta0.ensure(static_cast<size_t>(n_db) * q_rows * 4));
+    pp.neg_inf_words = a->theta0.as<float>();
+    pp.n_neg_inf = static_cast<int>(n_db * q_rows);
+  }
+  const unsigned blocks = static_cast<unsigned>(std::min<long long>((nq * 32 + 255) / 256, 4096));  // a warp per query
+  CKS(launch_k(a->use_pdl, k_prep_rows, dim3(blocks), dim3(256), 0, st, pp));
+  a->stats.launches++;
+  return 0;
 }
 
 // The scoring kernel in the instantiation sp asks for: gallery ranking (rk_lo), top-k with
 // exclusion (ex_rows: tests each tile against the query's excluded rows) or the plain top-k.
-int launch_score(keds_index* a, keds_index* const* dbs, int n_db, const Plan& pl, const ScoreParams& sp,
-                 cudaStream_t st) {
-  const keds_index* x1 = n_db > 1 ? dbs[1] : dbs[0];
+int launch_score(const Call& c, const Plan& pl, const ScoreParams& sp, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const keds_index* x0 = c.dbs[0];
+  const keds_index* x1 = c.n_db > 1 ? c.dbs[1] : c.dbs[0];
   if (pl.pair)
-    return launch_kc(a->use_pdl, 2,
-                     sp.rk_lo ? k_score_topk<true, true> : sp.ex_rows ? k_score_topk<true, false, true> : k_score_topk<true>,
-                     dim3(pl.grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, dbs[0]->tm_xh,
-                     x1->tm_xh, sp);
-  return launch_k(a->use_pdl,
-                  sp.rk_lo ? k_score_topk<false, true> : sp.ex_rows ? k_score_topk<false, false, true> : k_score_topk<false>,
-                  dim3(pl.grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, dbs[0]->tm_x, x1->tm_x, sp);
+    CKS(launch_kc(a->use_pdl, 2,
+                  sp.rk_lo ? k_score_topk<true, true> : sp.ex_rows ? k_score_topk<true, false, true> : k_score_topk<true>,
+                  dim3(pl.grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, x0->tm_xh, x1->tm_xh, sp));
+  else
+    CKS(launch_k(a->use_pdl,
+                 sp.rk_lo ? k_score_topk<false, true> : sp.ex_rows ? k_score_topk<false, false, true> : k_score_topk<false>,
+                 dim3(pl.grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, x0->tm_x, x1->tm_x, sp));
+  a->stats.launches++;
+  CK(cudaGetLastError());
+  return 0;
 }
 
 // Candidate capacity per query of the re-rank and hits blocks: room for the band a recent search
@@ -677,22 +752,188 @@ int cand_capacity(int k, unsigned int band_hint) {
   return rmax;
 }
 
-// One pass (<= Q_PASS_MAX queries) of a call; q, D and I are device memory.
+// The top-k from the candidate lists: exact fp32 scores of the rows at or above the certified
+// threshold, the queries the certificate rejects flagged for the fallback.
+int launch_rerank(const Call& c, const Plan& pl, const ScoreParams& sp, unsigned int band_hint,
+                  unsigned long long* tchain, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const int n_db = c.n_db, k = c.k;
+  const int64_t nq = c.nq;
+  RerankParams rp;
+  memset(&rp, 0, sizeof rp);
+  rp.n_db = n_db;
+  rp.n_qt = pl.n_qt;
+  rp.S = pl.S * pl.sub;  // candidate lines per (database, query)
+  rp.nq = static_cast<int>(nq);
+  rp.k = k;
+  rp.d = a->d;
+  rp.metric = c.metric();
+  rp.cand = sp.cand;
+  rp.cand_cnt = sp.cand_cnt;
+  rp.cand_theta = sp.cand_theta;
+  rp.q_f32 = c.q;
+  rp.qstat = a->qstat.as<float4>();
+  for (int i = 0; i < n_db; ++i) {
+    rp.x_f32[i] = c.dbs[i]->x_f32.as<float>();
+    rp.dbstat[i] = c.dbs[i]->dbstat.as<unsigned int>();
+    rp.D[i] = c.D[i];
+    rp.I[i] = c.I[i];
+    rp.id_offset[i] = c.dbs[i]->id_offset;
+    rp.flagged[i] = a->flagged[i].as<int>();
+    rp.n_flagged[i] = reinterpret_cast<int*>(a->ctrl_cur) + i;
+  }
+  rp.eps_scale = a->eps_scale;
+  rp.band_max = a->ctrl_cur + CTRL_BAND;
+  // A single wave (the latency variant) has the shared memory to spare: full candidate capacity.
+  // Large batches live on blocks per SM, so they start small and follow the band a recent search reported.
+  const int rmax = pl.small_batch ? R_MAX : cand_capacity(k, band_hint);
+  rp.rmax = rmax;
+  rp.peer = c.peer;
+  rp.cons = c.cons;
+  rp.timing = tchain ? tchain + 4 : nullptr;
+  const size_t slots = static_cast<size_t>(pl.S) * pl.sub * LKEEP;
+  // qvec | part | okey | keys, ids | smax | a_key, a_id, sel_id, sel_sc | hist | red | bcast | counters | top_*
+  const size_t smem = static_cast<size_t>((a->d + 3) & ~3) * 4 + static_cast<size_t>(c.cons.part4) * 16 +
+                      static_cast<size_t>(rmax) * 24 + slots * 8 + pl.S * pl.sub * 4 + 256 * 4 + 32 * 4 + 16 + 16 +
+                      static_cast<size_t>(k) * 12;
+  if (smem > 200 * 1024) return fail(KEDS_ERR_ARG, "re-rank shared memory %zu too large", smem);
+  if (pl.small_batch)
+    CKS(launch_k(a->use_pdl, k_select_rerank<3, 2>, dim3(static_cast<unsigned>(nq), n_db),
+                 dim3(RERANK_THREADS), smem, st, rp));
+  else if (k >= 128 && a->rerank_threads_large == 128)
+    // hundreds of fp32 rows per query: two rows per warp in flight (80 registers, six blocks per
+    // SM) measured 0.82-0.87 ms against 0.95-1.0 at 10,000 x 50k, k = 200; at k = 16 / 64 the
+    // 64-register variant below is 5-10 % faster
+    CKS(launch_k(a->use_pdl, k_select_rerank<2, 6, 128>, dim3(static_cast<unsigned>(nq), n_db),
+                 dim3(128), smem, st, rp));
+  else
+    CKS(launch_k(a->use_pdl, k_select_rerank<1, 4>, dim3(static_cast<unsigned>(nq), n_db),
+                 dim3(a->rerank_threads_large), smem, st, rp));
+  a->stats.launches++;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// Label hits at the cut points instead of the ranked rows (label_hits.cuh): same lists, same
+// certificate, exact scores only for the rows inside the error band around a cut.
+int launch_hits(const Call& c, const Plan& pl, const ScoreParams& sp, unsigned int band_hint,
+                unsigned long long* tchain, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const HitsMode& hm = c.hits;
+  HitsParams hp;
+  memset(&hp, 0, sizeof hp);
+  hp.n_qt = pl.n_qt;
+  hp.S = pl.S * pl.sub;
+  hp.nq = static_cast<int>(c.nq);
+  hp.d = a->d;
+  hp.metric = c.metric();
+  hp.nks = hm.nks;
+  for (int j = 0; j < hm.nks; ++j) hp.ks[j] = hm.ks[j];
+  const int rmax = cand_capacity(c.k, band_hint);
+  hp.rmax = rmax;
+  hp.cand = sp.cand;
+  hp.cand_cnt = sp.cand_cnt;
+  hp.cand_theta = sp.cand_theta;
+  hp.q_f32 = c.q;
+  hp.qstat = a->qstat.as<float4>();
+  hp.x_f32 = c.dbs[0]->x_f32.as<float>();
+  hp.dbstat = c.dbs[0]->dbstat.as<unsigned int>();
+  hp.row_labels = hm.row_labels;
+  hp.qlabel = hm.qlabel;
+  hp.hits = hm.hits;
+  hp.flagged = a->flagged[0].as<int>();
+  hp.n_flagged = reinterpret_cast<int*>(a->ctrl_cur);
+  hp.eps_scale = a->eps_scale;
+  hp.band_max = a->ctrl_cur + CTRL_BAND;
+  hp.timing = tchain ? tchain + 4 : nullptr;
+  const size_t hslots = static_cast<size_t>(pl.S) * pl.sub * LKEEP;
+  // qvec | cs | keys, ids | c_sc, c_info, amb | hist | red | bcast | counters | n_cert, band_end, n_hit
+  const size_t hsmem = static_cast<size_t>((a->d + 3) & ~3) * 4 + hslots * 8 + static_cast<size_t>(rmax) * 20 +
+                       1024 * 4 + 32 * 4 + 16 + 16 + 3 * HITS_MAX_CUTS * 4;
+  if (hsmem > 200 * 1024) return fail(KEDS_ERR_ARG, "label-hits shared memory %zu too large", hsmem);
+  // <2 rows in flight per warp, 6 blocks per SM>: measured 0.55 ms at 10,000 x 50k against 0.68 (<3, 4>) / 0.57 (<1, 8>)
+  CKS(launch_k(a->use_pdl, k_select_hits<2, 6>, dim3(static_cast<unsigned>(c.nq)), dim3(HITS_THREADS), hsmem, st, hp));
+  a->stats.launches++;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// Label hits behind the exact fallback: the queued queries' exact rows (written by the fallback
+// just now) -> their hits.
+int launch_hits_from_rows(const Call& c, cudaStream_t st) {
+  keds_index* a = c.owner;
+  HitsParams hp;
+  memset(&hp, 0, sizeof hp);
+  hp.nks = c.hits.nks;
+  for (int j = 0; j < c.hits.nks; ++j) hp.ks[j] = c.hits.ks[j];
+  hp.hits = c.hits.hits;
+  CKS(launch_k(a->use_pdl, k_hits_from_rows, dim3(static_cast<unsigned>(std::min<int64_t>((c.nq + 127) / 128, 64))),
+               dim3(128), 0, st, a->flagged[0].as<int>(), reinterpret_cast<int*>(a->ctrl_cur), c.I[0], c.k,
+               c.dbs[0]->id_offset, c.hits.row_labels, c.hits.qlabel, hp));
+  a->stats.launches++;
+  return 0;
+}
+
+// Shared memory of k_gallery_rank: 8 queries per block
+size_t gallery_rank_smem(int d) { return static_cast<size_t>((d + 3) & ~3) * 4 * 8; }
+
+// Gallery ranking, before the scoring kernel: each query's exact fp32 target score and the error
+// band around it, which the scoring kernel's counting epilogue reads.
+int launch_rank_targets(const Call& c, ScoreParams& sp, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const keds_index* g = c.dbs[0];
+  const int64_t nq = c.nq;
+  CKS(a->rk.ensure(static_cast<size_t>(nq) * 5 * 4));
+  float* rk_st = a->rk.as<float>();
+  float* rk_lo = rk_st + nq;
+  float* rk_hi = rk_lo + nq;
+  int* rk_t = reinterpret_cast<int*>(rk_hi + nq);
+  int* rk_e = rk_t + nq;
+  CKS(launch_k(a->use_pdl, k_rank_targets, dim3(static_cast<unsigned>((nq * 32 + 255) / 256)), dim3(256), 0, st, c.q,
+               nq, g->x_f32.as<float>(), g->d, c.rank.target, c.rank.exclude, a->qstat.as<float4>(),
+               g->dbstat.as<unsigned int>(), a->eps_scale, rk_st, rk_lo, rk_hi, rk_t, rk_e));
+  a->stats.launches++;
+  sp.rk_lo = rk_lo;
+  sp.rk_hi = rk_hi;
+  sp.rk_target = rk_t;
+  sp.rk_exclude = c.rank.exclude ? rk_e : nullptr;
+  return 0;
+}
+
+// Gallery ranking, after the scoring kernel: the lists' certain counts plus the band rows settled
+// exactly (k_rank_finish), then the exact recount of the queries whose band overflowed a list
+// (k_gallery_rank over the queue; none, normally: its blocks leave at once).
+int launch_rank_count(const Call& c, const Plan& pl, const ScoreParams& sp, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const keds_index* g = c.dbs[0];
+  const int64_t nq = c.nq;
+  int* queue = a->flagged[0].as<int>();
+  int* n_queue = reinterpret_cast<int*>(a->ctrl_cur);
+  CKS(launch_k(a->use_pdl, k_rank_finish, dim3(static_cast<unsigned>((nq * 32 + 255) / 256)), dim3(256), 0, st, c.q,
+               nq, g->x_f32.as<float>(), g->d, pl.S * pl.sub, pl.n_qt, sp.cand, sp.cand_cnt, sp.cand_theta,
+               a->rk.as<float>(), sp.rk_target, c.rank.out, queue, n_queue));
+  CKS(launch_k(a->use_pdl, k_gallery_rank, dim3(static_cast<unsigned>((nq + 7) / 8)), dim3(256), gallery_rank_smem(g->d),
+               st, c.q, nq, g->x_f32.as<float>(), g->n, g->d, c.rank.target, c.rank.exclude, c.rank.out, queue, n_queue));
+  a->stats.launches += 2;
+  CK(cudaGetLastError());
+  return 0;
+}
+
+// One pass (<= Q_PASS_MAX queries) of a call; q, D and I are device memory. The chain: prep, the
+// scoring kernel and its epilogue (re-rank, label hits or the rank count), the exact fallback.
 int search_pass(const Call& c, cudaStream_t st) {
   keds_index* a = c.owner;
   keds_index* const* ix = c.dbs;
-  const int n_db = c.n_db, k = c.k, metric = c.metric();
+  const int n_db = c.n_db;
   const int64_t nq = c.nq;
   CKS(set_kernel_attrs(a));
   // in-kernel %globaltimer stamps, one {min start, max end} pair per kernel of this chain
   // (prep, score, rerank, exact scores, exact select); the first TIMING_RING searches are timed
   unsigned long long* tchain = nullptr;
-  if (a->timing_on && a->timing_launches < TIMING_RING && !c.dump) {
+  if (a->timing_on && a->timing_launches < TIMING_RING && !c.dump && !c.rank.out) {
     tchain = a->timing.as<unsigned long long>() + TIMING_PAIRS * 2 * a->timing_launches;
     a->timing_launches++;
   }
-  // (a multi-pass call sizes the status blocks of all its passes before the first launch)
-  CKS(a->ctrl.ensure(static_cast<size_t>(c.pass + 1) * CTRL_STRIDE * 4));
   a->ctrl_cur = a->ctrl.as<unsigned int>() + static_cast<size_t>(c.pass) * CTRL_STRIDE;
   a->ctrl_passes = c.pass + 1;
   a->ctrl_slot = c.slot0;
@@ -704,197 +945,25 @@ int search_pass(const Call& c, cudaStream_t st) {
     n_max = std::max(n_max, ix[1]->n);
   }
   const unsigned int band_hint = a->h_feedback ? *static_cast<volatile unsigned int*>(a->h_feedback) : 0u;
-  Plan pl = make_plan(a, n_db, nq, k, n_min, n_max, c.flags, band_hint);
+  const Plan pl = c.rank.out ? rank_plan(a, nq) : make_plan(a, n_db, nq, c.k, n_min, n_max, c.flags, band_hint);
   if (c.dump && pl.exact_only) return fail(KEDS_ERR_ARG, "debug_scores needs at least one 256-row tile");
-  ExcludeStage exs;
-  memset(&exs, 0, sizeof exs);
-  if (c.ex) {
-    CKS(a->ex_rows.ensure(static_cast<size_t>(n_db) * nq * c.n_ex * 4));
-    exs.labels = c.ex;
-    exs.nq = nq;
-    exs.n_ex = c.n_ex;
-    exs.n_db = n_db;
-    exs.rows = a->ex_rows.as<int>();
-    for (int i = 0; i < n_db; ++i) {
-      exs.id_offset[i] = ix[i]->id_offset;
-      exs.n_rows[i] = ix[i]->n;
-    }
-  }
   a->stats.exact_only = pl.exact_only;
   a->stats.slices = pl.S;
   a->stats.items = pl.n_items;
   a->stats.grid = pl.grid;
 
-  if (pl.exact_only) {
-    if (c.q_src) CK(cudaMemcpyAsync(const_cast<float*>(c.q), c.q_src, static_cast<size_t>(nq) * a->d * 4, cudaMemcpyDefault, st));
-    CK(cudaMemsetAsync(a->ctrl_cur, 0, CTRL_STRIDE * 4, st));
-    for (int i = 0; i < n_db; ++i) {
-      k_flag_all<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, st>>>(
-          a->flagged[i].as<int>(), reinterpret_cast<int*>(a->ctrl_cur) + i, static_cast<int>(nq));
-      a->stats.launches++;
-    }
-    if (c.ex) {
-      // the staging half of k_prep_rows alone (no query rows to prepare on this route)
-      const unsigned blocks = static_cast<unsigned>(std::min<long long>((nq + 255) / 256, 1024));
-      k_prep_rows<<<blocks, 256, 0, st>>>(nullptr, 0, a->d, a->d_pad, a->fmt, nullptr, nullptr, nullptr, nullptr,
-                                          nullptr, 0, nullptr, 0, nullptr, nullptr, exs);
-      a->stats.launches++;
-    }
-  } else {
-    // operands: bf16 queries + per-query residual norms
-    const int64_t q_rows = static_cast<int64_t>(pl.n_qt) * BM;
-    CKS(ensure_q_map(a, q_rows, st));
-    CKS(a->qstat.ensure(static_cast<size_t>(nq) * sizeof(float4)));
-    const int64_t theta_ld = q_rows;
-    CKS(a->theta0.ensure(static_cast<size_t>(n_db) * theta_ld * 4));
-    {
-      CKS(prof_mark(a, st, 0));
-      const int threads = 256;
-      const long long warps_needed = nq;
-      const unsigned blocks =
-          static_cast<unsigned>(std::min<long long>((warps_needed * 32 + threads - 1) / threads, 4096));
-      CKS(launch_k(a->use_pdl, k_prep_rows, dim3(blocks), dim3(threads), 0, st, c.q_src ? c.q_src : c.q,
-                   static_cast<long long>(nq), a->d, a->d_pad, a->fmt, a->q_bf16.as<uint16_t>(),
-                   a->qstat.as<float4>(), static_cast<float*>(nullptr), static_cast<unsigned int*>(nullptr),
-                   a->ctrl_cur, CTRL_STRIDE, a->theta0.as<float>(), static_cast<int>(n_db * theta_ld), tchain,
-                   c.q_src ? const_cast<float*>(c.q) : static_cast<float*>(nullptr), exs));
-      a->stats.launches++;
-    }
+  CKS(launch_prep(c, pl, tchain, st));
+  if (!pl.exact_only) {
     CKS(ensure_cand(a, static_cast<size_t>(n_db) * pl.S * pl.sub * pl.n_qt));
-    ScoreParams sp = score_params(a, ix, n_db, pl, nq, a->ctrl_cur + 2);
-    for (int i = 0; i < n_db; ++i) sp.bias[i] = metric == METRIC_L2 ? ix[i]->bias.as<float>() : nullptr;
-    sp.theta0 = a->warm_start ? a->theta0.as<float>() : nullptr;
-    sp.theta_ld = static_cast<int>(theta_ld);
-    sp.dump = c.dump;
-    sp.ld_dump = c.ld_dump;
-    sp.timing = tchain ? tchain + 2 : nullptr;
-    if (c.ex) {
-      sp.ex_rows = exs.rows;
-      sp.n_ex = c.n_ex;
-      sp.ex_ld = static_cast<long long>(nq) * c.n_ex;
-    }
-    CKS(prof_mark(a, st, 1));
-    CKS(launch_score(a, ix, n_db, pl, sp, st));
-    CKS(prof_mark(a, st, 2));
-    a->stats.launches++;
-    CK(cudaGetLastError());
+    ScoreParams sp = score_params(c, pl, tchain);
+    if (c.rank.out) CKS(launch_rank_targets(c, sp, st));
+    CKS(launch_score(c, pl, sp, st));
     if (c.dump) return 0;
-
-    if (c.hits.nks) {
-      // label hits at the cut points instead of the ranked rows (label_hits.cuh): same lists, same
-      // certificate, exact scores only for the rows inside the error band around a cut
-      const HitsMode& hm = c.hits;
-      HitsParams hp;
-      memset(&hp, 0, sizeof hp);
-      hp.n_qt = pl.n_qt;
-      hp.S = pl.S * pl.sub;
-      hp.nq = static_cast<int>(nq);
-      hp.d = a->d;
-      hp.metric = metric;
-      hp.nks = hm.nks;
-      for (int j = 0; j < hm.nks; ++j) hp.ks[j] = hm.ks[j];
-      const int rmax = cand_capacity(k, band_hint);
-      hp.rmax = rmax;
-      hp.cand = sp.cand;
-      hp.cand_cnt = sp.cand_cnt;
-      hp.cand_theta = sp.cand_theta;
-      hp.q_f32 = c.q;
-      hp.qstat = a->qstat.as<float4>();
-      hp.x_f32 = ix[0]->x_f32.as<float>();
-      hp.dbstat = ix[0]->dbstat.as<unsigned int>();
-      hp.row_labels = hm.row_labels;
-      hp.qlabel = hm.qlabel;
-      hp.hits = hm.hits;
-      hp.flagged = a->flagged[0].as<int>();
-      hp.n_flagged = reinterpret_cast<int*>(a->ctrl_cur);
-      hp.eps_scale = a->eps_scale;
-      hp.band_max = a->ctrl_cur + CTRL_BAND;
-      hp.timing = tchain ? tchain + 4 : nullptr;
-      const size_t hslots = static_cast<size_t>(pl.S) * pl.sub * LKEEP;
-      // qvec | cs | keys, ids | c_sc, c_info, amb | hist | red | bcast | counters | n_cert, band_end, n_hit
-      const size_t hsmem = static_cast<size_t>((a->d + 3) & ~3) * 4 + hslots * 8 + static_cast<size_t>(rmax) * 20 +
-                           1024 * 4 + 32 * 4 + 16 + 16 + 3 * HITS_MAX_CUTS * 4;
-      if (hsmem > 200 * 1024) return fail(KEDS_ERR_ARG, "label-hits shared memory %zu too large", hsmem);
-      // <2 rows in flight per warp, 6 blocks per SM>: measured 0.55 ms at 10,000 x 50k against 0.68 (<3, 4>) / 0.57 (<1, 8>)
-      CKS(launch_k(a->use_pdl, k_select_hits<2, 6>, dim3(static_cast<unsigned>(nq)), dim3(HITS_THREADS), hsmem, st, hp));
-      CKS(prof_mark(a, st, 3));
-      a->stats.launches++;
-      CK(cudaGetLastError());
-    } else {
-    RerankParams rp;
-    memset(&rp, 0, sizeof rp);
-    rp.n_db = n_db;
-    rp.n_qt = pl.n_qt;
-    rp.S = pl.S * pl.sub;  // candidate lines per (database, query)
-    rp.nq = static_cast<int>(nq);
-    rp.k = k;
-    rp.d = a->d;
-    rp.metric = metric;
-    rp.cand = sp.cand;
-    rp.cand_cnt = sp.cand_cnt;
-    rp.cand_theta = sp.cand_theta;
-    rp.q_f32 = c.q;
-    rp.qstat = a->qstat.as<float4>();
-    for (int i = 0; i < n_db; ++i) {
-      rp.x_f32[i] = ix[i]->x_f32.as<float>();
-      rp.dbstat[i] = ix[i]->dbstat.as<unsigned int>();
-      rp.D[i] = c.D[i];
-      rp.I[i] = c.I[i];
-      rp.id_offset[i] = ix[i]->id_offset;
-      rp.flagged[i] = a->flagged[i].as<int>();
-      rp.n_flagged[i] = reinterpret_cast<int*>(a->ctrl_cur) + i;
-    }
-    rp.eps_scale = a->eps_scale;
-    rp.band_max = a->ctrl_cur + CTRL_BAND;
-    // one wave of blocks (two per SM): the latency variant; more: the four-per-SM throughput variant
-    const bool small_batch = pl.small_batch;
-    // A single wave has the shared memory to spare: full candidate capacity. Large batches live on
-    // blocks per SM, so they start small and follow the band a recent search reported.
-    const int rmax = small_batch ? R_MAX : cand_capacity(k, band_hint);
-    rp.rmax = rmax;
-    rp.peer = c.peer;
-    rp.cons = c.cons;
-    rp.timing = tchain ? tchain + 4 : nullptr;
-    const size_t slots = static_cast<size_t>(pl.S) * pl.sub * LKEEP;
-    // qvec | part | okey | keys, ids | smax | a_key, a_id, sel_id, sel_sc | hist | red | bcast | counters | top_*
-    const size_t smem = static_cast<size_t>((a->d + 3) & ~3) * 4 + static_cast<size_t>(c.cons.part4) * 16 +
-                        static_cast<size_t>(rmax) * 24 + slots * 8 + pl.S * pl.sub * 4 + 256 * 4 + 32 * 4 + 16 + 16 +
-                        static_cast<size_t>(k) * 12;
-    if (smem > 200 * 1024) return fail(KEDS_ERR_ARG, "re-rank shared memory %zu too large", smem);
-    if (small_batch)
-      CKS(launch_k(a->use_pdl, k_select_rerank<3, 2>, dim3(static_cast<unsigned>(nq), n_db),
-                   dim3(RERANK_THREADS), smem, st, rp));
-    else if (k >= 128 && a->rerank_threads_large == 128)
-      // hundreds of fp32 rows per query: two rows per warp in flight (80 registers, six blocks per
-      // SM) measured 0.82-0.87 ms against 0.95-1.0 at 10,000 x 50k, k = 200; at k = 16 / 64 the
-      // 64-register variant below is 5-10 % faster
-      CKS(launch_k(a->use_pdl, k_select_rerank<2, 6, 128>, dim3(static_cast<unsigned>(nq), n_db),
-                   dim3(128), smem, st, rp));
-    else
-      CKS(launch_k(a->use_pdl, k_select_rerank<1, 4>, dim3(static_cast<unsigned>(nq), n_db),
-                   dim3(a->rerank_threads_large), smem, st, rp));
-    CKS(prof_mark(a, st, 3));
-    a->stats.launches++;
-    CK(cudaGetLastError());
-    }
+    if (c.rank.out) return launch_rank_count(c, pl, sp, st);
+    CKS(c.hits.nks ? launch_hits(c, pl, sp, band_hint, tchain, st) : launch_rerank(c, pl, sp, band_hint, tchain, st));
   }
-  if (!(c.flags & KEDS_SEARCH_NO_FALLBACK) || pl.exact_only) {
-    CKS(launch_exact(c, tchain ? tchain + 6 : nullptr, st));
-    CKS(prof_mark(a, st, 4));
-  }
-  if (c.hits.nks) {
-    // the queued queries' exact rows (written by the fallback just now) -> their hits
-    HitsParams hp;
-    memset(&hp, 0, sizeof hp);
-    hp.nks = c.hits.nks;
-    for (int j = 0; j < c.hits.nks; ++j) hp.ks[j] = c.hits.ks[j];
-    hp.hits = c.hits.hits;
-    CKS(launch_k(a->use_pdl, k_hits_from_rows, dim3(static_cast<unsigned>(std::min<int64_t>((nq + 127) / 128, 64))),
-                 dim3(128), 0, st, static_cast<const int*>(a->flagged[0].as<int>()),
-                 static_cast<const int*>(reinterpret_cast<int*>(a->ctrl_cur)), static_cast<const long long*>(c.I[0]), k,
-                 static_cast<long long>(ix[0]->id_offset), c.hits.row_labels, c.hits.qlabel, hp));
-    a->stats.launches++;
-  }
+  if (!(c.flags & KEDS_SEARCH_NO_FALLBACK) || pl.exact_only) CKS(launch_exact(c, tchain ? tchain + 6 : nullptr, st));
+  if (c.hits.nks) CKS(launch_hits_from_rows(c, st));
   CK(cudaGetLastError());
   return 0;
 }
@@ -937,13 +1006,20 @@ Call slice(const Call& c, int64_t q0, int64_t nb) {
     p.hits.qlabel += q0;
     p.hits.hits += q0 * p.hits.nks;
   }
+  if (p.rank.out) {
+    p.rank.target += q0;
+    if (p.rank.exclude) p.rank.exclude += q0;
+    p.rank.out += q0;
+  }
   return p;
 }
 
 // Every pass of a call, queued back to back: each pass has its own status block and the scratch is
 // reused in stream order (each kernel of a chain waits for its predecessor to complete), so the
-// passes need no host round trip between them.
+// passes need no host round trip between them. The status blocks are sized before the first launch:
+// growing them later would free memory that kernels of an earlier pass still write.
 int run_passes(const Call& c, cudaStream_t st) {
+  CKS(c.owner->ctrl.ensure(static_cast<size_t>((c.nq + Q_PASS_MAX - 1) / Q_PASS_MAX) * CTRL_STRIDE * 4));
   for (int64_t q0 = 0; q0 < c.nq; q0 += Q_PASS_MAX)
     CKS(search_pass(slice(c, q0, std::min<int64_t>(Q_PASS_MAX, c.nq - q0)), st));
   return 0;
@@ -1059,8 +1135,7 @@ int search_impl(Call c, Io io, void* stream) {
     c.D[i] = a->D_stage[i].as<float>();
     c.I[i] = a->I_stage[i].as<long long>();
   }
-  // status blocks of every pass, sized before the first launch (growing them later would free
-  // memory that kernels of an earlier pass still write)
+  // status blocks of every pass (the empty-database route clears them)
   const int n_passes = static_cast<int>((nq + Q_PASS_MAX - 1) / Q_PASS_MAX);
   CKS(a->ctrl.ensure(static_cast<size_t>(n_passes) * CTRL_STRIDE * 4));
   if (ix[0]->n == 0 || (n_db > 1 && ix[1]->n == 0)) {
@@ -1205,7 +1280,6 @@ void keds_index_free(keds_index_t* ix) {
   ix->h_q.release();
   ix->h_out.release();
   if (ix->h_feedback) cudaFreeHost(ix->h_feedback);
-  for (cudaEvent_t e : ix->prof_ev) cudaEventDestroy(e);
   delete ix;
 }
 
@@ -1235,10 +1309,17 @@ static int prep_db_rows(keds_index* ix, int64_t r0, int64_t r1) {
   const size_t d = ix->d, dp = ix->d_pad;
   const int64_t n = r1 - r0;
   const unsigned blocks = static_cast<unsigned>(std::min<int64_t>((n * 32 + 255) / 256, ix->num_sms * 16));
-  k_prep_rows<<<blocks, 256>>>(ix->x_f32.as<float>() + r0 * d, n, ix->d, ix->d_pad, ix->fmt,
-                               ix->x_bf16.as<uint16_t>() + r0 * dp, nullptr, ix->bias.as<float>() + r0,
-                               ix->dbstat.as<unsigned int>(), nullptr, 0, nullptr, 0, nullptr, nullptr,
-                               ExcludeStage{});
+  PrepParams pp;
+  memset(&pp, 0, sizeof pp);
+  pp.x = ix->x_f32.as<float>() + r0 * d;
+  pp.n = n;
+  pp.d = ix->d;
+  pp.d_pad = ix->d_pad;
+  pp.fmt = ix->fmt;
+  pp.out = ix->x_bf16.as<uint16_t>() + r0 * dp;
+  pp.bias = ix->bias.as<float>() + r0;
+  pp.gmax = ix->dbstat.as<unsigned int>();
+  k_prep_rows<<<blocks, 256>>>(pp);
   CK(cudaGetLastError());
   return 0;
 }
@@ -1498,9 +1579,8 @@ int keds_index_sync(keds_index_t* ix, void* stream) {
 
 int keds_index_set_profiling(keds_index_t* ix, int enable) {
   if (!ix) return fail(KEDS_ERR_ARG, "set_profiling: null handle");
+  if (enable != 0 && enable != 1) return fail(KEDS_ERR_ARG, "set_profiling: mode must be 0 (off) or 1 (in-kernel timer)");
   DeviceGuard g(ix->device);
-  ix->profiling = enable == 2;  // stage marks (stream events between the kernels)
-  ix->prof_used = 0;
   ix->timing_on = enable == 1;  // in-kernel timer of the scoring kernel, launch chain untouched
   ix->timing_launches = 0;
   if (ix->timing_on) {
@@ -1555,41 +1635,12 @@ int keds_index_profile_chain(keds_index_t* ix, double* dur_ms, double* gap_ms, i
 
 int keds_index_profile(keds_index_t* ix, double* score_ms_total, int64_t* score_launches) {
   if (!ix || !score_ms_total || !score_launches) return fail(KEDS_ERR_ARG, "profile: null argument");
-  if (ix->timing_on) {
-    double dur[TIMING_PAIRS], gap[TIMING_PAIRS];
-    int64_t n = 0;
-    CKS(keds_index_profile_chain(ix, dur, gap, &n, TIMING_PAIRS));
-    *score_ms_total = dur[1] * static_cast<double>(n);
-    *score_launches = n;
-    return keds_index_set_profiling(ix, 1);  // re-arm the ring
-  }
-  double ms[PROF_STAGES];
-  int64_t cnt[PROF_STAGES];
-  CKS(keds_index_profile_stages(ix, ms, cnt, PROF_STAGES));
-  *score_ms_total = ms[2];
-  *score_launches = cnt[2];
-  return 0;
-}
-
-int keds_index_profile_stages(keds_index_t* ix, double* ms_total, int64_t* launches, int n_stages) {
-  if (!ix || !ms_total || !launches || n_stages < PROF_STAGES)
-    return fail(KEDS_ERR_ARG, "profile_stages: need room for %d stages", PROF_STAGES);
-  DeviceGuard g(ix->device);
-  for (int t = 0; t < n_stages; ++t) {
-    ms_total[t] = 0.0;
-    launches[t] = 0;
-  }
-  for (size_t i = 1; i < ix->prof_used; ++i) {
-    const int tag = ix->prof_tag[i];
-    if (tag <= 0 || tag >= PROF_STAGES) continue;  // tag 0 opens a new search
-    CK(cudaEventSynchronize(ix->prof_ev[i]));
-    float ms = 0.f;
-    CK(cudaEventElapsedTime(&ms, ix->prof_ev[i - 1], ix->prof_ev[i]));
-    ms_total[tag] += ms;
-    launches[tag]++;
-  }
-  ix->prof_used = 0;
-  return 0;
+  double dur[TIMING_PAIRS], gap[TIMING_PAIRS];
+  int64_t n = 0;
+  CKS(keds_index_profile_chain(ix, dur, gap, &n, TIMING_PAIRS));
+  *score_ms_total = dur[1] * static_cast<double>(n);
+  *score_launches = n;
+  return keds_index_set_profiling(ix, 1);  // re-arm the ring
 }
 
 int keds_index_last_stats(const keds_index_t* ix, keds_search_stats* out) {
@@ -1608,7 +1659,7 @@ int keds_debug_scores(keds_index_t* ix, const float* q, int64_t nq, float* out, 
   Call c = call(1, ix, nullptr, q, nq, 1, nullptr, nullptr, nullptr, nullptr, 0u);
   c.dump = out;
   c.ld_dump = ix->n;
-  CKS(search_pass(c, st));
+  CKS(run_passes(c, st));
   return finish_sync(ix, st);
 }
 
@@ -2080,83 +2131,29 @@ int keds_index_rank(keds_index_t* ix, const float* q, int64_t nq, const int64_t*
   DeviceGuard g(ix->device);
   if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  CKS(set_kernel_attrs(ix));
-  const float* G = ix->x_f32.as<float>();
-  const long long* tg = reinterpret_cast<const long long*>(target);
-  const long long* ex = reinterpret_cast<const long long*>(exclude);
-  long long* out = reinterpret_cast<long long*>(rank_out);
   const int d = ix->d;
-  const size_t simt_smem = static_cast<size_t>((d + 3) & ~3) * 4 * 8;  // 8 queries per block
-  if (simt_smem > 48 * 1024) return fail(KEDS_ERR_ARG, "index_rank: d too large");
-  const int T = static_cast<int>((ix->n + BN - 1) / BN);
-  if (T < 2) {
+  if (gallery_rank_smem(d) > 48 * 1024) return fail(KEDS_ERR_ARG, "index_rank: d too large");
+  const RankMode rm{reinterpret_cast<const long long*>(target), reinterpret_cast<const long long*>(exclude),
+                    reinterpret_cast<long long*>(rank_out)};
+  if (ix->n <= BN) {
     // less than two row tiles: nothing for the tensor cores to win
-    k_gallery_rank<<<static_cast<unsigned>((nq + 7) / 8), 256, simt_smem, st>>>(q, nq, G, ix->n, d, tg, ex, out,
-                                                                                  nullptr, nullptr);
+    k_gallery_rank<<<static_cast<unsigned>((nq + 7) / 8), 256, gallery_rank_smem(d), st>>>(
+        q, nq, ix->x_f32.as<float>(), ix->n, d, rm.target, rm.exclude, rm.out, nullptr, nullptr);
     CK(cudaGetLastError());
     return 0;
   }
+  memset(&ix->stats, 0, sizeof ix->stats);
+  Call c = call(1, ix, nullptr, q, nq, 0, nullptr, nullptr, nullptr, nullptr, 0u);
+  c.rank = rm;
   // warp_exact_score sums in float4 chunks only when q is 16-byte aligned: a query tensor that
   // starts elsewhere is scored from an aligned copy (left by k_prep_rows), so that its ranks do not
   // depend on where it starts and equal those of the recount, which reads q from shared memory
-  const bool q_copy = (d & 3) == 0 && (reinterpret_cast<uintptr_t>(q) & 15) != 0;
-  for (int64_t q0 = 0; q0 < nq; q0 += Q_PASS_MAX) {
-    const int64_t nb = std::min<int64_t>(Q_PASS_MAX, nq - q0);
-    const float* qsrc = q + q0 * d;
-    if (q_copy) CKS(ix->q_f32.ensure(static_cast<size_t>(nb) * d * 4));
-    float* qcopy = q_copy ? ix->q_f32.as<float>() : nullptr;
-    const float* qp = q_copy ? qcopy : qsrc;
-    Plan pl{geometry(ix, 1, nb)};
-    // as many candidate lists as the tiles allow: the band around a mid-ranked target is crowded
-    pl.set_slices(1, static_cast<int>(std::max<long long>(1, std::min<long long>(std::min(T, S_MAX), pl.s_mem))));
-    const int n_lists = pl.S * pl.sub;
-    CKS(ix->ctrl.ensure(CTRL_STRIDE * 4));  // (finish_sync reads whole status blocks)
-    ix->ctrl_passes = 1;
-    ix->ctrl_slot = 0;
-    CKS(ix->flagged[0].ensure(static_cast<size_t>(nb) * 4));
-    CKS(ensure_q_map(ix, static_cast<int64_t>(pl.n_qt) * BM, st));
-    CKS(ix->qstat.ensure(static_cast<size_t>(nb) * sizeof(float4)));
-    CKS(ix->rk.ensure(static_cast<size_t>(nb) * 5 * 4));
-    CKS(ensure_cand(ix, static_cast<size_t>(n_lists) * pl.n_qt));
-    float* rk_st = ix->rk.as<float>();
-    float* rk_lo = rk_st + nb;
-    float* rk_hi = rk_lo + nb;
-    int* rk_t = reinterpret_cast<int*>(rk_hi + nb);
-    int* rk_e = rk_t + nb;
-    {
-      const unsigned blocks = static_cast<unsigned>(std::min<long long>((nb * 32 + 255) / 256, 4096));
-      CKS(launch_k(ix->use_pdl, k_prep_rows, dim3(blocks), dim3(256), 0, st, qsrc, static_cast<long long>(nb), d,
-                   ix->d_pad, ix->fmt, ix->q_bf16.as<uint16_t>(), ix->qstat.as<float4>(), static_cast<float*>(nullptr),
-                   static_cast<unsigned int*>(nullptr), ix->ctrl.as<unsigned int>(), CTRL_WORDS,
-                   static_cast<float*>(nullptr), 0, static_cast<unsigned long long*>(nullptr), qcopy,
-                   ExcludeStage{}));
-    }
-    const unsigned wblocks = static_cast<unsigned>((nb * 32 + 255) / 256);
-    CKS(launch_k(ix->use_pdl, k_rank_targets, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,
-                 tg + q0, ex ? ex + q0 : nullptr, ix->qstat.as<float4>(), ix->dbstat.as<unsigned int>(), ix->eps_scale,
-                 rk_st, rk_lo, rk_hi, rk_t, rk_e));
-    ScoreParams sp = score_params(ix, &ix, 1, pl, nb, ix->ctrl.as<unsigned int>() + 2);
-    sp.rk_lo = rk_lo;
-    sp.rk_hi = rk_hi;
-    sp.rk_target = rk_t;
-    sp.rk_exclude = ex ? rk_e : nullptr;
-    CKS(launch_score(ix, &ix, 1, pl, sp, st));
-    CKS(launch_k(ix->use_pdl, k_rank_finish, dim3(wblocks), dim3(256), 0, st, qp, static_cast<long long>(nb), G, d,
-                 n_lists, pl.n_qt, static_cast<const uint2*>(sp.cand), static_cast<const int*>(sp.cand_cnt),
-                 static_cast<const float*>(sp.cand_theta), static_cast<const float*>(rk_st),
-                 static_cast<const int*>(rk_t), out + q0, ix->flagged[0].as<int>(), ix->ctrl.as<int>()));
-    // exact recount of the queries whose band overflowed a list (none, normally: the blocks leave at once)
-    CKS(launch_k(ix->use_pdl, k_gallery_rank, dim3(static_cast<unsigned>((nb + 7) / 8)), dim3(256), simt_smem, st, qp,
-                 static_cast<long long>(nb), G, static_cast<long long>(ix->n), d, tg + q0, ex ? ex + q0 : nullptr,
-                 out + q0, static_cast<const int*>(ix->flagged[0].as<int>()), static_cast<const int*>(ix->ctrl.as<int>())));
-    ix->stats.launches = 5;
-    ix->stats.slices = pl.S;
-    ix->stats.items = pl.n_items;
-    ix->stats.grid = pl.grid;
-    if (q0 + nb < nq) CKS(finish_sync(ix, st));  // the scratch is reused by the next pass
+  if ((d & 3) == 0 && (reinterpret_cast<uintptr_t>(q) & 15) != 0) {
+    CKS(ix->q_f32.ensure(static_cast<size_t>(nq) * d * 4));
+    c.q_src = q;
+    c.q = ix->q_f32.as<float>();
   }
-  CK(cudaGetLastError());
-  return 0;
+  return run_passes(c, st);
 }
 
 int keds_index_label_hits(keds_index_t* ix, const float* q, int64_t nq, const int64_t* row_labels,
@@ -2176,8 +2173,6 @@ int keds_index_label_hits(keds_index_t* ix, const float* q, int64_t nq, const in
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   memset(&ix->stats, 0, sizeof ix->stats);
   const int kmax = ks[nks - 1];
-  const int n_passes = static_cast<int>((nq + Q_PASS_MAX - 1) / Q_PASS_MAX);
-  CKS(ix->ctrl.ensure(static_cast<size_t>(n_passes) * CTRL_STRIDE * 4));
   // exact rows of the queries the certificate queues (the fallback writes them, k_hits_from_rows counts them)
   const int64_t nb_max = std::min<int64_t>(nq, Q_PASS_MAX);
   CKS(ix->D_stage[0].ensure(static_cast<size_t>(nb_max) * kmax * 4));

@@ -180,12 +180,40 @@ struct ExcludeStage {
   int* rows;                // [n_db][nq][n_ex]
 };
 
-__global__ void k_prep_rows(const float* __restrict__ x, long long n, int d, int d_pad, int fmt,
-                            uint16_t* __restrict__ out, float4* __restrict__ stat,
-                            float* __restrict__ bias, unsigned int* __restrict__ gmax,
-                            unsigned int* __restrict__ zero_words, int n_zero,
-                            float* __restrict__ neg_inf_words, int n_neg_inf,
-                            unsigned long long* timing, float* __restrict__ copy_f32, const ExcludeStage ex) {
+// fp32 rows -> 16-bit operand rows and their statistics (queries per search, database rows at add);
+// every output is optional (nullptr: not written)
+struct PrepParams {
+  const float* x;                // [n][d]
+  long long n;
+  int d, d_pad, fmt;
+  uint16_t* out;                 // [n][d_pad] 16-bit rows
+  float4* stat;                  // [n] {|x|^2, |x16|, |x - x16|, 0}
+  float* bias;                   // [n] -|x|^2 / 2 (L2)
+  unsigned int* gmax;            // [3] running maxima of the statistics (float bits, atomicMax)
+  unsigned int* zero_words;      // [n_zero] cleared by block 0 (a status block)
+  int n_zero;
+  float* neg_inf_words;          // [n_neg_inf] set to -inf (the warm-start thresholds)
+  int n_neg_inf;
+  unsigned long long* timing;
+  float* copy_f32;               // [n][d] device copy of x (x in page-locked host memory or misaligned)
+  ExcludeStage ex;
+};
+
+__global__ void k_prep_rows(const PrepParams p) {
+  const float* __restrict__ x = p.x;
+  const long long n = p.n;
+  const int d = p.d, d_pad = p.d_pad, fmt = p.fmt;
+  uint16_t* __restrict__ out = p.out;
+  float4* __restrict__ stat = p.stat;
+  float* __restrict__ bias = p.bias;
+  unsigned int* __restrict__ gmax = p.gmax;
+  unsigned int* __restrict__ zero_words = p.zero_words;
+  const int n_zero = p.n_zero;
+  float* __restrict__ neg_inf_words = p.neg_inf_words;
+  const int n_neg_inf = p.n_neg_inf;
+  unsigned long long* timing = p.timing;
+  float* __restrict__ copy_f32 = p.copy_f32;
+  const ExcludeStage& ex = p.ex;
   const int lane = threadIdx.x & 31;
   griddep_wait();               // earlier kernels of the stream may still read what is rewritten here
   griddep_launch_dependents();  // the scoring kernel may start its prologue

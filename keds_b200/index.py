@@ -302,7 +302,7 @@ class GpuIndexFlat:
         }
 
     def set_profiling(self, mode: int) -> None:
-        """0 off; 1 in-kernel timer of the scoring kernel (launch chain untouched); 2 stage marks."""
+        """0 off; 1 in-kernel timer of the scoring kernel (launch chain untouched)."""
         _capi.check(self._lib.keds_index_set_profiling(self._h, int(mode)))
 
     def profile(self):
@@ -321,15 +321,6 @@ class GpuIndexFlat:
         out = {name: {"ms": float(dur[i]), "gap_ms": float(gap[i])} for i, name in enumerate(self.CHAIN)}
         out["searches"] = int(n.value)
         return out
-
-    STAGES = ("", "k_prep_rows", "k_score_topk", "k_select_rerank", "k_exact_fallback", "")
-
-    def profile_stages(self) -> dict:
-        """{kernel: (summed ms, launches)} since set_profiling(True); stream time per stage."""
-        ms = (C.c_double * 6)()
-        n = (C.c_int64 * 6)()
-        _capi.check(self._lib.keds_index_profile_stages(self._h, ms, n, 6))
-        return {self.STAGES[i]: (float(ms[i]), int(n[i])) for i in range(1, 5)}
 
     def rows_ptr(self) -> int:
         """Device address of the resident fp32 rows [ntotal, d]."""

@@ -9,7 +9,9 @@ and times, round after round in rotating order on the same device-resident input
            itself out (training without self-retrieval)
 
 on three shapes: config 2 (retrieve2, 128 queries x 2 databases x 0.5M rows, k = 16, gathered
-neighbours), config 1 (search, 4096 x 50k, k = 16) and 4096 x 0.5M. Times are per call from CUDA
+neighbours), config 1 (search, 4096 x 50k, k = 16) and 4096 x 0.5M; and base against plain (no
+exclude variant) for gallery ranking at 4181 x 2297 (one pass) and 17,000 x 2297 (two passes) and
+label hits at 10,000 x 50k (cut points 1, 5, 10, 50). Times are per call from CUDA
 events around a back-to-back loop; the spread is the range over rounds, and the differences are
 the median (and quartiles) of the per-round ratios of variants that ran back to back. Also checks that base and
 plain return the same bits. Writes one JSON document (card name and power limit included).
@@ -25,6 +27,8 @@ import os
 import statistics
 import subprocess
 import sys
+
+import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -86,9 +90,9 @@ def main() -> None:
         x = torch.randn(n, D, generator=g, device=dev)
         return x / x.norm(dim=1, keepdim=True)
 
-    big_a, big_b, small = unit(500_000), unit(500_000), unit(50_000)
-    idx = {name: {"a": make_index(lib, big_a), "b": make_index(lib, big_b), "s": make_index(lib, small)}
-           for name, lib in libs.items()}
+    big_a, big_b, small, gal = unit(500_000), unit(500_000), unit(50_000), unit(2297)
+    idx = {name: {"a": make_index(lib, big_a), "b": make_index(lib, big_b), "s": make_index(lib, small),
+                  "g": make_index(lib, gal)} for name, lib in libs.items()}
     torch.cuda.synchronize()
 
     perm = torch.randperm(K, generator=torch.Generator().manual_seed(1)).to(dev, torch.int32)
@@ -99,8 +103,24 @@ def main() -> None:
         q = (big_a if n == 500_000 else small)[rows.to(dev)].contiguous()
         ex = rows.to(dev, torch.int64).reshape(nq, 1).contiguous()
         shapes[cfg] = (nq, q, ex)
+    # gallery ranking: queries near random gallery rows, mid-ranked random targets, one excluded row each
+    for cfg, nq in (("rank_4181x2297", 4181), ("rank_17000x2297", 17_000)):
+        sel = torch.randint(0, 2297, (nq,), generator=g, device=dev)
+        q = gal[sel] + 0.05 * unit(nq)
+        q = (q / q.norm(dim=1, keepdim=True)).contiguous()
+        tg_ex = torch.randint(0, 2297, (2, nq), generator=g, device=dev)
+        shapes[cfg] = (nq, q, tg_ex)
+    row_labels = torch.randint(0, 100, (50_000,), generator=g, device=dev)
+    ks = np.array([1, 5, 10, 50], np.int32)  # (read on the host)
+    rows = torch.randperm(50_000, generator=torch.Generator().manual_seed(7))[:10_000].to(dev)
+    shapes["hits_10000x50k"] = (10_000, small[rows].contiguous(),
+                                torch.randint(0, 100, (10_000,), generator=g, device=dev))
 
-    def outputs(nq, feats):
+    def outputs(cfg, nq, feats):
+        if cfg.startswith("rank"):
+            return [torch.empty(nq, dtype=torch.int64, device=dev)]
+        if cfg.startswith("hits"):
+            return [torch.empty((nq, len(ks)), dtype=torch.int32, device=dev)]
         o = [torch.empty((nq, K), dtype=torch.float32, device=dev), torch.empty((nq, K), dtype=torch.int64, device=dev),
              torch.empty((nq, K), dtype=torch.float32, device=dev), torch.empty((nq, K), dtype=torch.int64, device=dev)]
         if feats:
@@ -113,6 +133,12 @@ def main() -> None:
         ix = idx["base" if variant == "base" else "new"]
         o = outs[(cfg, variant)]
         p = [t.data_ptr() for t in o]
+        if cfg.startswith("rank"):
+            return lambda: check(lib, lib.keds_index_rank(ix["g"], q.data_ptr(), nq, ex[0].data_ptr(), ex[1].data_ptr(),
+                                                          p[0], st))
+        if cfg.startswith("hits"):
+            return lambda: check(lib, lib.keds_index_label_hits(ix["s"], q.data_ptr(), nq, row_labels.data_ptr(),
+                                                                ex.data_ptr(), ks.ctypes.data, len(ks), p[0], st))
         if cfg.startswith("cfg2"):
             common = (ix["a"], ix["b"], q.data_ptr(), nq, K, perm.data_ptr(), None, 0, 100.0, p[0], p[1], p[2], p[3],
                       p[4], p[5], None, None)
@@ -125,10 +151,12 @@ def main() -> None:
                                                                     0, st))
         return lambda: check(lib, lib.keds_index_search_ex(h, q.data_ptr(), nq, K, p[0], p[1], 0, st))
 
-    variants = ("base", "plain", "exclude")
-    outs = {(c, v): outputs(shapes[c][0], c.startswith("cfg2")) for c in shapes for v in variants}
-    fns = {(c, v): call(c, v) for c in shapes for v in variants}
-    iters = {"cfg2_retrieve2_128x2x500k": 50, "cfg1_search_4096x50k": 20, "search_4096x500k": 5}
+    variants = {c: ("base", "plain") if c.startswith(("rank", "hits")) else ("base", "plain", "exclude")
+                for c in shapes}
+    outs = {(c, v): outputs(c, shapes[c][0], c.startswith("cfg2")) for c in shapes for v in variants[c]}
+    fns = {(c, v): call(c, v) for c in shapes for v in variants[c]}
+    iters = {"cfg2_retrieve2_128x2x500k": 50, "cfg1_search_4096x50k": 20, "search_4096x500k": 5,
+             "rank_4181x2297": 20, "rank_17000x2297": 10, "hits_10000x50k": 10}
     for f in fns.values():  # warm-up: modules, scratch sizes, planner feedback
         for _ in range(5):
             f()
@@ -138,7 +166,8 @@ def main() -> None:
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for r in range(args.rounds):
         for c in shapes:
-            order = variants[r % 3:] + variants[:r % 3]
+            vs = variants[c]
+            order = vs[r % len(vs):] + vs[:r % len(vs)]
             for v in order:
                 f = fns[(c, v)]
                 f()
@@ -155,15 +184,17 @@ def main() -> None:
     result = {"card": card(), "rounds": args.rounds, "unit": "us per call", "configs": {}}
     for c in shapes:
         same = all(torch.equal(a, b) for a, b in zip(outs[(c, "base")], outs[(c, "plain")]))
-        nq, _, ex = shapes[c]
-        I_ex = outs[(c, "exclude")][1]
-        row = {"base_plain_outputs_identical": bool(same),
-               "exclude_never_returns_self": bool(not (I_ex == ex).any().item())}
-        for v in variants:
+        row = {"base_plain_outputs_identical": bool(same)}
+        if "exclude" in variants[c]:
+            I_ex = outs[(c, "exclude")][1]
+            row["exclude_never_returns_self"] = bool(not (I_ex == shapes[c][2]).any().item())
+        for v in variants[c]:
             t = times[(c, v)]
             row[v] = {"median": round(statistics.median(t), 2), "min": round(min(t), 2), "max": round(max(t), 2)}
         # paired within each round (the three variants ran back to back): median and range of the ratios
         for name, num, den in (("plain_vs_base_pct", "plain", "base"), ("exclude_vs_plain_pct", "exclude", "plain")):
+            if num not in variants[c]:
+                continue
             r = [100.0 * (a / b - 1.0) for a, b in zip(times[(c, num)], times[(c, den)])]
             row[name] = {"median": round(statistics.median(r), 2), "p25": round(statistics.quantiles(r, n=4)[0], 2),
                          "p75": round(statistics.quantiles(r, n=4)[2], 2)}

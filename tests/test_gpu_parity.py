@@ -775,7 +775,8 @@ def test_gallery_rank_tensor_core_path_equals_the_exact_count():
     """keds_index_rank: the tensor-core count + exact settlement of the band rows must give the
     ranks of the plain fp32 count (keds_gallery_rank's SIMT kernel on the same inputs) bit for bit:
     mid-ranked random targets (crowded bands), a 50k-row gallery, a batch below one query tile, an
-    inflated error bound that overflows the band lists (exact recount queue), and no exclusions."""
+    inflated error bound that overflows the band lists (exact recount queue), no exclusions, and a
+    batch of two passes (17,000 queries)."""
     lib = _capi.load()
 
     def simt(q, gal, tgt, ref):
@@ -785,7 +786,7 @@ def test_gallery_rank_tensor_core_path_equals_the_exact_count():
         torch.cuda.synchronize()
         return out[:60]   # below 64 queries the C entry point keeps to the fp32 SIMT kernel
 
-    for ng, nq, seed in ((2297, 4181, 1), (50000, 1000, 2), (700, 100, 3)):
+    for ng, nq, seed in ((2297, 4181, 1), (50000, 1000, 2), (700, 100, 3), (2297, 17000, 4)):
         gal = torch.from_numpy(unit(ng, 768, 900 + seed)).cuda()
         q = torch.from_numpy(unit(nq, 768, 910 + seed)).cuda()
         rng = np.random.default_rng(seed)
