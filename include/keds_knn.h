@@ -109,7 +109,14 @@ int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t
  *   feat_s[b][j][:] = rows_s[I_s[b][perm_s ? perm_s[j] : j]][:]      (nullable; [nq][k][d])
  *   pool_s[b][:]    = sum_j w_j rows_s[I_s[b][j]][:]                 (nullable; [nq][d])
  * pool_mode 0: no pool; 1: w = 1/k; 2: w = softmax_j(+-tau * D_s[b][j]) (minus under L2).
- * Each neighbour row is read once for both outputs. perm_*: device int32[k] or NULL. */
+ * Padding (I = -1, fewer than k rows to return) is a zero row in feat and in the pool: mean pools
+ * still divide by k, softmax pools give it weight 0.
+ * Each neighbour row is read once for both outputs. perm_*: device int32[k] or NULL, and it must be a
+ * permutation of 0..k-1. It is not checked (that would need a synchronisation): the pool is summed
+ * over output slots, slot j adding w_{perm[j]} * rows_s[I_s[b][perm[j]]], so a repeated entry counts
+ * one neighbour twice and drops another; an entry outside [0, k) gives a zero row in feat and adds
+ * nothing but w_0 * 0 to the pool. The Python wrappers refuse a host perm that is not a permutation.
+ * The summation order of the pool depends on the route a query takes (DESIGN.md section 3). */
 int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
                    const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
                    float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,

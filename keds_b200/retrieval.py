@@ -30,6 +30,19 @@ from . import _capi
 from .index import GpuIndexFlat, METRIC_INNER_PRODUCT, METRIC_L2, check_exclude, search2, _exclude_arg, _stream_ptr
 
 
+def check_perm(perm: Optional[torch.Tensor], k: int, name: str = "perm") -> None:
+    """Raise ValueError unless a host `perm` is a permutation of range(k). The fused consumer pools
+    over output slots (slot j adds the neighbour perm[j] shows), so a repeated entry would count one
+    neighbour twice and drop another. A device perm is not read here: that would synchronise the
+    stream (and is illegal inside a CUDA graph capture); its caller guarantees the same property."""
+    if perm is None or perm.is_cuda:
+        return
+    if perm.dim() != 1 or perm.numel() != k or perm.is_floating_point() or perm.is_complex():
+        raise ValueError(f"{name}: expected an integer tensor of {k} entries, got {perm.dtype} {tuple(perm.shape)}")
+    if not torch.equal(torch.sort(perm.to(torch.int64)).values, torch.arange(k)):
+        raise ValueError(f"{name}: not a permutation of range({k}): {perm.tolist()[:32]}")
+
+
 def gather_rows(index: GpuIndexFlat, I: torch.Tensor, perm: Optional[torch.Tensor] = None) -> torch.Tensor:
     """out[b, j, :] = rows[I[b, perm[j]], :] from the index's resident fp32 rows (device tensors)."""
     lib = _capi.load()
@@ -217,7 +230,17 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
 
     exclude: int64 [B] or [B, E] (E <= 8) labels each query must not retrieve from either base, -1 =
     none; the neighbours, gathers and pools are those of the exact search over the remaining rows.
-    On the host-I/O path it may be a pinned CPU tensor, read through the mapping like `q`."""
+    On the host-I/O path it may be a pinned CPU tensor, read through the mapping like `q`.
+
+    perm_img / perm_txt: permutations of range(topk). A CPU tensor that is not one raises ValueError;
+    a CUDA tensor is used as it is (checking it would synchronise), and one that repeats or leaves out
+    an entry corrupts the pool: the pool adds, per output slot j, the neighbour perm[j] shows.
+
+    `out` tensors are reused when they have the expected shape, dtype and device and are contiguous;
+    any other tensor under a key is replaced by a new one in the dict (the kernels write dense rows)."""
+    k = int(topk)
+    check_perm(perm_img, k, "retrieve2: perm_img")
+    check_perm(perm_txt, k, "retrieve2: perm_txt")
     lib = _capi.load()
     hostio = host_out is not None or not q.is_cuda
     if q.is_cuda:
@@ -227,12 +250,13 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
         if not q.is_pinned() or q.dtype != torch.float32 or q.dim() != 2 or q.shape[1] != image_index.d or not q.is_contiguous():
             raise TypeError("retrieve2: a host query must be a pinned, contiguous float32 [B, d] tensor")
         dev = torch.device("cuda", image_index.device)
-    B, d, k = q.shape[0], image_index.d, int(topk)
+    B, d = q.shape[0], image_index.d
     o = out if out is not None else {}
 
     def buf(name, shape, dtype):
         t = o.get(name)
-        if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev:
+        if (t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev
+                or not t.is_contiguous()):
             t = torch.empty(shape, dtype=dtype, device=dev)
             o[name] = t
         return t
@@ -288,12 +312,17 @@ class RetrievalStep:
     a pinned `exclude_host` [batch, n_exclude] int64 (-1 = none) that `run(q, exclude=...)` fills or
     the caller writes directly; the graph reads it on every replay, so changing it needs no
     re-capture.
+
+    perm_img must be a permutation of range(topk) (ValueError otherwise): it is checked here, once,
+    because the captured call uses its device copy, which retrieve2 does not read.
     """
 
     def __init__(self, image_index: GpuIndexFlat, text_index: GpuIndexFlat, batch: int, topk: int = 16,
                  perm_img: Optional[torch.Tensor] = None, want_feats: bool = True,
                  pool_mode: int = POOL_NONE, tau: float = 100.0, copy_nodes: Optional[bool] = None,
                  n_exclude: int = 0) -> None:
+        # the graph replays retrieve2 with the device copy of perm_img, which it cannot check there
+        check_perm(None if perm_img is None else perm_img.cpu(), int(topk), "RetrievalStep: perm_img")
         self.ia, self.ib = image_index, text_index
         # copy_nodes=False: no copies in the graph -- the first kernel reads the pinned queries through
         # the mapping and the ranking blocks store (D, I) into the pinned result block next to the

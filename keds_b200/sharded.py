@@ -22,6 +22,7 @@ import torch.distributed as dist
 
 from . import _capi
 from .index import GpuIndexFlat, _exclude_arg, _stream_ptr
+from .retrieval import check_perm
 
 
 def shard_bounds(n: int, world: int, rank: int) -> Tuple[int, int]:
@@ -327,7 +328,10 @@ class ShardedKnowledgeBase:
         by perm_img) and pool_img / pool_txt [hi-lo, d] (pool_mode 1 mean, 2 softmax(+-tau*D)).
         exclude: int64 [Bt] or [Bt, E] (E <= 8) global labels each query must not retrieve from
         either base, -1 = none. Collective: every rank calls it with the same q, k and exclusion.
-        `out` may carry the tensors of a previous call (keys as returned)."""
+        `out` may carry the tensors of a previous call (keys as returned); a tensor of another shape,
+        dtype or device, or a non-contiguous one, is replaced in the dict.
+        perm_img / perm_txt: permutations of range(k); a CPU tensor that is not one raises ValueError,
+        a CUDA tensor is trusted (the pool adds, per output slot j, the neighbour perm[j] shows)."""
         if not isinstance(q, torch.Tensor) or q.dtype != torch.float32 or q.dim() != 2 or q.shape[1] != self.d:
             raise TypeError(f"retrieve2: q must be a float32 [Bt, {self.d}] tensor")
         if q.device != self.device:
@@ -347,6 +351,7 @@ class ShardedKnowledgeBase:
             if p is not None and (not isinstance(p, torch.Tensor) or p.dim() != 1 or p.numel() != k
                                   or p.dtype not in (torch.int32, torch.int64)):
                 raise TypeError(f"retrieve2: {name} must be an integer tensor of {k} entries")
+            check_perm(p, k, f"retrieve2: {name}")
             perms.append(None if p is None else p.to(device=self.device, dtype=torch.int32).contiguous())
         ex = None
         if exclude is not None:
@@ -361,7 +366,8 @@ class ShardedKnowledgeBase:
 
         def buf(name, shape, dtype):
             t = o.get(name)
-            if t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev:
+            if (t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev
+                    or not t.is_contiguous()):
                 t = torch.empty(shape, dtype=dtype, device=dev)
                 o[name] = t
             return t

@@ -1,6 +1,8 @@
 """GPU (-m gpu): the row-sharded retrieval step (ShardedKnowledgeBase.retrieve2) on two ranks, each
 against retrieval.retrieve2 on a full copy of both bases on its own GPU: D, I and the gathered rows
-bit for bit, pools within 2e-6 of a float64 pool recomputed from the returned D and rows. Covers IP /
+bit for bit, pools within 2e-6 of a float64 pool recomputed from the returned D and rows, mean pools
+bit for bit against the emulation of the latency re-rank's summation order (oracle/pool_exact.py) and
+softmax pools within that module's bound. Covers IP /
 L2, k = 16 / 64, pool modes 0 / 1 / 2, perm_img, exclusion (own rows, E = 1; E = 8), two passes
 (more than 16,384 queries), the exact fallback, an exact-only tiny shard, an empty shard, consecutive
 steps, a strict sub-range of query rows, re-attachment after an add, the refusal when rows changed
@@ -56,6 +58,7 @@ class Case:
 
         kb = ShardedKnowledgeBase(D, metric, device=self.dev.index)
         kb.add(img, txt)
+        self.rows = {"img": img.to(self.dev), "txt": txt.to(self.dev)}
         refs = []
         for x in (img, txt):
             r = GpuIndexFlat(D, metric, self.dev.index)
@@ -64,14 +67,16 @@ class Case:
             refs.append(r)
         return kb, refs
 
-    def check(self, kb, refs, q, k, perm=None, pool_mode=0, ex=None, flags=0, tau=50.0, rows=None):
+    def check(self, kb, refs, q, k, perm=None, pool_mode=0, ex=None, flags=0, tau=50.0, rows=None, out=None):
         from keds_b200 import retrieval as kr
+        from oracle import pool_exact as pe
 
         Bt = q.shape[0]
         lo, hi = rows if rows is not None else (self.rank * Bt // self.world, (self.rank + 1) * Bt // self.world)
         q = q.to(self.dev)
         exd = None if ex is None else ex.to(self.dev)
-        out = kb.retrieve2(q, k, perm_img=perm, pool_mode=pool_mode, tau=tau, flags=flags, exclude=exd, rows=(lo, hi))
+        out = kb.retrieve2(q, k, perm_img=perm, pool_mode=pool_mode, tau=tau, flags=flags, exclude=exd, rows=(lo, hi),
+                           out=out)
         kb.exchange_stats()  # synchronises; raises if a peer never delivered
         l2 = kb.metric_type == 1
         if refs[0].ntotal == 0:
@@ -91,11 +96,21 @@ class Case:
             if ex is not None:
                 I = out["I_" + s].cpu()
                 assert not ((I[:, :, None] == ex[:, None, :]) & (ex[:, None, :] >= 0)).any()
-            if pool_mode:
+            if pool_mode and hi > lo:
                 p = pool_ref(out["D_" + s][lo:hi], out["I_" + s][lo:hi], out["feat_" + s],
                              perm if s == "img" else None, pool_mode, tau, l2)
-                err = (out["pool_" + s].double() - p).abs().max().item() if hi > lo else 0.0
+                err = (out["pool_" + s].double() - p).abs().max().item()
                 assert err <= 2e-6, (s, err)
+                # k_shard_consume sums in the latency re-rank's order (8 warps, two rows in flight), on
+                # any shard count: mean pools bit for bit, softmax pools within the bound of D
+                rows_s, I_s = self.rows[s], out["I_" + s][lo:hi]
+                ps = perm if s == "img" else None
+                if pool_mode == 1:
+                    want = pe.mean_pool(rows_s, I_s, ps, *pe.SHARD)
+                    assert bool(pe.equal_rows(out["pool_" + s], want).all()), ("mean pool bits", s)
+                else:
+                    p64, bound = pe.softmax_pool_bound(rows_s, I_s, out["D_" + s][lo:hi], ps, tau, l2, 8)
+                    assert bool(((out["pool_" + s].double() - p64).abs() <= bound).all()), ("softmax bound", s)
         return out
 
 
@@ -121,6 +136,13 @@ def run_cases(rank, world, dev):
         ex8 = torch.cat([sel[:, None], torch.randint(0, N, (sel.numel(), 6), generator=g),
                          torch.full((sel.numel(), 1), -1)], 1)
         c.check(kb, refs, q, 16, pool_mode=1, ex=ex8)
+        # out= with column slices of wider buffers: replaced by dense tensors, the buffers untouched
+        nb = 128                                # this rank's block of the 128 * world queries
+        wide_p = torch.full((nb, 2 * D), 7.0, device=dev)
+        wide_f = torch.full((nb, 16, 2 * D), 7.0, device=dev)
+        o = {"pool_img": wide_p[:, D:], "feat_txt": wide_f[:, :, :D]}
+        assert c.check(kb, refs, unit(128 * world, 44), 16, perm=perm16, pool_mode=1, out=o) is o
+        assert (wide_p == 7.0).all() and (wide_f == 7.0).all() and o["pool_img"].is_contiguous()
         # a strict sub-range of rows, different on each rank
         c.check(kb, refs, unit(128 * world, 45), 16, perm=perm16, pool_mode=2, rows=(37 + 5 * rank, 101 + 3 * rank))
         # the bare sharded search with exclusion against GpuIndexFlat.search on a full copy

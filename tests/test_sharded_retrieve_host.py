@@ -94,6 +94,8 @@ def test_retrieve2_argument_checks(tmp_path):
             (ValueError, dict(rows=(-1, 2))),
             (TypeError, dict(perm_img=torch.arange(5))),
             (TypeError, dict(perm_txt=torch.zeros(4, dtype=torch.float32))),
+            (ValueError, dict(perm_img=torch.tensor([0, 0, 1, 2]))),     # not a permutation
+            (ValueError, dict(perm_txt=torch.tensor([0, 1, 2, 4]))),
             (TypeError, dict(exclude=torch.zeros(6, dtype=torch.int32))),
             (ValueError, dict(exclude=torch.zeros(5, 1, dtype=torch.int64))),
             (ValueError, dict(exclude=torch.zeros(6, 9, dtype=torch.int64))),
