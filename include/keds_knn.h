@@ -378,6 +378,26 @@ int keds_consumer_forward_train(keds_consumer_t* c, const float* feat, const flo
                                 const int64_t* I_txt, const int32_t* perm, int64_t B, int k,
                                 const float* const* masks, float* tokens, void* cuda_stream);
 int keds_consumer_backward(keds_consumer_t* c, const float* dtokens, float* grads, void* cuda_stream);
+
+/* The consumer over two row-sharded bases (keds_retrieve2_sharded): the neighbour rows are read in
+ * place from the rank that owns them (its own fp32 rows, or a peer's over NVLink through the mapping
+ * of keds_exchange_attach_rows), so no [B][k][d] features are materialised.
+ *   I_img / I_txt   [B][k] GLOBAL labels, e.g. this rank's rows of the merged I of
+ *                   keds_retrieve2_sharded; a label no shard holds (-1 padding) reads as a zero row.
+ *   img / txt       this rank's index handles of the two bases (databases 0 and 1 of ex).
+ * Everything else as keds_consumer_forward / keds_consumer_forward_train; keds_consumer_backward
+ * follows either unchanged (it reads only the assembled MLP input). Refused with KEDS_ERR_ARG before
+ * anything is queued: a NULL argument or a buffer that is not device memory, a base not attached to
+ * ex, this rank's rows moved or grown since the attach (re-attach after every add), an index width
+ * other than d_in, consumer / indices / exchange on different devices. No flag guards the peers'
+ * rows: they do not change between adds, and an add synchronises every rank first. */
+int keds_consumer_forward_sharded(keds_consumer_t* c, keds_index_t* img, keds_index_t* txt, keds_exchange_t* ex,
+                                  const float* feat, const int64_t* I_img, const int64_t* I_txt,
+                                  const int32_t* perm, int64_t B, int k, float* tokens, void* cuda_stream);
+int keds_consumer_forward_train_sharded(keds_consumer_t* c, keds_index_t* img, keds_index_t* txt,
+                                        keds_exchange_t* ex, const float* feat, const int64_t* I_img,
+                                        const int64_t* I_txt, const int32_t* perm, int64_t B, int k,
+                                        const float* const* masks, float* tokens, void* cuda_stream);
 /* Test hook: hidden activations [B(1+2k)][d_mid] of IM2TEXT layer `layer` as the last forward_train
  * left them (after dropout and ReLU). Their signs are the ReLU gates the backward uses; a tf32
  * forward and a float64 one disagree on them for pre-activations within rounding of zero, so a

@@ -148,6 +148,14 @@ SIGNATURES = {
         [_vp, _vp, _vp, C.c_int64, _vp, C.c_int64, _vp, _vp, _vp, C.c_int64, C.c_int, C.POINTER(_vp), _vp, _vp],
     ),
     "keds_consumer_backward": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "keds_consumer_forward_sharded": (
+        C.c_int,
+        [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp],
+    ),
+    "keds_consumer_forward_train_sharded": (
+        C.c_int,
+        [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.POINTER(_vp), _vp, _vp],
+    ),
     "keds_consumer_debug_hidden": (C.c_int, [_vp, C.c_int, _vp, C.c_int64, _vp]),
     "keds_consumer_set_debug": (C.c_int, [_vp, C.c_int]),
     "keds_consumer_debug_timeline": (C.c_int, [_vp, C.c_int, _vp, C.c_int64]),

@@ -44,6 +44,35 @@ def _count_prefix(sd: Mapping[str, torch.Tensor], fmt: str) -> int:
     return n
 
 
+def _sharded_kb(image_index, text_index):
+    """The ShardedKnowledgeBase whose two bases are (image_index, text_index); None for two local
+    indices. A mixed pair, or the bases of two different knowledge bases, raise TypeError."""
+    from .sharded import ShardedIndex
+
+    sharded = (isinstance(image_index, ShardedIndex), isinstance(text_index, ShardedIndex))
+    if not any(sharded):
+        return None
+    kb = image_index._kb if sharded[0] else None
+    if not all(sharded) or kb is None or kb.image is not image_index or kb.text is not text_index:
+        raise TypeError("image_index and text_index must both be GpuIndexFlat, or be the `image` and `text` "
+                        "indices of one ShardedKnowledgeBase")
+    return kb
+
+
+def _call_forward(lib, name, h, feature, image_index, text_index, tail):
+    """keds_consumer_<name> with (base, n) of two local indices, or keds_consumer_<name>_sharded with
+    the local shards and the exchange of a ShardedKnowledgeBase; `tail` = the arguments from I_img on."""
+    kb = _sharded_kb(image_index, text_index)
+    if kb is None:
+        return getattr(lib, "keds_consumer_" + name)(h, feature.data_ptr(), image_index.rows_ptr(), image_index.ntotal,
+                                                     text_index.rows_ptr(), text_index.ntotal, *tail)
+    if kb._fx is None:
+        raise RuntimeError("the ShardedKnowledgeBase has no exchange yet: run kb.retrieve2 first (its labels are "
+                           "what the consumer reads)")
+    return getattr(lib, "keds_consumer_" + name + "_sharded")(h, kb.image.local._h, kb.text.local._h, kb._fx.handle,
+                                                              feature.data_ptr(), *tail)
+
+
 class NeighbourConsumer:
     """img2text + retrieval_fuse + text_condition in one launch sequence (tf32 tensor cores)."""
 
@@ -108,7 +137,10 @@ class NeighbourConsumer:
                  I_img: torch.Tensor, I_txt: torch.Tensor, perm: Optional[torch.Tensor] = None,
                  out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """tokens [B, 3, d_tok] = cat(fused, text_conditioned, mapped) for query features [B, d_in]
-        and neighbour ids I_img / I_txt [B, k] (int64, device) into the two resident databases."""
+        and neighbour ids I_img / I_txt [B, k] (int64, device) into the two resident databases.
+        image_index / text_index may also be `kb.image, kb.text` of a ShardedKnowledgeBase after a
+        kb.retrieve2: I_* are then global labels (the merged I it returns), and each neighbour row is
+        read from the rank that owns it."""
         if not (feature.is_cuda and feature.dtype == torch.float32 and feature.dim() == 2
                 and feature.shape[1] == self.d_in):
             raise TypeError(f"feature must be a CUDA float32 [B, {self.d_in}] tensor")
@@ -128,10 +160,9 @@ class NeighbourConsumer:
             perm = perm.to(device=feature.device, dtype=torch.int32).contiguous()
             assert perm.numel() == k
             pp = perm.data_ptr()
-        _capi.check(self._lib.keds_consumer_forward(
-            self._h, feature.data_ptr(), image_index.rows_ptr(), image_index.ntotal, text_index.rows_ptr(),
-            text_index.ntotal, I_img.data_ptr(), I_txt.data_ptr(), pp, B, k, out.data_ptr(),
-            _stream_ptr(self.device)))
+        _capi.check(_call_forward(self._lib, "forward", self._h, feature, image_index, text_index,
+                                  (I_img.data_ptr(), I_txt.data_ptr(), pp, B, k, out.data_ptr(),
+                                   _stream_ptr(self.device))))
         return out
 
     def from_features(self, image_features: torch.Tensor, database, topk: int = 16,
@@ -143,13 +174,29 @@ class NeighbourConsumer:
         img2text sees them as given. shuffle: the batch-shared randperm of :218-219 (it cannot
         change the result beyond fp32 summation order). exclude: int64 [B] or [B, E] rows each query
         must not retrieve (e.g. database.rows_of(names), training without self-retrieval); None:
-        the reference's search."""
-        from .index import search2
+        the reference's search.
 
-        image_index, text_index = database[3], database[4]
+        A row-sharded `database` (a ShardedKnowledgeBase, or a sequence whose [3] / [4] are its
+        `image` / `text`) runs the DDP step of retrieval.get_retrieved_features: every rank calls
+        this with its own batch (sizes may differ), the queries and exclusions are all-gathered, one
+        kb.retrieve2 without feature gathers merges the labels, and each rank runs the consumer over
+        its own rows of them with its own randperm. Returns this rank's [B_r, 3, d_tok]."""
+        from .index import search2
+        from .sharded import ShardedKnowledgeBase, gather_ddp_step
+
+        if isinstance(database, ShardedKnowledgeBase):
+            image_index, text_index = database.image, database.text
+        else:
+            image_index, text_index = database[3], database[4]
+        kb = _sharded_kb(image_index, text_index)
         feats = image_features.detach().to(device=torch.device("cuda", self.device), dtype=torch.float32).contiguous()
         q = feats / feats.norm(dim=1, keepdim=True)
-        (_, I_img), (_, I_txt) = search2(image_index, text_index, q, topk, exclude=exclude)
+        if kb is None:
+            (_, I_img), (_, I_txt) = search2(image_index, text_index, q, topk, exclude=exclude)
+        else:
+            q_all, ex_all, (lo, hi) = gather_ddp_step(q, exclude, kb.group, kb.device)
+            res = kb.retrieve2(q_all, topk, want_feats=False, pool_mode=0, exclude=ex_all, rows=(lo, hi))
+            I_img, I_txt = res["I_img"][lo:hi], res["I_txt"][lo:hi]
         perm = torch.randperm(topk) if shuffle else None
         return self(feats, image_index, text_index, I_img, I_txt, perm)
 
@@ -194,10 +241,9 @@ class _ConsumerFn(torch.autograd.Function):
         if masks is not None:
             mp = (C.c_void_p * mod.n_hidden)(*[0 if m is None else m.data_ptr() for m in masks])
         pp = 0 if perm is None else perm.data_ptr()
-        _capi.check(mod._lib.keds_consumer_forward_train(
-            mod._h, feature.data_ptr(), image_index.rows_ptr(), image_index.ntotal, text_index.rows_ptr(),
-            text_index.ntotal, I_img.data_ptr(), I_txt.data_ptr(), pp, B, k, mp, tokens.data_ptr(),
-            _stream_ptr(mod.device)))
+        _capi.check(_call_forward(mod._lib, "forward_train", mod._h, feature, image_index, text_index,
+                                  (I_img.data_ptr(), I_txt.data_ptr(), pp, B, k, mp, tokens.data_ptr(),
+                                   _stream_ptr(mod.device))))
         ctx.mod, ctx.keep = mod, (masks, feature, I_img, I_txt, perm)   # alive until the backward has run
         return tokens
 
@@ -222,7 +268,13 @@ class TrainableNeighbourConsumer(torch.nn.Module):
     `flat` holds every weight and bias (layout: keds_consumer_param_offset); `state_dicts()` hands them
     back under the reference's parameter names (views), `load_state_dicts` takes them in. In train()
     mode IM2TEXT's dropout (src/model/model.py:110-116, p = `dropout`) is applied with masks drawn
-    by torch's generator; eval() runs the plain forward."""
+    by torch's generator; eval() runs the plain forward.
+
+    On row-sharded bases the indices are `kb.image, kb.text` of a ShardedKnowledgeBase and the ids
+    global labels (neighbour rows read from their owners), e.g. per DDP rank:
+
+        out = kb.retrieve2(q_all, 16, want_feats=False, exclude=ex_all, rows=(lo, hi))
+        tokens = consumer(feature, kb.image, kb.text, out["I_img"][lo:hi], out["I_txt"][lo:hi], perm)"""
 
     def __init__(self, img2text_sd: Mapping[str, torch.Tensor], retrieval_fuse_sd: Mapping[str, torch.Tensor],
                  text_condition_sd: Mapping[str, torch.Tensor], heads: int = 8, device: int = 0,

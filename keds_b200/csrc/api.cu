@@ -1832,11 +1832,11 @@ int ex_check_rows(const keds_exchange* ex, keds_index* const* dbs, int n_db) {
     const ShardRowsDb& rd = ex->rows[i];
     const int me = ex->my_rank;
     if (!ex->attached[i])
-      return fail(KEDS_ERR_ARG, "retrieve2_sharded: database %d has no rows attached to the exchange", i);
+      return fail(KEDS_ERR_ARG, "sharded: database %d has no rows attached to the exchange", i);
     if (rd.n[me] != dbs[i]->n || rd.lo[me] != dbs[i]->id_offset ||
         (dbs[i]->n > 0 && rd.base[me] != dbs[i]->x_f32.as<float>()))
       return fail(KEDS_ERR_ARG,
-                  "retrieve2_sharded: the rows of database %d changed since keds_exchange_attach_rows "
+                  "sharded: the rows of database %d changed since keds_exchange_attach_rows "
                   "(re-attach on every rank after each add)", i);
   }
   return 0;

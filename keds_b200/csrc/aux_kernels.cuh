@@ -826,10 +826,21 @@ __global__ void k_gather_rows(const float* __restrict__ base, long long n_base, 
 
 // The neighbour consumer's MLP input in one launch: rows [queries | image neighbours | text
 // neighbours] = [B | B k | B k] x d (src/trainer.py:59-65 feeds the same three blocks through
-// IM2TEXT). One warp per row; image neighbours follow the shared permutation; ids outside their
-// base give zero rows.
-__global__ void k_consumer_rows(const float* __restrict__ q, const float* __restrict__ base_img, long long n_img,
-                                const float* __restrict__ base_txt, long long n_txt,
+// IM2TEXT). One warp per row; image neighbours follow the shared permutation; `rows` resolves a
+// neighbour id of either stream to its row, or to nullptr (a zero row): ConsumerLocalRows for bases
+// resident on this GPU, ConsumerShardRows (p2p_exchange.cuh) for row-sharded bases.
+struct ConsumerLocalRows {
+  const float* __restrict__ base_img;
+  long long n_img;
+  const float* __restrict__ base_txt;
+  long long n_txt;
+  __device__ __forceinline__ const float* operator()(bool img, long long id, int d) const {
+    return id >= 0 && id < (img ? n_img : n_txt) ? (img ? base_img : base_txt) + id * d : nullptr;
+  }
+};
+
+template <class Rows>
+__global__ void k_consumer_rows(const float* __restrict__ q, const Rows rows,
                                 const long long* __restrict__ I_img, const long long* __restrict__ I_txt,
                                 const int* __restrict__ perm, long long B, int k, int d, float* __restrict__ out) {
   const int lane = threadIdx.x & 31;
@@ -846,7 +857,7 @@ __global__ void k_consumer_rows(const float* __restrict__ q, const float* __rest
     const int j = static_cast<int>(r % k);
     const int pj = (img && perm) ? perm[j] : j;
     const long long id = static_cast<unsigned int>(pj) < static_cast<unsigned int>(k) ? (img ? I_img : I_txt)[b * k + pj] : -1;
-    if (id >= 0 && id < (img ? n_img : n_txt)) src = (img ? base_img : base_txt) + id * d;
+    src = rows(img, id, d);
   }
   float* o = out + w * d;
   if ((d & 3) == 0 && src != nullptr && ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(o)) & 15) == 0) {

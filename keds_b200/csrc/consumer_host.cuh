@@ -393,26 +393,62 @@ int keds_consumer_finalize(keds_consumer_t* c) {
 
 namespace {
 
+// Where the neighbour rows come from: the two resident bases of keds_consumer_forward[_train]
+// (local ids), or every rank's rows of two row-sharded bases (global labels; sharded = true).
+struct ConsumerRowSource {
+  bool sharded = false;
+  ConsumerLocalRows local{};
+  ConsumerShardRows shard{};
+};
+
+ConsumerRowSource local_rows(const float* base_img, int64_t n_img, const float* base_txt, int64_t n_txt) {
+  ConsumerRowSource src;
+  src.local = ConsumerLocalRows{base_img, static_cast<long long>(n_img), base_txt, static_cast<long long>(n_txt)};
+  return src;
+}
+
+// img / txt: this rank's shards of the two bases of `ex` (databases 0 and 1). Refuses, before
+// anything is queued, what the rows of the exchange cannot serve: another device or width, a base
+// that is not attached, this rank's rows moved or grown since the attach.
+int shard_rows(const keds_consumer* c, keds_index* img, keds_index* txt, const keds_exchange* ex,
+               ConsumerRowSource* src) {
+  if (!c || !img || !txt || !ex) return fail(KEDS_ERR_ARG, "consumer_forward_sharded: NULL argument");
+  if (img->device != c->device || txt->device != c->device || ex->device != c->device)
+    return fail(KEDS_ERR_ARG, "consumer_forward_sharded: consumer, indices and exchange live on different devices");
+  if (img->d != c->d_in || txt->d != c->d_in)
+    return fail(KEDS_ERR_ARG, "consumer_forward_sharded: database widths %d / %d differ from the consumer's d_in %d",
+                img->d, txt->d, c->d_in);
+  keds_index* const dbs[2] = {img, txt};
+  CKS(ex_check_rows(ex, dbs, 2));
+  src->sharded = true;
+  src->shard.db[0] = ex->rows[0];
+  src->shard.db[1] = ex->rows[1];
+  src->shard.n_ranks = ex->n_ranks;
+  return 0;
+}
+
 // The forward pass. train = false: eval (dropout is the identity), scratch reused across layers.
 // train = true: hidden activations, per-layer queries / attention outputs and layer inputs are
 // kept for keds_consumer_backward; masks[i] (nullable) is hidden layer i's dropout multiplier.
-int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_img, int64_t n_img,
-                          const float* base_txt, int64_t n_txt, const int64_t* I_img, const int64_t* I_txt,
-                          const int32_t* perm, int64_t B, int k, float* tokens, void* stream, bool train,
-                          const float* const* masks) {
-  if (!c || !q || !base_img || !base_txt || !I_img || !I_txt || !tokens)
+int consumer_forward_impl(keds_consumer_t* c, const float* q, const ConsumerRowSource& src, const int64_t* I_img,
+                          const int64_t* I_txt, const int32_t* perm, int64_t B, int k, float* tokens, void* stream,
+                          bool train, const float* const* masks) {
+  const ConsumerLocalRows& lr = src.local;
+  if (!c || !q || !I_img || !I_txt || !tokens || (!src.sharded && (!lr.base_img || !lr.base_txt)))
     return fail(KEDS_ERR_ARG, "consumer_forward: NULL argument");
   if (!c->finalized) return fail(KEDS_ERR_ARG, "consumer_forward: call keds_consumer_finalize first");
-  if (B < 0 || k <= 0 || k > 1024 || n_img < 0 || n_txt < 0) return fail(KEDS_ERR_ARG, "consumer_forward: bad B or k");
+  if (B < 0 || k <= 0 || k > 1024 || (!src.sharded && (lr.n_img < 0 || lr.n_txt < 0)))
+    return fail(KEDS_ERR_ARG, "consumer_forward: bad B or k");
   if (B == 0) return 0;
   if (B * (1 + 2 * (int64_t)k) > (int64_t(1) << 30)) return fail(KEDS_ERR_ARG, "consumer_forward: batch too large");
   if (attend_smem(c, k) > static_cast<size_t>(c->attend_max))
     return fail(KEDS_ERR_ARG, "consumer_forward: heads * (dim_head + k) too large for the attention kernel");
   if (train && attend_bwd_smem(c, k) > static_cast<size_t>(c->attend_max))
     return fail(KEDS_ERR_ARG, "consumer_forward_train: heads * (dim_head + k) too large for the attention backward");
-  for (const void* ptr : {(const void*)q, (const void*)base_img, (const void*)base_txt, (const void*)I_img,
+  for (const void* ptr : {(const void*)q, (const void*)lr.base_img, (const void*)lr.base_txt, (const void*)I_img,
                           (const void*)I_txt, (const void*)tokens})
-    if (!locate(ptr)) return fail(KEDS_ERR_ARG, "consumer_forward: all buffers must be device memory");
+    if ((ptr || !src.sharded) && !locate(ptr))
+      return fail(KEDS_ERR_ARG, "consumer_forward: all buffers must be device memory");
   DeviceGuard g(c->device);
   if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -453,9 +489,12 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const float* base_
   // rows of the MLP input: [queries | image neighbours | text neighbours], one launch
   float* xin = c->xin.as<float>();
   const unsigned gblocks = static_cast<unsigned>(((B + 2 * Bk) * 32 + 255) / 256);
-  k_consumer_rows<<<gblocks, 256, 0, st>>>(q, base_img, static_cast<long long>(n_img), base_txt,
-                                           static_cast<long long>(n_txt), reinterpret_cast<const long long*>(I_img),
-                                           reinterpret_cast<const long long*>(I_txt), perm, B, k, c->d_in, xin);
+  const long long* Ii = reinterpret_cast<const long long*>(I_img);
+  const long long* It = reinterpret_cast<const long long*>(I_txt);
+  if (src.sharded)
+    k_consumer_rows<<<gblocks, 256, 0, st>>>(q, src.shard, Ii, It, perm, B, k, c->d_in, xin);
+  else
+    k_consumer_rows<<<gblocks, 256, 0, st>>>(q, src.local, Ii, It, perm, B, k, c->d_in, xin);
   CK(cudaGetLastError());
   c->launches += 1;
 
@@ -553,8 +592,16 @@ extern "C" {
 int keds_consumer_forward(keds_consumer_t* c, const float* q, const float* base_img, int64_t n_img,
                           const float* base_txt, int64_t n_txt, const int64_t* I_img, const int64_t* I_txt,
                           const int32_t* perm, int64_t B, int k, float* tokens, void* stream) {
-  return consumer_forward_impl(c, q, base_img, n_img, base_txt, n_txt, I_img, I_txt, perm, B, k, tokens, stream, false,
-                               nullptr);
+  return consumer_forward_impl(c, q, local_rows(base_img, n_img, base_txt, n_txt), I_img, I_txt, perm, B, k, tokens,
+                               stream, false, nullptr);
+}
+
+int keds_consumer_forward_sharded(keds_consumer_t* c, keds_index_t* img, keds_index_t* txt, keds_exchange_t* ex,
+                                  const float* feat, const int64_t* I_img, const int64_t* I_txt, const int32_t* perm,
+                                  int64_t B, int k, float* tokens, void* stream) {
+  ConsumerRowSource src;
+  CKS(shard_rows(c, img, txt, ex, &src));
+  return consumer_forward_impl(c, feat, src, I_img, I_txt, perm, B, k, tokens, stream, false, nullptr);
 }
 
 int keds_consumer_set_debug(keds_consumer_t* c, int enable) {

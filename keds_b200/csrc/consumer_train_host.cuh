@@ -204,8 +204,17 @@ int keds_consumer_forward_train(keds_consumer_t* c, const float* feat, const flo
                                 const float* base_txt, int64_t n_txt, const int64_t* I_img, const int64_t* I_txt,
                                 const int32_t* perm, int64_t B, int k, const float* const* masks, float* tokens,
                                 void* stream) {
-  return consumer_forward_impl(c, feat, base_img, n_img, base_txt, n_txt, I_img, I_txt, perm, B, k, tokens, stream, true,
-                               masks);
+  return consumer_forward_impl(c, feat, local_rows(base_img, n_img, base_txt, n_txt), I_img, I_txt, perm, B, k, tokens,
+                               stream, true, masks);
+}
+
+int keds_consumer_forward_train_sharded(keds_consumer_t* c, keds_index_t* img, keds_index_t* txt, keds_exchange_t* ex,
+                                        const float* feat, const int64_t* I_img, const int64_t* I_txt,
+                                        const int32_t* perm, int64_t B, int k, const float* const* masks,
+                                        float* tokens, void* stream) {
+  ConsumerRowSource src;
+  CKS(shard_rows(c, img, txt, ex, &src));
+  return consumer_forward_impl(c, feat, src, I_img, I_txt, perm, B, k, tokens, stream, true, masks);
 }
 
 int keds_consumer_debug_hidden(keds_consumer_t* c, int layer, float* out, int64_t n, void* stream) {

@@ -73,6 +73,25 @@ struct ShardRowsDb {
   long long n[P2P_MAX_RANKS];
 };
 
+// Where global label `lab` lives: row lab - lo[r] of the rank r with lo[r] <= lab < lo[r] + n[r], read
+// in place from that rank's fp32 master; nullptr when no shard holds it (-1 padding included).
+__device__ __forceinline__ const float* shard_row(const ShardRowsDb& rd, int n_ranks, long long lab, int d) {
+  const float* row = nullptr;
+  for (int r = 0; r < n_ranks; ++r)
+    if (lab >= rd.lo[r] && lab < rd.lo[r] + rd.n[r]) row = rd.base[r] + (lab - rd.lo[r]) * d;
+  return row;
+}
+
+// Row source of k_consumer_rows for row-sharded bases: ids are global labels, resolved per stream
+// (0 image, 1 text) through the owners' rows as keds_exchange_attach_rows mapped them.
+struct ConsumerShardRows {
+  ShardRowsDb db[2];
+  int n_ranks;
+  __device__ __forceinline__ const float* operator()(bool img, long long id, int d) const {
+    return shard_row(db[img ? 0 : 1], n_ranks, id, d);
+  }
+};
+
 struct ShardConsume {
   ConsumeParams cons;  // feat / pool of the output rows [0, gridDim.x)
   int n_ranks, k, d, metric;
@@ -105,10 +124,7 @@ k_shard_consume(const ShardConsume p) {
   for (int r = 0; r < p.n_ranks; ++r) bits |= reinterpret_cast<uintptr_t>(rd.base[r]);
   griddep_wait();  // the merged rows are complete
   for (int j = threadIdx.x; j < p.k; j += blockDim.x) {
-    const long long lab = p.I[s][q * p.k + j];
-    const float* row = nullptr;
-    for (int r = 0; r < p.n_ranks; ++r)
-      if (lab >= rd.lo[r] && lab < rd.lo[r] + rd.n[r]) row = rd.base[r] + (lab - rd.lo[r]) * p.d;
+    const float* row = shard_row(rd, p.n_ranks, p.I[s][q * p.k + j], p.d);
     ptr[j] = row;
     top_id[j] = row != nullptr ? static_cast<unsigned int>(j) : 0xFFFFFFFFu;  // -1 padding: a zero row
     top_d[j] = p.D[s][q * p.k + j];
