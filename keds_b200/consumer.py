@@ -32,6 +32,8 @@ import torch
 
 from . import _capi
 from .index import GpuIndexFlat, _stream_ptr
+from .retrieval import _device_perm
+from .sharded import ShardedKnowledgeBase, _sharded_kb
 
 KIND_MLP, KIND_TO_Q, KIND_TO_K, KIND_TO_V, KIND_TO_OUT = 0, 1, 2, 3, 4
 STACK_IMAGE, STACK_TEXT = 0, 1
@@ -42,21 +44,6 @@ def _count_prefix(sd: Mapping[str, torch.Tensor], fmt: str) -> int:
     while fmt.format(n) in sd:
         n += 1
     return n
-
-
-def _sharded_kb(image_index, text_index):
-    """The ShardedKnowledgeBase whose two bases are (image_index, text_index); None for two local
-    indices. A mixed pair, or the bases of two different knowledge bases, raise TypeError."""
-    from .sharded import ShardedIndex
-
-    sharded = (isinstance(image_index, ShardedIndex), isinstance(text_index, ShardedIndex))
-    if not any(sharded):
-        return None
-    kb = image_index._kb if sharded[0] else None
-    if not all(sharded) or kb is None or kb.image is not image_index or kb.text is not text_index:
-        raise TypeError("image_index and text_index must both be GpuIndexFlat, or be the `image` and `text` "
-                        "indices of one ShardedKnowledgeBase")
-    return kb
 
 
 def _call_forward(lib, name, h, feature, image_index, text_index, tail):
@@ -155,14 +142,10 @@ class NeighbourConsumer:
         B, k = I_img.shape
         if out is None:
             out = torch.empty((B, 3, self.d_tok), dtype=torch.float32, device=feature.device)
-        pp = 0
-        if perm is not None:
-            perm = perm.to(device=feature.device, dtype=torch.int32).contiguous()
-            assert perm.numel() == k
-            pp = perm.data_ptr()
+        perm = _device_perm(perm, k, feature.device)
         _capi.check(_call_forward(self._lib, "forward", self._h, feature, image_index, text_index,
-                                  (I_img.data_ptr(), I_txt.data_ptr(), pp, B, k, out.data_ptr(),
-                                   _stream_ptr(self.device))))
+                                  (I_img.data_ptr(), I_txt.data_ptr(), 0 if perm is None else perm.data_ptr(), B, k,
+                                   out.data_ptr(), _stream_ptr(self.device))))
         return out
 
     def from_features(self, image_features: torch.Tensor, database, topk: int = 16,
@@ -182,7 +165,6 @@ class NeighbourConsumer:
         kb.retrieve2 without feature gathers merges the labels, and each rank runs the consumer over
         its own rows of them with its own randperm. Returns this rank's [B_r, 3, d_tok]."""
         from .index import search2
-        from .sharded import ShardedKnowledgeBase, gather_ddp_step
 
         if isinstance(database, ShardedKnowledgeBase):
             image_index, text_index = database.image, database.text
@@ -194,8 +176,7 @@ class NeighbourConsumer:
         if kb is None:
             (_, I_img), (_, I_txt) = search2(image_index, text_index, q, topk, exclude=exclude)
         else:
-            q_all, ex_all, (lo, hi) = gather_ddp_step(q, exclude, kb.group, kb.device)
-            res = kb.retrieve2(q_all, topk, want_feats=False, pool_mode=0, exclude=ex_all, rows=(lo, hi))
+            res, (lo, hi) = kb.retrieve2_ddp(q, topk, exclude, want_feats=False, pool_mode=0)
             I_img, I_txt = res["I_img"][lo:hi], res["I_txt"][lo:hi]
         perm = torch.randperm(topk) if shuffle else None
         return self(feats, image_index, text_index, I_img, I_txt, perm)

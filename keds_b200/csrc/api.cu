@@ -313,6 +313,7 @@ int set_kernel_attrs(keds_index* ix) {
   CK(cudaFuncSetAttribute(k_select_rerank<2, 6, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   CK(cudaFuncSetAttribute(k_exact_fallback, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
   CK(cudaFuncSetAttribute(k_select_hits<2, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+  CK(cudaFuncSetAttribute(k_shard_consume, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
   const char* no_pdl = getenv("KEDS_NO_PDL");
   ix->use_pdl = !(no_pdl && no_pdl[0] == '1');
   if (const char* ws = getenv("KEDS_NO_WARM_START")) ix->warm_start = !(ws[0] == '1');
@@ -1477,6 +1478,30 @@ int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q,
 
 namespace {
 
+// The fused consumer's description (enabled: something to consume); `fn` names the entry point in
+// the refusals of its limits.
+int consume_params(const char* fn, const keds_index* img, int k, const int32_t* perm_img, const int32_t* perm_txt,
+                   int pool_mode, float tau, float* feat_img, float* feat_txt, float* pool_img, float* pool_txt,
+                   ConsumeParams& cp) {
+  if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "%s: pool_mode must be 0, 1 or 2", fn);
+  if (k > 1024) return fail(KEDS_ERR_ARG, "%s: k=%d too large for the fused consumer", fn, k);
+  const bool want_pool = pool_mode != 0 && (pool_img || pool_txt);
+  memset(&cp, 0, sizeof cp);
+  cp.enabled = (feat_img || feat_txt || want_pool) ? 1 : 0;
+  cp.mode = want_pool ? pool_mode : 0;
+  cp.tau = tau;
+  cp.perm[0] = perm_img;
+  cp.perm[1] = perm_txt;
+  cp.feat[0] = feat_img;
+  cp.feat[1] = feat_txt;
+  cp.pool[0] = want_pool ? pool_img : nullptr;
+  cp.pool[1] = want_pool ? pool_txt : nullptr;
+  // one warp per neighbour row; per-warp partial pools meet in shared memory ([warps][d/4] float4)
+  static_assert(RERANK_THREADS == EXACT_THREADS, "the consumer scratch is sized for one block shape");
+  cp.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
+  return 0;
+}
+
 // The fused consumer on top of a two-database call (c: both handles, q, the device results and
 // the exclusion); hostio: q may be page-locked host memory and the results get host mirrors.
 int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
@@ -1485,15 +1510,13 @@ int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* 
   keds_index* img = c.dbs[0];
   if (!img || !c.dbs[1] || !c.q || !c.D[0] || !c.I[0] || !c.D[1] || !c.I[1])
     return fail(KEDS_ERR_ARG, "retrieve2: null handle, query or result pointer");
-  if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "retrieve2: pool_mode must be 0, 1 or 2");
+  ConsumeParams cp;
+  CKS(consume_params("retrieve2", img, c.k, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt,
+                     cp));
   if ((!hostio && !locate(c.q)) || !locate(c.D[0]) || !locate(c.I[0]) || !locate(c.D[1]) || !locate(c.I[1]))
     return fail(KEDS_ERR_ARG, "retrieve2: device pointers only");
   if ((Dh_img == nullptr) != (Ih_img == nullptr) || (Dh_txt == nullptr) != (Ih_txt == nullptr))
     return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host mirror needs both its D and its I block");
-  if (c.k > 1024) return fail(KEDS_ERR_ARG, "retrieve2: k=%d too large for the fused consumer", c.k);
-  const bool want_pool = pool_mode != 0 && (pool_img || pool_txt);
-  ConsumeParams cp;
-  memset(&cp, 0, sizeof cp);
   {
     DeviceGuard g(img->device);
     if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", img->device);
@@ -1509,18 +1532,7 @@ int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* 
     cp.host_D[1] = static_cast<float*>(mirror[2]);
     cp.host_I[1] = static_cast<long long*>(mirror[3]);
   }
-  cp.enabled = (feat_img || feat_txt || want_pool || Dh_img || Dh_txt) ? 1 : 0;
-  cp.mode = want_pool ? pool_mode : 0;
-  cp.tau = tau;
-  cp.perm[0] = perm_img;
-  cp.perm[1] = perm_txt;
-  cp.feat[0] = feat_img;
-  cp.feat[1] = feat_txt;
-  cp.pool[0] = want_pool ? pool_img : nullptr;
-  cp.pool[1] = want_pool ? pool_txt : nullptr;
-  // one warp per neighbour row; per-warp partial pools meet in shared memory ([warps][d/4] float4)
-  static_assert(RERANK_THREADS == EXACT_THREADS, "the consumer scratch is sized for one block shape");
-  cp.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
+  if (Dh_img || Dh_txt) cp.enabled = 1;  // the host mirrors are the consumer's too
   if (cp.enabled) c.cons = cp;
   return search_impl(c, hostio ? IO_MAPPED : IO_DEVICE, stream);
 }
@@ -2043,16 +2055,16 @@ int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t
                            const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
   if (!img || !txt || !ex || !q || !D_img || !I_img || !D_txt || !I_txt || nq <= 0 || k <= 0)
     return fail(KEDS_ERR_ARG, "retrieve2_sharded: null handle / pointer or bad nq / k");
-  if (k > 1024) return fail(KEDS_ERR_ARG, "retrieve2_sharded: k=%d too large for the fused consumer", k);
-  if (pool_mode < 0 || pool_mode > 2) return fail(KEDS_ERR_ARG, "retrieve2_sharded: pool_mode must be 0, 1 or 2");
+  ConsumeParams cp;
+  CKS(consume_params("retrieve2_sharded", img, k, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img,
+                     pool_txt, cp));
   if (row_lo < 0 || row_hi < row_lo || row_hi > nq)
     return fail(KEDS_ERR_ARG, "retrieve2_sharded: rows [%lld, %lld) outside [0, %lld)", (long long)row_lo,
                 (long long)row_hi, (long long)nq);
   if (ex->device != img->device || txt->device != img->device)
     return fail(KEDS_ERR_ARG, "retrieve2_sharded: exchange and indices live on different devices");
-  const bool want_pool = pool_mode != 0 && (pool_img || pool_txt);
-  const void* dev_ptrs[] = {q, D_img, I_img, D_txt, I_txt, feat_img, feat_txt, want_pool ? pool_img : nullptr,
-                            want_pool ? pool_txt : nullptr, perm_img, perm_txt};
+  const void* dev_ptrs[] = {q, D_img, I_img, D_txt, I_txt, feat_img, feat_txt, cp.pool[0], cp.pool[1], perm_img,
+                            perm_txt};
   for (const void* p : dev_ptrs)
     if (p && locate(p).device != img->device)
       return fail(KEDS_ERR_ARG, "retrieve2_sharded: device pointers of the indices' GPU only");
@@ -2063,19 +2075,10 @@ int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t
   int64_t* I[2] = {I_img, I_txt};
   CKS(sharded_search(c, ex, D, I, stream));
   const int64_t nb = row_hi - row_lo;
-  if (nb == 0 || !(feat_img || feat_txt || want_pool)) return 0;
+  if (nb == 0 || !cp.enabled) return 0;
   ShardConsume sc;
   memset(&sc, 0, sizeof sc);
-  sc.cons.enabled = 1;
-  sc.cons.mode = want_pool ? pool_mode : 0;
-  sc.cons.tau = tau;
-  sc.cons.perm[0] = perm_img;
-  sc.cons.perm[1] = perm_txt;
-  sc.cons.feat[0] = feat_img;
-  sc.cons.feat[1] = feat_txt;
-  sc.cons.pool[0] = want_pool ? pool_img : nullptr;
-  sc.cons.pool[1] = want_pool ? pool_txt : nullptr;
-  sc.cons.part4 = (img->d & 3) == 0 ? (RERANK_THREADS / 32) * (img->d >> 2) : 0;
+  sc.cons = cp;
   sc.n_ranks = ex->n_ranks;
   sc.k = k;
   sc.d = img->d;
@@ -2088,11 +2091,8 @@ int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t
   }
   const size_t smem = static_cast<size_t>(sc.cons.part4) * 16 + static_cast<size_t>(k) * 20;
   DeviceGuard g(img->device);
-  static std::atomic<bool> attr[64];
-  if (img->device >= 64 || !attr[img->device].load(std::memory_order_acquire)) {
-    CK(cudaFuncSetAttribute(k_shard_consume, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    if (img->device < 64) attr[img->device].store(true, std::memory_order_release);
-  }
+  // (with both of this rank's shards empty no search pass ran to set the attributes)
+  CKS(set_kernel_attrs(img));
   CKS(launch_k(img->use_pdl, k_shard_consume, dim3(static_cast<unsigned>(nb), 2), dim3(RERANK_THREADS), smem,
                static_cast<cudaStream_t>(stream), sc));
   return 0;

@@ -43,6 +43,33 @@ def check_perm(perm: Optional[torch.Tensor], k: int, name: str = "perm") -> None
         raise ValueError(f"{name}: not a permutation of range({k}): {perm.tolist()[:32]}")
 
 
+def _device_perm(perm: Optional[torch.Tensor], k: int, device) -> Optional[torch.Tensor]:
+    """`perm` as the contiguous int32 tensor on `device` that the kernels read (None stays None). The
+    caller keeps the result referenced until the native call that reads it has been queued."""
+    if perm is None:
+        return None
+    perm = perm.to(device=device, dtype=torch.int32).contiguous()
+    assert perm.numel() == k
+    return perm
+
+
+def _step_outputs(o: dict, device, nq: int, nb: int, k: int, d: int, want_feats: bool, pool_mode: int):
+    """The retrieve2 outputs in `o` (D_* / I_* [nq, k], feat_* [nb, k, d], pool_* [nb, d] for the nb consumer
+    rows; None when not asked for), reused or replaced as retrieve2 documents."""
+    f32, i64 = torch.float32, torch.int64
+    feat, pool = ((nb, k, d) if want_feats else None), ((nb, d) if pool_mode != POOL_NONE else None)
+    res = []
+    for name, shape, dtype in (("D_img", (nq, k), f32), ("I_img", (nq, k), i64), ("D_txt", (nq, k), f32),
+                               ("I_txt", (nq, k), i64), ("feat_img", feat, f32), ("feat_txt", feat, f32),
+                               ("pool_img", pool, f32), ("pool_txt", pool, f32)):
+        t = None if shape is None else o.get(name)
+        if shape is not None and (t is None or tuple(t.shape) != shape or t.dtype != dtype or t.device != device
+                                  or not t.is_contiguous()):
+            t = o[name] = torch.empty(shape, dtype=dtype, device=device)
+        res.append(t)
+    return res
+
+
 def gather_rows(index: GpuIndexFlat, I: torch.Tensor, perm: Optional[torch.Tensor] = None) -> torch.Tensor:
     """out[b, j, :] = rows[I[b, perm[j]], :] from the index's resident fp32 rows (device tensors)."""
     lib = _capi.load()
@@ -50,14 +77,10 @@ def gather_rows(index: GpuIndexFlat, I: torch.Tensor, perm: Optional[torch.Tenso
     I = I.contiguous()
     B, k = I.shape
     out = torch.empty((B, k, index.d), dtype=torch.float32, device=I.device)
-    p = 0
-    if perm is not None:
-        perm = perm.to(device=I.device, dtype=torch.int32).contiguous()
-        assert perm.numel() == k
-        p = perm.data_ptr()
+    perm = _device_perm(perm, k, I.device)
     _capi.check(
-        lib.keds_gather_pool(index.rows_ptr(), index.ntotal, I.data_ptr(), 0, p, B, k, 1, index.d,
-                             out.data_ptr(), _stream_ptr(index.device))
+        lib.keds_gather_pool(index.rows_ptr(), index.ntotal, I.data_ptr(), 0, 0 if perm is None else perm.data_ptr(),
+                             B, k, 1, index.d, out.data_ptr(), _stream_ptr(index.device))
     )
     return out
 
@@ -183,31 +206,25 @@ def get_retrieved_features(feature, database, args=None, topk: int = 16, use_fai
     sharded step over all of them and each gets the [B, topk, d] pair of its own block of rows, its
     image stream permuted by its own torch.randperm(topk) as the reference does per rank."""
     image_base, text_base, basenames, image_index, text_index = (database[i] for i in range(5))
-    from .sharded import ShardedIndex, gather_ddp_step
+    from .sharded import ShardedIndex, _sharded_kb
 
+    kb = None
     if isinstance(image_index, ShardedIndex) and isinstance(text_index, ShardedIndex):
-        kb = image_index._kb
-        if kb is None or kb.image is not image_index or kb.text is not text_index:
-            raise TypeError("database[3] and database[4] must be the image and text indices of one ShardedKnowledgeBase")
-        if use_faiss:
-            feature = feature / feature.norm(dim=1, keepdim=True)  # src/trainer.py:206
-        flags = 0 if use_faiss else _capi.SEARCH_FORCE_IP
-        perm = torch.randperm(topk) if use_faiss else None
-        q_all, ex_all, rows = gather_ddp_step(feature.detach(), exclude, kb.group, kb.device)
-        out = kb.retrieve2(q_all, topk, perm_img=perm, want_feats=True, pool_mode=0, flags=flags, exclude=ex_all,
-                           rows=rows)
-        return out["feat_img"].to(feature.device), out["feat_txt"].to(feature.device)
-    if not (_native(image_index) and _native(text_index)):
+        kb = _sharded_kb(image_index, text_index,
+                         "database[3] and database[4] must be the image and text indices of one ShardedKnowledgeBase")
+    elif not (_native(image_index) and _native(text_index)):
         raise TypeError("database[3] and database[4] must be keds_b200 GPU indices or the two indices of a "
                         "ShardedKnowledgeBase (no CPU path)")
     if use_faiss:
         feature = feature / feature.norm(dim=1, keepdim=True)  # src/trainer.py:206
-    dev = torch.device("cuda", image_index.device)
-    q = feature.detach().to(device=dev, dtype=torch.float32).contiguous()
     flags = 0 if use_faiss else _capi.SEARCH_FORCE_IP  # the torch branch ranks by raw inner product
     perm = torch.randperm(topk) if use_faiss else None  # CPU generator, like the reference (:218)
-    out = retrieve2(image_index, text_index, q, topk, perm_img=perm, want_feats=True, pool_mode=0, flags=flags,
-                    exclude=exclude)
+    kw = dict(perm_img=perm, want_feats=True, pool_mode=0, flags=flags)
+    if kb is not None:
+        out, _ = kb.retrieve2_ddp(feature.detach(), topk, exclude, **kw)
+    else:
+        q = feature.detach().to(device=torch.device("cuda", image_index.device), dtype=torch.float32).contiguous()
+        out = retrieve2(image_index, text_index, q, topk, exclude=exclude, **kw)
     return out["feat_img"].to(feature.device), out["feat_txt"].to(feature.device)
 
 
@@ -250,34 +267,10 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
         if not q.is_pinned() or q.dtype != torch.float32 or q.dim() != 2 or q.shape[1] != image_index.d or not q.is_contiguous():
             raise TypeError("retrieve2: a host query must be a pinned, contiguous float32 [B, d] tensor")
         dev = torch.device("cuda", image_index.device)
-    B, d = q.shape[0], image_index.d
+    B = q.shape[0]
     o = out if out is not None else {}
-
-    def buf(name, shape, dtype):
-        t = o.get(name)
-        if (t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev
-                or not t.is_contiguous()):
-            t = torch.empty(shape, dtype=dtype, device=dev)
-            o[name] = t
-        return t
-
-    Di, Ii = buf("D_img", (B, k), torch.float32), buf("I_img", (B, k), torch.int64)
-    Dt, It = buf("D_txt", (B, k), torch.float32), buf("I_txt", (B, k), torch.int64)
-    fi = ft = pi = pt = None
-    if want_feats:
-        fi, ft = buf("feat_img", (B, k, d), torch.float32), buf("feat_txt", (B, k, d), torch.float32)
-    if pool_mode != POOL_NONE:
-        pi, pt = buf("pool_img", (B, d), torch.float32), buf("pool_txt", (B, d), torch.float32)
-
-    def perm_ptr(p):
-        if p is None:
-            return 0, None
-        p = p.to(device=dev, dtype=torch.int32).contiguous()
-        assert p.numel() == k
-        return p.data_ptr(), p
-
-    pi_ptr, _keep1 = perm_ptr(perm_img)
-    pt_ptr, _keep2 = perm_ptr(perm_txt)
+    Di, Ii, Dt, It, fi, ft, pi, pt = _step_outputs(o, dev, B, B, k, image_index.d, want_feats, pool_mode)
+    perm_i, perm_t = _device_perm(perm_img, k, dev), _device_perm(perm_txt, k, dev)
     ptr = lambda t: 0 if t is None else t.data_ptr()
     ex = None if exclude is None else _exclude_arg(exclude, B, image_index.device, pinned_ok=hostio)
     mirrors = []
@@ -288,7 +281,7 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
             if t is not None and not (t.is_pinned() and t.dtype == dt and t.is_contiguous() and t.numel() == B * k):
                 raise TypeError(f"retrieve2: host_out[{name!r}] must be a pinned contiguous {dt} tensor of {B * k} elements")
             mirrors.append(ptr(t))
-    args = [image_index._h, text_index._h, q.data_ptr(), B, k, pi_ptr, pt_ptr, int(pool_mode), float(tau),
+    args = [image_index._h, text_index._h, q.data_ptr(), B, k, ptr(perm_i), ptr(perm_t), int(pool_mode), float(tau),
             Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), *mirrors, ptr(fi), ptr(ft), ptr(pi), ptr(pt)]
     if ex is not None:
         args += [ex.data_ptr(), ex.shape[1]]

@@ -22,7 +22,7 @@ import torch.distributed as dist
 
 from . import _capi
 from .index import GpuIndexFlat, _exclude_arg, _stream_ptr
-from .retrieval import check_perm
+from .retrieval import _device_perm, _step_outputs, check_perm
 
 
 def shard_bounds(n: int, world: int, rank: int) -> Tuple[int, int]:
@@ -37,6 +37,10 @@ def packed_layout(nq: int, k: int) -> Tuple[int, int, int]:
     d_bytes = nq * k * 4
     off_i = (d_bytes + 7) // 8 * 8
     return off_i + nq * k * 8, off_i, d_bytes
+
+
+def _exchange_name(exchange):
+    return "fused" if exchange == "p2p" else exchange  # the fused exchange's former name
 
 
 class _FusedExchange:
@@ -103,6 +107,18 @@ class _FusedExchange:
             self.handle = None
 
 
+def _grow_exchange(owner, need: int, floor: int) -> bool:
+    """Give `owner` (a lone ShardedIndex or a ShardedKnowledgeBase) an exchange of at least `need` entries,
+    at least `floor` when it allocates; True if it did. Collective: every rank grows at the same call."""
+    if owner._fx is not None and owner._fx.capacity >= need:
+        return False
+    if owner._fx is not None:  # peers may still be using the old buffers for a step in flight
+        torch.cuda.synchronize(owner.device)
+        dist.barrier(group=owner.group)
+    owner._fx = _FusedExchange(owner.world, owner.rank, max(need, floor), owner.device, owner.group)
+    return True
+
+
 class ShardedIndex:
     """exchange="fused" (default on GPUs): no collective call and no copy kernel in the step -- the
     search kernels store every finished result row straight into the peers' buffers over NVLink,
@@ -114,8 +130,7 @@ class ShardedIndex:
                  exchange: str = "fused", _local_index=None, _merge: Optional[Callable] = None) -> None:
         if not dist.is_initialized():
             raise RuntimeError("ShardedIndex needs an initialised torch.distributed process group")
-        if exchange == "p2p":
-            exchange = "fused"
+        exchange = _exchange_name(exchange)
         if exchange not in ("nccl", "fused"):
             raise ValueError("exchange must be 'nccl' or 'fused'")
         self.group = group
@@ -203,12 +218,7 @@ class ShardedIndex:
         lib = _capi.load()
         q = self.local._check_q_tensor(q)
         ex = None if exclude is None else _exclude_arg(exclude, nq, self.device.index)
-        if self._fx is None or self._fx.capacity < nq * k:
-            # (re)allocation is collective: every rank sees the same shapes in the same order
-            if self._fx is not None:
-                torch.cuda.synchronize(self.device)
-                dist.barrier(group=self.group)
-            self._fx = _FusedExchange(self.world, self.rank, max(nq * k, 8192), self.device, self.group)
+        fx = self._exchange(nq * k)
         if out is not None:
             Dg, Ig = out
             assert Dg.is_cuda and Ig.is_cuda and Dg.is_contiguous() and Ig.is_contiguous()
@@ -217,13 +227,20 @@ class ShardedIndex:
             Dg = torch.empty((nq, k), dtype=torch.float32, device=q.device)
             Ig = torch.empty((nq, k), dtype=torch.int64, device=q.device)
         if ex is None:
-            _capi.check(lib.keds_index_search_sharded(self.local._h, self._fx.handle, q.data_ptr(), nq, k,
+            _capi.check(lib.keds_index_search_sharded(self.local._h, fx.handle, q.data_ptr(), nq, k,
                                                       Dg.data_ptr(), Ig.data_ptr(), _stream_ptr(self.device.index)))
         else:
-            _capi.check(lib.keds_index_search_sharded_exclude(self.local._h, self._fx.handle, q.data_ptr(), nq, k,
+            _capi.check(lib.keds_index_search_sharded_exclude(self.local._h, fx.handle, q.data_ptr(), nq, k,
                                                               Dg.data_ptr(), Ig.data_ptr(), ex.data_ptr(), ex.shape[1],
                                                               _stream_ptr(self.device.index)))
         return Dg, Ig
+
+    def _exchange(self, need: int) -> _FusedExchange:
+        """The knowledge base's exchange for one of its bases (one set of peer buffers), else its own."""
+        if self._kb is not None:
+            return self._kb._exchange(need)
+        _grow_exchange(self, need, 8192)
+        return self._fx
 
     def exchange_stats(self) -> dict:
         """Synchronise and report how long the merge waited for the peers (rank skew); raises if a
@@ -234,6 +251,21 @@ class ShardedIndex:
 
     def check_exchange(self) -> None:
         self.exchange_stats()
+
+
+def _sharded_kb(image_index, text_index,
+                refusal: str = "image_index and text_index must both be GpuIndexFlat, or be the `image` and `text` "
+                               "indices of one ShardedKnowledgeBase"):
+    """The ShardedKnowledgeBase whose two bases are (image_index, text_index); None for two indices
+    that are not sharded. A mixed pair, or the bases of two different knowledge bases, raise
+    TypeError(refusal)."""
+    sharded = (isinstance(image_index, ShardedIndex), isinstance(text_index, ShardedIndex))
+    if not any(sharded):
+        return None
+    kb = image_index._kb if sharded[0] else None
+    if not all(sharded) or kb is None or kb.image is not image_index or kb.text is not text_index:
+        raise TypeError(refusal)
+    return kb
 
 
 def rank_block(batch_sizes, rank: int) -> Tuple[int, int, int]:
@@ -261,8 +293,7 @@ class ShardedKnowledgeBase:
 
     def __init__(self, d: int, metric: int, device: Optional[int] = None, group=None, exchange: str = "fused",
                  _local_index: Optional[Callable] = None, _retrieve: Optional[Callable] = None) -> None:
-        if exchange == "p2p":
-            exchange = "fused"
+        exchange = _exchange_name(exchange)
         if exchange != "fused":
             raise ValueError("ShardedKnowledgeBase: the retrieval step needs exchange='fused' (peer memory); "
                              f"got {exchange!r}")
@@ -305,15 +336,9 @@ class ShardedKnowledgeBase:
         n = (C.c_int64 * self.world)(*[e[2] for e in every])
         _capi.check(lib.keds_exchange_attach_rows(self._fx.handle, db, handles, lo, n))
 
-    def _exchange(self, need: int) -> "_FusedExchange":
-        if self._fx is None or self._fx.capacity < need:
-            # (re)allocation is collective: every rank sees the same shapes in the same order
-            if self._fx is not None:
-                torch.cuda.synchronize(self.device)
-                dist.barrier(group=self.group)
-            self._fx = _FusedExchange(self.world, self.rank, max(need, 16384), self.device, self.group)
-            for ix in (self.image, self.text):
-                ix._fx = self._fx
+    def _exchange(self, need: int) -> _FusedExchange:
+        if _grow_exchange(self, need, 16384):
+            self.image._fx = self.text._fx = self._fx
             self._attach_rows(0)
             self._attach_rows(1)
         return self._fx
@@ -352,7 +377,7 @@ class ShardedKnowledgeBase:
                                   or p.dtype not in (torch.int32, torch.int64)):
                 raise TypeError(f"retrieve2: {name} must be an integer tensor of {k} entries")
             check_perm(p, k, f"retrieve2: {name}")
-            perms.append(None if p is None else p.to(device=self.device, dtype=torch.int32).contiguous())
+            perms.append(_device_perm(p, k, self.device))
         ex = None
         if exclude is not None:
             ex = _exclude_arg(exclude, Bt, self.device.index) if self.device.type == "cuda" else \
@@ -362,31 +387,21 @@ class ShardedKnowledgeBase:
             return self._retrieve(q, k, perms[0], perms[1], want_feats, pool_mode, tau, flags, ex, (lo, hi))
         fx = self._exchange(2 * Bt * k)
         o = out if out is not None else {}
-        dev, d = self.device, self.d
-
-        def buf(name, shape, dtype):
-            t = o.get(name)
-            if (t is None or tuple(t.shape) != tuple(shape) or t.dtype != dtype or t.device != dev
-                    or not t.is_contiguous()):
-                t = torch.empty(shape, dtype=dtype, device=dev)
-                o[name] = t
-            return t
-
-        Di, Ii = buf("D_img", (Bt, k), torch.float32), buf("I_img", (Bt, k), torch.int64)
-        Dt, It = buf("D_txt", (Bt, k), torch.float32), buf("I_txt", (Bt, k), torch.int64)
-        fi = ft = pi = pt = None
-        if want_feats:
-            fi, ft = buf("feat_img", (hi - lo, k, d), torch.float32), buf("feat_txt", (hi - lo, k, d), torch.float32)
-        if pool_mode != 0:
-            pi, pt = buf("pool_img", (hi - lo, d), torch.float32), buf("pool_txt", (hi - lo, d), torch.float32)
+        Di, Ii, Dt, It, fi, ft, pi, pt = _step_outputs(o, self.device, Bt, hi - lo, k, self.d, want_feats, pool_mode)
         ptr = lambda t: 0 if t is None else t.data_ptr()
         lib = _capi.load()
         _capi.check(lib.keds_retrieve2_sharded(
             self.image.local._h, self.text.local._h, fx.handle, q.data_ptr(), Bt, k, ptr(perms[0]), ptr(perms[1]),
             int(pool_mode), float(tau), lo, hi, Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(),
             ptr(fi), ptr(ft), ptr(pi), ptr(pt), ptr(ex), 0 if ex is None else ex.shape[1], int(flags),
-            _stream_ptr(dev.index)))
+            _stream_ptr(self.device.index)))
         return o
+
+    def retrieve2_ddp(self, q: torch.Tensor, k: int, exclude=None, **kw):
+        """The DDP step: every rank passes its own queries [B_r, d] and exclusion; gather_ddp_step, then one
+        retrieve2(**kw) over every rank's queries with rows = this rank's block. Returns (out, (lo, hi))."""
+        q_all, ex_all, rows = gather_ddp_step(q, exclude, self.group, self.device)
+        return self.retrieve2(q_all, k, exclude=ex_all, rows=rows, **kw), rows
 
     def exchange_stats(self) -> dict:
         """Synchronise and report how long the merges waited for the peers; raises if a peer failed

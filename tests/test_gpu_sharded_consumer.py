@@ -9,9 +9,9 @@ Covers eval tokens (IP / L2, k = 16 / 64, with and without perm, labels with -1 
 12-row base at k = 16 and with E = 8 exclusions, labels outside every shard, an empty shard),
 from_features on the sharded base against from_features on an unsharded KnowledgeBase (unequal
 batches 48 / 37, with and without exclusion), training forward + backward in train() (dropout) and
-eval() (tokens and flat.grad), a step that grows the exchange before a consumer call, and the
-refusals: rows changed without a re-attach, a mixed or foreign index pair, a width mismatch, a base
-that has run no step.
+eval() (tokens and flat.grad), a step and a search of one base that grow the knowledge base's one
+exchange before a consumer call, and the refusals: rows changed without a re-attach, a mixed or
+foreign index pair, a width mismatch, a base that has run no step.
 
 The harness is that of test_gpu_sharded_retrieve.py: two GPUs over NCCL, or two processes sharing
 one GPU over gloo (peer reads then go through the cudaIpc mapping of the other process, on the same
@@ -168,6 +168,15 @@ def run_cases(rank, world, dev):
     assert kb._fx.capacity > cap
     c.eval_tokens(kb, refs, I_img, I_txt, perm16, 53)
     c.training(kb, refs, I_img[:96], I_txt[:96], perm16, 54)
+    # a search of one base that outgrows the exchange grows the knowledge base's one exchange
+    cap = kb._fx.capacity
+    q = unit(cap // 16 + 1, 55).to(dev)
+    Ds, Is = kb.image.search(q, 16)
+    Dr, Ir = refs[0].search(q, 16)
+    assert same_bits(Ds, Dr) and torch.equal(Is, Ir)
+    assert kb._fx.capacity > cap and kb.image._fx is kb.text._fx is kb._fx
+    I_img, I_txt = c.labels(kb, unit(16 * world, 56), 16)
+    c.eval_tokens(kb, refs, I_img, I_txt, perm16, 57)
     # -1 padding: k above the rows of a 12-row base, and E = 8 exclusions on it; an empty shard
     for n in (12, world - 1):
         for metric in (IP, L2):

@@ -36,7 +36,7 @@ def test_sharded_consumer_entry_points_refuse_null_arguments_without_a_gpu():
 
 
 def test_mixed_index_pair_is_a_type_error():
-    from keds_b200.consumer import _sharded_kb
+    from keds_b200.sharded import _sharded_kb
     from keds_b200.sharded import ShardedIndex
 
     local = object()
