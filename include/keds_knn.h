@@ -163,6 +163,27 @@ int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const fl
                                   int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img,
                                   float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude,
                                   int n_exclude, uint32_t flags, void* cuda_stream);
+/* ---- range search ------------------------------------------------------------------------------
+ * lims, D, I = index.range_search(q, radius) (Faiss' RangeSearchResult layout): every row n with
+ *   IP: s(n) > radius        L2: d(n) < radius (squared distance)
+ * strictly, where s / d is the library's exact fp32 score -- the same bits keds_index_search reports
+ * for that (query, row). Query i owns entries [lims[i], lims[i+1]) of D / I, ordered best first,
+ * ties by lower label (Faiss leaves this order open; here it is fixed). Labels include id_offset;
+ * KEDS_SEARCH_FORCE_IP is the only flag that applies. The tensor-core pass lists every row whose
+ * 16-bit-operand score lies above the radius minus the certificate's error bound and the rounding of
+ * the fp32 score (DESIGN.md section 3), and those rows are re-scored in fp32, so the answer is exact
+ * for every query, including queries the 16-bit format cannot hold.
+ * The result size is known only after the search, so the call has two steps:
+ *   range_search   q [nq][d] float32 and lims int64 [nq + 1]: host or device memory. Runs the search
+ *                  on cuda_stream, writes lims and synchronises the stream before it returns (it
+ *                  reads counts back between its kernels). D and I stay in handle-owned buffers.
+ *   range_results  copies the lims[nq] results out: D float32, I int64, host or device memory
+ *                  (device pointers: stream-ordered; host pointers: synchronous).
+ * The results stay valid until the next call on idx; a results buffer that grows bumps generation. */
+int keds_index_range_search(keds_index_t* idx, const float* q, int64_t nq, float radius, int64_t* lims,
+                            uint32_t flags, void* cuda_stream);
+int keds_index_range_results(keds_index_t* idx, float* D, int64_t* I, void* cuda_stream);
+
 /* Wait for the last asynchronous search on idx and report its device status. */
 int keds_index_sync(keds_index_t* idx, void* cuda_stream);
 int keds_index_last_stats(const keds_index_t* idx, keds_search_stats* out);

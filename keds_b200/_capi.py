@@ -98,6 +98,8 @@ SIGNATURES = {
         [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
          _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
     ),
+    "keds_index_range_search": (C.c_int, [_vp, _vp, C.c_int64, C.c_float, _vp, C.c_uint32, _vp]),
+    "keds_index_range_results": (C.c_int, [_vp, _vp, _vp, _vp]),
     "keds_index_label_hits": (C.c_int, [_vp, _vp, C.c_int64, _vp, _vp, _vp, C.c_int, _vp, _vp]),
     "keds_index_sync": (C.c_int, [_vp, _vp]),
     "keds_index_last_stats": (C.c_int, [_vp, C.POINTER(SearchStats)]),

@@ -14,6 +14,7 @@
 #include <vector>
 
 #include "aux_kernels.cuh"
+#include "range_search.cuh"
 
 using namespace keds;
 
@@ -193,9 +194,10 @@ PtrLoc locate(const void* p) {
   return l;
 }
 
-// [0],[1] n_flagged per db, [2] err word, [3..5] spare, [6] largest candidate band |C| of the search
-// (planner feedback), [7] spare
+// [0],[1] n_flagged per db, [2] err word, [3] spare, [4..5] range search: candidates found (64 bit),
+// [6] largest candidate band |C| of the search (planner feedback), [7] spare
 constexpr int CTRL_WORDS = 8;
+constexpr int CTRL_RANGE = 4;
 constexpr int CTRL_BAND = 6;
 // One block of status words per pass of a multi-pass call, so that no pass has to be read back
 // before the next one starts. Behind the status words: the exact fallback's work counters, one set
@@ -224,6 +226,13 @@ struct RankMode {
   const long long* target;   // [nq]
   const long long* exclude;  // [nq] or nullptr
   long long* out;            // [nq] ranks
+};
+
+// keds_index_range_search: the scoring kernel appends the rows inside each query's band, which are
+// re-scored, kept when strictly inside the radius, and ordered per query (range_search.cuh)
+struct RangeMode {
+  float radius;
+  long long* lims;  // [nq + 1] handle scratch; a pass writes its queries' entries and the one behind them
 };
 
 // How the scoring kernel covers nq queries: which kernel, its work units and query groups, and
@@ -268,6 +277,10 @@ struct keds_index {
   // per-call scratch (one search in flight per handle)
   DevBuf q_f32, q_bf16, qstat, cand, cand_cnt, cand_theta, flagged[2], ctrl, exact_scratch, rk, theta0;
   DevBuf ex_rows;  // search with exclusion: the staged local row ids [n_db][nq][n_ex] of the pass
+  // range search: band thresholds, candidates, order keys (two halves), per-query counts and offsets,
+  // read-back words, and the results of the last call (rg_total entries, valid until the next call)
+  DevBuf rg_thr, rg_cand, rg_key, rg_qcnt, rg_off, rg_word, rg_lims, rg_D, rg_I;
+  int64_t rg_total = 0;
   bool warm_start = true;  // lists start at a finished list's threshold (KEDS_NO_WARM_START=1: every list cold)
   DevBuf D_stage[2], I_stage[2];
   HostBuf h_q, h_out;  // pinned staging for host-pointer calls
@@ -305,6 +318,10 @@ int set_kernel_attrs(keds_index* ix) {
   CK(cudaFuncSetAttribute(k_score_topk<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)SCORE_SMEM_BYTES));
   CK(cudaFuncSetAttribute(k_score_topk<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)SCORE_PAIR_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(k_score_range<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                          (int)SCORE_SMEM_BYTES));
+  CK(cudaFuncSetAttribute(k_score_range<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                           (int)SCORE_PAIR_SMEM_BYTES));
   const char* no_pair = getenv("KEDS_NO_PAIR");
   ix->use_pair = !(no_pair && no_pair[0] == '1');
@@ -496,6 +513,7 @@ struct Call {
   int n_ex = 0;                   // k_prep_rows stages them as local row ids in owner->ex_rows
   HitsMode hits{};                // label hits at cut points in the re-rank's place
   RankMode rank{};                // gallery ranks in the top-k's place (rank.out set)
+  RangeMode range{};              // range search in the top-k's place (range.lims set)
   float* dump = nullptr;          // debug_scores: the raw scores, ld_dump per query
   int64_t ld_dump = 0;
 
@@ -725,18 +743,25 @@ int launch_prep(const Call& c, const Plan& pl, unsigned long long* tchain, cudaS
 }
 
 // The scoring kernel in the instantiation sp asks for: gallery ranking (rk_lo), top-k with
-// exclusion (ex_rows: tests each tile against the query's excluded rows) or the plain top-k.
+// exclusion (ex_rows: tests each tile against the query's excluded rows), range search (rg_out) or
+// the plain top-k.
 int launch_score(const Call& c, const Plan& pl, const ScoreParams& sp, cudaStream_t st) {
   keds_index* a = c.owner;
   const keds_index* x0 = c.dbs[0];
   const keds_index* x1 = c.n_db > 1 ? c.dbs[1] : c.dbs[0];
   if (pl.pair)
     CKS(launch_kc(a->use_pdl, 2,
-                  sp.rk_lo ? k_score_topk<true, true> : sp.ex_rows ? k_score_topk<true, false, true> : k_score_topk<true>,
+                  sp.rk_lo     ? k_score_topk<true, true>
+                  : sp.ex_rows ? k_score_topk<true, false, true>
+                  : sp.rg_out  ? k_score_range<true>
+                               : k_score_topk<true>,
                   dim3(pl.grid), dim3(SCORE_PAIR_THREADS), SCORE_PAIR_SMEM_BYTES, st, a->tm_q, x0->tm_xh, x1->tm_xh, sp));
   else
     CKS(launch_k(a->use_pdl,
-                 sp.rk_lo ? k_score_topk<false, true> : sp.ex_rows ? k_score_topk<false, false, true> : k_score_topk<false>,
+                 sp.rk_lo     ? k_score_topk<false, true>
+                 : sp.ex_rows ? k_score_topk<false, false, true>
+                 : sp.rg_out  ? k_score_range<false>
+                              : k_score_topk<false>,
                  dim3(pl.grid), dim3(SCORE_THREADS), SCORE_SMEM_BYTES, st, a->tm_q, x0->tm_x, x1->tm_x, sp));
   a->stats.launches++;
   CK(cudaGetLastError());
@@ -920,6 +945,132 @@ int launch_rank_count(const Call& c, const Plan& pl, const ScoreParams& sp, cuda
   return 0;
 }
 
+// Range search: row slices for the scoring kernel alone (there are no candidate lists to certify),
+// by the top-k planner's balance term.
+Plan range_plan(const keds_index* ix, int64_t nq) {
+  Plan pl{geometry(ix, 1, nq)};
+  const int T = static_cast<int>((ix->n + BN - 1) / BN);
+  double best = 1e300;
+  for (int S = 1; S <= std::min(T, S_MAX); ++S) {
+    const long long items = static_cast<long long>(pl.n_qg) * S;
+    const long long G = std::min<long long>(items, pl.units);
+    const long long per_cta = (items + G - 1) / G;
+    const double cost = static_cast<double>(per_cta) * ((T + S - 1) / S) + 0.35 * per_cta;
+    if (cost < best - 1e-9) {
+      best = cost;
+      pl.S = S;
+    }
+  }
+  pl.set_slices(1, pl.S);
+  return pl;
+}
+
+// Blocks for a grid-stride kernel over n work items of `per` threads each.
+unsigned stride_grid(const keds_index* a, long long n, int per) {
+  const long long want = (std::max(1ll, n) * per + 255) / 256;
+  return static_cast<unsigned>(std::min<long long>(want, 16ll * a->num_sms));
+}
+
+// Wait for the queued work and read n 64-bit device words; a fired watchdog is the call's error.
+int range_read(keds_index* a, const unsigned long long* words, unsigned long long* out, int n, cudaStream_t st) {
+  uint32_t err = 0;
+  CK(cudaMemcpyAsync(out, words, static_cast<size_t>(n) * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(&err, a->ctrl_cur + 2, 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  a->stats.err_word = err;
+  if (err != 0) return fail(KEDS_ERR_KERNEL, "device watchdog fired (range search): error word 0x%x", err);
+  return 0;
+}
+
+// One pass of a range search. The result size is known only once the pass has run, so it reads
+// back twice: the candidate count (a buffer that overflowed is grown and the scoring kernel rerun,
+// so no candidate is ever dropped), then the hit count (the results grow, keeping earlier passes).
+int range_pass(const Call& c, cudaStream_t st) {
+  keds_index* a = c.owner;
+  const keds_index* x = c.dbs[0];
+  const int64_t nq = c.nq;
+  const int metric = c.metric();
+  const float radius = c.range.radius;
+  const Plan pl = range_plan(a, nq);
+  a->stats.slices = pl.S;
+  a->stats.items = pl.n_items;
+  a->stats.grid = pl.grid;
+
+  CKS(launch_prep(c, pl, nullptr, st));  // also clears the status block, the candidate count included
+  CKS(a->rg_thr.ensure(static_cast<size_t>(nq) * 4));
+  CKS(launch_k(a->use_pdl, k_range_band, dim3(static_cast<unsigned>((nq + 255) / 256)), dim3(256), 0, st,
+               a->qstat.as<float4>(), x->dbstat.as<unsigned int>(), static_cast<int>(nq), a->d_pad, metric, radius,
+               a->eps_scale, a->rg_thr.as<float>()));
+  ScoreParams sp = score_params(c, pl, nullptr);
+  sp.theta0 = nullptr;
+  sp.rg_thr = a->rg_thr.as<float>();
+  unsigned long long* count = reinterpret_cast<unsigned long long*>(a->ctrl_cur + CTRL_RANGE);
+  sp.rg_count = count;
+  CKS(a->rg_cand.ensure(static_cast<size_t>(std::max<int64_t>(int64_t(1) << 16, nq * 64)) * 8));
+  sp.rg_out = a->rg_cand.as<uint2>();
+  sp.rg_cap = a->rg_cand.cap / 8;
+  CKS(launch_score(c, pl, sp, st));
+  a->stats.launches += 2;
+  unsigned long long n_cand = 0;
+  CKS(range_read(a, count, &n_cand, 1, st));
+  if (n_cand > sp.rg_cap) {
+    CKS(a->rg_cand.ensure(static_cast<size_t>(n_cand + n_cand / 4) * 8));
+    sp.rg_out = a->rg_cand.as<uint2>();
+    sp.rg_cap = a->rg_cand.cap / 8;
+    CK(cudaMemsetAsync(count, 0, 8, st));
+    CKS(launch_score(c, pl, sp, st));
+    CKS(range_read(a, count, &n_cand, 1, st));
+  }
+  const long long nc = static_cast<long long>(n_cand);
+
+  // exact scores, hits per query, offsets (and this pass's lims)
+  CKS(a->rg_qcnt.ensure(static_cast<size_t>(nq) * 4));
+  CKS(a->rg_off.ensure(static_cast<size_t>(nq + 1) * 8));
+  CKS(a->rg_key.ensure(static_cast<size_t>(std::max(nc, 1ll)) * 16));
+  CKS(a->rg_word.ensure(16));
+  CK(cudaMemsetAsync(a->rg_qcnt.p, 0, static_cast<size_t>(nq) * 4, st));
+  int* qcnt = a->rg_qcnt.as<int>();
+  long long* off = a->rg_off.as<long long>();
+  unsigned long long* k0 = a->rg_key.as<unsigned long long>();
+  unsigned long long* k1 = k0 + std::max(nc, 1ll);
+  if (nc > 0) {
+    k_range_rescore<<<stride_grid(a, nc, 32), 256, 0, st>>>(a->rg_cand.as<uint2>(), nc, c.q, x->x_f32.as<float>(),
+                                                            a->d, metric, radius, k0, qcnt);
+    a->stats.launches++;
+  }
+  k_range_scan<<<1, 1024, 0, st>>>(qcnt, static_cast<int>(nq), a->rg_total, off, c.range.lims,
+                                   a->rg_word.as<unsigned long long>());
+  a->stats.launches++;
+  unsigned long long w[2] = {0, 0};
+  CKS(range_read(a, a->rg_word.as<unsigned long long>(), w, 2, st));
+  const long long total = static_cast<long long>(w[0]), longest = static_cast<long long>(w[1]);
+  if (total == 0) return 0;
+
+  // the hits into their queries' segments, ordered by (score, label) inside each, then out
+  const size_t keep = static_cast<size_t>(a->rg_total);
+  const size_t need = keep + static_cast<size_t>(total);
+  if (need * 8 > a->rg_I.cap) {  // by half again at least, so that passes of one call rarely copy
+    CKS(a->rg_D.grow_keep(std::max(need * 4, a->rg_D.cap + a->rg_D.cap / 2), keep * 4));
+    CKS(a->rg_I.grow_keep(std::max(need * 8, a->rg_I.cap + a->rg_I.cap / 2), keep * 8));
+  }
+  k_range_scatter<<<stride_grid(a, nc, 1), 256, 0, st>>>(a->rg_cand.as<uint2>(), k0, nc, off, qcnt, k1);
+  unsigned long long* in = k1;
+  unsigned long long* out = k0;
+  k_range_sort_runs<<<stride_grid(a, total, 1), 256, 0, st>>>(in, out, total, off, static_cast<int>(nq));
+  std::swap(in, out);
+  a->stats.launches += 3;
+  for (long long run = RANGE_RUN; run < longest; run *= 2) {
+    k_range_merge<<<stride_grid(a, total, 1), 256, 0, st>>>(in, out, total, off, static_cast<int>(nq), run);
+    std::swap(in, out);
+    a->stats.launches++;
+  }
+  k_range_emit<<<stride_grid(a, total, 1), 256, 0, st>>>(in, total, metric, x->id_offset, a->rg_D.as<float>() + keep,
+                                                         a->rg_I.as<long long>() + keep);
+  CK(cudaGetLastError());
+  a->rg_total += total;
+  return 0;
+}
+
 // One pass (<= Q_PASS_MAX queries) of a call; q, D and I are device memory. The chain: prep, the
 // scoring kernel and its epilogue (re-rank, label hits or the rank count), the exact fallback.
 int search_pass(const Call& c, cudaStream_t st) {
@@ -938,6 +1089,7 @@ int search_pass(const Call& c, cudaStream_t st) {
   a->ctrl_cur = a->ctrl.as<unsigned int>() + static_cast<size_t>(c.pass) * CTRL_STRIDE;
   a->ctrl_passes = c.pass + 1;
   a->ctrl_slot = c.slot0;
+  if (c.range.lims) return range_pass(c, st);
   for (int i = 0; i < n_db; ++i) CKS(a->flagged[i].ensure(static_cast<size_t>(nq) * 4));
 
   int64_t n_min = ix[0]->n, n_max = ix[0]->n;
@@ -1012,6 +1164,7 @@ Call slice(const Call& c, int64_t q0, int64_t nb) {
     if (p.rank.exclude) p.rank.exclude += q0;
     p.rank.out += q0;
   }
+  if (p.range.lims) p.range.lims += q0;
   return p;
 }
 
@@ -1263,7 +1416,8 @@ int keds_index_create(int d, int metric, int device, keds_index_t** out) {
   DevBuf* tracked[] = {&ix->x_f32, &ix->x_bf16, &ix->bias, &ix->q_f32, &ix->q_bf16, &ix->qstat, &ix->cand,
                        &ix->cand_cnt, &ix->cand_theta, &ix->flagged[0], &ix->flagged[1], &ix->ctrl,
                        &ix->exact_scratch, &ix->D_stage[0], &ix->D_stage[1], &ix->I_stage[0], &ix->I_stage[1],
-                       &ix->rk, &ix->theta0, &ix->ex_rows};
+                       &ix->rk, &ix->theta0, &ix->ex_rows, &ix->rg_thr, &ix->rg_cand, &ix->rg_key,
+                       &ix->rg_qcnt, &ix->rg_off, &ix->rg_word, &ix->rg_lims, &ix->rg_D, &ix->rg_I};
   for (DevBuf* b : tracked) b->gen = &ix->generation;
   *out = ix;
   return 0;
@@ -1276,7 +1430,8 @@ void keds_index_free(keds_index_t* ix) {
                     &ix->qstat, &ix->cand, &ix->cand_cnt, &ix->cand_theta, &ix->flagged[0],
                     &ix->flagged[1], &ix->ctrl, &ix->exact_scratch, &ix->D_stage[0], &ix->D_stage[1],
                     &ix->I_stage[0], &ix->I_stage[1], &ix->timing, &ix->probe, &ix->rk, &ix->theta0,
-                    &ix->ex_rows};
+                    &ix->ex_rows, &ix->rg_thr, &ix->rg_cand, &ix->rg_key, &ix->rg_qcnt, &ix->rg_off,
+                    &ix->rg_word, &ix->rg_lims, &ix->rg_D, &ix->rg_I};
   for (DevBuf* b : bufs) b->release();
   ix->h_q.release();
   ix->h_out.release();
@@ -2115,6 +2270,60 @@ int keds_exchange_stats(keds_exchange_t* ex, void* stream, double* wait_us_avg, 
   if (w[1] != 0)
     return fail(KEDS_ERR_KERNEL, "sharded exchange: peer %u did not deliver within the watchdog window (error word 0x%x)",
                 w[1] - 0x500u, w[1]);
+  return 0;
+}
+
+int keds_index_range_search(keds_index_t* ix, const float* q, int64_t nq, float radius, int64_t* lims,
+                            uint32_t flags, void* stream) {
+  if (!ix || !lims || nq < 0 || (nq > 0 && !q)) return fail(KEDS_ERR_ARG, "range_search: null handle/query/lims or nq < 0");
+  if (flags & ~KEDS_SEARCH_FORCE_IP) return fail(KEDS_ERR_ARG, "range_search: flags 0x%x; only KEDS_SEARCH_FORCE_IP applies", flags);
+  if (radius != radius) return fail(KEDS_ERR_ARG, "range_search: radius is NaN");
+  if (ix->n > 0x7fffffffll - BN) return fail(KEDS_ERR_ARG, "index too large for 32-bit row ids");
+  DeviceGuard g(ix->device);
+  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  memset(&ix->stats, 0, sizeof ix->stats);
+  ix->rg_total = 0;
+  const PtrLoc ll = locate(lims);
+  if (ll && ll.device != ix->device) return fail(KEDS_ERR_ARG, "range_search: lims on device %d, index on %d", ll.device, ix->device);
+  CKS(ix->rg_lims.ensure(static_cast<size_t>(nq + 1) * 8));
+  Call c = call(1, ix, nullptr, q, nq, 1, nullptr, nullptr, nullptr, nullptr, flags);
+  c.range.radius = radius;
+  c.range.lims = ix->rg_lims.as<long long>();
+  if (nq == 0 || ix->n == 0) {
+    CK(cudaMemsetAsync(ix->rg_lims.p, 0, static_cast<size_t>(nq + 1) * 8, st));
+  } else {
+    const PtrLoc lq = locate(q);
+    if (lq && lq.device != ix->device) return fail(KEDS_ERR_ARG, "range_search: q on device %d, index on %d", lq.device, ix->device);
+    // host queries, and device queries off a 16-byte boundary (warp_exact_score would take its scalar
+    // order and so differ from search()), are scored from the handle's copy
+    if (!lq || (reinterpret_cast<uintptr_t>(q) & 15) != 0) {
+      const size_t qb = static_cast<size_t>(nq) * ix->d * 4;
+      CKS(ix->q_f32.ensure(qb));
+      CK(cudaMemcpyAsync(ix->q_f32.p, q, qb, cudaMemcpyDefault, st));
+      c.q = ix->q_f32.as<float>();
+    }
+    CKS(run_passes(c, st));
+  }
+  CK(cudaMemcpyAsync(lims, ix->rg_lims.p, static_cast<size_t>(nq + 1) * 8, cudaMemcpyDefault, st));
+  CK(cudaStreamSynchronize(st));
+  return 0;
+}
+
+int keds_index_range_results(keds_index_t* ix, float* D, int64_t* I, void* stream) {
+  if (!ix) return fail(KEDS_ERR_ARG, "range_results: null handle");
+  if (ix->rg_total == 0) return 0;
+  if (!D || !I) return fail(KEDS_ERR_ARG, "range_results: null output for %lld results", (long long)ix->rg_total);
+  DeviceGuard g(ix->device);
+  if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", ix->device);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const PtrLoc ld = locate(D), li = locate(I);
+  if ((ld && ld.device != ix->device) || (li && li.device != ix->device))
+    return fail(KEDS_ERR_ARG, "range_results: outputs on another device than the index");
+  const size_t n = static_cast<size_t>(ix->rg_total);
+  CK(cudaMemcpyAsync(D, ix->rg_D.p, n * 4, cudaMemcpyDefault, st));
+  CK(cudaMemcpyAsync(I, ix->rg_I.p, n * 8, cudaMemcpyDefault, st));
+  if (!ld || !li) CK(cudaStreamSynchronize(st));
   return 0;
 }
 

@@ -108,6 +108,14 @@ struct ScoreParams {
   const int* ex_rows;
   int n_ex;
   long long ex_ld;           // ints per database
+  // kRange only (range search, database 0): per query the band threshold in approximate-score
+  // space (range_search.cuh: k_range_band); every row scoring at or above it is appended as
+  // {query, row} to rg_out. rg_count counts every such row, also past rg_cap (overflow: the host
+  // grows the buffer and reruns the pass).
+  const float* rg_thr;
+  uint2* rg_out;
+  unsigned long long* rg_count;
+  unsigned long long rg_cap;
 };
 
 struct ItemCoord {
@@ -203,11 +211,17 @@ __device__ __noinline__ CandState compact_candidates(uint32_t slot0, int cnt, fl
 //                rows or -1 (overflow), cand_theta = the certain count (as int bits).
 // kExclude = true (top-k search only): rows listed per query in p.ex_rows never enter a list. A
 //                separate instantiation, so that the plain search keeps its code and registers.
-template <bool kPair, bool kRank = false, bool kExclude = false>
-__global__ void __launch_bounds__(ScoreCfg<kPair>::kThreads, 1)
-k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_x0,
-             const __grid_constant__ CUtensorMap tm_x1, const ScoreParams p) {
+// kRange = true: range search (kernel k_score_range). No candidate lists: every (query, row) whose
+//                approximate score (L2 bias included) is not below the query's band threshold
+//                p.rg_thr[q] is appended to p.rg_out, one atomic per warp and 32-column chunk that
+//                has any.
+// The kernels below are thin entry points around this body: the tensor maps are their
+// __grid_constant__ parameters, p their parameter block.
+template <bool kPair, bool kRank, bool kExclude, bool kRange>
+__device__ __forceinline__ void score_topk_body(const CUtensorMap& tm_q, const CUtensorMap& tm_x0,
+                                                const CUtensorMap& tm_x1, const ScoreParams& p) {
   static_assert(!(kRank && kExclude), "exclusion is a top-k search option");
+  static_assert(!(kRange && (kRank || kExclude)), "range search is a mode of its own");
   using Cfg = ScoreCfg<kPair>;
   constexpr int NSTAGE = Cfg::kStages;
   extern __shared__ uint8_t smem_raw[];
@@ -401,7 +415,7 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
       // eight appends -- which is what made short slices (k = 200 galleries: two tiles per item)
       // spend more time warming lists than scoring. Any stale value is still a valid start.
       float* th0 = nullptr;
-      if constexpr (!kRank) {
+      if constexpr (!kRank && !kRange) {
         if (active && p.theta0 != nullptr) {
           th0 = p.theta0 + static_cast<long long>(c.db) * p.theta_ld + q_glob;
           theta = __ldcg(th0);
@@ -418,6 +432,10 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
           rk_t = p.rk_target[q_glob];
           rk_e = p.rk_exclude != nullptr ? p.rk_exclude[q_glob] : -1;
         }
+      }
+      [[maybe_unused]] float rg_thr = 0.f;
+      if constexpr (kRange) {
+        if (active) rg_thr = p.rg_thr[q_glob];
       }
       // Exclusion: this query's excluded rows of this database, in registers (statically indexed:
       // every loop over them is unrolled). An excluded row is not a row of this query's problem --
@@ -506,6 +524,35 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
                 if ((xm >> j) & 1u) v[j] = 0xff800000u;
             }
           }
+          if constexpr (kRange) {
+            // "not below" rather than ">=": a threshold of -inf (a query with an unbounded error)
+            // takes every row, -inf and NaN scores included; rows past n_rows are padding
+            uint32_t m = 0;
+#pragma unroll
+            for (int j = 0; j < CHUNK; ++j)
+              m |= (active && !(__uint_as_float(v[j]) < rg_thr) && static_cast<int>(idx0) + j < n_rows) ? (1u << j) : 0u;
+            if (__any_sync(0xffffffffu, m != 0u)) {
+              // warp-wide exclusive prefix of the hit counts, one atomic for the warp's whole chunk
+              const int nh = __popc(m);
+              int incl = nh;
+#pragma unroll
+              for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += t;
+              }
+              unsigned long long base = 0;
+              if (lane == 31) base = atomicAdd(p.rg_count, static_cast<unsigned long long>(incl));
+              base = __shfl_sync(0xffffffffu, base, 31);
+              unsigned long long pos = base + static_cast<unsigned long long>(incl - nh);
+              while (m != 0u) {
+                const int j = __ffs(m) - 1;
+                m &= m - 1u;
+                if (pos < p.rg_cap) p.rg_out[pos] = make_uint2(static_cast<uint32_t>(q_glob), idx0 + j);
+                ++pos;
+              }
+            }
+            continue;
+          }
           if constexpr (kRank) {
             // count the certain winners; rows inside the band are rare and take a plain branch
 #pragma unroll
@@ -567,6 +614,7 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
       // LKEEP-th best, which becomes theta). They leave as one 128-byte line per (slice, query):
       // [(db, s, qt)][query][LKEEP] {score bits, row id}, padded with {-inf, ~0}; the re-rank
       // kernel reads a slice with a single coalesced half-warp load.
+      if constexpr (kRange) continue;  // the candidates are out already
       if constexpr (!kRank) {
         if (__any_sync(0xffffffffu, cnt >= LKEEP)) {
           const CandState st = compact_candidates<CAP>(slot0, cnt, theta);
@@ -611,6 +659,21 @@ k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ C
     tc_fence_after();
     if constexpr (kPair) tmem_dealloc_2sm(tmem_base, TMEM_COLS); else tmem_dealloc(tmem_base, TMEM_COLS);
   }
+}
+
+template <bool kPair, bool kRank = false, bool kExclude = false>
+__global__ void __launch_bounds__(ScoreCfg<kPair>::kThreads, 1)
+k_score_topk(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_x0,
+             const __grid_constant__ CUtensorMap tm_x1, const ScoreParams p) {
+  score_topk_body<kPair, kRank, kExclude, false>(tm_q, tm_x0, tm_x1, p);
+}
+
+// Range search: the same mainloop with the range epilogue (database 0 only).
+template <bool kPair>
+__global__ void __launch_bounds__(ScoreCfg<kPair>::kThreads, 1)
+k_score_range(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_x0,
+              const __grid_constant__ CUtensorMap tm_x1, const ScoreParams p) {
+  score_topk_body<kPair, false, false, true>(tm_q, tm_x0, tm_x1, p);
 }
 
 }  // namespace keds

@@ -64,6 +64,37 @@ def build_knowledge_base(image_rows: torch.Tensor, text_rows: torch.Tensor, name
     return kb
 
 
+def drop_near_duplicates(image_rows: torch.Tensor, text_rows: torch.Tensor, names: Sequence[str], radius: float,
+                         device: int = 0, batch: int = 65536):
+    """Leave out the later copies of near-duplicate images (CC3M holds one photo under several names,
+    and a copy of a query's own pair would come back as its first neighbour). Row j is dropped when
+    some row i < j has a normalised-image inner product > radius with it: a range self-join of the
+    base on the GPU, exact in fp32, in query batches of `batch` rows. The rule depends neither on the
+    batch size nor on the order of the batches. Returns (image_rows, text_rows, names, dropped_rows)
+    with the kept rows in their order and dropped_rows an int64 tensor of the dropped row numbers."""
+    from .index import METRIC_INNER_PRODUCT, GpuIndexFlat
+
+    n = int(image_rows.shape[0])
+    if int(text_rows.shape[0]) != n or len(names) != n:
+        raise ValueError(f"drop_near_duplicates: {n} image rows, {int(text_rows.shape[0])} text rows, {len(names)} names")
+    if int(batch) <= 0:
+        raise ValueError("drop_near_duplicates: batch must be positive")
+    dev = torch.device("cuda", device)
+    index = GpuIndexFlat(int(image_rows.shape[1]), METRIC_INNER_PRODUCT, device)
+    index.add(image_rows.to(dev, torch.float32).contiguous(), normalize=True)
+    drop = torch.zeros(n, dtype=torch.bool, device=dev)
+    for b0 in range(0, n, int(batch)):
+        b1 = min(n, b0 + int(batch))
+        q = torch.from_numpy(index.get_rows(b0, b1 - b0)).to(dev)
+        lims, _, I = index.range_search(q, radius)
+        row = torch.repeat_interleave(torch.arange(b0, b1, device=dev), lims[1:] - lims[:-1])
+        drop[row[I < row]] = True
+    del index
+    keep = (~drop).cpu()
+    kept_names = [nm for nm, k in zip(names, keep.tolist()) if k]
+    return image_rows[keep], text_rows[keep], kept_names, drop.nonzero().flatten().cpu()
+
+
 def save_artefacts(kb: KnowledgeBase, out_dir: str) -> Tuple[str, str, str]:
     """Write cc_image_databases.pt / cc_text_databases.pt / database_names.txt (README.md:17)."""
     os.makedirs(out_dir, exist_ok=True)

@@ -123,6 +123,10 @@ class GpuMultipleClonerOptions(GpuClonerOptions):
         self.shard = False
 
 
+_NO_CPU_SEARCH = ("keds_b200 has no CPU search path: move the index to a GPU with "
+                  "index_cpu_to_gpu / index_cpu_to_all_gpus first")
+
+
 class IndexFlat:
     """Host-side flat index: collects rows until it is cloned to a GPU (no CPU search)."""
 
@@ -145,10 +149,10 @@ class IndexFlat:
         self._blocks = []
 
     def search(self, x, k):
-        raise RuntimeError(
-            "keds_b200 has no CPU search path: move the index to a GPU with "
-            "index_cpu_to_gpu / index_cpu_to_all_gpus first"
-        )
+        raise RuntimeError(_NO_CPU_SEARCH)
+
+    def range_search(self, x, radius):
+        raise RuntimeError(_NO_CPU_SEARCH)
 
 
 class IndexFlatIP(IndexFlat):
@@ -275,13 +279,42 @@ class GpuIndexFlat:
         _capi.check(call(a.ctypes.data, a.shape[0], D.ctypes.data, I.ctypes.data))
         return D, I
 
-    def _check_q_tensor(self, x):
+    def range_search(self, x, radius: float, flags: int = 0):
+        """Faiss' index.range_search(x, radius) -> (lims, D, I): every row with score > radius (IP)
+        or squared distance < radius (L2), radius rounded to float32, exact in fp32; query i owns
+        [lims[i], lims[i+1]) of D and I, best first, ties by lower label. numpy in -> numpy out.
+        CUDA tensor in -> CUDA tensors out; the call synchronises the stream once the search has run,
+        to size D and I."""
+        radius = float(radius)
+        if radius != radius:
+            raise ValueError("radius must not be NaN")
+        stream = _stream_ptr(self.device)
+        if _is_tensor(x) and x.is_cuda:
+            q = self._check_q_tensor(x, "range_search")
+            lims = torch.empty(q.shape[0] + 1, dtype=torch.int64, device=q.device)
+            _capi.check(self._lib.keds_index_range_search(self._h, q.data_ptr(), q.shape[0], radius, lims.data_ptr(),
+                                                          flags, stream))
+            n = int(lims[-1].item())
+            D = torch.empty(n, dtype=torch.float32, device=q.device)
+            I = torch.empty(n, dtype=torch.int64, device=q.device)
+            _capi.check(self._lib.keds_index_range_results(self._h, D.data_ptr(), I.data_ptr(), stream))
+            return lims, D, I
+        a = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, self.d, "range_search")
+        lims = np.empty(a.shape[0] + 1, dtype=np.int64)
+        _capi.check(self._lib.keds_index_range_search(self._h, a.ctypes.data, a.shape[0], radius, lims.ctypes.data,
+                                                      flags, stream))
+        D = np.empty(int(lims[-1]), dtype=np.float32)
+        I = np.empty(int(lims[-1]), dtype=np.int64)
+        _capi.check(self._lib.keds_index_range_results(self._h, D.ctypes.data, I.ctypes.data, stream))
+        return lims, D, I
+
+    def _check_q_tensor(self, x, what: str = "search"):
         if x.dim() != 2 or x.shape[1] != self.d:
-            raise AssertionError(f"search: shape {tuple(x.shape)} does not match d={self.d}")
+            raise AssertionError(f"{what}: shape {tuple(x.shape)} does not match d={self.d}")
         if x.dtype != torch.float32:
-            raise TypeError(f"search: expected float32, got {x.dtype}")
+            raise TypeError(f"{what}: expected float32, got {x.dtype}")
         if x.device.index != self.device:
-            raise ValueError(f"search: query on cuda:{x.device.index}, index on cuda:{self.device}")
+            raise ValueError(f"{what}: query on cuda:{x.device.index}, index on cuda:{self.device}")
         return x.contiguous()
 
     def sync(self) -> None:
@@ -411,6 +444,21 @@ class IndexReplicas:
         res = _run_parallel([lambda s=s, lo=lo, hi=hi: s.search(a[lo:hi], k) for s, lo, hi in parts])
         return np.concatenate([r[0] for r in res]), np.concatenate([r[1] for r in res])
 
+    def range_search(self, x, radius: float):
+        """The queries split across the replicas as in `search`; each part's lims are shifted by the
+        results of the parts before it, so the result equals one index's (numpy out)."""
+        a = _as_f32_matrix(x.cpu().numpy() if _is_tensor(x) else x, self.d, "range_search")
+        n = a.shape[0]
+        bounds = np.linspace(0, n, len(self.subs) + 1).astype(np.int64)
+        parts = [(s, int(lo), int(hi)) for s, lo, hi in zip(self.subs, bounds[:-1], bounds[1:]) if hi > lo]
+        res = _run_parallel([lambda s=s, lo=lo, hi=hi: s.range_search(a[lo:hi], radius) for s, lo, hi in parts])
+        lims, shift = [np.zeros(1, np.int64)], 0
+        for r in res:
+            lims.append(np.asarray(r[0][1:], dtype=np.int64) + shift)
+            shift += int(r[0][-1])
+        return (np.concatenate(lims), np.concatenate([np.zeros(0, np.float32)] + [r[1] for r in res]),
+                np.concatenate([np.zeros(0, np.int64)] + [r[2] for r in res]))
+
 
 class IndexShards:
     """Row shards across the GPUs of one process (GpuMultipleClonerOptions.shard=True): every GPU
@@ -445,6 +493,10 @@ class IndexShards:
         for s in self.subs:
             s.reset()
         self._ntotal = 0
+
+    def range_search(self, x, radius: float):
+        raise NotImplementedError("IndexShards.range_search is not implemented: use one GpuIndexFlat or "
+                                  "IndexReplicas (index_cpu_to_all_gpus without shard=True)")
 
     def search(self, x, k: int):
         if torch is None:

@@ -172,6 +172,10 @@ class ShardedIndex:
         lo, hi = shard_bounds(int(x.shape[0]), self.world, self.rank)
         self.add_local(x[lo:hi], lo, int(x.shape[0]))
 
+    def range_search(self, q, radius: float):
+        raise NotImplementedError("ShardedIndex.range_search is not implemented: range-search an unsharded "
+                                  "GpuIndexFlat, or each rank's `local` index (its labels are global)")
+
     def search(self, q: torch.Tensor, k: int, out=None, exclude=None):
         """q: [nq, d] float32 on this rank's device, identical on all ranks. Returns (D, I);
         `out=(D, I)` may name preallocated contiguous device tensors to fill (fused exchange).
