@@ -387,7 +387,8 @@ int keds_consumer_check(keds_consumer_t* c, void* cuda_stream, int64_t* launches
  *                   text neighbours), applied between Linear and ReLU as in IM2TEXT
  *                   (src/model/model.py:110-116); they must stay alive until the backward.
  *                   Refuses (before queuing anything) a k whose attention backward, heads x
- *                   (2 dim_head + 2k) floats of shared memory, would not fit one block.
+ *                   (2 dim_head + 2k) floats of shared memory, would not fit one block. Every
+ *                   other batch it accepts (B (1 + 2k) <= 2^30 rows) also runs its backward.
  *   backward        dtokens [B][3][d_tok] -> grads (param_count floats, same layout, overwritten).
  *                   One backward per forward_train. tf32 tensor-core products, fp32 accumulation. */
 int64_t keds_consumer_param_count(const keds_consumer_t* c);
@@ -472,6 +473,21 @@ int keds_consumer_debug_linear(keds_consumer_t* c, int variant, const float* A0,
                                int64_t M, int K, const float* W0, const float* W1, const float* b0,
                                const float* b1, int N, int relu, float* C0, float* C1, int64_t ldc, int nz,
                                void* cuda_stream);
+/* Test hook for the single-query cross-attention alone: one launch over both stacks z = 0, 1 (as the
+ * forward and backward launch it), heads and dim_head of the handle, scale 1.0f / sqrtf(dim_head).
+ * Q[z], out[z] (and dO[z]) [B][heads * dim_head]; KV[z] [B * k][ld_kv] with the keys of head h at
+ * columns k_off + h * dim_head and its values at v_off + h * dim_head.
+ *   backward = 0: out[z] = O = softmax(scale q K^T) V per head. variant 0 = the production choice,
+ *     1 forces k_cross_attend<0>, 2 forces k_cross_attend<64> (dim_head 64, ld_kv, k_off and v_off
+ *     multiples of 4, KV 16-byte aligned; refused otherwise).
+ *   backward = 1 (variant 0 only): out[z] = dQ, and dK / dV of every neighbour row written to dKV[z]
+ *     at the same columns as K / V in KV[z] (ld_kv); nothing else of dKV[z] is touched.
+ * Refused before any launch: NULL or non-device buffers, k outside [1, 1024], key / value columns
+ * beyond ld_kv, shared memory beyond what one block can have. Asynchronous on cuda_stream. */
+int keds_consumer_debug_attend(keds_consumer_t* c, int variant, int backward, int64_t B, int k, const float* Q0,
+                               const float* Q1, const float* KV0, const float* KV1, int64_t ld_kv, int k_off,
+                               int v_off, const float* dO0, const float* dO1, float* out0, float* out1,
+                               float* dKV0, float* dKV1, void* cuda_stream);
 /* Programmatic dependent launch between the kernels of a search (default on; env KEDS_NO_PDL=1
  * turns the default off). Tuning/diagnostic switch; results do not depend on it. */
 int keds_index_set_pdl(keds_index_t* idx, int enable);

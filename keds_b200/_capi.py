@@ -176,6 +176,11 @@ SIGNATURES = {
         [_vp, C.c_int, _vp, _vp, C.c_int64, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp, _vp,
          C.c_int64, C.c_int, _vp],
     ),
+    "keds_consumer_debug_attend": (
+        C.c_int,
+        [_vp, C.c_int, C.c_int, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_int64, C.c_int, C.c_int, _vp, _vp, _vp,
+         _vp, _vp, _vp, _vp],
+    ),
     "keds_index_set_eps_scale": (C.c_int, [_vp, C.c_float]),
     "keds_index_set_pdl": (C.c_int, [_vp, C.c_int]),
     "keds_last_error": (C.c_char_p, []),

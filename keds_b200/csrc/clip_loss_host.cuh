@@ -150,7 +150,7 @@ int keds_clip_loss_forward_backward(keds_clip_loss_t* h, const float* I_all, con
     float* Itb = Ttb + static_cast<size_t>(d) * N3;
     float* Gra = h->Ga.as<float>();         // [B][3N], [hi|lo|hi]
     float* Gca = Gra + B * N3;
-    const dim3 tg(static_cast<unsigned>((d + 31) / 32), static_cast<unsigned>((N + 31) / 32));
+    const dim3 tg = transpose_grid(N, d);
     k_transpose_f32<<<tg, dim3(32, 8), 0, st>>>(T_all, d, static_cast<int>(N), d, Tt, N);
     k_transpose_f32<<<tg, dim3(32, 8), 0, st>>>(I_all, d, static_cast<int>(N), d, It, N);
     const unsigned s1 = static_cast<unsigned>((static_cast<long long>(d) * N + 255) / 256);

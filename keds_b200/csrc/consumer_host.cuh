@@ -137,6 +137,9 @@ int linear_variant(int64_t M, int N, int nz, int num_sms) {
   const long long mt = (M + LIN_M - 1) / LIN_M;
   const long long c128 = mt * ((N + 127) / 128) * nz, c256 = mt * ((N + 255) / 256) * nz;
   const long long sms = std::max(1, num_sms);
+  // the one-tile and split-K kernels put the row tiles on grid.y (at most 65 535); the persistent
+  // kernel walks a flat tile list, so it takes any M the consumer accepts (B (1 + 2k) <= 2^30)
+  if (mt > 65535) return LIN_PERSISTENT;
   const bool wide = ((c256 + sms - 1) / sms) * 48 < ((c128 + sms - 1) / sms) * 32;
   // a handful of tiles only: 32-column tiles with the K range split over a cluster of SK_SPLIT CTAs
   if (c128 * 6 <= sms && num_sms >= SK_MAX_SPLIT) {
@@ -207,6 +210,25 @@ int64_t round4(int64_t x) { return (x + 3) & ~int64_t(3); }
 // accepts only what its backward can also launch
 size_t attend_smem(const keds_consumer* c, int k) { return static_cast<size_t>(c->heads) * (c->dim_head + k) * 4; }
 size_t attend_bwd_smem(const keds_consumer* c, int k) { return 2 * attend_smem(c, k); }
+
+// Which attention forward runs: k_cross_attend<64> (every key row read with 16-byte loads) for the
+// reference's dim_head = 64 when every key / value row is 16-byte aligned, k_cross_attend<0> otherwise.
+bool attend_dh64(int dim_head, int64_t ld_kv, int k_off, int v_off, const float* KV0, const float* KV1) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(KV0) | reinterpret_cast<uintptr_t>(KV1);
+  return dim_head == 64 && (ld_kv & 3) == 0 && (k_off & 3) == 0 && (v_off & 3) == 0 && (a & 15) == 0;
+}
+
+// opt the attention kernels into the device's whole shared memory per block, once per handle
+int attend_init(keds_consumer* c) {
+  if (c->attend_max != 0) return 0;
+  int optin = 0;
+  CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+  CK(cudaFuncSetAttribute(k_cross_attend<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+  CK(cudaFuncSetAttribute(k_cross_attend<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+  CK(cudaFuncSetAttribute(k_cross_attend_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
+  c->attend_max = optin;
+  return 0;
+}
 
 // C[z] = act(A[z] W[z]^T + b[z]) for z < nz; A[z]: [M][K] with lda floats between rows
 int consumer_linear(keds_consumer* c, const float* A0, const float* A1, int64_t lda, int64_t M,
@@ -347,14 +369,7 @@ int keds_consumer_finalize(keds_consumer_t* c) {
       if (!c->wq[z][l].set || !c->wk[z][l].set || !c->wv[z][l].set || !c->wo[z][l].set)
         return fail(KEDS_ERR_ARG, "consumer_finalize: attention stack %d layer %d incomplete", z, l);
   CKS(linear_init(c));
-  if (c->attend_max == 0) {
-    int optin = 0;
-    CK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
-    CK(cudaFuncSetAttribute(k_cross_attend<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
-    CK(cudaFuncSetAttribute(k_cross_attend<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
-    CK(cudaFuncSetAttribute(k_cross_attend_bwd, cudaFuncAttributeMaxDynamicSharedMemorySize, optin));
-    c->attend_max = optin;
-  }
+  CKS(attend_init(c));
   const size_t wl = static_cast<size_t>(c->inner) * c->d_tok;  // one to_k or to_v matrix
   for (int z = 0; z < 2; ++z) {
     LinearW& kv = c->wkv[z];
@@ -553,8 +568,7 @@ int consumer_forward_impl(keds_consumer_t* c, const float* q, const ConsumerRowS
     ap.k_off = (2 * l) * inner;
     ap.v_off = (2 * l + 1) * inner;
     ap.scale = 1.0f / sqrtf(static_cast<float>(c->dim_head));
-    // fast path: the reference's dim_head = 64 with 16-byte aligned key / value rows
-    const bool dh64 = c->dim_head == 64 && (kvw & 3) == 0;
+    const bool dh64 = attend_dh64(c->dim_head, kvw, ap.k_off, ap.v_off, kv0, kv1);
     CKS(launch_k(true, dh64 ? k_cross_attend<64> : k_cross_attend<0>, dim3(static_cast<unsigned>(B), 2),
                  dim3(32 * c->heads), attend_smem(c, k), st, ap));
     c->launches++;
@@ -680,6 +694,79 @@ int keds_consumer_debug_linear(keds_consumer_t* c, int variant, const float* A0,
   }
   return linear_launch(c, variant, ta[0], ta[1], tw[0], tw[1], M, N, K, b0, b1, relu, C0, C1, ldc, nz,
                        static_cast<cudaStream_t>(stream));
+}
+
+int keds_consumer_debug_attend(keds_consumer_t* c, int variant, int backward, int64_t B, int k, const float* Q0,
+                               const float* Q1, const float* KV0, const float* KV1, int64_t ld_kv, int k_off,
+                               int v_off, const float* dO0, const float* dO1, float* out0, float* out1, float* dKV0,
+                               float* dKV1, void* stream) {
+  if (!c || variant < 0 || variant > 2 || (backward && variant != 0) || B < 1 || B > INT32_MAX || k < 1 || k > 1024)
+    return fail(KEDS_ERR_ARG, "consumer_debug_attend: bad handle, variant, B or k");
+  const int inner = c->inner;
+  if (k_off < 0 || v_off < 0 || ld_kv < static_cast<int64_t>(std::max(k_off, v_off)) + inner)
+    return fail(KEDS_ERR_ARG, "consumer_debug_attend: key / value columns outside ld_kv");
+  const float* need[] = {Q0, Q1, KV0, KV1, out0, out1, backward ? dO0 : Q0, backward ? dO1 : Q0,
+                         backward ? dKV0 : Q0, backward ? dKV1 : Q0};
+  for (const float* p : need)
+    if (!p) return fail(KEDS_ERR_ARG, "consumer_debug_attend: NULL buffer");
+  for (const float* p : need)
+    if (!locate(p)) return fail(KEDS_ERR_ARG, "consumer_debug_attend: all buffers must be device memory");
+  if (variant == 2 && !attend_dh64(c->dim_head, ld_kv, k_off, v_off, KV0, KV1))
+    return fail(KEDS_ERR_ARG, "consumer_debug_attend: k_cross_attend<64> needs dim_head 64, ld_kv, k_off, v_off "
+                              "multiples of 4 and 16-byte aligned KV");
+  DeviceGuard g(c->device);
+  if (!g.ok) return fail(KEDS_ERR_CUDA, "cudaSetDevice(%d) failed", c->device);
+  CKS(attend_init(c));
+  const size_t smem = backward ? attend_bwd_smem(c, k) : attend_smem(c, k);
+  if (smem > static_cast<size_t>(c->attend_max))
+    return fail(KEDS_ERR_ARG, "consumer_debug_attend: heads * (dim_head + k) too large for the attention kernel");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const float scale = 1.0f / sqrtf(static_cast<float>(c->dim_head));  // as the forward and backward compute it
+  const dim3 grid(static_cast<unsigned>(B), 2), block(32 * c->heads);
+  if (backward) {
+    AttendBwdParams ap;
+    memset(&ap, 0, sizeof ap);
+    ap.B = static_cast<int>(B);
+    ap.k = k;
+    ap.heads = c->heads;
+    ap.dim_head = c->dim_head;
+    ap.Q[0] = Q0;
+    ap.Q[1] = Q1;
+    ap.KV[0] = KV0;
+    ap.KV[1] = KV1;
+    ap.dO[0] = dO0;
+    ap.dO[1] = dO1;
+    ap.dQ[0] = out0;
+    ap.dQ[1] = out1;
+    ap.dKV[0] = dKV0;
+    ap.dKV[1] = dKV1;
+    ap.ld_kv = ld_kv;
+    ap.k_off = k_off;
+    ap.v_off = v_off;
+    ap.scale = scale;
+    CKS(launch_k(true, k_cross_attend_bwd, grid, block, smem, st, ap));
+  } else {
+    AttendParams ap;
+    memset(&ap, 0, sizeof ap);
+    ap.B = static_cast<int>(B);
+    ap.k = k;
+    ap.heads = c->heads;
+    ap.dim_head = c->dim_head;
+    ap.Q[0] = Q0;
+    ap.Q[1] = Q1;
+    ap.KV[0] = KV0;
+    ap.KV[1] = KV1;
+    ap.O[0] = out0;
+    ap.O[1] = out1;
+    ap.ld_kv = ld_kv;
+    ap.k_off = k_off;
+    ap.v_off = v_off;
+    ap.scale = scale;
+    const bool dh64 = variant == 0 ? attend_dh64(c->dim_head, ld_kv, k_off, v_off, KV0, KV1) : variant == 2;
+    CKS(launch_k(true, dh64 ? k_cross_attend<64> : k_cross_attend<0>, grid, block, smem, st, ap));
+  }
+  c->launches++;
+  return 0;
 }
 
 }  // extern "C"

@@ -67,8 +67,7 @@ int train_weight(keds_consumer* c, const float* W, int out, int in, int64_t ld, 
 // out[c][r] = in[r][c]
 int train_transpose(keds_consumer* c, const float* in, int64_t ld_in, int64_t rows, int cols, float* out, int64_t ld_out,
                     cudaStream_t st) {
-  const dim3 grid(static_cast<unsigned>((cols + 31) / 32), static_cast<unsigned>((rows + 31) / 32));
-  CKS(launch_k(true, k_transpose_f32, grid, dim3(32, 8), 0, st, in, static_cast<long long>(ld_in),
+  CKS(launch_k(true, k_transpose_f32, transpose_grid(rows, cols), dim3(32, 8), 0, st, in, static_cast<long long>(ld_in),
                static_cast<int>(rows), cols, out, static_cast<long long>(ld_out)));
   c->launches++;
   return 0;

@@ -91,21 +91,30 @@ __global__ void k_clip_grad_rows(const float* __restrict__ L, long long ld, int 
   }
 }
 
-// out[c][r] = in[r][c]  (in: [rows][cols] with ld_in, out: [cols][ld_out]); 32 x 32 tiles
+// out[c][r] = in[r][c]  (in: [rows][cols] with ld_in, out: [cols][ld_out]); 32 x 32 tiles. A block
+// walks the row tiles blockIdx.y, blockIdx.y + gridDim.y, ...: grid.y stops at 65 535, the rows of a
+// consumer backward (B (1 + 2k) up to 2^30) do not. Launch with transpose_grid.
 __global__ void k_transpose_f32(const float* __restrict__ in, long long ld_in, int rows, int cols,
                                 float* __restrict__ out, long long ld_out) {
   griddep_wait();
   __shared__ float tile[32][33];
-  const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int r = r0 + i, c = c0 + threadIdx.x;
-    tile[i][threadIdx.x] = (r < rows && c < cols) ? in[static_cast<long long>(r) * ld_in + c] : 0.f;
+  const int c0 = blockIdx.x * 32;
+  for (int r0 = blockIdx.y * 32; r0 < rows; r0 += gridDim.y * 32) {
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int r = r0 + i, c = c0 + threadIdx.x;
+      tile[i][threadIdx.x] = (r < rows && c < cols) ? in[static_cast<long long>(r) * ld_in + c] : 0.f;
+    }
+    __syncthreads();
+    for (int i = threadIdx.y; i < 32; i += blockDim.y) {
+      const int c = c0 + i, r = r0 + threadIdx.x;
+      if (c < cols && r < rows) out[static_cast<long long>(c) * ld_out + r] = tile[threadIdx.x][i];
+    }
+    __syncthreads();  // the next row tile reuses `tile`
   }
-  __syncthreads();
-  for (int i = threadIdx.y; i < 32; i += blockDim.y) {
-    const int c = c0 + i, r = r0 + threadIdx.x;
-    if (c < cols && r < rows) out[static_cast<long long>(c) * ld_out + r] = tile[threadIdx.x][i];
-  }
+}
+
+inline dim3 transpose_grid(long long rows, int cols) {
+  return dim3(static_cast<unsigned>((cols + 31) / 32), static_cast<unsigned>(std::min((rows + 31) / 32, 65535LL)));
 }
 
 // fp32-accurate products on the tf32 tensor cores: x = hi + lo with hi = tf32(x) (10-bit mantissa,

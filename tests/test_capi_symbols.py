@@ -61,6 +61,8 @@ def test_bad_arguments_are_rejected_without_a_gpu():
     assert lib.keds_index_ntotal(None) == -1
     assert lib.keds_index_search(None, None, 1, 1, None, None, None) == -1
     assert lib.keds_gather_pool(None, 0, None, None, None, 1, 1, 1, 1, None, None) == -1
+    assert lib.keds_consumer_debug_attend(None, 0, 0, 1, 16, None, None, None, None, 64, 0, 32, None, None, None, None,
+                                          None, None, None) == -1
 
 
 def test_library_is_sm100a_tcgen05_code():

@@ -240,3 +240,69 @@ def test_forward_train_accepts_only_what_the_backward_can_run():
     assert mod.flat.grad is None
     ref = NeighbourConsumer(*mod.state_dicts(), heads=32, device=0)
     assert torch.isfinite(ref(f, ix_i, ix_t, Ii, It)).all()
+
+
+# rows past which a 32-row-tile transpose (65 535 x 32) and a 128-row-tile GEMM (65 535 x 128) would
+# need more than grid.y's 65 535 blocks
+TRANSPOSE_ROWS, GEMM_ROWS = 65535 * 32, 65535 * 128
+
+
+def far_queries(B, k):
+    """the first and last query, and the first whose image neighbours, text neighbours or dK/dV rows
+    start beyond each of the two limits (rows: queries | image neighbours | text neighbours)"""
+    qs = {0, B - 1}
+    for T in (TRANSPOSE_ROWS, GEMM_ROWS):
+        for first_row, rows_per_query in ((B, k), (B + B * k, k), (0, k)):
+            b = max(0, -(-(T - first_row) // rows_per_query))
+            if b < B:
+                qs.add(b)
+    return sorted(qs)
+
+
+@pytest.mark.parametrize("B,k", [(1100, 1024), (4100, 1024)])
+def test_the_largest_batches_train(B, k):
+    """forward_train accepts any B (1 + 2k) <= 2^30 rows, and the backward has to run them: its
+    transposes once B (1 + 2k) > 65 535 x 32, the GEMMs' row tiles once it exceeds 65 535 x 128 (both
+    past grid.y's limit). At widths of 16 (one head of 4) B = 4100, k = 1024 is 8.4M rows in about
+    5 GB. dtokens are non-zero for a few queries only, the first, the last, and those whose rows lie
+    beyond the two limits; every other query then contributes exact zeros, and tokens and gradients
+    must match the tf32 oracle evaluated on those queries alone. The eval forward runs the same shape."""
+    M = B * (1 + 2 * k)
+    sds = corc.random_state_dicts(16, 16, 16, 1, 1, 1, 4, seed=B)
+    rng = np.random.default_rng(B)
+    n = 2000
+    base_img = rng.standard_normal((n, 16)).astype(np.float32)
+    base_txt = rng.standard_normal((n, 16)).astype(np.float32)
+    feat = rng.standard_normal((B, 16)).astype(np.float32)
+    I_img = rng.integers(0, n, (B, k)).astype(np.int64)
+    I_txt = rng.integers(0, n, (B, k)).astype(np.int64)
+    sel = far_queries(B, k)
+    dtok = np.zeros((B, 3, 16), np.float32)
+    dtok[sel] = rng.standard_normal((len(sel), 3, 16)).astype(np.float32)
+    mod, ix_i, ix_t, f, Ii, It = run(sds, 1, feat, base_img, base_txt, I_img, I_txt, dtok, dropout=0.0)
+    tokens = mod(f, ix_i, ix_t, Ii, It)
+    tokens.backward(torch.from_numpy(dtok).cuda())
+    assert mod.check() > 0
+    # the oracle on the selected queries, with the native forward's ReLU gates of their rows
+    rows = np.concatenate([np.array(sel)] + [B + np.arange(b * k, (b + 1) * k) for b in sel] +
+                          [B + B * k + np.arange(b * k, (b + 1) * k) for b in sel])
+    gate = (mod.debug_hidden(0, M)[torch.from_numpy(rows).cuda()] > 0).double().cpu().numpy()
+    nb_i, nb_t = base_img[I_img[sel]], base_txt[I_txt[sel]]
+    want_tok, want = cto.tokens_and_grads(sds[0], sds[1], sds[2], 1, feat[sel], nb_i, nb_t, dtok[sel], None, [gate],
+                                          tf32=True)
+    got_tok = tokens.detach()[torch.tensor(sel, device="cuda")].cpu().numpy()
+    errs = {"tokens": rel(got_tok, want_tok)}
+    gi, gf, gc = mod.state_dicts(grads=True)
+    scale = 1e-3 * max(float(np.abs(v).max()) for v in want.values())
+    for prefix, gsd in (("img2text", gi), ("retrieval_fuse", gf), ("text_condition", gc)):
+        for name, t in gsd.items():
+            errs[f"{prefix}/{name}"] = rel(t.cpu().numpy(), want[f"{prefix}/{name}"], scale)
+    print(f"B={B} k={k} M={M} queries {sel}: worst", sorted(errs.items(), key=lambda kv: -kv[1])[:3])
+    assert errs["tokens"] < TF32_TOK_TOL, errs
+    assert max(errs.values()) < TF32_GRAD_TOL, errs
+    del tokens
+    mod.flat.grad = None
+    ref = NeighbourConsumer(*mod.state_dicts(), heads=1, device=0)
+    got_eval = ref(f, ix_i, ix_t, Ii, It)
+    assert ref.check() > 0
+    assert rel(got_eval[torch.tensor(sel, device="cuda")].cpu().numpy(), want_tok) < TF32_TOK_TOL

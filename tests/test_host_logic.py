@@ -218,3 +218,17 @@ def test_linear_chooser_rejects_bad_arguments():
     for args in [(0, 4, 1, 148), (4, 0, 1, 148), (4, 4, 3, 148), (4, 4, 1, 0)]:
         assert lib.keds_debug_linear_plan(*args, C.byref(v)) == -1
     assert lib.keds_debug_linear_plan(4, 4, 1, 148, None) == -1
+
+
+@pytest.mark.parametrize("sms", [1, 4, 148])
+@pytest.mark.parametrize("nz", [1, 2])
+@pytest.mark.parametrize("N", [4, 16, 80, 768])
+def test_linear_chooser_takes_the_persistent_kernel_past_grid_y(N, nz, sms):
+    """The one-tile and split-K kernels put the 128-row tiles on grid.y, at most 65 535 of them; the
+    persistent kernel walks a flat tile list. Past that edge, up to the 2^30 rows the consumer accepts,
+    only the persistent kernel may be chosen; at the edge d_tok = 80 still takes 128-column tiles."""
+    edge = 65535 * 128
+    for M in (edge + 1, 4100 * 2049, 1 << 30):
+        assert _linear_plan(M, N, nz, sms) == PERSISTENT, M
+    if N == 80 and nz == 1 and sms == 148:
+        assert _linear_plan(edge, N, nz, sms) == TILE128
