@@ -94,18 +94,28 @@ uint64_t keds_index_generation(const keds_index_t* idx);
  * D, I = index.search(q, k) (src/trainer.py:213,221,271; src/eval_utils.py:169,177).
  * q: [nq][d] float32. D: [nq][k] float32 (inner products, or squared L2 distances). I: [nq][k]
  * int64 labels, best first; ties by lower label; rows past ntotal are padded with label -1 and
- * D = -FLT_MAX (IP) / +FLT_MAX (L2). Results equal an exact fp32 flat search. */
+ * D = -FLT_MAX (IP) / +FLT_MAX (L2). Results equal an exact fp32 flat search.
+ *
+ * Exclusion (every search call but keds_index_search): rows left out per query (training without
+ * self-retrieval: a query whose own pair is in the knowledge base must not retrieve it).
+ * exclude: NULL with n_exclude = 0 for none, or int64 [nq][n_exclude], 1 <= n_exclude <= 8, labels
+ * as I returns them (id_offset included); -1 = unused slot, a label the index does not hold excludes
+ * nothing. Device memory of the index's GPU (keds_retrieve2 also takes page-locked host memory). In
+ * two-database calls one array applies to both databases (aligned row for row: a pair's image row
+ * and caption row share a label). Each query's result equals an exact fp32 flat search over the rows
+ * it does not exclude: same order, same ties, -1 / -+FLT_MAX padding when fewer than k rows remain;
+ * an excluded row is never returned. Gather, pool and host mirrors follow the returned I. */
 int keds_index_search(keds_index_t* idx, const float* q, int64_t nq, int k, float* D, int64_t* I,
                       void* cuda_stream);
 int keds_index_search_ex(keds_index_t* idx, const float* q, int64_t nq, int k, float* D, int64_t* I,
-                         uint32_t flags, void* cuda_stream);
+                         const int64_t* exclude, int n_exclude, uint32_t flags, void* cuda_stream);
 /* Two indices, one query batch: the image-DB and text-DB searches of src/trainer.py:213 and :221
  * fused into one pass over the queries. Both indices share d, metric and device. */
 int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k,
-                       float* Da, int64_t* Ia, float* Db, int64_t* Ib, uint32_t flags,
-                       void* cuda_stream);
-/* The whole retrieval operator of src/trainer.py:198-230 in one call (device pointers only):
- * search both databases, then per stream s in {img, txt}
+                       float* Da, int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude,
+                       int n_exclude, uint32_t flags, void* cuda_stream);
+/* The whole retrieval operator of src/trainer.py:198-230 in one call: search both databases, then
+ * per stream s in {img, txt}
  *   feat_s[b][j][:] = rows_s[I_s[b][perm_s ? perm_s[j] : j]][:]      (nullable; [nq][k][d])
  *   pool_s[b][:]    = sum_j w_j rows_s[I_s[b][j]][:]                 (nullable; [nq][d])
  * pool_mode 0: no pool; 1: w = 1/k; 2: w = softmax_j(+-tau * D_s[b][j]) (minus under L2).
@@ -116,53 +126,24 @@ int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t
  * over output slots, slot j adding w_{perm[j]} * rows_s[I_s[b][perm[j]]], so a repeated entry counts
  * one neighbour twice and drops another; an entry outside [0, k) gives a zero row in feat and adds
  * nothing but w_0 * 0 to the pool. The Python wrappers refuse a host perm that is not a permutation.
- * The summation order of the pool depends on the route a query takes (DESIGN.md section 3). */
-int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                   const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                   float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
-                   float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags,
-                   void* cuda_stream);
-/* The same operator for a caller whose queries and results live on the HOST, as the reference's do
- * (q.cpu().numpy() in, numpy (D, I) out, src/trainer.py:207-221), without copies around the search:
+ * The summation order of the pool depends on the route a query takes (DESIGN.md section 3).
+ * D_*, I_*, feat_*, pool_*: device memory. For a caller whose queries and results live on the HOST,
+ * as the reference's do (q.cpu().numpy() in, numpy (D, I) out, src/trainer.py:207-221), the call
+ * also runs without copies around the search:
  *   q        may be page-locked host memory (cudaHostAlloc / cudaHostRegister / torch pin_memory):
- *            the first kernel of the chain reads it through the device mapping, once;
+ *            the first kernel of the chain reads it through the device mapping, once; so may
+ *            exclude, read through the mapping once per call, like q;
  *   Dh_x, Ih_x (nullable, in pairs) page-locked host blocks [nq][k]: the block that finishes a query's
  *            row stores it there as well as into D_x, I_x (posted writes that travel while the
  *            neighbour gather of that query runs).
- * Stream-ordered and asynchronous like keds_retrieve2: the host blocks are complete once the stream
- * has been synchronised (or the graph that captured the call has finished). */
-int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                          const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                          float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
-                          int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img,
-                          float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags,
-                          void* cuda_stream);
-/* ---- search with exclusion -------------------------------------------------------------------
- * The four calls above with rows left out per query (training without self-retrieval: a query
- * whose own pair is in the knowledge base must not retrieve it). exclude: int64 [nq][n_exclude],
- * 1 <= n_exclude <= 8, labels as I returns them (id_offset included); -1 = unused slot, a label the
- * index does not hold excludes nothing. Device memory of the index's GPU; the hostio variant also
- * takes page-locked host memory, read through the mapping once per call, like q. In two-database
- * calls one array applies to both databases (aligned row for row: a pair's image row and caption
- * row share a label). Each query's result equals an exact fp32 flat search over the rows it does
- * not exclude: same order, same ties, -1 / -+FLT_MAX padding when fewer than k rows remain; an
- * excluded row is never returned. Gather, pool and host mirrors follow the returned I. */
-int keds_index_search_exclude(keds_index_t* idx, const float* q, int64_t nq, int k, float* D, int64_t* I,
-                              const int64_t* exclude, int n_exclude, uint32_t flags, void* cuda_stream);
-int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k,
-                               float* Da, int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude,
-                               int n_exclude, uint32_t flags, void* cuda_stream);
-int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                           const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                           float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
-                           float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude,
-                           int n_exclude, uint32_t flags, void* cuda_stream);
-int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                                  const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                                  float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
-                                  int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img,
-                                  float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude,
-                                  int n_exclude, uint32_t flags, void* cuda_stream);
+ * Stream-ordered and asynchronous: the host blocks are complete once the stream has been
+ * synchronised (or the graph that captured the call has finished). */
+int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                   const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                   float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
+                   int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
+                   float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
+                   uint32_t flags, void* cuda_stream);
 /* ---- range search ------------------------------------------------------------------------------
  * lims, D, I = index.range_search(q, radius) (Faiss' RangeSearchResult layout): every row n with
  *   IP: s(n) > radius        L2: d(n) < radius (squared distance)
@@ -252,6 +233,9 @@ int keds_topk_merge_wait(const float* D_parts, const int64_t* I_parts, int64_t s
  *   exchange_capacity largest nq * k one search may carry.
  *   search_sharded    q [nq][d], D [nq][k], I [nq][k]: device memory; idx holds this rank's rows
  *                     with keds_index_set_id_offset(first global row). Asynchronous on cuda_stream.
+ *                     exclude (nullable, as keds_index_search_ex): [nq][n_exclude] global labels in
+ *                     device memory, the same on every rank; each shard leaves out the ones it holds,
+ *                     so the merged result equals keds_index_search_ex on an unsharded index.
  *   exchange_stats    synchronises; average / maximum time (us) block 0 of the merge waited for the
  *                     peers since the last call (rank skew), merges counted, and the error word
  *                     (non-zero: a peer never delivered). */
@@ -261,15 +245,9 @@ int keds_exchange_create(int n_ranks, int my_rank, int device, void* const* peer
 void keds_exchange_free(keds_exchange_t* ex);
 int64_t keds_exchange_capacity(const keds_exchange_t* ex);
 int keds_index_search_sharded(keds_index_t* idx, keds_exchange_t* ex, const float* q, int64_t nq, int k,
-                              float* D, int64_t* I, void* cuda_stream);
+                              float* D, int64_t* I, const int64_t* exclude, int n_exclude, void* cuda_stream);
 int keds_exchange_stats(keds_exchange_t* ex, void* cuda_stream, double* wait_us_avg, double* wait_us_max,
                         int64_t* steps, uint32_t* err_word);
-/* search_sharded with exclusion: exclude [nq][n_exclude] global labels (device memory, -1 = none,
- * 1 <= n_exclude <= 8), the same on every rank; each shard leaves out the ones it holds, so the
- * merged result equals keds_index_search_exclude on an unsharded index. */
-int keds_index_search_sharded_exclude(keds_index_t* idx, keds_exchange_t* ex, const float* q, int64_t nq, int k,
-                                      float* D, int64_t* I, const int64_t* exclude, int n_exclude,
-                                      void* cuda_stream);
 
 /* Row-sharded retrieval step: keds_retrieve2 over two row-sharded bases that share one exchange.
  *   index_rows_ipc      cudaIpcMemHandle_t (64 bytes) of the index's fp32 rows; all zero for an

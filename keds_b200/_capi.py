@@ -53,9 +53,7 @@ SIGNATURES = {
     "keds_exchange_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.POINTER(_vp), C.c_int64, C.POINTER(_vp)]),
     "keds_exchange_free": (None, [_vp]),
     "keds_exchange_capacity": (C.c_int64, [_vp]),
-    "keds_index_search_sharded": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp]),
-    "keds_index_search_sharded_exclude": (
-        C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int, _vp]),
+    "keds_index_search_sharded": (C.c_int, [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int, _vp]),
     "keds_index_rows_ipc": (C.c_int, [_vp, _vp]),
     "keds_exchange_attach_rows": (C.c_int, [_vp, C.c_int, C.POINTER(_vp), _i64p, _i64p]),
     "keds_retrieve2_sharded": (
@@ -68,32 +66,12 @@ SIGNATURES = {
         [_vp, _vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_int64), C.POINTER(C.c_uint32)],
     ),
     "keds_index_search": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp]),
-    "keds_index_search_ex": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_uint32, _vp]),
+    "keds_index_search_ex": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp]),
     "keds_index_search2": (
-        C.c_int,
-        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, C.c_uint32, _vp],
-    ),
-    "keds_retrieve2": (
-        C.c_int,
-        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
-         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint32, _vp],
-    ),
-    "keds_retrieve2_hostio": (
-        C.c_int,
-        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
-         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint32, _vp],
-    ),
-    "keds_index_search_exclude": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp]),
-    "keds_index_search2_exclude": (
         C.c_int,
         [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
     ),
-    "keds_retrieve2_exclude": (
-        C.c_int,
-        [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
-         _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],
-    ),
-    "keds_retrieve2_hostio_exclude": (
+    "keds_retrieve2": (
         C.c_int,
         [_vp, _vp, _vp, C.c_int64, C.c_int, _vp, _vp, C.c_int, C.c_float,
          _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_uint32, _vp],

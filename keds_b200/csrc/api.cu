@@ -518,9 +518,11 @@ struct Call {
   int64_t ld_dump = 0;
 
   int metric() const { return (flags & KEDS_SEARCH_FORCE_IP) ? METRIC_IP : owner->metric; }
+  // the entry points' (exclude, n_exclude): NULL with 0 = no exclusion
   int exclude(const int64_t* labels, int n) {
-    if (!labels || n < 1 || n > EXCLUDE_MAX)
-      return fail(KEDS_ERR_ARG, "exclude must be a non-null [nq][n_exclude] array, 1 <= n_exclude <= %d", EXCLUDE_MAX);
+    if (labels ? n < 1 || n > EXCLUDE_MAX : n != 0)
+      return fail(KEDS_ERR_ARG, "exclude must be NULL with n_exclude = 0, or an [nq][n_exclude] array with 1 <= n_exclude <= %d",
+                  EXCLUDE_MAX);
     ex = reinterpret_cast<const long long*>(labels);
     n_ex = n;
     return 0;
@@ -1238,7 +1240,7 @@ int search_impl(Call c, Io io, void* stream) {
 
   const PtrLoc lq = io == IO_DEVICE ? PtrLoc{a->device, nullptr} : locate(c.q);
   if (!lq && io == IO_MAPPED && !lq.mapped)
-    return fail(KEDS_ERR_ARG, "retrieve2_hostio: q is neither device memory nor page-locked host memory");
+    return fail(KEDS_ERR_ARG, "retrieve2: q is neither device memory nor page-locked host memory");
   bool out_dev = true;
   for (int i = 0; io == IO_HOST && i < n_db; ++i) {
     const bool dd = static_cast<bool>(locate(c.D[i])), di = static_cast<bool>(locate(c.I[i]));
@@ -1250,7 +1252,7 @@ int search_impl(Call c, Io io, void* stream) {
     const PtrLoc lex = locate(c.ex);
     if (lex.device != a->device) {
       if (io != IO_MAPPED || !lex.mapped)
-        return fail(KEDS_ERR_ARG, io == IO_MAPPED ? "retrieve2_hostio: exclude is neither device memory of the index's GPU "
+        return fail(KEDS_ERR_ARG, io == IO_MAPPED ? "retrieve2: exclude is neither device memory of the index's GPU "
                                                     "nor page-locked host memory"
                                                   : "search: exclude must be device memory of the index's GPU");
       c.ex = static_cast<const long long*>(lex.mapped);
@@ -1259,7 +1261,7 @@ int search_impl(Call c, Io io, void* stream) {
   // Host in, host out (the reference's numpy call): the call synchronises before it returns, so
   // page-locked staging buffers can be reused call after call (one real DMA each way instead of
   // the driver's chunked pageable copies). Letting the kernels work on those buffers through the
-  // mapping (as keds_retrieve2_hostio does for RetrievalStep) was measured here too and is no
+  // mapping (as keds_retrieve2 does with host mirrors for RetrievalStep) was measured here too and is no
   // faster for this path (two searches of 128 queries: 403-411 us with copies, 413-425 us mapped):
   // the call is dominated by its host side.
   // one database's I (8 B) and D (4 B) blocks in the staged result, labels first (8-byte aligned)
@@ -1355,7 +1357,7 @@ int search_impl(Call c, Io io, void* stream) {
 extern "C" {
 
 const char* keds_last_error(void) { return g_err.c_str(); }
-const char* keds_version(void) { return "keds-knn-b200 0.1 (sm_100a)"; }
+const char* keds_version(void) { return "keds-knn-b200 0.2 (sm_100a)"; }
 
 int keds_device_count(void) {
   int n = 0;
@@ -1599,31 +1601,19 @@ int keds_index_set_eps_scale(keds_index_t* ix, float scale) {
 
 int keds_index_search(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
                       void* stream) {
-  return keds_index_search_ex(ix, q, nq, k, D, I, 0u, stream);
+  return keds_index_search_ex(ix, q, nq, k, D, I, nullptr, 0, 0u, stream);
 }
 
 int keds_index_search_ex(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
-                         uint32_t flags, void* stream) {
-  Call c = call(1, ix, nullptr, q, nq, k, D, I, nullptr, nullptr, flags);
-  return search_impl(c, IO_HOST, stream);
-}
-
-int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
-                       int64_t* Ia, float* Db, int64_t* Ib, uint32_t flags, void* stream) {
-  Call c = call(2, a, b, q, nq, k, Da, Ia, Db, Ib, flags);
-  return search_impl(c, IO_HOST, stream);
-}
-
-int keds_index_search_exclude(keds_index_t* ix, const float* q, int64_t nq, int k, float* D, int64_t* I,
-                              const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
+                         const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
   Call c = call(1, ix, nullptr, q, nq, k, D, I, nullptr, nullptr, flags);
   CKS(c.exclude(exclude, n_exclude));
   return search_impl(c, IO_HOST, stream);
 }
 
-int keds_index_search2_exclude(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
-                               int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude, int n_exclude,
-                               uint32_t flags, void* stream) {
+int keds_index_search2(keds_index_t* a, keds_index_t* b, const float* q, int64_t nq, int k, float* Da,
+                       int64_t* Ia, float* Db, int64_t* Ib, const int64_t* exclude, int n_exclude, uint32_t flags,
+                       void* stream) {
   Call c = call(2, a, b, q, nq, k, Da, Ia, Db, Ib, flags);
   CKS(c.exclude(exclude, n_exclude));
   return search_impl(c, IO_HOST, stream);
@@ -1657,21 +1647,29 @@ int consume_params(const char* fn, const keds_index* img, int k, const int32_t* 
   return 0;
 }
 
-// The fused consumer on top of a two-database call (c: both handles, q, the device results and
-// the exclusion); hostio: q may be page-locked host memory and the results get host mirrors.
-int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                   float* feat_img, float* feat_txt, float* pool_img, float* pool_txt, float* Dh_img, int64_t* Ih_img,
-                   float* Dh_txt, int64_t* Ih_txt, void* stream) {
-  keds_index* img = c.dbs[0];
-  if (!img || !c.dbs[1] || !c.q || !c.D[0] || !c.I[0] || !c.D[1] || !c.I[1])
+}  // namespace
+
+extern "C" {
+
+// The fused consumer on top of the two-database search, always on the mapped route: device queries
+// and labels are used in place, page-locked host ones are read through the mapping.
+int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
+                   const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
+                   float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
+                   int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
+                   float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude, uint32_t flags,
+                   void* stream) {
+  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
+  CKS(c.exclude(exclude, n_exclude));
+  if (!img || !txt || !q || !D_img || !I_img || !D_txt || !I_txt)
     return fail(KEDS_ERR_ARG, "retrieve2: null handle, query or result pointer");
   ConsumeParams cp;
-  CKS(consume_params("retrieve2", img, c.k, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt,
+  CKS(consume_params("retrieve2", img, k, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt,
                      cp));
-  if ((!hostio && !locate(c.q)) || !locate(c.D[0]) || !locate(c.I[0]) || !locate(c.D[1]) || !locate(c.I[1]))
-    return fail(KEDS_ERR_ARG, "retrieve2: device pointers only");
+  if (!locate(D_img) || !locate(I_img) || !locate(D_txt) || !locate(I_txt))
+    return fail(KEDS_ERR_ARG, "retrieve2: D and I must be device memory");
   if ((Dh_img == nullptr) != (Ih_img == nullptr) || (Dh_txt == nullptr) != (Ih_txt == nullptr))
-    return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host mirror needs both its D and its I block");
+    return fail(KEDS_ERR_ARG, "retrieve2: a host mirror needs both its D and its I block");
   {
     DeviceGuard g(img->device);
     if (!g.ok) return fail(KEDS_ERR_NO_GPU, "cannot select CUDA device %d", img->device);
@@ -1680,7 +1678,7 @@ int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* 
     for (void*& m : mirror) {
       if (!m) continue;
       m = locate(m).mapped;
-      if (!m) return fail(KEDS_ERR_ARG, "retrieve2_hostio: a host result pointer is not page-locked (cudaHostAlloc / pin_memory)");
+      if (!m) return fail(KEDS_ERR_ARG, "retrieve2: a host result pointer is not page-locked (cudaHostAlloc / pin_memory)");
     }
     cp.host_D[0] = static_cast<float*>(mirror[0]);
     cp.host_I[0] = static_cast<long long*>(mirror[1]);
@@ -1689,53 +1687,7 @@ int retrieve2_impl(Call c, bool hostio, const int32_t* perm_img, const int32_t* 
   }
   if (Dh_img || Dh_txt) cp.enabled = 1;  // the host mirrors are the consumer's too
   if (cp.enabled) c.cons = cp;
-  return search_impl(c, hostio ? IO_MAPPED : IO_DEVICE, stream);
-}
-
-}  // namespace
-
-extern "C" {
-
-int keds_retrieve2(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                   const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                   float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
-                   float* feat_txt, float* pool_img, float* pool_txt, uint32_t flags, void* stream) {
-  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
-  return retrieve2_impl(c, false, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, nullptr,
-                        nullptr, nullptr, nullptr, stream);
-}
-
-int keds_retrieve2_hostio(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                          const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                          float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
-                          int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
-                          float* pool_img, float* pool_txt, uint32_t flags, void* stream) {
-  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
-  return retrieve2_impl(c, true, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, Dh_img,
-                        Ih_img, Dh_txt, Ih_txt, stream);
-}
-
-int keds_retrieve2_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                           const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                           float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* feat_img,
-                           float* feat_txt, float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
-                           uint32_t flags, void* stream) {
-  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
-  CKS(c.exclude(exclude, n_exclude));
-  return retrieve2_impl(c, false, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, nullptr,
-                        nullptr, nullptr, nullptr, stream);
-}
-
-int keds_retrieve2_hostio_exclude(keds_index_t* img, keds_index_t* txt, const float* q, int64_t nq, int k,
-                                  const int32_t* perm_img, const int32_t* perm_txt, int pool_mode, float tau,
-                                  float* D_img, int64_t* I_img, float* D_txt, int64_t* I_txt, float* Dh_img,
-                                  int64_t* Ih_img, float* Dh_txt, int64_t* Ih_txt, float* feat_img, float* feat_txt,
-                                  float* pool_img, float* pool_txt, const int64_t* exclude, int n_exclude,
-                                  uint32_t flags, void* stream) {
-  Call c = call(2, img, txt, q, nq, k, D_img, I_img, D_txt, I_txt, flags);
-  CKS(c.exclude(exclude, n_exclude));
-  return retrieve2_impl(c, true, perm_img, perm_txt, pool_mode, tau, feat_img, feat_txt, pool_img, pool_txt, Dh_img,
-                        Ih_img, Dh_txt, Ih_txt, stream);
+  return search_impl(c, IO_MAPPED, stream);
 }
 
 int keds_index_sync(keds_index_t* ix, void* stream) {
@@ -2188,18 +2140,13 @@ int keds_exchange_attach_rows(keds_exchange_t* ex, int db, const void* const* ha
 }
 
 int keds_index_search_sharded(keds_index_t* ix, keds_exchange_t* ex, const float* q, int64_t nq, int k, float* D,
-                              int64_t* I, void* stream) {
-  return keds_index_search_sharded_exclude(ix, ex, q, nq, k, D, I, nullptr, 0, stream);
-}
-
-int keds_index_search_sharded_exclude(keds_index_t* ix, keds_exchange_t* ex, const float* q, int64_t nq, int k,
-                                      float* D, int64_t* I, const int64_t* exclude, int n_exclude, void* stream) {
+                              int64_t* I, const int64_t* exclude, int n_exclude, void* stream) {
+  Call c = call(1, ix, nullptr, q, nq, k, nullptr, nullptr, nullptr, nullptr, 0u);
+  CKS(c.exclude(exclude, n_exclude));
   if (!ix || !ex || !q || !D || !I || nq <= 0 || k <= 0)
     return fail(KEDS_ERR_ARG, "search_sharded: null handle / pointer or bad nq / k");
   if (ex->device != ix->device) return fail(KEDS_ERR_ARG, "search_sharded: exchange and index live on different devices");
   if (!locate(q) || !locate(D) || !locate(I)) return fail(KEDS_ERR_ARG, "search_sharded: device pointers only");
-  Call c = call(1, ix, nullptr, q, nq, k, nullptr, nullptr, nullptr, nullptr, 0u);
-  if (exclude) CKS(c.exclude(exclude, n_exclude));
   return sharded_search(c, ex, &D, &I, stream);
 }
 
@@ -2208,6 +2155,8 @@ int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t
                            int64_t row_lo, int64_t row_hi, float* D_img, int64_t* I_img, float* D_txt,
                            int64_t* I_txt, float* feat_img, float* feat_txt, float* pool_img, float* pool_txt,
                            const int64_t* exclude, int n_exclude, uint32_t flags, void* stream) {
+  Call c = call(2, img, txt, q, nq, k, nullptr, nullptr, nullptr, nullptr, flags);
+  CKS(c.exclude(exclude, n_exclude));
   if (!img || !txt || !ex || !q || !D_img || !I_img || !D_txt || !I_txt || nq <= 0 || k <= 0)
     return fail(KEDS_ERR_ARG, "retrieve2_sharded: null handle / pointer or bad nq / k");
   ConsumeParams cp;
@@ -2223,8 +2172,6 @@ int keds_retrieve2_sharded(keds_index_t* img, keds_index_t* txt, keds_exchange_t
   for (const void* p : dev_ptrs)
     if (p && locate(p).device != img->device)
       return fail(KEDS_ERR_ARG, "retrieve2_sharded: device pointers of the indices' GPU only");
-  Call c = call(2, img, txt, q, nq, k, nullptr, nullptr, nullptr, nullptr, flags);
-  if (exclude) CKS(c.exclude(exclude, n_exclude));
   CKS(ex_check_rows(ex, c.dbs, 2));
   float* D[2] = {D_img, D_txt};
   int64_t* I[2] = {I_img, I_txt};

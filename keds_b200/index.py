@@ -77,8 +77,11 @@ def check_exclude(exclude, nq: int):
 
 
 def _exclude_arg(exclude, nq: int, device: int, pinned_ok: bool = False):
-    """check_exclude, then a contiguous int64 tensor the native call can read: on `device`, or a
-    pinned host tensor as it is when `pinned_ok` (the hostio path reads it through the mapping)."""
+    """None for None; else check_exclude, then a contiguous int64 tensor the native call can read:
+    on `device`, or a pinned host tensor as it is when `pinned_ok` (retrieve2's host I/O reads it
+    through the mapping). Keep it alive until the native call has been queued."""
+    if exclude is None:
+        return None
     ex = check_exclude(exclude, nq)
     if torch is None:
         raise RuntimeError("search with exclusion needs torch for the device copy of `exclude`")
@@ -91,6 +94,25 @@ def _exclude_arg(exclude, nq: int, device: int, pinned_ok: bool = False):
     if pinned_ok and ex.is_pinned() and ex.is_contiguous():
         return ex
     return ex.to(torch.device("cuda", device), non_blocking=False).contiguous()
+
+
+def _exclude_ptrs(ex) -> Tuple[int, int]:
+    """The native calls' (exclude, n_exclude) for a result of _exclude_arg: (0, 0) = no exclusion."""
+    return (0, 0) if ex is None else (ex.data_ptr(), int(ex.shape[1]))
+
+
+def _check_out(out, n: int):
+    """A caller's out=(D, I): contiguous CUDA float32 / int64 tensors of n elements each."""
+    D, I = out
+    assert D.is_cuda and I.is_cuda and D.is_contiguous() and I.is_contiguous()
+    assert D.dtype == torch.float32 and I.dtype == torch.int64
+    assert D.numel() == n and I.numel() == n
+    return D, I
+
+
+def _ptr(a) -> int:
+    """Address of the data of a tensor or a numpy array."""
+    return a.data_ptr() if _is_tensor(a) else a.ctypes.data
 
 
 def _stream_ptr(device: int) -> int:
@@ -253,30 +275,20 @@ class GpuIndexFlat:
         k = int(k)
         if k <= 0:
             raise ValueError("k must be positive")
-
-        def call(qp, nq, Dp, Ip):
-            if exclude is None:
-                return self._lib.keds_index_search_ex(self._h, qp, nq, k, Dp, Ip, flags, _stream_ptr(self.device))
-            ex = _exclude_arg(exclude, nq, self.device)
-            return self._lib.keds_index_search_exclude(self._h, qp, nq, k, Dp, Ip, ex.data_ptr(), ex.shape[1], flags,
-                                                       _stream_ptr(self.device))
-
         if _is_tensor(x) and x.is_cuda:
             q = self._check_q_tensor(x)
             if out is not None:
-                D, I = out
-                assert D.is_cuda and I.is_cuda and D.is_contiguous() and I.is_contiguous()
-                assert D.dtype == torch.float32 and I.dtype == torch.int64
-                assert D.numel() == q.shape[0] * k and I.numel() == q.shape[0] * k
+                D, I = _check_out(out, q.shape[0] * k)
             else:
                 D = torch.empty((q.shape[0], k), dtype=torch.float32, device=q.device)
                 I = torch.empty((q.shape[0], k), dtype=torch.int64, device=q.device)
-            _capi.check(call(q.data_ptr(), q.shape[0], D.data_ptr(), I.data_ptr()))
-            return D, I
-        a = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, self.d, "search")
-        D = np.empty((a.shape[0], k), dtype=np.float32)
-        I = np.empty((a.shape[0], k), dtype=np.int64)
-        _capi.check(call(a.ctypes.data, a.shape[0], D.ctypes.data, I.ctypes.data))
+        else:
+            q = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, self.d, "search")
+            D = np.empty((q.shape[0], k), dtype=np.float32)
+            I = np.empty((q.shape[0], k), dtype=np.int64)
+        ex = _exclude_arg(exclude, q.shape[0], self.device)
+        _capi.check(self._lib.keds_index_search_ex(self._h, _ptr(q), q.shape[0], k, _ptr(D), _ptr(I),
+                                                   *_exclude_ptrs(ex), flags, _stream_ptr(self.device)))
         return D, I
 
     def range_search(self, x, radius: float, flags: int = 0):
@@ -375,29 +387,17 @@ def search2(a: GpuIndexFlat, b: GpuIndexFlat, x, k: int, flags: int = 0, exclude
     exclude: as GpuIndexFlat.search; one array for both databases (aligned row for row)."""
     lib = _capi.load()
     k = int(k)
-
-    def call(qp, nq, Da, Ia, Db, Ib):
-        if exclude is None:
-            return lib.keds_index_search2(a._h, b._h, qp, nq, k, Da, Ia, Db, Ib, flags, _stream_ptr(a.device))
-        ex = _exclude_arg(exclude, nq, a.device)
-        return lib.keds_index_search2_exclude(a._h, b._h, qp, nq, k, Da, Ia, Db, Ib, ex.data_ptr(), ex.shape[1],
-                                              flags, _stream_ptr(a.device))
-
     if _is_tensor(x) and x.is_cuda:
         q = a._check_q_tensor(x)
-        outs = []
-        for _ in range(2):
-            outs.append(torch.empty((q.shape[0], k), dtype=torch.float32, device=q.device))
-            outs.append(torch.empty((q.shape[0], k), dtype=torch.int64, device=q.device))
-        _capi.check(call(q.data_ptr(), q.shape[0], outs[0].data_ptr(), outs[1].data_ptr(), outs[2].data_ptr(),
-                         outs[3].data_ptr()))
-        return (outs[0], outs[1]), (outs[2], outs[3])
-    arr = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, a.d, "search2")
-    Da = np.empty((arr.shape[0], k), np.float32)
-    Ia = np.empty((arr.shape[0], k), np.int64)
-    Db = np.empty_like(Da)
-    Ib = np.empty_like(Ia)
-    _capi.check(call(arr.ctypes.data, arr.shape[0], Da.ctypes.data, Ia.ctypes.data, Db.ctypes.data, Ib.ctypes.data))
+        Da, Db = (torch.empty((q.shape[0], k), dtype=torch.float32, device=q.device) for _ in range(2))
+        Ia, Ib = (torch.empty((q.shape[0], k), dtype=torch.int64, device=q.device) for _ in range(2))
+    else:
+        q = _as_f32_matrix(x.numpy() if _is_tensor(x) else x, a.d, "search2")
+        Da, Db = (np.empty((q.shape[0], k), np.float32) for _ in range(2))
+        Ia, Ib = (np.empty((q.shape[0], k), np.int64) for _ in range(2))
+    ex = _exclude_arg(exclude, q.shape[0], a.device)
+    _capi.check(lib.keds_index_search2(a._h, b._h, _ptr(q), q.shape[0], k, _ptr(Da), _ptr(Ia), _ptr(Db), _ptr(Ib),
+                                       *_exclude_ptrs(ex), flags, _stream_ptr(a.device)))
     return (Da, Ia), (Db, Ib)
 
 

@@ -27,7 +27,8 @@ import numpy as np
 import torch
 
 from . import _capi
-from .index import GpuIndexFlat, METRIC_INNER_PRODUCT, METRIC_L2, check_exclude, search2, _exclude_arg, _stream_ptr
+from .index import (GpuIndexFlat, METRIC_INNER_PRODUCT, METRIC_L2, check_exclude, search2, _exclude_arg, _exclude_ptrs,
+                    _stream_ptr)
 
 
 def check_perm(perm: Optional[torch.Tensor], k: int, name: str = "perm") -> None:
@@ -240,7 +241,7 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
     [B, d].  `out` may carry preallocated tensors from a previous call (keys as returned) so a
     steady-state loop allocates nothing.
 
-    Host I/O without copies (keds_retrieve2_hostio): `q` may be a pinned CPU tensor -- the first
+    Host I/O without copies (keds_retrieve2's host mirrors): `q` may be a pinned CPU tensor -- the first
     kernel reads it through the device mapping -- and `host_out` may hold pinned CPU tensors
     D_img / I_img / D_txt / I_txt ([B, k]) that the kernels fill next to the device results; they
     are complete once the stream has been synchronised.
@@ -272,22 +273,17 @@ def retrieve2(image_index: GpuIndexFlat, text_index: GpuIndexFlat, q: torch.Tens
     Di, Ii, Dt, It, fi, ft, pi, pt = _step_outputs(o, dev, B, B, k, image_index.d, want_feats, pool_mode)
     perm_i, perm_t = _device_perm(perm_img, k, dev), _device_perm(perm_txt, k, dev)
     ptr = lambda t: 0 if t is None else t.data_ptr()
-    ex = None if exclude is None else _exclude_arg(exclude, B, image_index.device, pinned_ok=hostio)
-    mirrors = []
-    if hostio:
-        ho = host_out or {}
-        for name, dt in (("D_img", torch.float32), ("I_img", torch.int64), ("D_txt", torch.float32), ("I_txt", torch.int64)):
-            t = ho.get(name)
-            if t is not None and not (t.is_pinned() and t.dtype == dt and t.is_contiguous() and t.numel() == B * k):
-                raise TypeError(f"retrieve2: host_out[{name!r}] must be a pinned contiguous {dt} tensor of {B * k} elements")
-            mirrors.append(ptr(t))
-    args = [image_index._h, text_index._h, q.data_ptr(), B, k, ptr(perm_i), ptr(perm_t), int(pool_mode), float(tau),
-            Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), *mirrors, ptr(fi), ptr(ft), ptr(pi), ptr(pt)]
-    if ex is not None:
-        args += [ex.data_ptr(), ex.shape[1]]
-    fn = {(False, False): lib.keds_retrieve2, (True, False): lib.keds_retrieve2_hostio,
-          (False, True): lib.keds_retrieve2_exclude, (True, True): lib.keds_retrieve2_hostio_exclude}[(hostio, ex is not None)]
-    _capi.check(fn(*args, int(flags), _stream_ptr(image_index.device)))
+    ex = _exclude_arg(exclude, B, image_index.device, pinned_ok=hostio)
+    ho, mirrors = host_out or {}, []
+    for name, dt in (("D_img", torch.float32), ("I_img", torch.int64), ("D_txt", torch.float32), ("I_txt", torch.int64)):
+        t = ho.get(name)
+        if t is not None and not (t.is_pinned() and t.dtype == dt and t.is_contiguous() and t.numel() == B * k):
+            raise TypeError(f"retrieve2: host_out[{name!r}] must be a pinned contiguous {dt} tensor of {B * k} elements")
+        mirrors.append(ptr(t))
+    _capi.check(lib.keds_retrieve2(
+        image_index._h, text_index._h, q.data_ptr(), B, k, ptr(perm_i), ptr(perm_t), int(pool_mode), float(tau),
+        Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(), *mirrors, ptr(fi), ptr(ft), ptr(pi), ptr(pt),
+        *_exclude_ptrs(ex), int(flags), _stream_ptr(image_index.device)))
     return o
 
 
@@ -319,7 +315,7 @@ class RetrievalStep:
         self.ia, self.ib = image_index, text_index
         # copy_nodes=False: no copies in the graph -- the first kernel reads the pinned queries through
         # the mapping and the ranking blocks store (D, I) into the pinned result block next to the
-        # device one (keds_retrieve2_hostio). True: H2D + D2H copy nodes around the search (the
+        # device one (keds_retrieve2's host mirrors). True: H2D + D2H copy nodes around the search (the
         # round-1 layout). None (default): capture both once and keep the faster on THIS box -- SM
         # loads over PCIe beat the copy engines' set-up cost on most boxes (7 of 8 measured), but how
         # the pinned pages sit relative to the GPU's root complex decides it; the answers are the same.

@@ -21,7 +21,7 @@ import torch
 import torch.distributed as dist
 
 from . import _capi
-from .index import GpuIndexFlat, _exclude_arg, _stream_ptr
+from .index import GpuIndexFlat, _check_out, _exclude_arg, _exclude_ptrs, _stream_ptr
 from .retrieval import _device_perm, _step_outputs, check_perm
 
 
@@ -221,22 +221,15 @@ class ShardedIndex:
         only publish step t+1 after finishing its merge of step t)."""
         lib = _capi.load()
         q = self.local._check_q_tensor(q)
-        ex = None if exclude is None else _exclude_arg(exclude, nq, self.device.index)
+        ex = _exclude_arg(exclude, nq, self.device.index)
         fx = self._exchange(nq * k)
         if out is not None:
-            Dg, Ig = out
-            assert Dg.is_cuda and Ig.is_cuda and Dg.is_contiguous() and Ig.is_contiguous()
-            assert Dg.dtype == torch.float32 and Ig.dtype == torch.int64 and Dg.numel() == nq * k == Ig.numel()
+            Dg, Ig = _check_out(out, nq * k)
         else:
             Dg = torch.empty((nq, k), dtype=torch.float32, device=q.device)
             Ig = torch.empty((nq, k), dtype=torch.int64, device=q.device)
-        if ex is None:
-            _capi.check(lib.keds_index_search_sharded(self.local._h, fx.handle, q.data_ptr(), nq, k,
-                                                      Dg.data_ptr(), Ig.data_ptr(), _stream_ptr(self.device.index)))
-        else:
-            _capi.check(lib.keds_index_search_sharded_exclude(self.local._h, fx.handle, q.data_ptr(), nq, k,
-                                                              Dg.data_ptr(), Ig.data_ptr(), ex.data_ptr(), ex.shape[1],
-                                                              _stream_ptr(self.device.index)))
+        _capi.check(lib.keds_index_search_sharded(self.local._h, fx.handle, q.data_ptr(), nq, k, Dg.data_ptr(),
+                                                  Ig.data_ptr(), *_exclude_ptrs(ex), _stream_ptr(self.device.index)))
         return Dg, Ig
 
     def _exchange(self, need: int) -> _FusedExchange:
@@ -397,7 +390,7 @@ class ShardedKnowledgeBase:
         _capi.check(lib.keds_retrieve2_sharded(
             self.image.local._h, self.text.local._h, fx.handle, q.data_ptr(), Bt, k, ptr(perms[0]), ptr(perms[1]),
             int(pool_mode), float(tau), lo, hi, Di.data_ptr(), Ii.data_ptr(), Dt.data_ptr(), It.data_ptr(),
-            ptr(fi), ptr(ft), ptr(pi), ptr(pt), ptr(ex), 0 if ex is None else ex.shape[1], int(flags),
+            ptr(fi), ptr(ft), ptr(pi), ptr(pt), *_exclude_ptrs(ex), int(flags),
             _stream_ptr(self.device.index)))
         return o
 

@@ -3,14 +3,17 @@
 Loads a reference build (--base-lib, e.g. the parent commit's) and this tree's build into one
 process (scripts/perf_exclude.py's loader) and runs each call on both, each build on its own
 handles over the same rows: search with flags 0 / exact-only / no-fallback / force-IP, search2,
-host (numpy-style) and device I/O, the four exclusion variants, retrieve2 with gathered
-neighbours, pools and host mirrors, label hits (one and two passes), rank (one and two passes;
-misaligned queries; an inflated error bound that sends queries to the exact recount), debug_scores
-and a one-rank sharded search, over B = 7 .. 17,000, k = 16 / 200 / 600, IP and L2, fp16 and bf16.
+host (numpy-style) and device I/O, exclusion in search, search2 and retrieve2 (device and
+page-locked host labels), retrieve2 with gathered neighbours, pools and host mirrors, label hits
+(one and two passes), rank (one and two passes; misaligned queries; an inflated error bound that
+sends queries to the exact recount), debug_scores and a one-rank sharded search, over
+B = 7 .. 17,000, k = 16 / 200 / 600, IP and L2, fp16 and bf16. A reference build of the 0.1 ABI,
+which had one entry point per optional search input, is called through the loader's ParentAbi.
 Every output and every last_stats field must be identical, except launches and n_flagged of a
-multi-pass rank call (summed over its passes; a reference build may report its last pass's). A two-database search whose first
-database is empty is checked against the CPU oracle instead (its status is reported differently
-by design). Writes one JSON document (card name and power limit included); exits 1 on a mismatch.
+multi-pass rank call (summed over its passes; a reference build may report its last pass's). A
+two-database search whose first database is empty is checked against the CPU oracle instead (its
+status is reported differently by design). Writes one JSON document (card name and power limit
+included); exits 1 on a mismatch.
 
     python scripts/ab_entry_points.py --base-lib /path/to/parent/libkeds_knn.so --out ab.json
 """
@@ -121,7 +124,7 @@ def main() -> None:
                     outs = {n: dev_out(B, k) for n in libs}
                     compare(f"search m{metric} f{fmt} B{B} k{k}",
                             lambda n, lib, hs: check(lib, lib.keds_index_search_ex(
-                                hs[0], q.data_ptr(), B, k, outs[n][0].data_ptr(), outs[n][1].data_ptr(), 0, st)),
+                                hs[0], q.data_ptr(), B, k, outs[n][0].data_ptr(), outs[n][1].data_ptr(), None, 0, 0, st)),
                             [("a", metric, fmt)], lambda n: outs[n])
     for flags in (_capi.SEARCH_EXACT_ONLY, _capi.SEARCH_NO_FALLBACK, _capi.SEARCH_FORCE_IP):
         for B in (128, 4096):
@@ -129,7 +132,7 @@ def main() -> None:
             outs = {n: dev_out(B, 16) for n in libs}
             compare(f"search flags{flags} B{B}",
                     lambda n, lib, hs: check(lib, lib.keds_index_search_ex(
-                        hs[0], q.data_ptr(), B, 16, outs[n][0].data_ptr(), outs[n][1].data_ptr(), flags, st)),
+                        hs[0], q.data_ptr(), B, 16, outs[n][0].data_ptr(), outs[n][1].data_ptr(), None, 0, flags, st)),
                     [("a", _capi.METRIC_L2, 1)], lambda n: outs[n])
 
     # host I/O (numpy-style): search and search2
@@ -138,11 +141,11 @@ def main() -> None:
         outs = {n: [np.empty((B, 16), dt) for _ in range(2) for dt in (np.float32, np.int64)] for n in libs}
         compare(f"search host B{B}",
                 lambda n, lib, hs: check(lib, lib.keds_index_search_ex(
-                    hs[0], qh.ctypes.data, B, 16, outs[n][0].ctypes.data, outs[n][1].ctypes.data, 0, st)),
+                    hs[0], qh.ctypes.data, B, 16, outs[n][0].ctypes.data, outs[n][1].ctypes.data, None, 0, 0, st)),
                 [("a", _capi.METRIC_IP, 1)], lambda n: outs[n][:2])
         compare(f"search2 host B{B}",
                 lambda n, lib, hs: check(lib, lib.keds_index_search2(
-                    hs[0], hs[1], qh.ctypes.data, B, 16, *[o.ctypes.data for o in outs[n]], 0, st)),
+                    hs[0], hs[1], qh.ctypes.data, B, 16, *[o.ctypes.data for o in outs[n]], None, 0, 0, st)),
                 [("a", _capi.METRIC_IP, 1), ("b", _capi.METRIC_IP, 1)], lambda n: outs[n])
 
     # search2 and the exclusion variants on device memory
@@ -154,10 +157,10 @@ def main() -> None:
             p = lambda n: [o.data_ptr() for o in outs[n]]  # noqa: E731
             two = [("a", _capi.METRIC_IP, 1), ("b", _capi.METRIC_IP, 1)]
             compare(f"search2 B{B} k{k}", lambda n, lib, hs: check(lib, lib.keds_index_search2(
-                hs[0], hs[1], q.data_ptr(), B, k, *p(n), 0, st)), two, lambda n: outs[n])
-            compare(f"search_exclude B{B} k{k}", lambda n, lib, hs: check(lib, lib.keds_index_search_exclude(
+                hs[0], hs[1], q.data_ptr(), B, k, *p(n), None, 0, 0, st)), two, lambda n: outs[n])
+            compare(f"search_exclude B{B} k{k}", lambda n, lib, hs: check(lib, lib.keds_index_search_ex(
                 hs[0], q.data_ptr(), B, k, *p(n)[:2], ex.data_ptr(), 2, 0, st)), two[:1], lambda n: outs[n][:2])
-            compare(f"search2_exclude B{B} k{k}", lambda n, lib, hs: check(lib, lib.keds_index_search2_exclude(
+            compare(f"search2_exclude B{B} k{k}", lambda n, lib, hs: check(lib, lib.keds_index_search2(
                 hs[0], hs[1], q.data_ptr(), B, k, *p(n), ex.data_ptr(), 2, 0, st)), two, lambda n: outs[n])
 
     # retrieve2: gathered neighbours, pools, host mirrors, exclusion
@@ -179,15 +182,10 @@ def main() -> None:
                 o = [t.data_ptr() for t in outs[n]]
                 head = (hs[0], hs[1], (qp if "hostio" in variant else q).data_ptr(), B, 16, perm.data_ptr(), None, 2,
                         100.0, *o[:4])
-                feats = (o[4], o[5], o[6], o[7])
-                if variant == "plain":
-                    check(lib, lib.keds_retrieve2(*head, *feats, 0, st))
-                elif variant == "exclude":
-                    check(lib, lib.keds_retrieve2_exclude(*head, *feats, ex.data_ptr(), 2, 0, st))
-                elif variant == "hostio":
-                    check(lib, lib.keds_retrieve2_hostio(*head, *o[8:12], *feats, 0, st))
-                else:
-                    check(lib, lib.keds_retrieve2_hostio_exclude(*head, *o[8:12], *feats, exp_.data_ptr(), 2, 0, st))
+                mirrors = o[8:12] if "hostio" in variant else (None,) * 4
+                exclusion = {"plain": (None, 0), "exclude": (ex.data_ptr(), 2), "hostio": (None, 0),
+                             "hostio_exclude": (exp_.data_ptr(), 2)}[variant]
+                check(lib, lib.keds_retrieve2(*head, *mirrors, o[4], o[5], o[6], o[7], *exclusion, 0, st))
             compare(f"retrieve2 {variant} B{B}", run, two,
                     lambda n, outs=outs, variant=variant: outs[n] if "hostio" in variant else outs[n][:8])
 
@@ -238,7 +236,7 @@ def main() -> None:
                                             C.byref(h)))
         exch[n] = h
     compare("search_sharded 1 rank 4096x50k", lambda n, lib, hs: check(lib, lib.keds_index_search_sharded(
-        hs[0], exch[n], q.data_ptr(), 4096, 16, outs[n][0].data_ptr(), outs[n][1].data_ptr(), st)),
+        hs[0], exch[n], q.data_ptr(), 4096, 16, outs[n][0].data_ptr(), outs[n][1].data_ptr(), None, 0, st)),
         [("a", _capi.METRIC_IP, 1)], lambda n: outs[n])
 
     # the empty-database route: against the oracle (the status of the call is reported differently)
@@ -251,11 +249,8 @@ def main() -> None:
 
             def run(n, lib, hs, outs=outs, ex=ex, excl=excl, q=q, B=B):
                 p = [o.data_ptr() for o in outs[n]]
-                if excl:
-                    check(lib, lib.keds_index_search2_exclude(hs[0], hs[1], q.data_ptr(), B, 16, *p, ex.data_ptr(), 2,
-                                                              0, st))
-                else:
-                    check(lib, lib.keds_index_search2(hs[0], hs[1], q.data_ptr(), B, 16, *p, 0, st))
+                exclusion = (ex.data_ptr(), 2) if excl else (None, 0)
+                check(lib, lib.keds_index_search2(hs[0], hs[1], q.data_ptr(), B, 16, *p, *exclusion, 0, st))
 
             def oracle(o, q=q, ex=ex, excl=excl):
                 if not (o[1] == -1).all():

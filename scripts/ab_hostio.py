@@ -1,6 +1,6 @@
 """Same-process A/B of the end-to-end retrieval step (RetrievalStep: pinned host queries in, (D, I)
 on the host out, one graph launch + one stream sync per step): copy nodes around the search vs
-host I/O through the mapping (keds_retrieve2_hostio), interleaved.
+host I/O through the mapping (keds_retrieve2 with host mirrors), interleaved.
 -> gpurun_out/ab_hostio.json"""
 from __future__ import annotations
 

@@ -5,8 +5,8 @@ and times, round after round in rotating order on the same device-resident input
 
   base     the plain entry point of a reference build (--base-lib, e.g. the parent commit's)
   plain    the plain entry point of this tree's build
-  exclude  this tree's *_exclude entry point, E = 1: every query is a row of the base and leaves
-           itself out (training without self-retrieval)
+  exclude  the same entry point of this tree's build with an exclusion array, E = 1: every query is
+           a row of the base and leaves itself out (training without self-retrieval)
 
 on three shapes: config 2 (retrieve2, 128 queries x 2 databases x 0.5M rows, k = 16, gathered
 neighbours), config 1 (search, 4096 x 50k, k = 16) and 4096 x 0.5M; and base against plain (no
@@ -41,13 +41,57 @@ D = 768
 K = 16
 
 
-def load(path: str) -> C.CDLL:
+class ParentAbi:
+    """A build of the 0.1 ABI behind this build's calls. That ABI had one entry point per optional
+    search input: each unified call goes to the one its arguments need (`_exclude` for an exclusion
+    array, `_hostio` for retrieve2 with host mirrors), without the arguments that one lacks."""
+
+    # unified call -> (position of exclude, n_exclude; position of retrieve2's four host mirrors)
+    CALLS = {"keds_index_search_ex": (6, None), "keds_index_search2": (9, None),
+             "keds_index_search_sharded": (7, None), "keds_retrieve2": (21, 13)}
+
+    def __init__(self, lib):
+        self._lib = lib
+        self._twins = {}
+
+    def _twin(self, name, exclude, hostio):
+        """(the 0.1 entry point, the positions of the unified arguments it takes), set up once"""
+        key = (name, exclude, hostio)
+        if key not in self._twins:
+            at_ex, at_mirrors = self.CALLS[name]
+            drop = set() if exclude else {at_ex, at_ex + 1}
+            if at_mirrors is not None and not hostio:
+                drop |= set(range(at_mirrors, at_mirrors + 4))
+            twin = name
+            if exclude or hostio:
+                twin = name.removesuffix("_ex") + ("_hostio" if hostio else "") + ("_exclude" if exclude else "")
+            args = _capi.SIGNATURES[name][1]
+            keep = [i for i in range(len(args)) if i not in drop]
+            fn = getattr(self._lib, twin)
+            fn.restype, fn.argtypes = C.c_int, [args[i] for i in keep]
+            self._twins[key] = (fn, keep)
+        return self._twins[key]
+
+    def __getattr__(self, name):
+        if name not in self.CALLS:
+            return getattr(self._lib, name)
+        at_ex, at_mirrors = self.CALLS[name]
+
+        def call(*args):
+            hostio = at_mirrors is not None and any(args[at_mirrors:at_mirrors + 4])
+            fn, keep = self._twin(name, bool(args[at_ex]), hostio)
+            return fn(*[args[i] for i in keep])
+        return call
+
+
+def load(path: str):
+    """One build of the library with this tree's signatures (a build of the 0.1 ABI behind ParentAbi)."""
     lib = C.CDLL(path)
     for name, (res, args) in _capi.SIGNATURES.items():
         if hasattr(lib, name):
             fn = getattr(lib, name)
             fn.restype, fn.argtypes = res, args
-    return lib
+    return ParentAbi(lib) if lib.keds_version().split()[1] == b"0.1" else lib
 
 
 def check(lib, rc):
@@ -81,7 +125,6 @@ def main() -> None:
     args = ap.parse_args()
     assert torch.cuda.is_available(), "needs a CUDA device"
     libs = {"base": load(os.path.abspath(args.base_lib)), "new": load(os.path.abspath(args.lib))}
-    assert hasattr(libs["new"], "keds_index_search_exclude"), "--lib is not a build with exclusion"
     dev = torch.device("cuda", 0)
     st = torch.cuda.current_stream(dev).cuda_stream
     g = torch.Generator(device=dev).manual_seed(0)
@@ -139,17 +182,13 @@ def main() -> None:
         if cfg.startswith("hits"):
             return lambda: check(lib, lib.keds_index_label_hits(ix["s"], q.data_ptr(), nq, row_labels.data_ptr(),
                                                                 ex.data_ptr(), ks.ctypes.data, len(ks), p[0], st))
+        exclusion =(ex.data_ptr(), 1) if variant == "exclude" else (None, 0)
         if cfg.startswith("cfg2"):
-            common = (ix["a"], ix["b"], q.data_ptr(), nq, K, perm.data_ptr(), None, 0, 100.0, p[0], p[1], p[2], p[3],
-                      p[4], p[5], None, None)
-            if variant == "exclude":
-                return lambda: check(lib, lib.keds_retrieve2_exclude(*common, ex.data_ptr(), 1, 0, st))
-            return lambda: check(lib, lib.keds_retrieve2(*common, 0, st))
+            return lambda: check(lib, lib.keds_retrieve2(ix["a"], ix["b"], q.data_ptr(), nq, K, perm.data_ptr(), None, 0,
+                                                         100.0, p[0], p[1], p[2], p[3], None, None, None, None, p[4],
+                                                         p[5], None, None, *exclusion, 0, st))
         h = ix["s"] if cfg.startswith("cfg1") else ix["a"]
-        if variant == "exclude":
-            return lambda: check(lib, lib.keds_index_search_exclude(h, q.data_ptr(), nq, K, p[0], p[1], ex.data_ptr(), 1,
-                                                                    0, st))
-        return lambda: check(lib, lib.keds_index_search_ex(h, q.data_ptr(), nq, K, p[0], p[1], 0, st))
+        return lambda: check(lib, lib.keds_index_search_ex(h, q.data_ptr(), nq, K, p[0], p[1], *exclusion, 0, st))
 
     variants = {c: ("base", "plain") if c.startswith(("rank", "hits")) else ("base", "plain", "exclude")
                 for c in shapes}

@@ -1,6 +1,8 @@
 """CPU: search with exclusion -- the exclusion reference (the oracle's search for k + E rows with
 the excluded labels dropped) against a brute-force argsort, the Python argument checks,
 KnowledgeBase.rows_of, the exported C surface, and a spill-free sm_100a compile."""
+import ctypes as C
+
 import numpy as np
 import pytest
 import torch
@@ -112,22 +114,27 @@ def test_rows_of():
     assert kb.rows_of(["a.jpg", "c.jpg"]).tolist() == [1, -1]
 
 
-def test_exclude_symbols_in_ctypes_table():
-    for name in ("keds_index_search_exclude", "keds_index_search2_exclude", "keds_retrieve2_exclude",
-                 "keds_retrieve2_hostio_exclude"):
-        assert name in _capi.SIGNATURES
-        assert hasattr(_capi.load(), name)
+def test_search_calls_take_exclusion_arguments():
+    """Every search call with exclusion is exported and takes (exclude, n_exclude) as (pointer, int)."""
+    lib = _capi.load()
+    for name, at in (("keds_index_search_ex", 6), ("keds_index_search2", 9), ("keds_retrieve2", 21),
+                     ("keds_index_search_sharded", 7), ("keds_retrieve2_sharded", 20)):
+        assert hasattr(lib, name)
+        assert _capi.SIGNATURES[name][1][at:at + 2] == [C.c_void_p, C.c_int], name
 
 
-def test_exclude_entry_points_refuse_bad_arrays_without_a_gpu():
+def test_search_calls_refuse_bad_exclusion_without_a_gpu():
     lib = _capi.load()
     ex = np.zeros((1, 1), np.int64)
-    # a null array or E outside 1..8 is refused before anything else
-    assert lib.keds_index_search_exclude(None, None, 1, 1, None, None, None, 1, 0, None) == -1
-    assert lib.keds_index_search_exclude(None, None, 1, 1, None, None, ex.ctypes.data, 0, 0, None) == -1
-    assert lib.keds_index_search_exclude(None, None, 1, 1, None, None, ex.ctypes.data, 9, 0, None) == -1
-    assert lib.keds_index_search2_exclude(None, None, None, 1, 1, None, None, None, None, None, 1, 0, None) == -1
-    assert "exclude" in _capi.last_error()
+    # a null array with n_exclude != 0, or an array with n_exclude outside 1..8, is refused before anything else
+    for e, n in ((None, 1), (ex.ctypes.data, 0), (ex.ctypes.data, 9)):
+        assert lib.keds_index_search_ex(None, None, 1, 1, None, None, e, n, 0, None) == -1
+        assert "exclude" in _capi.last_error()
+        assert lib.keds_index_search2(None, None, None, 1, 1, None, None, None, None, e, n, 0, None) == -1
+        assert "exclude" in _capi.last_error()
+        assert lib.keds_retrieve2(None, None, None, 1, 16, None, None, 0, 1.0, None, None, None, None, None, None, None,
+                                  None, None, None, None, None, e, n, 0, None) == -1
+        assert "exclude" in _capi.last_error()
 
 
 def test_scoring_and_fallback_kernels_do_not_spill(tmp_path):

@@ -626,7 +626,7 @@ def test_search_gather_returns_neighbours_or_their_weighted_pool():
 
 
 def test_host_io_through_the_mapping_equals_the_copy_path():
-    """keds_retrieve2_hostio: pinned host queries read by the first kernel through the mapping and
+    """keds_retrieve2 with host I/O: pinned host queries read by the first kernel through the mapping and
     (D, I) mirrored into pinned host blocks by the ranking blocks -- same answers as device queries
     + copies, for certified queries, for flagged ones (mirrored by the exact fallback), for a
     database small enough to go to the exact kernels only, and across a pass seam."""

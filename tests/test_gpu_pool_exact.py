@@ -256,7 +256,7 @@ def test_padding():
 
 
 def test_host_io_and_graph_replays():
-    """Pinned host queries and results (keds_retrieve2_hostio), and RetrievalStep replays in both
+    """Pinned host queries and results (keds_retrieve2's host mirrors), and RetrievalStep replays in both
     copy-node layouts: pools and feats equal to the stream path and to the emulation."""
     d, k, nq = 768, 16, 128
     xs = rows(d)

@@ -163,14 +163,22 @@ def test_get_retrieved_features_gathers_pads_and_returns_own_block(metric, use_e
     assert out.get(0) is True and out.get(1) is True, dict(out)
 
 
-def test_sharded_entry_points_refuse_bad_arguments_without_a_gpu():
+def test_sharded_calls_refuse_bad_arguments_and_exclusion_without_a_gpu():
     lib = _capi.load()
-    for name in ("keds_retrieve2_sharded", "keds_index_search_sharded_exclude", "keds_index_rows_ipc",
+    for name in ("keds_retrieve2_sharded", "keds_index_search_sharded", "keds_index_rows_ipc",
                  "keds_exchange_attach_rows"):
         assert name in _capi.SIGNATURES and hasattr(lib, name)
     assert lib.keds_retrieve2_sharded(None, None, None, None, 1, 16, None, None, 0, 1.0, 0, 1, None, None, None, None,
                                       None, None, None, None, None, 0, 0, None) == -1
-    assert lib.keds_index_search_sharded_exclude(None, None, None, 1, 1, None, None, None, 0, None) == -1
+    assert lib.keds_index_search_sharded(None, None, None, 1, 1, None, None, None, 0, None) == -1
+    # exclusion arrays: a null array with n_exclude != 0, or n_exclude outside 1..8, are refused first
+    ex = np.zeros((1, 1), np.int64)
+    for e, n in ((None, 1), (ex.ctypes.data, 0), (ex.ctypes.data, 9)):
+        assert lib.keds_retrieve2_sharded(None, None, None, None, 1, 16, None, None, 0, 1.0, 0, 1, None, None, None,
+                                          None, None, None, None, None, e, n, 0, None) == -1
+        assert "exclude" in _capi.last_error()
+        assert lib.keds_index_search_sharded(None, None, None, 1, 1, None, None, e, n, None) == -1
+        assert "exclude" in _capi.last_error()
     assert lib.keds_index_rows_ipc(None, None) == -1
     assert lib.keds_exchange_attach_rows(None, 0, None, None, None) == -1
 
